@@ -2,15 +2,17 @@
 """bench.py -- BASELINE.json's metric: raycast fwd+bwd rays/s, % of the HBM roofline, train chunks/s (SURVEY.md section 8(d)).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c5]
+                    [--dump-outputs DIR]
 
-A "step" is one pass of the hot path over one batch of synthetic input:
+A "step" is one pass of the hot path over one batch of synthetic input; every timed region below that counts steps runs
+exactly K of them:
   c3 (default, BASELINE configs[2])  8 chunks 64x64x128 x 5 views 320x256 (3 276 800 rays): raycast forward with the depth /
                                      colour / 2D-semantic losses fused in, and its backward (voxel gradients)
   c2 (BASELINE configs[1])           one chunk, one view; also reported inside the default line as `c2`
   c5 (BASELINE configs[4])           whole-room 2 cm inference by sliding chunks with multi-view semantic rendering
 `value`   rays/s with every input already resident in HBM, the step replayed from a CUDA graph (no host launch latency in
           the device number); distinct input sets are rotated so that consecutive steps never find their data in the
-          126 MB L2; the timed region is at least MIN_REGION_S long whatever --steps says.
+          126 MB L2.
 `e2e`     the same metric through the public Python API with HOST buffers: every step copies its voxel tensors, cameras
           and target frames from pinned host memory (copy stream, double-buffered) and reads the loss back.
 `roofline`     the dominant kernel (raycast forward) timed with CUDA events on its launch stream (C-ABI timing hook),
@@ -25,6 +27,10 @@ A "step" is one pass of the hot path over one batch of synthetic input:
           path, so its arm is its CUDA extension (falls back to the CPU port if the extension is not on the box).
 One process per GPU (torchrun sets RANK/LOCAL_RANK/WORLD_SIZE); units are independent chunk x view batches, so ranks shard
 them with no data-path collective ("scaling": "weak"); time is the max over ranks.
+--dump-outputs DIR  after the timed steps of `value`, rank 0 writes what the last of them returned to its caller as
+          DIR/<name>.npy (float32 / float64): the loss terms and the voxel gradients (c2/c3; rows sampled with a fixed seed
+          when all of them would exceed DUMP_MAX_BYTES, their indices in voxel_rows.npy), or the room's label histogram
+          (c5).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -45,8 +51,8 @@ import torch.distributed as dist  # noqa: E402
 
 MAX_LOCS = 640000      # train.py:136 max_num_locs_per_sample (sizes the reference's memsets)
 E2E_REPEATS = 3        # timed regions of the end-to-end leg (median reported), both arms
-MIN_REGION_S = 0.5     # the device-resident timed region lasts at least this long
 TRAIN_BATCH = 8        # chunks per GPU and step of the train leg (BASELINE configs[2]/[3])
+DUMP_MAX_BYTES = 64 * 1000 * 1000  # --dump-outputs: all files together stay below this
 
 
 def bind_to_gpu_numa_node(dev):
@@ -73,7 +79,7 @@ def bind_to_gpu_numa_node(dev):
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=700)  # ~0.5 s of device-resident c3 steps on a B200
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c3", choices=["c2", "c3", "c5"])
@@ -81,7 +87,13 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train", action="store_true", help="skip the train-step leg (configs[3])")
     ap.add_argument("--no-secondary", action="store_true", help="skip the c2 / un-fused secondary numbers")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs is implemented for --impl ours")
+    return args
 
 
 class ClockSampler(threading.Thread):
@@ -164,14 +176,14 @@ def reduce_max_ms(ms, dev, world):
     return ms
 
 
-def timed_replays(graph, replays, dev, world):
-    """`replays` graph launches bracketed by barrier + synchronize, CUDA-event time, max over ranks."""
+def timed_replays(graphs, dev, world):
+    """One launch of each graph in order, bracketed by barrier + synchronize, CUDA-event time, max over ranks."""
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     a.record()
-    for _ in range(replays):
+    for graph in graphs:
         graph.replay()
     b.record()
     torch.cuda.synchronize()
@@ -181,8 +193,9 @@ def timed_replays(graph, replays, dev, world):
     return ms
 
 
-def capture_rotation(step, num_sets, dev, warmup):
-    """Warm up, then capture one rotation over all input sets into a CUDA graph."""
+def capture_rotation(step, num_steps, dev, warmup):
+    """Warm up, then capture steps 0 .. num_steps-1 (one rotation over the input sets, or its first part) into a CUDA
+    graph."""
     for i in range(max(warmup, 3)):
         step(i)
     torch.cuda.synchronize()
@@ -193,7 +206,7 @@ def capture_rotation(step, num_sets, dev, warmup):
         step(0)
         side.synchronize()
         with torch.cuda.graph(graph, stream=side):
-            for i in range(num_sets):
+            for i in range(num_steps):
                 step(i)
     torch.cuda.current_stream(dev).wait_stream(side)
     for _ in range(2):
@@ -202,13 +215,13 @@ def capture_rotation(step, num_sets, dev, warmup):
     return graph
 
 
-def measure_resident(step, num_sets, dev, world, want_steps, warmup):
-    """(ms, steps) of a device-resident loop: graph replays covering >= want_steps steps and >= MIN_REGION_S."""
+def measure_resident(step, num_sets, dev, world, steps, warmup):
+    """(ms, graphs) of a device-resident loop of exactly `steps` steps: replays of one captured rotation over the input
+    sets, then a graph of the steps left over.  The graphs own the memory of what their steps returned."""
     graph = capture_rotation(step, num_sets, dev, warmup)
-    probe = timed_replays(graph, 2, dev, world) / 2.0  # ms per rotation
-    replays = max(1, int(math.ceil(want_steps / num_sets)), int(math.ceil(MIN_REGION_S * 1e3 / max(probe, 1e-3))))
-    ms = timed_replays(graph, replays, dev, world)
-    return ms, replays * num_sets, graph
+    rest = steps % num_sets
+    tail = [capture_rotation(step, rest, dev, 0)] if rest else []
+    return timed_replays([graph] * (steps // num_sets) + tail, dev, world), [graph] + tail
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -239,6 +252,7 @@ class Ours:
         self.nv = int(np.mean([d["locs"].shape[0] for d in self.devsets]))
         self.cw = torch.tensor(S.CLASS_WEIGHTS, dtype=torch.float32, device=dev)
         self.loss_sink = torch.zeros((), device=dev)
+        self.returned = {}
 
     def step_fused(self, i):
         """forward with the three 2D losses fused in + backward from the scalar loss (the north-star path)."""
@@ -247,10 +261,18 @@ class Ours:
         d, m = self.devsets[k], self.mods[k]
         # the two native calls of spsg_b200.losses (spsg_raycast_forward_loss + spsg_raycast_backward_loss) without the
         # autograd wrapper: voxel gradients land in the module's d_* rows, the loss in loss_out[3]
-        loss_out, _ = self.render_pair(m, d["locs"], d["sdf"], d["color"], d["normal"], d["semantic"], d["view"], d["intr"],
-                                       images_depth=d["t_depth"], images_color=d["t_color"], target2d_label=d["t_label"],
-                                       weight_semantic_class=self.cw, voxelsize=S.VOXELSIZE)
+        loss_out, grads = self.render_pair(m, d["locs"], d["sdf"], d["color"], d["normal"], d["semantic"], d["view"],
+                                           d["intr"], images_depth=d["t_depth"], images_color=d["t_color"],
+                                           target2d_label=d["t_label"], weight_semantic_class=self.cw, voxelsize=S.VOXELSIZE)
         self.loss_sink.copy_(loss_out[3])
+        self.returned[k] = (loss_out, grads)  # when captured: the tensors every replay of this step writes
+
+    def last_outputs(self, steps):
+        """What the last of `steps` fused steps returned: its loss_out and voxel gradients, as numpy arrays."""
+        loss_out, grads = self.returned[(steps - 1) % self.num_sets]
+        out = {"loss_out": loss_out}
+        out.update(zip(("d_sdf", "d_color", "d_normal", "d_semantic"), grads))
+        return {k: v.detach().cpu().numpy() for k, v in out.items()}
 
     def step_unfused(self, i):
         """forward + backward with upstream gradient images (the reference op boundary)."""
@@ -438,6 +460,26 @@ class Ours:
                 "backward_gather_us": round(g_ms / max(g_n, 1) * 1e3, 2),
                 "note": "not HBM-bound (traffic ~ algorithmic bytes): instruction issue / per-warp latency, see DESIGN.md "
                         "section 5 and profiles/README.md"}
+
+
+def dump_outputs(path, arrays):
+    """Write each array as path/<name>.npy (float32 stays float32; integers, so that counts stay exact, and everything
+    else become float64).  When the per-voxel arrays (those with the most rows) would take the files past DUMP_MAX_BYTES,
+    the same fixed, seeded sample of their rows is written and voxel_rows.npy holds its indices."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: a.astype(np.float32 if a.dtype == np.float32 else np.float64) for k, a in arrays.items()}
+    rows = max(a.shape[0] if a.ndim else 0 for a in arrays.values())
+    per_voxel = [k for k, a in arrays.items() if a.ndim and a.shape[0] == rows]
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_MAX_BYTES - 256 * (len(arrays) + 1)  # .npy headers
+    if total > budget:
+        row_bytes = sum(arrays[k].nbytes // rows for k in per_voxel) + 8  # + its float64 index
+        keep = (budget - (total - sum(arrays[k].nbytes for k in per_voxel))) // row_bytes
+        sel = np.sort(np.random.default_rng(0).choice(rows, size=keep, replace=False))
+        arrays = dict(arrays, voxel_rows=sel.astype(np.float64), **{k: arrays[k][sel] for k in per_voxel})
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def ncu_traffic(workload):
@@ -804,15 +846,7 @@ def run_room(args, dev, rank, world, base):
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
-    t0 = time.perf_counter()
-    R.render_room(predict, dims, dev, **kw)
-    torch.cuda.synchronize()
-    one = max(time.perf_counter() - t0, 1e-4)
-    reps = max(3, min(args.steps, 20), int(math.ceil(MIN_REGION_S / one)))  # a timed region of at least MIN_REGION_S
-    if world > 1:  # the same count on every rank
-        t = torch.tensor([reps], device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        reps = int(t.item())
+    reps = args.steps
     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     a.record()
     for _ in range(reps):
@@ -827,6 +861,8 @@ def run_room(args, dev, rank, world, base):
         dist.all_reduce(t)
         rays = float(t.item())
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"label_hist": out["label_hist"]})
         value = rays * reps / (ms * 1e-3)
         print(json.dumps(dict(base, value=value, steps=reps, ms_per_step=ms / reps, clocks=sampler.summary(),
                               e2e={"value": value, "unit": "rays/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 15 * 8,
@@ -884,7 +920,7 @@ def main():
         from oracle import ref_driver
         if ref_driver.available():
             r = Reference(dev, rank, B, F, num_sets)
-            steps = max(1, min(args.steps, 60 if B * F == 1 else 12))  # bounded: the reference step is 10-25x longer
+            steps = args.steps
             sampler = ClockSampler(dev.index)
             sampler.start()
             ms = r.resident(world, steps, args.warmup)
@@ -925,13 +961,16 @@ def main():
     o = Ours(dev, rank, B, F, num_sets)
     sampler = ClockSampler(dev.index)
     sampler.start()
-    ms, steps, _ = measure_resident(o.step_fused, num_sets, dev, world, args.steps, args.warmup)
+    steps = args.steps
+    ms, graphs = measure_resident(o.step_fused, num_sets, dev, world, steps, args.warmup)
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, o.last_outputs(steps))
+    del graphs
     value = world * o.rays * steps / (ms * 1e-3)
-    e2e_steps = max(10, min(args.steps, 60))
-    ms_e2e, last_loss, copy_only = o.e2e(world, e2e_steps, min(args.warmup, 5))
-    e2e = world * o.rays * e2e_steps / (ms_e2e * 1e-3)
-    roof = o.roofline(min(args.steps, 40), fused=True) if rank == 0 else None
+    ms_e2e, last_loss, copy_only = o.e2e(world, steps, min(args.warmup, 5))
+    e2e = world * o.rays * steps / (ms_e2e * 1e-3)
+    roof = o.roofline(steps, fused=True) if rank == 0 else None
     extra = {}
 
     def secondary(name, fn):
@@ -945,7 +984,7 @@ def main():
             extra[name] = {"error": "%s: %s" % (type(e).__name__, str(e)[:300])}
 
     def leg_flow():
-        n_f = max(10, min(args.steps, 40))
+        n_f = args.steps
         ms_f, loss_f, h2d_f = o.e2e_device_flow(world, n_f, 3)
         return {"value": world * o.rays * n_f / (ms_f * 1e-3), "unit": "rays/s", "ms_per_step": ms_f / n_f, "steps": n_f,
                 "h2d_bytes_per_step": h2d_f, "d2h_bytes_per_step": 4, "last_loss": loss_f,
@@ -954,17 +993,17 @@ def main():
                        "step's frames (depth, colour, labels, cameras) are copied from pinned host memory"}
 
     def leg_unfused():
-        ms_u, steps_u, _ = measure_resident(o.step_unfused, num_sets, dev, world, args.steps, 3)
-        return {"value": world * o.rays * steps_u / (ms_u * 1e-3), "unit": "rays/s", "ms_per_step": ms_u / steps_u,
-                "steps": steps_u, "note": "same workload at the reference op boundary: forward renders, backward takes four "
+        ms_u, _ = measure_resident(o.step_unfused, num_sets, dev, world, steps, 3)
+        return {"value": world * o.rays * steps / (ms_u * 1e-3), "unit": "rays/s", "ms_per_step": ms_u / steps,
+                "steps": steps, "note": "same workload at the reference op boundary: forward renders, backward takes four "
                                           "upstream gradient images (no fused losses)"}
 
     def leg_c2():
         sets2, _ = auto_sets(1, 1)
         o2 = Ours(dev, rank, 1, 1, sets2)
-        ms2, steps2, _ = measure_resident(o2.step_fused, sets2, dev, world, args.steps, 3)
+        ms2, _ = measure_resident(o2.step_fused, sets2, dev, world, steps, 3)
         return {"workload": "c2: one chunk x one 320x256 view (BASELINE configs[1]), fused losses", "unit": "rays/s",
-                "value": world * o2.rays * steps2 / (ms2 * 1e-3), "ms_per_step": ms2 / steps2, "steps": steps2}
+                "value": world * o2.rays * steps / (ms2 * 1e-3), "ms_per_step": ms2 / steps, "steps": steps}
 
     if not args.no_secondary:
         secondary("e2e_train_flow", leg_flow)
@@ -974,7 +1013,7 @@ def main():
     # per step: fill, index, cell classes, forward (its last CTA finalises the loss), gather
     launches = 5
     if not args.no_train:
-        o.mods, o.devsets = None, None
+        o.mods, o.devsets, o.returned = None, None, None
         torch.cuda.empty_cache()
         def leg_train():
             # the step as this package runs it on B200 (generator in NDHWC), and the same step with the generator left in
@@ -989,7 +1028,7 @@ def main():
         line = dict(base, value=value, steps=steps, ms_per_step=ms / steps, clocks=sampler.summary(),
                     e2e={"value": e2e, "unit": "rays/s", "h2d_bytes_per_step": copy_only.pop("h2d_bytes_per_step"),
                          "host_input_bytes_per_step": bytes_of(o.host[0], H2D_KEYS),
-                         "d2h_bytes_per_step": 4, "steps": e2e_steps, "ms_per_step": ms_e2e / e2e_steps,
+                         "d2h_bytes_per_step": 4, "steps": steps, "ms_per_step": ms_e2e / steps,
                          "api": "host inputs in the reference's formats -> spsg_b200.raycast_rgbd_cuda.pack_locs_host (int64 "
                                 "voxel rows -> uint32 cell indices, %d host threads, every step) -> one pinned staging buffer "
                                 "copied on a copy stream (double-buffered) -> spsg_b200.losses.render_with_2d_losses (fused "

@@ -11,10 +11,10 @@ from oracle import ref_driver as refdriver
 from tests.test_gpu_adversarial import _batch, _cameras
 from spsg_b200.raycast_rgbd import RaycastRGBD
 
-def run(cases=100, seed0=0, dev=None):
+def run(cases=100, seed0=0, dev=None, pinned=False):
     """Returns the number of mismatching cases."""
     dev = dev or torch.device("cuda", 0)
-    assert refdriver.available(), "oracle/_ref not built"
+    assert refdriver.available(pinned), "oracle/_ref not built"
     bad = skipped = 0
     t0 = time.time()
     for c in range(cases):
@@ -32,7 +32,7 @@ def run(cases=100, seed0=0, dev=None):
         f = float(rng.uniform(0.5, 1.5)) * w
         intr = torch.tensor([[f, f, (w - 1) / 2, (h - 1) / 2]] * (B * F), device=dev)
         mine = RaycastRGBD(B, dims, w, h, 0.0, 150.0, 50.0, inc, max_num_frames=F, max_num_locs_per_sample=n, device=dev)
-        ref = refdriver.RefRaycaster(B, dims, w, h, 0.0, 150.0, 50.0, inc, n, 64, device=dev)
+        ref = refdriver.RefRaycaster(B, dims, w, h, 0.0, 150.0, 50.0, inc, n, 64, device=dev, pinned=pinned)
         leaves = [t[k].clone().requires_grad_(True) for k in ("sdf", "color", "normal", "semantic")]
         out = mine(t["locs"], leaves[0], leaves[1], leaves[2], leaves[3], view, intr)
         g = torch.Generator(device=dev).manual_seed(c)

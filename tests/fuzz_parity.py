@@ -10,10 +10,10 @@ from tests.test_gpu_adversarial import _batch, _cameras
 from tests.common import count_bit_mismatch
 from spsg_b200.raycast_rgbd import RaycastRGBD
 
-def run(cases=100, seed0=0, dev=None, large=False):
+def run(cases=100, seed0=0, dev=None, large=False, pinned=False):
     """Returns the number of mismatching cases."""
     dev = dev or torch.device("cuda", 0)
-    assert refdriver.available(), "oracle/_ref not built"
+    assert refdriver.available(pinned), "oracle/_ref not built"
     bad = 0
     t0 = time.time()
     for c in range(cases):
@@ -42,7 +42,7 @@ def run(cases=100, seed0=0, dev=None, large=False):
         f = float(rng.uniform(0.4, 1.5)) * w
         intr = torch.tensor([[f, f * float(rng.uniform(0.9, 1.1)), (w - 1) / 2 + float(rng.uniform(-2, 2)), (h - 1) / 2]] * B, device=dev)
         mine = RaycastRGBD(B, dims, w, h, dmin, dmax, thresh, inc, max_num_frames=1, max_num_locs_per_sample=n, max_pixels_per_voxel=max_pix, device=dev)
-        ref = refdriver.RefRaycaster(B, dims, w, h, dmin, dmax, thresh, inc, n, max_pix, device=dev)
+        ref = refdriver.RefRaycaster(B, dims, w, h, dmin, dmax, thresh, inc, n, max_pix, device=dev, pinned=pinned)
         desc = "case %d: dims %s B %d img %dx%d inc %g dmin %g dmax %g thresh %g max_pix %d specs %s n %d" % (
             c, dims, B, w, h, inc, dmin, dmax, thresh, max_pix, specs, n)
         try:

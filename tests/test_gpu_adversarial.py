@@ -94,11 +94,11 @@ def _cameras(dims_zyx, count, seed, device, lattice=False):
 
 def _pair(device, batch, dims, w, h, n_max, dmin, dmax, inc, thresh, max_pix=64):
     from spsg_b200.raycast_rgbd import RaycastRGBD
-    if not refdriver.available():
+    if not refdriver.available(pinned=True):
         pytest.skip("oracle/_ref not built (run __graft_entry__.build() where /root/reference exists)")
     mine = RaycastRGBD(batch, dims, w, h, dmin, dmax, thresh, inc, max_num_frames=1, max_num_locs_per_sample=n_max,
                        max_pixels_per_voxel=max_pix, device=device)
-    ref = refdriver.RefRaycaster(batch, dims, w, h, dmin, dmax, thresh, inc, n_max, max_pix, device=device)
+    ref = refdriver.RefRaycaster(batch, dims, w, h, dmin, dmax, thresh, inc, n_max, max_pix, device=device, pinned=True)
     return mine, ref
 
 

@@ -19,13 +19,13 @@ B, F = 8, 5
 def _modules(device, n, batch=B, frames=F):
     from spsg_b200 import synthetic as S
     from spsg_b200.raycast_rgbd import RaycastRGBD
-    if not refdriver.available():
+    if not refdriver.available(pinned=True):
         pytest.skip("oracle/_ref not built (run __graft_entry__.build() where /root/reference exists)")
     n_max = n // batch + 1000
     mine = RaycastRGBD(batch, S.DIMS_ZYX, S.WIDTH, S.HEIGHT, S.DEPTH_MIN, S.DEPTH_MAX, S.THRESH_SAMPLE_DIST, S.RAY_INCREMENT,
                        max_num_frames=frames, max_num_locs_per_sample=n_max, device=device)
     ref = refdriver.RefRaycaster(batch, S.DIMS_ZYX, S.WIDTH, S.HEIGHT, S.DEPTH_MIN, S.DEPTH_MAX, S.THRESH_SAMPLE_DIST,
-                                 S.RAY_INCREMENT, n_max, 64, device=device)
+                                 S.RAY_INCREMENT, n_max, 64, device=device, pinned=True)
     return mine, ref
 
 

@@ -27,7 +27,7 @@ def _frames(device, batch=3, h=96, w=128, holes=0.03, seed=0, hole_blocks=True):
 
 
 def _need_ref():
-    if not refdriver.depth_available():
+    if not refdriver.depth_available(pinned=True):
         pytest.skip("oracle/_ref depth_utils not built (run __graft_entry__.build() where /root/reference exists)")
 
 
@@ -38,7 +38,7 @@ def _bits_equal(a, b):
 def test_individual_entry_points_bit_exact(cuda_device):
     _need_ref()
     from spsg_b200 import depth_utils_cuda as mine
-    ref = refdriver.depth_module()
+    ref = refdriver.depth_module(pinned=True)
     depth, intr = _frames(cuda_device)
     b, _, h, w = depth.shape
     fa, fb = torch.zeros_like(depth), torch.zeros_like(depth)
@@ -70,7 +70,7 @@ def test_depth2normals_pipeline_bit_exact(cuda_device, holes):
     mod = Depth2Normals(b, w, h, 0.1 / 0.02, 6.0 / 0.02, device=cuda_device)
     got = mod(d_mine, intr)
     filt, cam, nrm = torch.zeros_like(depth), torch.zeros(b, h, w, 3, device=cuda_device), torch.zeros(b, h, w, 3, device=cuda_device)
-    want = refdriver.ref_depth2normals(d_ref, intr, filt, cam, nrm)
+    want = refdriver.ref_depth2normals(d_ref, intr, filt, cam, nrm, pinned=True)
     assert (got is None) == (want is None)
     assert got is not None, "the synthetic holes are meant to be fillable"
     assert got.shape == (b, 3, h, w)
@@ -94,7 +94,7 @@ def test_depth2normals_returns_none_when_holes_remain(cuda_device):
     _need_ref()
     from spsg_b200 import depth_utils_cuda as mine
     from spsg_b200.depth_utils import Depth2Normals
-    ref = refdriver.depth_module()
+    ref = refdriver.depth_module(pinned=True)
     depth, intr = _frames(cuda_device, batch=1, holes=0.0, hole_blocks=False, seed=2)
     depth[:, :, 10:70, 20:100] = 0.0                 # far wider than what one fill round (2 x 5 pixels) can close
     b, _, h, w = depth.shape

@@ -8,26 +8,26 @@ pytestmark = pytest.mark.gpu
 
 def _need_ref():
     from oracle import ref_driver
-    if not ref_driver.available():
+    if not ref_driver.available(pinned=True):
         pytest.skip("oracle/_ref not built (run __graft_entry__.build() where /root/reference exists)")
 
 
 def test_fuzz_forward_bit_exact_slice(cuda_device):
     _need_ref()
     from tests import fuzz_parity
-    assert fuzz_parity.run(cases=200, seed0=20261, dev=cuda_device) == 0
+    assert fuzz_parity.run(cases=200, seed0=20261, dev=cuda_device, pinned=True) == 0
 
 
 def test_fuzz_forward_bit_exact_large_images(cuda_device):
     _need_ref()
     from tests import fuzz_parity
-    assert fuzz_parity.run(cases=24, seed0=977, dev=cuda_device, large=True) == 0
+    assert fuzz_parity.run(cases=24, seed0=977, dev=cuda_device, large=True, pinned=True) == 0
 
 
 def test_fuzz_backward_slice(cuda_device):
     _need_ref()
     from tests import fuzz_backward
-    assert fuzz_backward.run(cases=80, seed0=31, dev=cuda_device) == 0
+    assert fuzz_backward.run(cases=80, seed0=31, dev=cuda_device, pinned=True) == 0
 
 
 def test_fuzz_fused_losses_slice(cuda_device):

@@ -27,12 +27,12 @@ def _mine(device, batch_size, dims, w, h, n_max, dmin=None, dmax=None, thresh=No
 
 def _ref(device, batch_size, dims, w, h, n_max, dmin=None, dmax=None, thresh=None, inc=None, max_pix=64):
     from spsg_b200 import synthetic as S
-    if not refdriver.available():
+    if not refdriver.available(pinned=True):
         pytest.skip("oracle/_ref not built (run __graft_entry__.build() where /root/reference exists)")
     return refdriver.RefRaycaster(batch_size, dims, w, h, S.DEPTH_MIN if dmin is None else dmin,
                                   S.DEPTH_MAX if dmax is None else dmax,
                                   S.THRESH_SAMPLE_DIST if thresh is None else thresh,
-                                  S.RAY_INCREMENT if inc is None else inc, n_max, max_pix, device=device)
+                                  S.RAY_INCREMENT if inc is None else inc, n_max, max_pix, device=device, pinned=True)
 
 
 def _assert_render_equal(mine, ref, what=""):
@@ -213,7 +213,7 @@ def test_multi_view_equals_looped_reference(cuda_device):
 def test_raycast_occ_bit_exact(cuda_device):
     from spsg_b200 import synthetic as S
     from spsg_b200.raycast_rgbd import RaycastOcc
-    if not refdriver.available():
+    if not refdriver.available(pinned=True):
         pytest.skip("oracle/_ref not built")
     w, h = 160, 128
     sdf, _ = S.sdf_volume(3)
@@ -224,7 +224,7 @@ def test_raycast_occ_bit_exact(cuda_device):
     got = mine(occ, view, intr)
     want = torch.zeros_like(got)
     opts = torch.FloatTensor([w, h, S.DEPTH_MIN, S.DEPTH_MAX, S.RAY_INCREMENT, 64, 64, 128])
-    refdriver.module().raycast_occ(occ, want, view, intr, opts)
+    refdriver.module(pinned=True).raycast_occ(occ, want, view, intr, opts)
     assert torch.equal(got, want)
     assert 0.2 < got.float().mean().item() < 1.0
 

@@ -33,7 +33,7 @@ def test_room_windows_match_looped_reference_calls(cuda_device):
     and call), labels by the literal argmax(cat(render, ones)) of train.py:749-752."""
     from oracle import ref_driver
     from spsg_b200 import room as R, synthetic as S
-    if not ref_driver.available():
+    if not ref_driver.available(pinned=True):
         pytest.skip("oracle/_ref not built (run __graft_entry__.build() where /root/reference exists)")
     dims, F, w, h = (64, 96, 128), 3, 96, 64
     room = R.synthetic_room_sdf(dims, cuda_device, seed=3)
@@ -45,7 +45,7 @@ def test_room_windows_match_looped_reference_calls(cuda_device):
     view = torch.from_numpy(view_np).to(cuda_device)
     intr = torch.from_numpy(intr_np).to(cuda_device)
     ref = ref_driver.RefRaycaster(1, chunk_dims, w, h, S.DEPTH_MIN, S.DEPTH_MAX, S.THRESH_SAMPLE_DIST, S.RAY_INCREMENT,
-                                  200000, 64, device=cuda_device)
+                                  200000, 64, device=cuda_device, pinned=True)
     hist = np.zeros(S.NUM_CLASSES + 1)
     images = dict(got["images"])
     assert len(images) == got["rendered_windows"] > 6
