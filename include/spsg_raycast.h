@@ -195,6 +195,31 @@ SPSG_API int spsg_raycast_backward_loss(const spsg_raycast_params *p, const floa
                                         float *d_normal, float *d_semantic, void *workspace, size_t workspace_bytes,
                                         void *stream);
 
+/* Gradients of an objective with respect to the four renderings of a fused forward, from terms the library does not
+ * compute itself (a patch-GAN discriminator or a style loss on the rendered colour and normals). */
+typedef struct spsg_upstream_grads {   /* d objective / d rendering, same layouts as the images; NULL plane = 0 */
+    const float *grad_color;    /* (I,H,W,3)  */
+    const float *grad_depth;    /* (I,H,W)    */
+    const float *grad_normal;   /* (I,H,W,3)  */
+    const float *grad_semantic; /* (I,H,W,14), 8-byte aligned */
+} spsg_upstream_grads;
+
+/* spsg_raycast_backward_loss that also gathers caller-supplied upstream gradient images, in the same launch:
+ *     d_x[v] = sum over views of mean over the pixels registered to voxel v of
+ *              (recomputed 2D-loss gradient * grad_scale + upstream gradient)
+ * Upstream gradients are not multiplied by grad_scale.  Gradients at pixels that hit nothing are ignored, as in
+ * spsg_raycast_backward.  Loss targets switched off (NULL target pointers) give exactly spsg_raycast_backward of the
+ * upstream images; upstream NULL, or all four planes NULL, gives exactly spsg_raycast_backward_loss.  The renderings must be
+ * those of the matching spsg_raycast_forward_loss, unmodified. */
+SPSG_API int spsg_raycast_backward_loss_upstream(const spsg_raycast_params *p, const float *image_color,
+                                                 const float *image_depth, const float *image_semantic,
+                                                 const spsg_loss_targets *t, const float *loss_out,
+                                                 const float *grad_scale, const spsg_upstream_grads *upstream,
+                                                 const int32_t *sparse_mapping, const int32_t *mapping3dto2d,
+                                                 const int32_t *mapping3dto2d_num, float *d_color, float *d_depth,
+                                                 float *d_normal, float *d_semantic, void *workspace,
+                                                 size_t workspace_bytes, void *stream);
+
 /* == loss.compute_normals_sparse (reference torch/loss.py:285-306, with compute_normals_dense :261-267): per-voxel
  *    normals of the sparse SDF, the producer of the raycaster's vals_normals (train.py:542).  normals[i] =
  *    -normalize(R_chunk * central_difference(sdf at voxel i), eps 1e-5); absent neighbours count as 0, voxels on the

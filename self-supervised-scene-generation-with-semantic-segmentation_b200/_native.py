@@ -26,8 +26,8 @@ SPSG_DEPTH_MAX_FILL_ROUNDS = 64
 EXPORTS = (
     "spsg_version", "spsg_last_error", "spsg_workspace_bytes", "spsg_build_index", "spsg_raycast_forward",
     "spsg_raycast_forward_indexed", "spsg_raycast_backward", "spsg_raycast_occ", "spsg_raycast_forward_loss",
-    "spsg_raycast_backward_loss", "spsg_timing_enable", "spsg_timing_read", "spsg_normals_forward",
-    "spsg_normals_backward", "spsg_losses2d_forward", "spsg_losses2d_backward",
+    "spsg_raycast_backward_loss", "spsg_raycast_backward_loss_upstream", "spsg_timing_enable", "spsg_timing_read",
+    "spsg_normals_forward", "spsg_normals_backward", "spsg_losses2d_forward", "spsg_losses2d_backward",
     "spsg_depth_bilateral_filter", "spsg_depth_median_fill", "spsg_depth_to_cameraspace", "spsg_depth_to_normals",
     "spsg_depth_compute_normals",
     "spsg_sparsify_scratch_bytes", "spsg_sparsify_count", "spsg_sparsify_locs", "spsg_sparsify_locs_indexed",
@@ -72,6 +72,12 @@ class GradBuffers(ctypes.Structure):
                 ("d_semantic", ctypes.c_void_p)]
 
 
+class UpstreamGrads(ctypes.Structure):
+    """``spsg_upstream_grads``"""
+    _fields_ = [("grad_color", ctypes.c_void_p), ("grad_depth", ctypes.c_void_p), ("grad_normal", ctypes.c_void_p),
+                ("grad_semantic", ctypes.c_void_p)]
+
+
 def _load():
     if not os.path.isfile(LIB_PATH):
         raise ImportError(
@@ -102,6 +108,9 @@ def _load():
     lib.spsg_raycast_forward_loss.argtypes = [pp] + [vp] * 14 + [lt, vp, gb, vp, sz, vp]
     lib.spsg_raycast_backward_loss.restype = ctypes.c_int
     lib.spsg_raycast_backward_loss.argtypes = [pp, vp, vp, vp, lt, vp, vp] + [vp] * 7 + [vp, sz, vp]
+    lib.spsg_raycast_backward_loss_upstream.restype = ctypes.c_int
+    lib.spsg_raycast_backward_loss_upstream.argtypes = [pp, vp, vp, vp, lt, vp, vp, ctypes.POINTER(UpstreamGrads)] + \
+        [vp] * 7 + [vp, sz, vp]
     lib.spsg_normals_forward.restype = ctypes.c_int
     lib.spsg_normals_forward.argtypes = [vp, i64, vp, vp, vp, i32, i32, i32, i32, vp, vp]
     lib.spsg_normals_backward.restype = ctypes.c_int

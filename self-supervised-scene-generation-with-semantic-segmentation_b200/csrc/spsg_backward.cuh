@@ -22,6 +22,9 @@ struct BackwardArgs {
     int views, max_pixels;
     long long num_locs;
     int zero_blocks;  // leading CTAs of the launch that clear gradient rows instead of gathering
+    // fused variant with upstream images (kUpstream): d objective / d rendering added to the recomputed loss gradients;
+    // NULL plane = 0.  (Last in the struct: the other variants' parameter offsets stay where they were.)
+    const float *up_color, *up_depth, *up_normal, *up_semantic;
 };
 
 // Clears the 21 gradient slots of voxels [0, N) (replaces the 4 whole-buffer memsets of kernel.cu:557-560): a warp
@@ -144,6 +147,29 @@ __device__ __forceinline__ void pixel_grads_fused(const BackwardArgs &a, const F
     t[17] = gd; t[18] = 0.0f; t[19] = 0.0f; t[20] = 0.0f;
 }
 
+// kUpstream: the caller's gradient images of the same pixel added, in fp32, onto the row pixel_grads_fused just wrote
+// (read-modify-write of shared memory rather than 21 more live registers).  Which planes are present is the same for the
+// whole launch, so the branches do not diverge.  Not scaled by grad_scale: that is d objective / d loss_out[3] only.
+__device__ __forceinline__ void add_upstream_grads(const BackwardArgs &a, unsigned gpix, float *__restrict__ t) {
+    if (a.up_semantic) {
+        const float2 *s2 = reinterpret_cast<const float2 *>(a.up_semantic + (size_t)gpix * 14);
+#pragma unroll
+        for (int k = 0; k < 7; k++) {
+            const float2 v = __ldg(s2 + k);
+            t[2 * k] += v.x; t[2 * k + 1] += v.y;
+        }
+    }
+    if (a.up_color) {
+        const float *c = a.up_color + (size_t)gpix * 3;
+        t[14] += __ldg(c); t[15] += __ldg(c + 1); t[16] += __ldg(c + 2);
+    }
+    if (a.up_depth) t[17] += __ldg(a.up_depth + gpix);
+    if (a.up_normal) {
+        const float *n = a.up_normal + (size_t)gpix * 3;
+        t[18] += __ldg(n); t[19] += __ldg(n + 1); t[20] += __ldg(n + 2);
+    }
+}
+
 // The gather (kernel.cu:391-419 turned inside out).  Work items are the (voxel, view) pairs the forward listed; one
 // warp per item.  Lane k fetches the k-th registered pixel id (one coalesced load) and that pixel's 21 upstream
 // gradients (independent 8- and 4-byte loads), parks them in shared memory, and lane c then adds column c in
@@ -158,11 +184,13 @@ constexpr int kGatherWarps = 8;
 constexpr int kGatherGroup = SPSG_GATHER_GROUP;  // lanes per (voxel, view) item
 
 // kViews: 0 = one view per chunk; 1 = several, per-view means added with float atomics (fast); 2 = several, deterministic
-template <bool kFused, int kViews>
+// kUpstream (needs kFused): each pixel's row is the recomputed loss gradient plus the caller's upstream gradient images
+template <bool kFused, bool kUpstream, int kViews>
 #ifndef SPSG_GATHER_MIN_BLOCKS
 #define SPSG_GATHER_MIN_BLOCKS 8  // 32 registers: full occupancy hides the dependent gathers (the fused variant spills ~150 B and is still faster)
 #endif
 __global__ void __launch_bounds__(kGatherWarps * 32, SPSG_GATHER_MIN_BLOCKS) backward_gather_kernel(const BackwardArgs a) {
+    static_assert(kFused || !kUpstream, "upstream images are added to the fused variant's recomputed gradients");
     if ((int)blockIdx.x < a.zero_blocks) {
         zero_rows<true>(a, ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5, ((long long)a.zero_blocks * blockDim.x) >> 5);
         return;
@@ -219,6 +247,7 @@ __global__ void __launch_bounds__(kGatherWarps * 32, SPSG_GATHER_MIN_BLOCKS) bac
                         const unsigned gpix = pixbase + (unsigned)__ldg(prow + k0 + hl);
                         if (kFused) {
                             pixel_grads_fused(a, fc, gpix, tile + hl * 21);
+                            if (kUpstream) add_upstream_grads(a, gpix, tile + hl * 21);
                         } else {
                             float g[21];
                             pixel_grads(a, gpix, g);

@@ -261,12 +261,18 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
                     const float *grad_normal, const float *g_or_img_semantic, const spsg_loss_targets *targets,
                     const float *loss_out, const float *grad_scale, const int32_t *sparse_mapping,
                     const int32_t *mapping3dto2d, const int32_t *mapping3dto2d_num, float *d_color, float *d_depth,
-                    float *d_normal, float *d_semantic, void *workspace, size_t workspace_bytes, cudaStream_t st) {
+                    float *d_normal, float *d_semantic, void *workspace, size_t workspace_bytes, cudaStream_t st,
+                    const spsg_upstream_grads *upstream = nullptr) {
     if (int rc = check_params(p)) return rc;
     if (!g_or_img_color || !g_or_img_depth || !g_or_img_semantic || (!fused && !grad_normal) || !sparse_mapping ||
         !mapping3dto2d || !mapping3dto2d_num)
         return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL tensor pointer");
     if (fused && (!targets || !loss_out)) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL loss targets");
+    // upstream images (fused only): any plane may be NULL; none at all is exactly the fused backward without them
+    const bool up = fused && upstream &&
+                    (upstream->grad_color || upstream->grad_depth || upstream->grad_normal || upstream->grad_semantic);
+    if (up && (reinterpret_cast<uintptr_t>(upstream->grad_semantic) & 7u))
+        return fail(SPSG_ERR_INVALID_ARGUMENT, "upstream grad_semantic must be 8-byte aligned");
     if (p->max_pixels_per_voxel <= 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "max_pixels_per_voxel must be positive");
     if (p->num_locs == 0) return SPSG_OK;
     if (!d_color || !d_depth || !d_normal || !d_semantic) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL gradient pointer");
@@ -282,6 +288,10 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
         a.loss_out = loss_out;
         a.w_depth = targets->weight_depth; a.w_color = targets->weight_color_loss; a.w_sem = targets->weight_semantic;
         a.grad_scale = grad_scale;
+        if (up) {
+            a.up_color = upstream->grad_color; a.up_depth = upstream->grad_depth; a.up_normal = upstream->grad_normal;
+            a.up_semantic = upstream->grad_semantic;
+        }
     } else {
         a.grad_color = g_or_img_color; a.grad_depth = g_or_img_depth; a.grad_normal = grad_normal;
         a.grad_semantic = g_or_img_semantic;
@@ -300,12 +310,18 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
     const unsigned zero_blocks = (unsigned)std::min<long long>((p->num_locs + 255) / 256, (long long)sms * 4);
     const bool cleared = (p->flags & SPSG_FLAG_GRADS_CLEARED) != 0;  // the forward's fill pass cleared rows [0, N)
     const bool multi = p->views_per_chunk > 1, exact = (p->flags & SPSG_FLAG_DETERMINISTIC_GRADS) != 0;
-#define SPSG_GATHER(FUSED, VIEWS, BLOCKS) backward_gather_kernel<FUSED, VIEWS><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a)
-#define SPSG_GATHER_ANY(BLOCKS)                                                         \
-    do {                                                                                \
-        if (!multi) { if (fused) SPSG_GATHER(true, 0, BLOCKS); else SPSG_GATHER(false, 0, BLOCKS); }       \
-        else if (!exact) { if (fused) SPSG_GATHER(true, 1, BLOCKS); else SPSG_GATHER(false, 1, BLOCKS); }  \
-        else { if (fused) SPSG_GATHER(true, 2, BLOCKS); else SPSG_GATHER(false, 2, BLOCKS); }              \
+#define SPSG_GATHER(FUSED, UP, VIEWS, BLOCKS) backward_gather_kernel<FUSED, UP, VIEWS><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a)
+#define SPSG_GATHER_VIEWS(VIEWS, BLOCKS)                                                                          \
+    do {                                                                                                          \
+        if (up) SPSG_GATHER(true, true, VIEWS, BLOCKS);                                                           \
+        else if (fused) SPSG_GATHER(true, false, VIEWS, BLOCKS);                                                  \
+        else SPSG_GATHER(false, false, VIEWS, BLOCKS);                                                            \
+    } while (0)
+#define SPSG_GATHER_ANY(BLOCKS)                                                                                   \
+    do {                                                                                                          \
+        if (!multi) SPSG_GATHER_VIEWS(0, BLOCKS);                                                                 \
+        else if (!exact) SPSG_GATHER_VIEWS(1, BLOCKS);                                                            \
+        else SPSG_GATHER_VIEWS(2, BLOCKS);                                                                        \
     } while (0)
     if (cleared) {
         a.zero_blocks = 0;
@@ -324,6 +340,7 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
         SPSG_GATHER_ANY(gather_blocks);
     }
 #undef SPSG_GATHER_ANY
+#undef SPSG_GATHER_VIEWS
 #undef SPSG_GATHER
     CUDA_TRY(cudaGetLastError());
     return SPSG_OK;
@@ -477,6 +494,17 @@ int spsg_raycast_backward_loss(const spsg_raycast_params *p, const float *image_
     return launch_backward(p, true, image_color, image_depth, nullptr, image_semantic, t, loss_out, grad_scale,
                            sparse_mapping, mapping3dto2d, mapping3dto2d_num, d_color, d_depth, d_normal, d_semantic,
                            workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int spsg_raycast_backward_loss_upstream(const spsg_raycast_params *p, const float *image_color, const float *image_depth,
+                                        const float *image_semantic, const spsg_loss_targets *t, const float *loss_out,
+                                        const float *grad_scale, const spsg_upstream_grads *upstream,
+                                        const int32_t *sparse_mapping, const int32_t *mapping3dto2d,
+                                        const int32_t *mapping3dto2d_num, float *d_color, float *d_depth, float *d_normal,
+                                        float *d_semantic, void *workspace, size_t workspace_bytes, void *stream) {
+    return launch_backward(p, true, image_color, image_depth, nullptr, image_semantic, t, loss_out, grad_scale,
+                           sparse_mapping, mapping3dto2d, mapping3dto2d_num, d_color, d_depth, d_normal, d_semantic,
+                           workspace, workspace_bytes, (cudaStream_t)stream, upstream);
 }
 
 static int normals_check(const int64_t *locs, int64_t n, const float *sdf, const int32_t *index, int32_t num_chunks,

@@ -7,8 +7,9 @@ kernel, accumulates the reference's three 2D loss terms
     colour L1     mean |colour * w - target * w|            over hit pixels x 3 channels      loss.py:246-257
     semantic CE   sum w[y] * nll / sum w[y]                 over (hit & label < 14)           train.py:744-746
 
-Its backward never materialises the four gradient images: every registered pixel's upstream gradient is
-recomputed from (rendering, target, normalisers) inside the per-voxel gather.  No CPU path.
+Its backward never materialises the loss terms' gradient images: every registered pixel's gradient is recomputed from
+(rendering, target, normalisers) inside the per-voxel gather, which can also add the caller's own gradient images of the
+renderings (``differentiable_images=True``).  No CPU path.
 """
 import ctypes
 
@@ -113,31 +114,69 @@ def fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, v
     return p, tg, loss_out
 
 
-def fused_backward(m, p, tg, loss_out, grad_scale, grads_cleared):
-    """``spsg_raycast_backward_loss``: voxel gradients of ``grad_scale * total`` into rows [0, N) of ``m.d_*``."""
+def _upstream_struct(m, p, upstream):
+    """``spsg_upstream_grads`` of ``upstream`` = (grad_color, grad_depth, grad_normal, grad_semantic), any of them None:
+    contiguous float32 CUDA tensors shaped like the renderings of the forward ``p`` describes."""
+    images = p.num_chunks * p.views_per_chunk
+    px = images * p.height * p.width
+    ptrs = []
+    for g, ch, name in zip(upstream, (3, 1, 3, 14), ("grad_color", "grad_depth", "grad_normal", "grad_semantic")):
+        if g is not None:
+            rc._check_input(g, name)
+            rc._check_dtype(g, torch.float32, name)
+            if g.numel() != ch * px or g.device != m.image_depth.device:
+                raise RuntimeError("%s must hold %d x %d x %d x %d floats on %s" % (name, images, p.height, p.width, ch,
+                                                                                   m.image_depth.device))
+        ptrs.append(N.ptr(g))
+    return N.UpstreamGrads(*ptrs)
+
+
+def fused_backward(m, p, tg, loss_out, grad_scale, grads_cleared, upstream=None):
+    """``spsg_raycast_backward_loss``: voxel gradients of ``grad_scale * total`` into rows [0, N) of ``m.d_*``.
+    ``upstream`` = (grad_color, grad_depth, grad_normal, grad_semantic) gradient images of the renderings (any of them
+    None; contiguous float32): ``spsg_raycast_backward_loss_upstream`` then adds them, unscaled, in the same gather.
+    ``grad_scale`` None means 1."""
     if grads_cleared:
         p.flags |= N.SPSG_FLAG_GRADS_CLEARED
     dev = m.image_depth.device
-    rc._check_input(grad_scale, "grad_scale")
-    rc._check_dtype(grad_scale, torch.float32, "grad_scale")
+    if grad_scale is not None:
+        rc._check_input(grad_scale, "grad_scale")
+        rc._check_dtype(grad_scale, torch.float32, "grad_scale")
+    up = _upstream_struct(m, p, upstream) if upstream is not None else None
     owner = _module_workspace(m)
     with rc.device_guard(dev):
         ws = owner.check(p, N.workspace_bytes(p))  # the work list of the forward that rendered m's images
-        N.check(N.lib.spsg_raycast_backward_loss(
-            ctypes.byref(p), N.ptr(m.image_color), N.ptr(m.image_depth), N.ptr(m.image_semantic),
-            ctypes.byref(tg), N.ptr(loss_out), N.ptr(grad_scale), N.ptr(m.sparse_mapping), N.ptr(m.mapping3dto2d),
-            N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth), N.ptr(m.d_normal), N.ptr(m.d_semantic),
-            N.ptr(ws), ws.numel(), rc._stream(dev)))
+        if up is None:
+            N.check(N.lib.spsg_raycast_backward_loss(
+                ctypes.byref(p), N.ptr(m.image_color), N.ptr(m.image_depth), N.ptr(m.image_semantic),
+                ctypes.byref(tg), N.ptr(loss_out), N.ptr(grad_scale), N.ptr(m.sparse_mapping), N.ptr(m.mapping3dto2d),
+                N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth), N.ptr(m.d_normal), N.ptr(m.d_semantic),
+                N.ptr(ws), ws.numel(), rc._stream(dev)))
+        else:
+            N.check(N.lib.spsg_raycast_backward_loss_upstream(
+                ctypes.byref(p), N.ptr(m.image_color), N.ptr(m.image_depth), N.ptr(m.image_semantic),
+                ctypes.byref(tg), N.ptr(loss_out), N.ptr(grad_scale), ctypes.byref(up), N.ptr(m.sparse_mapping),
+                N.ptr(m.mapping3dto2d), N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth),
+                N.ptr(m.d_normal), N.ptr(m.d_semantic), N.ptr(ws), ws.numel(), rc._stream(dev)))
+
+
+def _targets_off(tg):
+    """A copy of the targets struct with every loss term switched off: the fused backward then gathers the upstream
+    images alone."""
+    return N.LossTargets(None, None, None, None, None, tg.voxelsize, tg.weight_depth, tg.weight_color_loss,
+                         tg.weight_semantic)
 
 
 class FusedRaycastLossFunction(Function):
     @staticmethod
     def forward(ctx, raycaster, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, view_matrix,
                 intrinsic_params, target_depth, target_color, weight_color, target_label, class_weight, voxelsize,
-                weights):
+                weights, differentiable_images=False):
         m = raycaster
         n = locs.shape[0]
         images = view_matrix.shape[0]
+        # gradients that do not reach an output stay None: no zero-filled image per non-differentiable rendering
+        ctx.set_materialize_grads(False)
         # a backward will follow: let the forward's fill pass clear the gradient rows it will write
         ctx.grads_cleared = any(ctx.needs_input_grad[2:6]) and n > 0
         p, tg, loss_out = fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, view_matrix,
@@ -146,21 +185,42 @@ class FusedRaycastLossFunction(Function):
         ctx.raycaster, ctx.params, ctx.targets, ctx.n, ctx.loss_out = m, p, tg, n, loss_out
         # keep the target tensors alive until backward (the struct only holds raw pointers)
         ctx.keep = (target_depth, target_color, weight_color, target_label, class_weight)
-        ctx.mark_non_differentiable(m.image_color, m.image_depth, m.image_normal, m.image_semantic)
+        ctx.differentiable_images = differentiable_images
         imgs = (m.image_color, m.image_depth, m.image_normal, m.image_semantic)
-        if images != m.image_depth.shape[0]:
-            imgs = tuple(i[:images] for i in imgs)
+        if not differentiable_images:
             ctx.mark_non_differentiable(*imgs)
+        if images != m.image_depth.shape[0] or differentiable_images:
+            # differentiable: always views, so that the module's buffers themselves never carry this node's history
+            # (the next forward of the module takes them as inputs, and must not link its graph to this one)
+            imgs = tuple(i[:images] for i in imgs)
+            if not differentiable_images:
+                ctx.mark_non_differentiable(*imgs)
+        if differentiable_images:
+            # the backward recomputes the loss gradients from these buffers: saving them makes an in-place change
+            # before backward() an error (autograd's version counter) instead of silently wrong gradients
+            ctx.save_for_backward(*imgs)
         terms = loss_out[:3]
         ctx.mark_non_differentiable(terms)
         return (loss_out[3], terms) + imgs
 
     @staticmethod
-    def backward(ctx, grad_total, grad_terms, *unused):
+    def backward(ctx, grad_total, grad_terms, *grad_images):
         m, n = ctx.raycaster, ctx.n
-        fused_backward(m, ctx.params, ctx.targets, ctx.loss_out, grad_total.to(torch.float32).contiguous(),
-                       ctx.grads_cleared)
-        return (None, None, m.d_depth[:n], m.d_color[:n], m.d_normal[:n], m.d_semantic[:n]) + (None,) * 9
+        upstream = None
+        if ctx.differentiable_images:
+            ctx.saved_tensors  # noqa: B018 -- raises if a rendering was modified in place since the forward
+            if any(g is not None for g in grad_images):
+                upstream = tuple(None if g is None else g.to(torch.float32).contiguous() for g in grad_images)
+        if grad_total is None and upstream is None:
+            return (None,) * 16
+        if grad_total is None:
+            # only the images feed the objective: no scale derived from the loss normalisers (an empty valid set would
+            # turn 0 * (w / 0) into NaN); the targets switched off leave the plain gather of the upstream images
+            fused_backward(m, ctx.params, _targets_off(ctx.targets), ctx.loss_out, None, ctx.grads_cleared, upstream)
+        else:
+            fused_backward(m, ctx.params, ctx.targets, ctx.loss_out, grad_total.to(torch.float32).contiguous(),
+                           ctx.grads_cleared, upstream)
+        return (None, None, m.d_depth[:n], m.d_color[:n], m.d_normal[:n], m.d_semantic[:n]) + (None,) * 10
 
 
 def render_loss_and_voxel_grads(raycaster, locs, vals_sdf, vals_colors, vals_normals, vals_semantics, view_matrix,
@@ -188,7 +248,8 @@ def render_loss_and_voxel_grads(raycaster, locs, vals_sdf, vals_colors, vals_nor
 def render_with_2d_losses(raycaster, locs, vals_sdf, vals_colors, vals_normals, vals_semantics, view_matrix,
                           intrinsic_params, images_depth=None, images_color=None, weight_color=None,
                           target2d_label=None, weight_semantic_class=None, voxelsize=0.02,
-                          weight_depth_loss=1.0, weight_color_loss=1.0, weight_semantic_loss=1.0):
+                          weight_depth_loss=1.0, weight_color_loss=1.0, weight_semantic_loss=1.0,
+                          differentiable_images=False):
     """Fused prediction raycast + 2D losses (train.py:626-643, 744-746 in one kernel pair).
 
     raycaster        a ``RaycastRGBD`` (owns the image / mapping / gradient buffers, as in the reference)
@@ -197,8 +258,15 @@ def render_with_2d_losses(raycaster, locs, vals_sdf, vals_colors, vals_normals, 
     weight_color     (I,H,W) or (I,1,H,W) per-pixel colour weight or None
     target2d_label   (I,H,W) or (I,H,W,1) uint8, 14 = ignore; None switches the semantic term off
     Returns (total, terms[3] = (depth, colour, semantic), (color, depth, normal, semantic) renderings).
-    ``total = weight_depth_loss*depth + weight_color_loss*colour + weight_semantic_loss*semantic``; gradients flow
-    from ``total`` only (``terms`` are reported values, like the ``.item()`` logging in train.py)."""
+    ``total = weight_depth_loss*depth + weight_color_loss*colour + weight_semantic_loss*semantic``; ``terms`` are
+    reported values, like the ``.item()`` logging in train.py.  Gradients flow from ``total`` and, with
+    ``differentiable_images=True``, from the four renderings too: terms the caller computes on them (a discriminator on
+    ``cat(colour, normal)``, a style loss) are gathered into the voxels by the same backward launch, per registered pixel.
+
+    The renderings are the raycaster's own buffers, as in the reference: any later forward of the same module overwrites
+    them, so this must be the last call on ``raycaster`` before ``backward()`` (clone what is needed beyond that).  With
+    ``differentiable_images=True`` they are saved for the backward, and modifying one in place before ``backward()``
+    raises autograd's version-counter error."""
     if vals_semantics is None:
         vals_semantics = torch.zeros(vals_sdf.shape[0], 14, device=vals_sdf.device)
     out = FusedRaycastLossFunction.apply(
@@ -207,7 +275,8 @@ def render_with_2d_losses(raycaster, locs, vals_sdf, vals_colors, vals_normals, 
         None if images_color is None else images_color.contiguous(),
         None if weight_color is None else weight_color.contiguous(),
         None if target2d_label is None else target2d_label.contiguous(),
-        weight_semantic_class, voxelsize, (weight_depth_loss, weight_color_loss, weight_semantic_loss))
+        weight_semantic_class, voxelsize, (weight_depth_loss, weight_color_loss, weight_semantic_loss),
+        bool(differentiable_images))
     return out[0], out[1], out[2:]
 
 

@@ -31,20 +31,28 @@ def prepare_generator(model):
 
 
 class ViewGuidedTrainStep:
-    """One training iteration past ``num_iters_geo_only`` with the 2D semantic branch (``--pred_3d_semantic ''``), GAN
-    and VGG style terms off (``train.py:740-747``).
+    """One training iteration past ``num_iters_geo_only`` with the 2D semantic branch (``--pred_3d_semantic ''``)
+    (``train.py:740-747``), with or without image-space terms such as the reference's GAN and VGG style losses.
 
     model       generator with the reference's call signature ``model(inputs, mask, pred_sdf=[..], pred_color=..,
                 pred_semantic=..) -> (occ, sdf, colour, semantic)`` dense heads (``model.py:345``); may be DDP-wrapped
     loss_util   module providing the reference's dense 3D losses (``loss.compute_targets``, ``compute_dense_geo_weights``,
                 ``compute_geo_occ_loss``, ``compute_geo_loss``; loss.py:8-146)
+    image_loss  None (GAN and style terms off), or a callable ``image_loss(pred, input2d) -> scalar`` added to the loss:
+                ``pred`` = the prediction's ``(color, depth, normal, semantic)`` renderings, differentiable (their
+                gradients are gathered into the voxels by the fused backward); ``input2d`` = the input scan's (I,6,H,W)
+                conditioning ``cat(colour * 2 - 1, normal)`` with misses set to 0, channels first, as in train.py:556-578,
+                or None with ``render_input=False``.  ``pred`` are the raycaster's buffers, valid until the next step.
+                The discriminator, its own update and the exact form of the GAN / style terms are the caller's: this
+                step only adds what ``image_loss`` returns.  Its value is recorded in ``self.last["image_loss"]``.
     """
 
     def __init__(self, model, loss_util, batch_size, dims3d, width, height, class_weight, voxelsize=0.02, truncation=3.0,
                  weight_occ_loss=1.0, weight_sdf_loss=0.1, weight_depth_loss=1.0, weight_color_loss=1.0,
                  weight_semantic_loss=0.1, weight_surf_geo=1.0, weight_missing_geo=5.0, logweight_sdf=True,
-                 max_num_locs_per_sample=640000, views_per_chunk=1, render_input=True, device=None):
+                 max_num_locs_per_sample=640000, views_per_chunk=1, render_input=True, device=None, image_loss=None):
         self.model, self.loss_util = model, loss_util
+        self.image_loss = image_loss
         self.batch_size, self.dims3d, self.width, self.height = batch_size, tuple(dims3d), width, height
         self.voxelsize, self.truncation = voxelsize, truncation
         self.w = dict(occ=weight_occ_loss, sdf=weight_sdf_loss, depth=weight_depth_loss, color=weight_color_loss,
@@ -73,8 +81,9 @@ class ViewGuidedTrainStep:
         return losses.labels_from_render(raycast_semantic)  # (I,H,W) uint8, 14 = miss / unlabeled
 
     def _render_input(self, inputs, view_matrix, intrinsics, transform):
-        """train.py:556-578: the input scan's colour / normal rendering (the discriminator's conditioning; nothing else reads it,
-        so with the GAN term off it only keeps the step's work like the reference's).  Its normals come from the sparse
+        """train.py:556-578: the input scan's colour / normal rendering (the discriminator's conditioning; with no
+        ``image_loss`` nothing reads it, it only keeps the step's work like the reference's).  Returns the raycaster's
+        buffers, which the next render overwrites.  Its normals come from the sparse
         normals kernel (absent neighbours count as 0), where the reference uses `loss.compute_normals` on the dense input
         volume (truncated neighbours count as +-truncation): the two differ at the rim of the input's band."""
         locs, vals, cols = sparsify.sparsify_predictions(inputs[:, :1].contiguous(), self.truncation, None,
@@ -82,6 +91,14 @@ class ViewGuidedTrainStep:
         input_normals = normals.compute_normals_sparse(locs, vals, self.dims3d, transform=transform)
         raycast_color, _, raycast_normal, _ = self.raycaster(locs, vals, cols, input_normals, None, view_matrix, intrinsics)
         return raycast_color, raycast_normal
+
+    @staticmethod
+    def _conditioning(raycast_color, raycast_normal):
+        """train.py:556-578 (baseline/ref_train_step.py:85-91): (I,6,H,W) = cat(colour * 2 - 1, normal), misses -> 0."""
+        miss = -float("inf")
+        color = torch.where(raycast_color == miss, torch.zeros_like(raycast_color), raycast_color * 2 - 1)
+        normal = torch.where(raycast_normal == miss, torch.zeros_like(raycast_normal), raycast_normal)
+        return torch.cat([color, normal], 3).permute(0, 3, 1, 2).contiguous()
 
     def __call__(self, sample, optimizer=None):
         """sample: dict with the reference dataloader's keys (scene_dataloader.py / data_util.py:862-902), all on the
@@ -114,8 +131,11 @@ class ViewGuidedTrainStep:
         if 0 < n <= self.raycaster.get_max_num_locs_per_sample() * self.batch_size:          # train.py:524-529
             view_matrix, intrinsics = sample["view_matrix"], sample["images_intrinsic"]
             transform = torch.inverse(view_matrix)                                             # train.py:544
+            input2d = None
             if self.render_input:
-                self._render_input(inputs, view_matrix, intrinsics, transform)
+                input_color, input_normal = self._render_input(inputs, view_matrix, intrinsics, transform)
+                if self.image_loss is not None:  # now: the two renders below overwrite these buffers
+                    input2d = self._conditioning(input_color, input_normal)
             with torch.no_grad():
                 target2d_label = self._target_labels(target_for_sdf, target_for_colors, target_for_semantics,
                                                      view_matrix, intrinsics, transform)
@@ -124,14 +144,18 @@ class ViewGuidedTrainStep:
             output_normals = normals.compute_normals_sparse(locs, sdf_vals, self.dims3d, transform=transform)
             color = (color_vals + 1) * 0.5                                                     # train.py:623
             # prediction raycast + depth L1 + colour L1 + 2D semantic CE (train.py:626-643, 744-746), one kernel pair
-            total2d, terms, _ = losses.render_with_2d_losses(
+            total2d, terms, pred = losses.render_with_2d_losses(
                 self.raycaster, locs, sdf_vals, color, output_normals, sem_vals, view_matrix, intrinsics,
                 images_depth=sample["images_depth"], images_color=sample["images_color"].permute(0, 2, 3, 1),
                 target2d_label=target2d_label, weight_semantic_class=self.class_weight, voxelsize=self.voxelsize,
                 weight_depth_loss=self.w["depth"], weight_color_loss=self.w["color"],
-                weight_semantic_loss=self.w["semantic"])
+                weight_semantic_loss=self.w["semantic"], differentiable_images=self.image_loss is not None)
             loss = loss + total2d
             self.last.update(terms2d=terms.detach())
+            if self.image_loss is not None:
+                loss_image = self.image_loss(pred, input2d)
+                loss = loss + loss_image
+                self.last.update(image_loss=loss_image.detach())
         if optimizer is not None:
             loss.backward()                                                                    # train.py:756
             optimizer.step()                                                                   # train.py:757
