@@ -336,6 +336,49 @@ SPSG_API int spsg_dense_gather(const spsg_dense_payload *payloads, int32_t count
 SPSG_API int spsg_dense_scatter(const spsg_dense_payload *payloads, int32_t count, const int64_t *locs, int64_t num_locs,
                                 int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx, void *stream);
 
+/* == The same glue on heads as a generator in channels_last_3d and/or under bfloat16 autocast produces them.
+ *
+ *    Compaction of a bfloat16 SDF head: spsg_sparsify_count_bf16 / spsg_sparsify_locs_bf16 /
+ *    spsg_sparsify_locs_indexed_bf16 take `sdf` as B*Dz*Dy*Dx bfloat16 values (raw bits; a (B,1,Dz,Dy,Dx) head is
+ *    contiguous in NCDHW and NDHWC alike), 16-byte aligned, and are otherwise exactly their float32 counterparts.  The
+ *    comparison is torch's for a bfloat16 tensor and a Python scalar: `truncation` is first rounded to bfloat16 (nearest
+ *    even), then |sdf| < rounded truncation is evaluated (NaN fails).  The indexed variant writes the widened value into
+ *    the float32 SDF brick, which equals the gathered vals_sdf below, so SPSG_FLAG_INDEX_PREBUILT holds as before.
+ *
+ *    Gather / scatter of strided heads: spsg_dense_gather_strided / spsg_dense_scatter_strided, up to 4 heads per call.
+ *    Element (b, c, z, y, x) of a head is at dense + b*strides[0] + c*strides[1] + z*strides[2] + y*strides[3] +
+ *    x*strides[4] (in elements of its dtype); NCDHW- and NDHWC-contiguous heads and channel slices of either are all
+ *    expressible.  gather: sparse[i, c] = (float) dense[b_i, c, z_i, y_i, x_i], exact (bfloat16 widens exactly).
+ *    scatter: the head's B*C*Dz*Dy*Dx elements are zeroed, then dense[b_i, c, z_i, y_i, x_i] = 0 + round(sparse[i, c]),
+ *    rounded to the head's dtype to nearest even; each cell takes at most one row, so this is autograd of
+ *    head[idx].float() bit for bit (including -0 -> +0).  The scatter's head must be packed: its strides a permutation of a
+ *    contiguous layout (dimensions of size 1 excepted).
+ *    SPSG_ERR_INVALID_ARGUMENT: NULL heads / dense / sparse (sparse may be NULL when num_locs == 0) / locs, an unknown
+ *    dtype, channels or grid sizes <= 0, a negative stride, a head whose last element lies at or beyond `extent`, a dense
+ *    pointer not aligned to its element size, a scatter head that is not packed, more than 4 heads. */
+enum { SPSG_DTYPE_F32 = 0, SPSG_DTYPE_BF16 = 1 };
+typedef struct spsg_dense_head {
+    void *dense;         /* the head, SPSG_DTYPE_* elements; read by gather, written by scatter */
+    float *sparse;       /* (N, channels) float32 contiguous; written by gather, read by scatter */
+    int64_t strides[5];  /* (b, c, z, y, x), in elements, >= 0 */
+    int64_t extent;      /* elements addressable from `dense` (the head's storage from `dense` on) */
+    int32_t channels;
+    int32_t dtype;       /* SPSG_DTYPE_F32 or SPSG_DTYPE_BF16 */
+} spsg_dense_head;
+SPSG_API int spsg_sparsify_count_bf16(const uint16_t *sdf, const uint8_t *empty, int64_t cells, float truncation,
+                                      void *scratch, size_t scratch_bytes, int64_t *total_out, void *stream);
+SPSG_API int spsg_sparsify_locs_bf16(const uint16_t *sdf, const uint8_t *empty, int32_t num_chunks, int32_t dimz,
+                                     int32_t dimy, int32_t dimx, float truncation, const void *scratch, int64_t *locs,
+                                     int64_t num_locs, void *stream);
+SPSG_API int spsg_sparsify_locs_indexed_bf16(const uint16_t *sdf, const uint8_t *empty, int32_t num_chunks, int32_t dimz,
+                                             int32_t dimy, int32_t dimx, float truncation, const void *scratch,
+                                             int64_t *locs, int64_t num_locs, int32_t *sparse_mapping,
+                                             void *raycast_workspace, void *stream);
+SPSG_API int spsg_dense_gather_strided(const spsg_dense_head *heads, int32_t count, const int64_t *locs, int64_t num_locs,
+                                       int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx, void *stream);
+SPSG_API int spsg_dense_scatter_strided(const spsg_dense_head *heads, int32_t count, const int64_t *locs, int64_t num_locs,
+                                        int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx, void *stream);
+
 /* == 2D label maps (reference torch/train.py:614-616 target2d_label, :749-752 pred2d_label):
  *        label = argmax(cat(raycast_semantic, ones), -1).to(uint8)
  *    = first index of the pixel's maximum among its 14 rendered values if that maximum is >= 1, else 14 (miss or

@@ -20,6 +20,8 @@ SPSG_FLAG_GLOBAL_MAPS = 1 << 6
 SPSG_FLAG_INDEX_PREBUILT = 1 << 7
 SPSG_FLAG_PACKED_LOCS = 1 << 8
 SPSG_LOSS_OUT_FLOATS = 8
+SPSG_DTYPE_F32 = 0
+SPSG_DTYPE_BF16 = 1
 SPSG_DEPTH_MAX_FILL_ROUNDS = 64
 
 # every symbol include/spsg_raycast.h declares (tests check the library exports them all)
@@ -32,6 +34,8 @@ EXPORTS = (
     "spsg_depth_compute_normals",
     "spsg_sparsify_scratch_bytes", "spsg_sparsify_count", "spsg_sparsify_locs", "spsg_sparsify_locs_indexed",
     "spsg_dense_gather", "spsg_dense_scatter",
+    "spsg_sparsify_count_bf16", "spsg_sparsify_locs_bf16", "spsg_sparsify_locs_indexed_bf16",
+    "spsg_dense_gather_strided", "spsg_dense_scatter_strided",
     "spsg_labels_from_render", "spsg_pack_locs_host",
 )
 
@@ -64,6 +68,12 @@ class DensePayload(ctypes.Structure):
     """``spsg_dense_payload``"""
     _fields_ = [("dense", ctypes.c_void_p), ("sparse", ctypes.c_void_p), ("channels", ctypes.c_int32),
                 ("reserved", ctypes.c_int32)]
+
+
+class DenseHead(ctypes.Structure):
+    """``spsg_dense_head``"""
+    _fields_ = [("dense", ctypes.c_void_p), ("sparse", ctypes.c_void_p), ("strides", ctypes.c_int64 * 5),
+                ("extent", ctypes.c_int64), ("channels", ctypes.c_int32), ("dtype", ctypes.c_int32)]
 
 
 class GradBuffers(ctypes.Structure):
@@ -145,6 +155,17 @@ def _load():
     lib.spsg_dense_gather.argtypes = [dp, i32, vp, i64, i32, i32, i32, i32, vp]
     lib.spsg_dense_scatter.restype = ctypes.c_int
     lib.spsg_dense_scatter.argtypes = [dp, i32, vp, i64, i32, i32, i32, i32, vp]
+    lib.spsg_sparsify_count_bf16.restype = ctypes.c_int
+    lib.spsg_sparsify_count_bf16.argtypes = [vp, vp, i64, f32, vp, sz, vp, vp]
+    lib.spsg_sparsify_locs_bf16.restype = ctypes.c_int
+    lib.spsg_sparsify_locs_bf16.argtypes = [vp, vp, i32, i32, i32, i32, f32, vp, vp, i64, vp]
+    lib.spsg_sparsify_locs_indexed_bf16.restype = ctypes.c_int
+    lib.spsg_sparsify_locs_indexed_bf16.argtypes = [vp, vp, i32, i32, i32, i32, f32, vp, vp, i64, vp, vp, vp]
+    dh = ctypes.POINTER(DenseHead)
+    lib.spsg_dense_gather_strided.restype = ctypes.c_int
+    lib.spsg_dense_gather_strided.argtypes = [dh, i32, vp, i64, i32, i32, i32, i32, vp]
+    lib.spsg_dense_scatter_strided.restype = ctypes.c_int
+    lib.spsg_dense_scatter_strided.argtypes = [dh, i32, vp, i64, i32, i32, i32, i32, vp]
     lib.spsg_labels_from_render.restype = ctypes.c_int
     lib.spsg_labels_from_render.argtypes = [vp, i64, vp, vp, vp]
     lib.spsg_timing_enable.restype = None

@@ -10,6 +10,11 @@
 // torch.nonzero's lexicographic (b,z,y,x) order, already in the raycaster's (z,y,x,b) column order) and one fused gather
 // over all heads; the backward is one scatter into zero-filled dense gradients.  Results are identical (integer rows;
 // values are copies).
+//
+// The heads may also be bfloat16 (a generator run under autocast) and NDHWC or channel slices (a generator in
+// channels_last_3d): the compaction has bfloat16 twins of its count and write passes, and the *_strided gather /
+// scatter pair reads and writes each head in its own dtype and strides, with float payloads on the sparse side.
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -39,16 +44,33 @@ Scratch carve(void *scratch, long long tiles) {
     return s;
 }
 
+// The SDF head's element types: float, or bfloat16 (raw bits; widening is exact, a shift by 16).
+__device__ __forceinline__ void load_cells8(const float *p, float (&v)[kCellsPerThread]) {
+    const float4 a = __ldg(reinterpret_cast<const float4 *>(p));
+    const float4 b = __ldg(reinterpret_cast<const float4 *>(p) + 1);
+    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+__device__ __forceinline__ void load_cells8(const uint16_t *p, float (&v)[kCellsPerThread]) {
+    const uint4 a = __ldg(reinterpret_cast<const uint4 *>(p));  // one 16-byte load: 8 cells
+    const unsigned w[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        v[2 * k] = __uint_as_float(w[k] << 16);
+        v[2 * k + 1] = __uint_as_float(w[k] & 0xffff0000u);
+    }
+}
+__device__ __forceinline__ float load_cell(const float *p) { return __ldg(p); }
+__device__ __forceinline__ float load_cell(const uint16_t *p) { return __uint_as_float((unsigned)__ldg(p) << 16); }
+
 // bit k of the result: cell (first + k) passes |sdf| < truncation (NaN fails, like torch) and is not marked empty;
-// v[k] = the cell's SDF value (NaN beyond the end of the grid)
-__device__ __forceinline__ unsigned thread_cells(const float *__restrict__ sdf, const uint8_t *__restrict__ empty,
+// v[k] = the cell's SDF value widened to float (NaN beyond the end of the grid)
+template <typename T>
+__device__ __forceinline__ unsigned thread_cells(const T *__restrict__ sdf, const uint8_t *__restrict__ empty,
                                                  long long first, long long cells, float truncation,
                                                  float (&v)[kCellsPerThread]) {
     unsigned m = 0u;
     if (first + kCellsPerThread <= cells) {  // (sdf is 16-byte aligned and first is a multiple of 8)
-        const float4 a = __ldg(reinterpret_cast<const float4 *>(sdf + first));
-        const float4 b = __ldg(reinterpret_cast<const float4 *>(sdf + first) + 1);
-        v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+        load_cells8(sdf + first, v);
 #pragma unroll
         for (int k = 0; k < 8; k++) m |= (fabsf(v[k]) < truncation ? 1u : 0u) << k;
         if (empty && m) {
@@ -64,7 +86,7 @@ __device__ __forceinline__ unsigned thread_cells(const float *__restrict__ sdf, 
         for (int k = 0; k < kCellsPerThread; k++) {
             v[k] = __int_as_float(0x7fffffff);
             if (first + k < cells) {
-                v[k] = __ldg(sdf + first + k);
+                v[k] = load_cell(sdf + first + k);
                 if (fabsf(v[k]) < truncation && !(empty && empty[first + k])) m |= 1u << k;
             }
         }
@@ -72,13 +94,15 @@ __device__ __forceinline__ unsigned thread_cells(const float *__restrict__ sdf, 
     return m;
 }
 
-__device__ __forceinline__ unsigned thread_mask(const float *__restrict__ sdf, const uint8_t *__restrict__ empty,
+template <typename T>
+__device__ __forceinline__ unsigned thread_mask(const T *__restrict__ sdf, const uint8_t *__restrict__ empty,
                                                 long long first, long long cells, float truncation) {
     float v[kCellsPerThread];
     return thread_cells(sdf, empty, first, cells, truncation, v);
 }
 
-__global__ void __launch_bounds__(kTileThreads) sparsify_count_kernel(const float *__restrict__ sdf,
+template <typename T>
+__global__ void __launch_bounds__(kTileThreads) sparsify_count_kernel(const T *__restrict__ sdf,
                                                                       const uint8_t *__restrict__ empty, long long cells,
                                                                       float truncation, int32_t *__restrict__ counts) {
     __shared__ int s_warp[kTileThreads / 32];
@@ -140,9 +164,10 @@ __global__ void __launch_bounds__(1024) sparsify_scan_kernel(const int32_t *__re
 // kIndexed: the same pass also writes, for EVERY cell, what the raycaster's fill + index passes derive from `locs`
 // (kernel.cu:346-362, 515 and the dense SDF brick of this implementation): index[cell] = row of the cell or -1,
 // brick[cell] = its SDF or NaN (absent) -- two coalesced 32-byte stores per thread instead of a 32-byte read and two
-// scattered 4-byte writes per row in a later launch.
-template <bool kIndexed>
-__global__ void __launch_bounds__(kTileThreads) sparsify_write_kernel(const float *__restrict__ sdf,
+// scattered 4-byte writes per row in a later launch.  (T = uint16_t: a bfloat16 head; the brick gets the widened value,
+// which is what the gather hands the raycaster as vals_sdf.)
+template <typename T, bool kIndexed>
+__global__ void __launch_bounds__(kTileThreads) sparsify_write_kernel(const T *__restrict__ sdf,
                                                                       const uint8_t *__restrict__ empty, long long cells,
                                                                       int dimz, int dimy, int dimx, float truncation,
                                                                       const long long *__restrict__ offsets,
@@ -271,6 +296,96 @@ __global__ void __launch_bounds__(256) dense_payload_kernel(const PayloadArgs a,
     }
 }
 
+struct HeadArgs {
+    void *dense[kMaxPayloads];
+    float *sparse[kMaxPayloads];
+    long long stride[kMaxPayloads][5];  // elements, (b, c, z, y, x)
+    int channels[kMaxPayloads];
+    int bf16[kMaxPayloads];
+    int count;
+};
+
+__device__ __forceinline__ float load_elem(const void *p, long long o, bool bf16) {
+    return bf16 ? __uint_as_float((unsigned)__ldg(static_cast<const uint16_t *>(p) + o) << 16)
+                : __ldg(static_cast<const float *>(p) + o);
+}
+
+// The gradient of head[idx].float() with respect to a head of either dtype: the row's gradient rounded to the head's
+// dtype (round-to-nearest-even, what the backward of .float() does) and added to the zero-filled dense gradient
+// (index_put with accumulate): 0 + g, so -0 becomes +0, exactly as autograd of the literal expression gives it.  (A
+// float32 NaN is stored as it comes, as the accumulation leaves it; a bfloat16 NaN is the conversion's.)
+__device__ __forceinline__ void store_elem(void *p, long long o, float g, bool bf16) {
+    if (bf16) {
+        const float r = __bfloat162float(__float2bfloat16_rn(g));
+        static_cast<__nv_bfloat16 *>(p)[o] = __float2bfloat16_rn(0.0f + r);
+    } else {
+        static_cast<float *>(p)[o] = g == 0.0f ? 0.0f : g;
+    }
+}
+
+// As dense_payload_kernel, for heads of any element strides and of dtype float or bfloat16; the sparse side is float.
+// A warp takes 32 consecutive voxels.  Heads whose channels are adjacent (stride 1: NDHWC, or a channel slice of it)
+// are moved voxel by voxel: lane e of a pass handles channel e % C of voxel e / C, so both sides are contiguous runs of
+// the warp's (mostly adjacent) voxels -- C * 2 or C * 4 bytes each on the dense side, one run of 32 * C floats on the
+// sparse side.  Other heads (channels a volume apart) go channel by channel through shared memory, as in
+// dense_payload_kernel.
+template <bool kScatter>
+__global__ void __launch_bounds__(256) strided_payload_kernel(const HeadArgs a, const longlong4 *__restrict__ locs,
+                                                              long long num_locs) {
+    __shared__ float s_vals[8][32 * 16 + 16];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    float *s = s_vals[warp];
+    const long long warps = (long long)gridDim.x * 8;
+    for (long long base = ((long long)blockIdx.x * 8 + warp) * 32; base < num_locs; base += warps * 32) {
+        const int n = (int)min((long long)32, num_locs - base);
+        longlong4 l = make_longlong4(0, 0, 0, 0);  // (z, y, x, b)
+        if (lane < n) l = locs[base + lane];
+        for (int p = 0; p < a.count; p++) {
+            const long long *st = a.stride[p];
+            const long long off = l.w * st[0] + l.x * st[2] + l.y * st[3] + l.z * st[4];
+            const int C = a.channels[p];
+            const bool bf = a.bf16[p] != 0;
+            void *dense = a.dense[p];
+            float *sparse = a.sparse[p] + base * C;
+            if (st[1] == 1 || C == 1) {
+                const int total = n * C;
+                for (int e0 = 0; e0 < total; e0 += 32) {
+                    const int e = e0 + lane;
+                    const int v = min(e / C, 31), c = e - v * C;
+                    const long long o = __shfl_sync(0xffffffffu, off, v) + c;
+                    if (e < total) {
+                        if (!kScatter) sparse[e] = load_elem(dense, o, bf);
+                        else store_elem(dense, o, __ldg(sparse + e), bf);
+                    }
+                }
+            } else {
+                const long long sc = st[1];
+                for (int c0 = 0; c0 < C; c0 += 16) {
+                    const int cc = min(16, C - c0);
+                    __syncwarp();
+                    if (!kScatter) {
+                        if (lane < n)
+                            for (int c = 0; c < cc; c++) s[lane * cc + c] = load_elem(dense, off + (c0 + c) * sc, bf);
+                        __syncwarp();
+                        for (int e = lane; e < n * cc; e += 32) {
+                            const int v = e / cc, c = e - v * cc;
+                            sparse[(long long)v * C + c0 + c] = s[e];
+                        }
+                    } else {
+                        for (int e = lane; e < n * cc; e += 32) {
+                            const int v = e / cc, c = e - v * cc;
+                            s[e] = __ldg(sparse + (long long)v * C + c0 + c);
+                        }
+                        __syncwarp();
+                        if (lane < n)
+                            for (int c = 0; c < cc; c++) store_elem(dense, off + (c0 + c) * sc, s[lane * cc + c], bf);
+                    }
+                }
+            }
+        }
+    }
+}
+
 int check_grid(int num_chunks, int dimz, int dimy, int dimx) {
     if (num_chunks <= 0 || dimz <= 0 || dimy <= 0 || dimx <= 0)
         return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "bad grid sizes");
@@ -303,18 +418,78 @@ int launch_payload(bool scatter, const spsg_dense_payload *payloads, int count, 
     return SPSG_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-SPSG_API size_t spsg_sparsify_scratch_bytes(int64_t cells) {
-    if (cells <= 0) return 0;
-    const long long tiles = num_tiles(cells);
-    return align_up((size_t)(tiles + 1) * 8, 256) + align_up((size_t)tiles * 4, 256);
+// the head's strides are a permutation of a packed layout of its B * C * Dz * Dy * Dx elements (dimensions of size 1
+// may carry any stride)
+bool packed(const int64_t *stride, const long long *size) {
+    int order[5] = {0, 1, 2, 3, 4};
+    std::sort(order, order + 5, [&](int i, int j) {
+        return size[i] == 1 ? false : size[j] == 1 ? true : stride[i] < stride[j];
+    });
+    long long expect = 1;
+    for (int k = 0; k < 5 && size[order[k]] != 1; k++) {
+        if (stride[order[k]] != expect) return false;
+        expect *= size[order[k]];
+    }
+    return true;
 }
 
-SPSG_API int spsg_sparsify_count(const float *sdf, const uint8_t *empty, int64_t cells, float truncation, void *scratch,
-                                 size_t scratch_bytes, int64_t *total_out, void *stream) {
+int launch_strided(bool scatter, const spsg_dense_head *heads, int count, const int64_t *locs, int64_t num_locs,
+                   int num_chunks, int dimz, int dimy, int dimx, cudaStream_t st) {
+    if (int rc = check_grid(num_chunks, dimz, dimy, dimx)) return rc;
+    if (count < 0 || count > kMaxPayloads) return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "at most 4 heads per call");
+    if (count > 0 && !heads) return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "NULL heads");
+    if (num_locs < 0 || (num_locs > 0 && !locs)) return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "bad locs");
+    if (reinterpret_cast<uintptr_t>(locs) & 15u) return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "locs must be 16-byte aligned");
+    HeadArgs a = {};
+    a.count = count;
+    for (int p = 0; p < count; p++) {
+        const spsg_dense_head &h = heads[p];
+        if (!h.dense || (num_locs > 0 && !h.sparse))
+            return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "NULL dense / sparse pointer of a head");
+        if (h.channels <= 0) return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "non-positive channels");
+        if (h.dtype != SPSG_DTYPE_F32 && h.dtype != SPSG_DTYPE_BF16)
+            return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "unknown head dtype");
+        const size_t esize = h.dtype == SPSG_DTYPE_BF16 ? 2 : 4;
+        if (reinterpret_cast<uintptr_t>(h.dense) & (esize - 1))
+            return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "dense head not aligned to its element size");
+        const long long size[5] = {num_chunks, h.channels, dimz, dimy, dimx};
+        long long last = 0;  // offset of the head's last element
+        for (int d = 0; d < 5; d++) {
+            if (h.strides[d] < 0) return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "negative head stride");
+            if (h.strides[d] > 0 && (size[d] - 1) > (INT64_MAX - last) / h.strides[d])
+                return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "head strides overflow");
+            last += (size[d] - 1) * h.strides[d];
+        }
+        if (last >= h.extent) return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "head strides leave the head's extent");
+        if (scatter && !packed(h.strides, size))
+            return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "the scatter's dense gradient must be packed");
+        a.dense[p] = h.dense;
+        a.sparse[p] = h.sparse;
+        for (int d = 0; d < 5; d++) a.stride[p][d] = h.strides[d];
+        a.channels[p] = h.channels;
+        a.bf16[p] = h.dtype == SPSG_DTYPE_BF16;
+    }
+    if (scatter)
+        for (int p = 0; p < count; p++) {
+            const size_t elems = (size_t)num_chunks * heads[p].channels * dimz * dimy * dimx;
+            SPSG_CUDA_TRY(cudaMemsetAsync(heads[p].dense, 0, elems * (heads[p].dtype == SPSG_DTYPE_BF16 ? 2 : 4), st));
+        }
+    if (num_locs == 0 || count == 0) return SPSG_OK;
+    const unsigned grid = (unsigned)std::min<long long>((num_locs + 255) / 256, (long long)spsg_internal_sm_count() * 16);
+    if (scatter) strided_payload_kernel<true><<<grid, 256, 0, st>>>(a, reinterpret_cast<const longlong4 *>(locs), num_locs);
+    else strided_payload_kernel<false><<<grid, 256, 0, st>>>(a, reinterpret_cast<const longlong4 *>(locs), num_locs);
+    SPSG_CUDA_TRY(cudaGetLastError());
+    return SPSG_OK;
+}
+
+// torch compares a bfloat16 tensor with a Python scalar in bfloat16: the scalar is rounded (double -> float -> bfloat16,
+// nearest-even) before |sdf| < truncation is evaluated.  A truncation bfloat16 cannot represent that rounds down
+// excludes the cells equal to the rounded value.
+float bf16_truncation(float t) { return __bfloat162float(__float2bfloat16_rn(t)); }
+
+template <typename T>
+int sparsify_count_impl(const T *sdf, const uint8_t *empty, int64_t cells, float truncation, void *scratch,
+                               size_t scratch_bytes, int64_t *total_out, void *stream) {
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (!sdf || cells <= 0) return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "bad sdf / cells");
     if ((reinterpret_cast<uintptr_t>(sdf) & 15u) || (empty && (reinterpret_cast<uintptr_t>(empty) & 7u)))
@@ -323,14 +498,15 @@ SPSG_API int spsg_sparsify_count(const float *sdf, const uint8_t *empty, int64_t
         return spsg_internal_fail(SPSG_ERR_WORKSPACE_TOO_SMALL, "sparsify scratch too small or not 256-byte aligned");
     const long long tiles = num_tiles(cells);
     const Scratch s = carve(scratch, tiles);
-    sparsify_count_kernel<<<(unsigned)tiles, kTileThreads, 0, st>>>(sdf, empty, cells, truncation, s.counts);
+    sparsify_count_kernel<T><<<(unsigned)tiles, kTileThreads, 0, st>>>(sdf, empty, cells, truncation, s.counts);
     SPSG_CUDA_TRY(cudaGetLastError());
     sparsify_scan_kernel<<<1, 1024, 0, st>>>(s.counts, tiles, s.offsets, reinterpret_cast<long long *>(total_out));
     SPSG_CUDA_TRY(cudaGetLastError());
     return SPSG_OK;
 }
 
-static int sparsify_locs_impl(const float *sdf, const uint8_t *empty, int32_t num_chunks, int32_t dimz, int32_t dimy,
+template <typename T>
+int sparsify_locs_impl(const T *sdf, const uint8_t *empty, int32_t num_chunks, int32_t dimz, int32_t dimy,
                               int32_t dimx, float truncation, const void *scratch, int64_t *locs, int64_t num_locs,
                               int32_t *index, float *brick, bool indexed, void *stream) {
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -350,13 +526,33 @@ static int sparsify_locs_impl(const float *sdf, const uint8_t *empty, int32_t nu
     const long long tiles = num_tiles(cells);
     const Scratch s = carve(const_cast<void *>(scratch), tiles);
     if (indexed)
-        sparsify_write_kernel<true><<<(unsigned)tiles, kTileThreads, 0, st>>>(sdf, empty, cells, dimz, dimy, dimx, truncation, s.offsets,
-                                                                              reinterpret_cast<longlong4 *>(locs), num_locs, index, brick);
+        sparsify_write_kernel<T, true><<<(unsigned)tiles, kTileThreads, 0, st>>>(sdf, empty, cells, dimz, dimy, dimx, truncation, s.offsets,
+                                                                                 reinterpret_cast<longlong4 *>(locs), num_locs, index, brick);
     else
-        sparsify_write_kernel<false><<<(unsigned)tiles, kTileThreads, 0, st>>>(sdf, empty, cells, dimz, dimy, dimx, truncation, s.offsets,
-                                                                               reinterpret_cast<longlong4 *>(locs), num_locs, nullptr, nullptr);
+        sparsify_write_kernel<T, false><<<(unsigned)tiles, kTileThreads, 0, st>>>(sdf, empty, cells, dimz, dimy, dimx, truncation, s.offsets,
+                                                                                  reinterpret_cast<longlong4 *>(locs), num_locs, nullptr, nullptr);
     SPSG_CUDA_TRY(cudaGetLastError());
     return SPSG_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+SPSG_API size_t spsg_sparsify_scratch_bytes(int64_t cells) {
+    if (cells <= 0) return 0;
+    const long long tiles = num_tiles(cells);
+    return align_up((size_t)(tiles + 1) * 8, 256) + align_up((size_t)tiles * 4, 256);
+}
+
+SPSG_API int spsg_sparsify_count(const float *sdf, const uint8_t *empty, int64_t cells, float truncation, void *scratch,
+                                 size_t scratch_bytes, int64_t *total_out, void *stream) {
+    return sparsify_count_impl(sdf, empty, cells, truncation, scratch, scratch_bytes, total_out, stream);
+}
+
+SPSG_API int spsg_sparsify_count_bf16(const uint16_t *sdf, const uint8_t *empty, int64_t cells, float truncation,
+                                      void *scratch, size_t scratch_bytes, int64_t *total_out, void *stream) {
+    return sparsify_count_impl(sdf, empty, cells, bf16_truncation(truncation), scratch, scratch_bytes, total_out, stream);
 }
 
 SPSG_API int spsg_sparsify_locs(const float *sdf, const uint8_t *empty, int32_t num_chunks, int32_t dimz, int32_t dimy,
@@ -374,6 +570,21 @@ SPSG_API int spsg_sparsify_locs_indexed(const float *sdf, const uint8_t *empty, 
                               static_cast<float *>(raycast_workspace), true, stream);
 }
 
+SPSG_API int spsg_sparsify_locs_bf16(const uint16_t *sdf, const uint8_t *empty, int32_t num_chunks, int32_t dimz,
+                                     int32_t dimy, int32_t dimx, float truncation, const void *scratch, int64_t *locs,
+                                     int64_t num_locs, void *stream) {
+    return sparsify_locs_impl(sdf, empty, num_chunks, dimz, dimy, dimx, bf16_truncation(truncation), scratch, locs, num_locs,
+                              nullptr, nullptr, false, stream);
+}
+
+SPSG_API int spsg_sparsify_locs_indexed_bf16(const uint16_t *sdf, const uint8_t *empty, int32_t num_chunks, int32_t dimz,
+                                             int32_t dimy, int32_t dimx, float truncation, const void *scratch,
+                                             int64_t *locs, int64_t num_locs, int32_t *sparse_mapping,
+                                             void *raycast_workspace, void *stream) {
+    return sparsify_locs_impl(sdf, empty, num_chunks, dimz, dimy, dimx, bf16_truncation(truncation), scratch, locs, num_locs,
+                              sparse_mapping, static_cast<float *>(raycast_workspace), true, stream);
+}
+
 SPSG_API int spsg_dense_gather(const spsg_dense_payload *payloads, int32_t count, const int64_t *locs, int64_t num_locs,
                                int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx, void *stream) {
     return launch_payload(false, payloads, count, locs, num_locs, num_chunks, dimz, dimy, dimx, static_cast<cudaStream_t>(stream));
@@ -382,6 +593,16 @@ SPSG_API int spsg_dense_gather(const spsg_dense_payload *payloads, int32_t count
 SPSG_API int spsg_dense_scatter(const spsg_dense_payload *payloads, int32_t count, const int64_t *locs, int64_t num_locs,
                                 int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx, void *stream) {
     return launch_payload(true, payloads, count, locs, num_locs, num_chunks, dimz, dimy, dimx, static_cast<cudaStream_t>(stream));
+}
+
+SPSG_API int spsg_dense_gather_strided(const spsg_dense_head *heads, int32_t count, const int64_t *locs, int64_t num_locs,
+                                       int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx, void *stream) {
+    return launch_strided(false, heads, count, locs, num_locs, num_chunks, dimz, dimy, dimx, static_cast<cudaStream_t>(stream));
+}
+
+SPSG_API int spsg_dense_scatter_strided(const spsg_dense_head *heads, int32_t count, const int64_t *locs, int64_t num_locs,
+                                        int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx, void *stream) {
+    return launch_strided(true, heads, count, locs, num_locs, num_chunks, dimz, dimy, dimx, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

@@ -14,6 +14,8 @@ caller's (the reference's own ``model.Generator`` / ``loss`` module in bench.py 
 outside the hot path (SURVEY.md section 8).  Data parallelism is ``torch.nn.parallel.DistributedDataParallel`` around the
 generator: its gradient all-reduce is the step's only collective (SURVEY.md section 8(e)).  No CPU path.
 """
+import contextlib
+
 import torch
 import torch.nn.functional as F
 
@@ -45,14 +47,20 @@ class ViewGuidedTrainStep:
                 or None with ``render_input=False``.  ``pred`` are the raycaster's buffers, valid until the next step.
                 The discriminator, its own update and the exact form of the GAN / style terms are the caller's: this
                 step only adds what ``image_loss`` returns.  Its value is recorded in ``self.last["image_loss"]``.
+    autocast_bf16  run the generator forward and the dense 3D losses under ``torch.autocast("cuda", dtype=torch.bfloat16)``.
+                The bfloat16 heads (NDHWC with ``prepare_generator``) go to the producer glue as they are; from the voxel
+                payloads on (normals, the three raycasts, the 2D losses, ``image_loss``) everything stays float32.  No
+                gradient scaler: bfloat16 has float32's exponent range.  False: the float32 step.
     """
 
     def __init__(self, model, loss_util, batch_size, dims3d, width, height, class_weight, voxelsize=0.02, truncation=3.0,
                  weight_occ_loss=1.0, weight_sdf_loss=0.1, weight_depth_loss=1.0, weight_color_loss=1.0,
                  weight_semantic_loss=0.1, weight_surf_geo=1.0, weight_missing_geo=5.0, logweight_sdf=True,
-                 max_num_locs_per_sample=640000, views_per_chunk=1, render_input=True, device=None, image_loss=None):
+                 max_num_locs_per_sample=640000, views_per_chunk=1, render_input=True, device=None, image_loss=None,
+                 autocast_bf16=False):
         self.model, self.loss_util = model, loss_util
         self.image_loss = image_loss
+        self.autocast_bf16 = autocast_bf16
         self.batch_size, self.dims3d, self.width, self.height = batch_size, tuple(dims3d), width, height
         self.voxelsize, self.truncation = voxelsize, truncation
         self.w = dict(occ=weight_occ_loss, sdf=weight_sdf_loss, depth=weight_depth_loss, color=weight_color_loss,
@@ -112,16 +120,19 @@ class ViewGuidedTrainStep:
         target_for_semantics = sample["semantics"]
         if optimizer is not None:
             optimizer.zero_grad(set_to_none=True)
-        output_occ, output_sdf, output_color, output_semantic = self.model(
-            inputs, mask, pred_sdf=[True, True], pred_color=True, pred_semantic=True)          # train.py:465
-        # ---- dense 3D losses (train.py:476-493), the caller's functions
-        input_occ = torch.abs(inputs[:, :1]) < (T - 0.01)
-        weight = lu.compute_dense_geo_weights(target_for_sdf, input_occ, T, self.weight_surf_geo, self.weight_missing_geo)
-        empty = torch.sigmoid(output_occ.detach()) < 0.5
-        weight[empty] = 0
-        loss_occ = lu.compute_geo_occ_loss(target_for_sdf, output_occ, known, weight, T)
-        loss_sdf = lu.compute_geo_loss(target_for_sdf, None, output_sdf, known, weight, self.logweight_sdf)
-        loss = self.w["occ"] * loss_occ + self.w["sdf"] * loss_sdf
+        dense_region = (torch.autocast("cuda", dtype=torch.bfloat16) if self.autocast_bf16 else contextlib.nullcontext())
+        with dense_region:
+            output_occ, output_sdf, output_color, output_semantic = self.model(
+                inputs, mask, pred_sdf=[True, True], pred_color=True, pred_semantic=True)      # train.py:465
+            # ---- dense 3D losses (train.py:476-493), the caller's functions
+            input_occ = torch.abs(inputs[:, :1]) < (T - 0.01)
+            weight = lu.compute_dense_geo_weights(target_for_sdf, input_occ, T, self.weight_surf_geo,
+                                                  self.weight_missing_geo)
+            empty = torch.sigmoid(output_occ.detach()) < 0.5
+            weight[empty] = 0
+            loss_occ = lu.compute_geo_occ_loss(target_for_sdf, output_occ, known, weight, T)
+            loss_sdf = lu.compute_geo_loss(target_for_sdf, None, output_sdf, known, weight, self.logweight_sdf)
+            loss = self.w["occ"] * loss_occ + self.w["sdf"] * loss_sdf
         # ---- dense heads -> sparse raycaster inputs (train.py:494-509)
         # (counted first, written after the other two renders of the step: the rows then feed the prediction render
         # directly -- voxel index and SDF brick written with them, see sparsify.sparse_locs)

@@ -1,10 +1,13 @@
 #!/usr/bin/env python
 """Compare the SASS of two builds of spsg_raycast.cu function by function, instruction offsets and encodings stripped
 (no GPU needed).  The backward gather's template gained a parameter (kUpstream); its old instantiations
-<kFused, kViews> are matched with <kFused, false, kViews>.
+<kFused, kViews> are matched with <kFused, false, kViews>.  The compaction kernels of spsg_sparsify.cu gained the SDF
+element type: the plain sparsify_count_kernel and sparsify_write_kernel<kIndexed> are matched with their <float>
+instantiations.
 
     nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -I include -Xptxas -v -cubin \\
          <package>/csrc/spsg_raycast.cu -o after.cubin          # and the same on the older tree -> before.cubin
+                                                                # (likewise spsg_sparsify.cu)
     python tools/sass_compare.py before.cubin after.cubin
 """
 import os
@@ -37,7 +40,15 @@ def functions(cubin):
 def key(name):
     name = re.sub(r"_GLOBAL__N__[0-9a-f]+_\d+_\w+?_cu_[0-9a-f]{8}", "", name)  # the anonymous namespace's per-build tag
     m = re.search(r"backward_gather_kernelI(Lb[01]E)(Lb[01]E)?(Li\dE)E", name)
-    return "backward_gather_kernel" + m.group(1) + (m.group(2) or "Lb0E") + m.group(3) if m else name
+    if m:
+        return "backward_gather_kernel" + m.group(1) + (m.group(2) or "Lb0E") + m.group(3)
+    m = re.search(r"sparsify_count_kernel(?:I([a-z])EEv)?", name)
+    if m:
+        return "sparsify_count_kernel<%s>" % (m.group(1) or "f")
+    m = re.search(r"sparsify_write_kernelI([a-z])?(Lb[01]E)E", name)
+    if m:
+        return "sparsify_write_kernel<%s,%s>" % (m.group(1) or "f", m.group(2))
+    return name
 
 
 def main(before, after):
