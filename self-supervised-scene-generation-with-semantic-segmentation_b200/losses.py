@@ -137,6 +137,7 @@ def fused_backward(m, p, tg, loss_out, grad_scale, grads_cleared, upstream=None)
     None; contiguous float32): ``spsg_raycast_backward_loss_upstream`` then adds them, unscaled, in the same gather.
     ``grad_scale`` None means 1."""
     if grads_cleared:
+        p = type(p).from_buffer_copy(p)  # the caller's params stay as the forward left them
         p.flags |= N.SPSG_FLAG_GRADS_CLEARED
     dev = m.image_depth.device
     if grad_scale is not None:
@@ -183,6 +184,7 @@ class FusedRaycastLossFunction(Function):
                                         intrinsic_params, (target_depth, target_color, weight_color, target_label,
                                                            class_weight, voxelsize, weights), ctx.grads_cleared)
         ctx.raycaster, ctx.params, ctx.targets, ctx.n, ctx.loss_out = m, p, tg, n, loss_out
+        ctx.forward_id = m.workspace.forwards
         # keep the target tensors alive until backward (the struct only holds raw pointers)
         ctx.keep = (target_depth, target_color, weight_color, target_label, class_weight)
         ctx.differentiable_images = differentiable_images
@@ -213,6 +215,7 @@ class FusedRaycastLossFunction(Function):
                 upstream = tuple(None if g is None else g.to(torch.float32).contiguous() for g in grad_images)
         if grad_total is None and upstream is None:
             return (None,) * 16
+        m.workspace.check_latest(ctx.forward_id)
         if grad_total is None:
             # only the images feed the objective: no scale derived from the loss normalisers (an empty valid set would
             # turn 0 * (w / 0) into NaN); the targets switched off leave the plain gather of the upstream images
@@ -220,7 +223,10 @@ class FusedRaycastLossFunction(Function):
         else:
             fused_backward(m, ctx.params, ctx.targets, ctx.loss_out, grad_total.to(torch.float32).contiguous(),
                            ctx.grads_cleared, upstream)
-        return (None, None, m.d_depth[:n], m.d_color[:n], m.d_normal[:n], m.d_semantic[:n]) + (None,) * 10
+        ctx.grads_cleared = False  # the forward cleared the rows once: a second backward (retain_graph) clears its own
+        grads = (m.d_depth[:n], m.d_color[:n], m.d_normal[:n], m.d_semantic[:n])
+        m.workspace.grad_views = grads  # leaves get copies, not the buffers (raycast_rgbd_cuda.ModuleWorkspace)
+        return (None, None) + grads + (None,) * 10
 
 
 def render_loss_and_voxel_grads(raycaster, locs, vals_sdf, vals_colors, vals_normals, vals_semantics, view_matrix,

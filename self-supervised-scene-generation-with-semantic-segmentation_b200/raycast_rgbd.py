@@ -46,6 +46,7 @@ class RayCastRGBDFunction(Function):
                                   clear_grads=(d_color, d_depth, d_normal, d_semantic) if ctx.grads_cleared else None,
                                   workspace_owner=workspace_owner)
         ctx.workspace_owner = workspace_owner
+        ctx.forward_id = None if workspace_owner is None else workspace_owner.forwards
         ctx.flags = flags
         ctx.dims = [sparse_mapping.shape[0], dims3d[2], dims3d[1], dims3d[0], num_locs]  # raycast_rgbd.py:30-31
         ctx.views_per_chunk = views_per_chunk
@@ -60,14 +61,20 @@ class RayCastRGBDFunction(Function):
     def backward(ctx, grad_color, grad_depth, grad_normal, grad_semantic):
         sparse_mapping, mapping3dto2d, mapping3dto2d_num, d_color, d_depth, d_normal, d_semantic = ctx.saved_tensors
         n = ctx.dims[4]
+        owner = ctx.workspace_owner
+        if owner is not None:
+            owner.check_latest(ctx.forward_id)
         raycast_rgbd_cuda.backward(
             grad_color.contiguous(), grad_depth.contiguous(), grad_normal.contiguous(), grad_semantic.contiguous(),
             sparse_mapping, mapping3dto2d, mapping3dto2d_num, ctx.dims, d_color, d_depth, d_normal, d_semantic,
-            views_per_chunk=ctx.views_per_chunk, grads_cleared=ctx.grads_cleared, workspace_owner=ctx.workspace_owner,
+            views_per_chunk=ctx.views_per_chunk, grads_cleared=ctx.grads_cleared, workspace_owner=owner,
             flags=ctx.flags)
+        ctx.grads_cleared = False  # the forward cleared the rows once: a second backward (retain_graph) clears its own
+        grads = (d_depth[:n], d_color[:n], d_normal[:n], d_semantic[:n])
+        if owner is not None:
+            owner.grad_views = grads  # leaves get copies, not the buffers (ModuleWorkspace)
         # raycast_rgbd.py:42-43: (locs, vals_sdf, vals_colors, vals_normals, vals_semantic, None...)
-        return (None, d_depth[:n], d_color[:n], d_normal[:n], d_semantic[:n]) + \
-               (None,) * (len(ctx.needs_input_grad) - 5)
+        return (None,) + grads + (None,) * (len(ctx.needs_input_grad) - 5)
 
 
 class RaycastRGBD(nn.Module):

@@ -125,10 +125,17 @@ def workspace(device, nbytes, owner=None, stamp=None, expect=None):
 
 
 class ModuleWorkspace:
-    """The workspace of one raycaster module: an explicit buffer it owns, stamped by every forward."""
+    """The workspace of one raycaster module: an explicit buffer it owns, stamped by every forward.
+
+    ``forwards`` counts the forwards that filled it: an autograd backward records the count its forward left and refuses
+    to gather once a later forward has overwritten the module's tables and images (``check_latest``).  ``grad_views``
+    holds the ``d_*`` row views the last autograd backward returned: with that extra reference, autograd copies them into
+    the ``.grad`` of leaf tensors instead of storing the module's buffers there (which the next forward clears)."""
 
     def __init__(self):
         self.ws, self.stamp, self._prebuilt = None, None, None
+        self.forwards = 0
+        self.grad_views = None
 
     def get(self, device, nbytes):
         if self.ws is None or self.ws.numel() < nbytes or self.ws.device != device:
@@ -153,6 +160,14 @@ class ModuleWorkspace:
 
     def filled(self, p):
         self.stamp = _stamp(p)
+        self.forwards += 1
+
+    def check_latest(self, forward):
+        """``forward`` = ``self.forwards`` right after the forward whose backward is about to run."""
+        if forward != self.forwards:
+            raise RuntimeError("raycast backward after a later forward on the same module: that forward overwrote the "
+                               "registration tables and renderings this backward gathers from (%d forwards since)"
+                               % (self.forwards - forward))
 
     def check(self, p, nbytes):
         if self.ws is None or self.stamp != _stamp(p) or self.ws.numel() < nbytes:
