@@ -61,8 +61,16 @@ enum {
     SPSG_FLAG_INDEX_PREBUILT = 1u << 7, /* forward: sparse_mapping and the workspace's dense SDF brick already hold exactly
                                           these locs / vals_sdf (written by spsg_sparsify_locs_indexed): skip the -1 / NaN
                                           fill and the index pass (only mapping3dto2d_num is reset)                          */
-    SPSG_FLAG_DETERMINISTIC_GRADS = 1u << 4 /* backward, several views per chunk: add a voxel's per-view means in view order
+    SPSG_FLAG_DETERMINISTIC_GRADS = 1u << 4, /* backward, several views per chunk: add a voxel's per-view means in view order
                                                without float atomics (bit-reproducible; the gather takes ~30 % longer) */
+    SPSG_FLAG_VIEW_NORMALS = 1u << 9    /* forward and backward, several views per chunk: one normal per (voxel, view).
+                                           vals_normal is (N,F,3) voxel-major: row (v, f) is voxel v's normal as image
+                                           chunk(v)*F + f sees it, and that image's normal rendering reads it (a row of
+                                           zeros renders -inf, per row).  d_normal is (N,F,3): row (v, f) is the mean of
+                                           grad_normal over view f's pixels registered to v -- not summed over views.  The
+                                           forward's clear_grads->d_normal must hold N*F rows.  Colour, depth and semantic
+                                           are unchanged.  With views_per_chunk == 1 the flag changes nothing.  Pass it
+                                           to the forward and to its backward alike. */
 };
 
 /* Replaces the reference's `opts` CPU tensor [W,H,depth_min,depth_max,thresh,ray_inc,Dx,Dy,Dz]
@@ -235,6 +243,24 @@ SPSG_API int spsg_normals_forward(const int64_t *locs, int64_t num_locs, const f
 SPSG_API int spsg_normals_backward(const int64_t *locs, int64_t num_locs, const float *vals_sdf, const float *transform,
                                    const int32_t *index, int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx,
                                    const float *grad_normals, float *scratch_u, float *d_sdf, void *stream);
+
+/* Per-view normals for renders with several views per chunk (SPSG_FLAG_VIEW_NORMALS): the central difference g is
+ *    computed once per voxel, then normals[(i*F + f)*3 ..] = -normalize(R_{b*F+f} * g), b = chunk of voxel i, with the
+ *    arithmetic of spsg_normals_forward.  normals: (N,F,3); transform: (B*F,4,4), the inverse view matrices of the
+ *    render's images in image order, required when F > 1.  views_per_chunk == 1 is exactly spsg_normals_forward.
+ *    views_per_chunk <= 0, or a NULL transform with F > 1, is SPSG_ERR_INVALID_ARGUMENT. */
+SPSG_API int spsg_normals_forward_views(const int64_t *locs, int64_t num_locs, const float *vals_sdf,
+                                        const float *transform, int32_t views_per_chunk, int32_t *index,
+                                        int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx, float *normals,
+                                        void *stream);
+
+/* Gradient of spsg_normals_forward_views w.r.t. vals_sdf.  grad_normals: (N,F,3).  Pass 1 writes u = dL/dg (N,3) into
+ *    scratch_u, the per-view terms of spsg_normals_backward summed in view order; pass 2 is spsg_normals_backward's
+ *    neighbour gather.  views_per_chunk == 1 is exactly spsg_normals_backward; same argument checks as the forward. */
+SPSG_API int spsg_normals_backward_views(const int64_t *locs, int64_t num_locs, const float *vals_sdf,
+                                         const float *transform, int32_t views_per_chunk, const int32_t *index,
+                                         int32_t num_chunks, int32_t dimz, int32_t dimy, int32_t dimx,
+                                         const float *grad_normals, float *scratch_u, float *d_sdf, void *stream);
 
 /* The 2D losses as stand-alone image-space ops, i.e. at the boundary the reference applies them: to rendered images
  *    (depth L1 train.py:635-638, colour L1 loss.compute_2dcolor_loss loss.py:246-257, 2D semantic CE train.py:744-746).

@@ -19,6 +19,7 @@ SPSG_FLAG_SMEM_MAPS = 1 << 5
 SPSG_FLAG_GLOBAL_MAPS = 1 << 6
 SPSG_FLAG_INDEX_PREBUILT = 1 << 7
 SPSG_FLAG_PACKED_LOCS = 1 << 8
+SPSG_FLAG_VIEW_NORMALS = 1 << 9
 SPSG_LOSS_OUT_FLOATS = 8
 SPSG_DTYPE_F32 = 0
 SPSG_DTYPE_BF16 = 1
@@ -29,7 +30,8 @@ EXPORTS = (
     "spsg_version", "spsg_last_error", "spsg_workspace_bytes", "spsg_build_index", "spsg_raycast_forward",
     "spsg_raycast_forward_indexed", "spsg_raycast_backward", "spsg_raycast_occ", "spsg_raycast_forward_loss",
     "spsg_raycast_backward_loss", "spsg_raycast_backward_loss_upstream", "spsg_timing_enable", "spsg_timing_read",
-    "spsg_normals_forward", "spsg_normals_backward", "spsg_losses2d_forward", "spsg_losses2d_backward",
+    "spsg_normals_forward", "spsg_normals_backward", "spsg_normals_forward_views", "spsg_normals_backward_views",
+    "spsg_losses2d_forward", "spsg_losses2d_backward",
     "spsg_depth_bilateral_filter", "spsg_depth_median_fill", "spsg_depth_to_cameraspace", "spsg_depth_to_normals",
     "spsg_depth_compute_normals",
     "spsg_sparsify_scratch_bytes", "spsg_sparsify_count", "spsg_sparsify_locs", "spsg_sparsify_locs_indexed",
@@ -125,6 +127,10 @@ def _load():
     lib.spsg_normals_forward.argtypes = [vp, i64, vp, vp, vp, i32, i32, i32, i32, vp, vp]
     lib.spsg_normals_backward.restype = ctypes.c_int
     lib.spsg_normals_backward.argtypes = [vp, i64, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp]
+    lib.spsg_normals_forward_views.restype = ctypes.c_int
+    lib.spsg_normals_forward_views.argtypes = [vp, i64, vp, vp, i32, vp, i32, i32, i32, i32, vp, vp]
+    lib.spsg_normals_backward_views.restype = ctypes.c_int
+    lib.spsg_normals_backward_views.argtypes = [vp, i64, vp, vp, i32, vp, i32, i32, i32, i32, vp, vp, vp, vp]
     lib.spsg_losses2d_forward.restype = ctypes.c_int
     lib.spsg_losses2d_forward.argtypes = [lt, vp, vp, vp, i64, vp, vp, sz, vp]
     lib.spsg_losses2d_backward.restype = ctypes.c_int

@@ -163,7 +163,9 @@ __device__ __forceinline__ void clear_span(float *__restrict__ p, size_t n, size
 // CTA i works on chunk i % B (then i % B + gridDim, ...): the chunk's cell-class bit planes and block map are pulled
 // into shared memory once by TMA bulk copies, so the march's "does this sample need arithmetic" lookups never leave
 // the SM; tiles of the chunk's images are dealt to warps first statically, then from a global counter.
-template <bool kLoss, bool kSmemMaps, int kWarps>
+// kViewNormals (SPSG_FLAG_VIEW_NORMALS, several views): vals_normal is (N,F,3) and image chunk*F + f reads row (hit, f); the
+// backward's normal rows to clear are N*F.
+template <bool kLoss, bool kSmemMaps, int kWarps, bool kViewNormals>
 __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const ForwardArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ float4 s_steps[kStepEntries];
@@ -181,7 +183,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
         const size_t wid = (size_t)blockIdx.x * kWarps + warp, nw = (size_t)gridDim.x * kWarps, n = (size_t)a.clear_rows;
         clear_span(a.clear.d_semantic, n * 14, wid, nw, lane);
         clear_span(a.clear.d_color, n * 3, wid, nw, lane);
-        clear_span(a.clear.d_normal, n * 3, wid, nw, lane);
+        clear_span(a.clear.d_normal, n * 3 * (kViewNormals ? (size_t)a.views : 1), wid, nw, lane);
         clear_span(a.clear.d_depth, n, wid, nw, lane);
     }
     if (threadIdx.x < kStepEntries) step_table_fill(s_steps, threadIdx.x, a.inc);
@@ -608,7 +610,8 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
                 float n0 = ninf, n1 = ninf, n2 = ninf;
                 bool first = false;
                 if (hit >= 0) {
-                    const float *c = a.vals_color + (size_t)hit * 3, *n = a.vals_normal + (size_t)hit * 3;
+                    const float *c = a.vals_color + (size_t)hit * 3;
+                    const float *n = a.vals_normal + (kViewNormals ? ((size_t)hit * a.views + view) * 3 : (size_t)hit * 3);
                     col0 = __ldg(c + 0); col1 = __ldg(c + 1); col2 = __ldg(c + 2);
                     const float m0 = __ldg(n + 0), m1 = __ldg(n + 1), m2 = __ldg(n + 2);
                     if (!(m0 == 0.0f && m1 == 0.0f && m2 == 0.0f)) { n0 = m0; n1 = m1; n2 = m2; }  // :220

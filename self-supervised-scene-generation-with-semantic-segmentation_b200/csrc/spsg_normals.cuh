@@ -16,7 +16,7 @@
 struct NormalsArgs {
     const longlong4 *locs;
     const float *sdf;
-    const float *transform;  // (B,4,4) row-major or NULL
+    const float *transform;  // (B,4,4) row-major or NULL; (B*F,4,4) for the per-view kernels
     const int32_t *index;    // (B,Dz,Dy,Dx) voxel -> row, -1 = absent
     const float *grad_out;   // backward: dL/d out (N,3)
     float *out;              // forward: normals (N,3); backward pass 1: u = dL/dg (N,3)
@@ -93,6 +93,58 @@ __global__ void __launch_bounds__(256) normals_backward_u_kernel(const NormalsAr
         ux = R[0] * dmx + R[3] * dmy + R[6] * dmz;  // R^T
         uy = R[1] * dmx + R[4] * dmy + R[7] * dmz;
         uz = R[2] * dmx + R[5] * dmy + R[8] * dmz;
+    }
+    a.out[i * 3 + 0] = ux; a.out[i * 3 + 1] = uy; a.out[i * 3 + 2] = uz;
+}
+
+// Per-view normals (SPSG_FLAG_VIEW_NORMALS renders): g once per voxel, then out[(i*F + f)*3 ..] = -normalize(R_{b*F+f} g)
+// with the arithmetic of normals_forward_kernel; transform is (B*F,4,4), one rotation per image.
+__global__ void __launch_bounds__(256) normals_forward_views_kernel(const NormalsArgs a, int views) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n) return;
+    const longlong4 l = a.locs[i];
+    float gx, gy, gz, R[9];
+    normals_gradient(a, l, gx, gy, gz);
+    for (int f = 0; f < views; f++) {
+        load_rotation(a, l.w * views + f, R);
+        const float mx = R[0] * gx + R[1] * gy + R[2] * gz, my = R[3] * gx + R[4] * gy + R[5] * gz,
+                    mz = R[6] * gx + R[7] * gy + R[8] * gz;
+        const float inv = 1.0f / fmaxf(sqrtf(mx * mx + my * my + mz * mz), 1e-5f);
+        float *o = a.out + ((size_t)i * views + f) * 3;
+        o[0] = -(mx * inv);
+        o[1] = -(my * inv);
+        o[2] = -(mz * inv);
+    }
+}
+
+// backward pass 1 of the per-view normals: u = sum over f, in view order, of view f's dL/dg (normals_backward_u_kernel's
+// formula with grad_out row (i, f) and image b*F+f's rotation)
+__global__ void __launch_bounds__(256) normals_backward_u_views_kernel(const NormalsArgs a, int views) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= a.n) return;
+    const longlong4 l = a.locs[i];
+    float gx, gy, gz, R[9];
+    float ux = 0.0f, uy = 0.0f, uz = 0.0f;
+    if (normals_gradient(a, l, gx, gy, gz)) {
+        for (int f = 0; f < views; f++) {
+            load_rotation(a, l.w * views + f, R);
+            const float mx = R[0] * gx + R[1] * gy + R[2] * gz, my = R[3] * gx + R[4] * gy + R[5] * gz,
+                        mz = R[6] * gx + R[7] * gy + R[8] * gz;
+            const float len = sqrtf(mx * mx + my * my + mz * mz);
+            const float *q = a.grad_out + ((size_t)i * views + f) * 3;
+            const float qx = __ldg(q + 0), qy = __ldg(q + 1), qz = __ldg(q + 2);
+            float dmx, dmy, dmz;
+            if (len > 1e-5f) {
+                const float inv = 1.0f / len;
+                const float hx = mx * inv, hy = my * inv, hz = mz * inv, dot = hx * qx + hy * qy + hz * qz;
+                dmx = -(qx - hx * dot) * inv; dmy = -(qy - hy * dot) * inv; dmz = -(qz - hz * dot) * inv;
+            } else {
+                dmx = -qx * 1e5f; dmy = -qy * 1e5f; dmz = -qz * 1e5f;
+            }
+            const float vx = R[0] * dmx + R[3] * dmy + R[6] * dmz, vy = R[1] * dmx + R[4] * dmy + R[7] * dmz,
+                        vz = R[2] * dmx + R[5] * dmy + R[8] * dmz;
+            ux += vx; uy += vy; uz += vz;
+        }
     }
     a.out[i * 3 + 0] = ux; a.out[i * 3 + 1] = uy; a.out[i * 3 + 2] = uz;
 }

@@ -221,6 +221,8 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
     const unsigned grid = (unsigned)std::max<long long>(1, std::min<long long>(sms, all_tiles));
     // CTA size: 24 warps when every warp gets about one tile (latency-bound), 28 when there are many tiles per SM
     const bool large = all_tiles >= (long long)sms * 4 * kFwdWarpsLarge;
+    // one normal per (voxel, view); with one view per chunk that is the shared-normals kernel
+    const bool view_normals = (p->flags & SPSG_FLAG_VIEW_NORMALS) && p->views_per_chunk > 1;
     const int warps = large ? kFwdWarpsLarge : kFwdWarps;
     const size_t dyn = fwd_smem_fixed(warps) + (a.maps_in_smem ? map_bytes : 0);
     {
@@ -230,21 +232,29 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
         CUDA_TRY(cudaGetDevice(&dev));
         std::lock_guard<std::mutex> lk(mu);
         if (dev < 0 || dev >= 64 || !configured[dev]) {
-#define SPSG_SET_SMEM(L, M, W) CUDA_TRY(cudaFuncSetAttribute(raycast_forward_kernel<L, M, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmemMax))
-            SPSG_SET_SMEM(true, true, kFwdWarps); SPSG_SET_SMEM(false, true, kFwdWarps);
-            SPSG_SET_SMEM(true, false, kFwdWarps); SPSG_SET_SMEM(false, false, kFwdWarps);
-            SPSG_SET_SMEM(true, true, kFwdWarpsLarge); SPSG_SET_SMEM(false, true, kFwdWarpsLarge);
-            SPSG_SET_SMEM(true, false, kFwdWarpsLarge); SPSG_SET_SMEM(false, false, kFwdWarpsLarge);
+#define SPSG_SET_SMEM(L, M, W, VN) CUDA_TRY(cudaFuncSetAttribute(raycast_forward_kernel<L, M, W, VN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmemMax))
+#define SPSG_SET_SMEM_ALL(VN)                                                                                   \
+    SPSG_SET_SMEM(true, true, kFwdWarps, VN); SPSG_SET_SMEM(false, true, kFwdWarps, VN);                         \
+    SPSG_SET_SMEM(true, false, kFwdWarps, VN); SPSG_SET_SMEM(false, false, kFwdWarps, VN);                       \
+    SPSG_SET_SMEM(true, true, kFwdWarpsLarge, VN); SPSG_SET_SMEM(false, true, kFwdWarpsLarge, VN);               \
+    SPSG_SET_SMEM(true, false, kFwdWarpsLarge, VN); SPSG_SET_SMEM(false, false, kFwdWarpsLarge, VN)
+            SPSG_SET_SMEM_ALL(false);
+            SPSG_SET_SMEM_ALL(true);
+#undef SPSG_SET_SMEM_ALL
 #undef SPSG_SET_SMEM
             if (dev >= 0 && dev < 64) configured[dev] = true;
         }
     }
     {
         ScopedKernelTimer timer(0, st);
+#define SPSG_LAUNCH_VN(L, M, VN)                                                                                  \
+    do {                                                                                                          \
+        if (large) raycast_forward_kernel<L, M, kFwdWarpsLarge, VN><<<grid, kFwdWarpsLarge * 32, dyn, st>>>(a);  \
+        else raycast_forward_kernel<L, M, kFwdWarps, VN><<<grid, kFwdWarps * 32, dyn, st>>>(a);                  \
+    } while (0)
 #define SPSG_LAUNCH(L, M)                                                                                         \
     do {                                                                                                          \
-        if (large) raycast_forward_kernel<L, M, kFwdWarpsLarge><<<grid, kFwdWarpsLarge * 32, dyn, st>>>(a);      \
-        else raycast_forward_kernel<L, M, kFwdWarps><<<grid, kFwdWarps * 32, dyn, st>>>(a);                      \
+        if (view_normals) SPSG_LAUNCH_VN(L, M, true); else SPSG_LAUNCH_VN(L, M, false);                           \
     } while (0)
         if (targets) {
             if (a.maps_in_smem) SPSG_LAUNCH(true, true); else SPSG_LAUNCH(true, false);
@@ -252,6 +262,7 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
             if (a.maps_in_smem) SPSG_LAUNCH(false, true); else SPSG_LAUNCH(false, false);
         }
 #undef SPSG_LAUNCH
+#undef SPSG_LAUNCH_VN
     }
     CUDA_TRY(cudaGetLastError());
     return SPSG_OK;
@@ -310,18 +321,21 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
     const unsigned zero_blocks = (unsigned)std::min<long long>((p->num_locs + 255) / 256, (long long)sms * 4);
     const bool cleared = (p->flags & SPSG_FLAG_GRADS_CLEARED) != 0;  // the forward's fill pass cleared rows [0, N)
     const bool multi = p->views_per_chunk > 1, exact = (p->flags & SPSG_FLAG_DETERMINISTIC_GRADS) != 0;
-#define SPSG_GATHER(FUSED, UP, VIEWS, BLOCKS) backward_gather_kernel<FUSED, UP, VIEWS><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a)
-#define SPSG_GATHER_VIEWS(VIEWS, BLOCKS)                                                                          \
+    const bool view_normals = multi && (p->flags & SPSG_FLAG_VIEW_NORMALS);  // d_normal (N,F,3), one row per view
+#define SPSG_GATHER(FUSED, UP, VIEWS, VN, BLOCKS) backward_gather_kernel<FUSED, UP, VIEWS, VN><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a)
+#define SPSG_GATHER_VIEWS(VIEWS, VN, BLOCKS)                                                                      \
     do {                                                                                                          \
-        if (up) SPSG_GATHER(true, true, VIEWS, BLOCKS);                                                           \
-        else if (fused) SPSG_GATHER(true, false, VIEWS, BLOCKS);                                                  \
-        else SPSG_GATHER(false, false, VIEWS, BLOCKS);                                                            \
+        if (up) SPSG_GATHER(true, true, VIEWS, VN, BLOCKS);                                                       \
+        else if (fused) SPSG_GATHER(true, false, VIEWS, VN, BLOCKS);                                              \
+        else SPSG_GATHER(false, false, VIEWS, VN, BLOCKS);                                                        \
     } while (0)
 #define SPSG_GATHER_ANY(BLOCKS)                                                                                   \
     do {                                                                                                          \
-        if (!multi) SPSG_GATHER_VIEWS(0, BLOCKS);                                                                 \
-        else if (!exact) SPSG_GATHER_VIEWS(1, BLOCKS);                                                            \
-        else SPSG_GATHER_VIEWS(2, BLOCKS);                                                                        \
+        if (!multi) SPSG_GATHER_VIEWS(0, false, BLOCKS);                                                          \
+        else if (view_normals && !exact) SPSG_GATHER_VIEWS(1, true, BLOCKS);                                      \
+        else if (view_normals) SPSG_GATHER_VIEWS(2, true, BLOCKS);                                                \
+        else if (!exact) SPSG_GATHER_VIEWS(1, false, BLOCKS);                                                     \
+        else SPSG_GATHER_VIEWS(2, false, BLOCKS);                                                                 \
     } while (0)
     if (cleared) {
         a.zero_blocks = 0;
@@ -334,7 +348,8 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
         SPSG_GATHER_ANY(zero_blocks + gather_blocks);
     } else {
         a.zero_blocks = 0;
-        backward_zero_kernel<<<zero_blocks, 256, 0, st>>>(a);
+        if (view_normals) backward_zero_view_normals_kernel<<<zero_blocks, 256, 0, st>>>(a);
+        else backward_zero_kernel<<<zero_blocks, 256, 0, st>>>(a);
         CUDA_TRY(cudaGetLastError());
         ScopedKernelTimer timer(1, st);
         SPSG_GATHER_ANY(gather_blocks);
@@ -547,6 +562,59 @@ int spsg_normals_backward(const int64_t *locs, int64_t num_locs, const float *va
     a.n = num_locs; a.dimx = dimx; a.dimy = dimy; a.dimz = dimz;
     const unsigned blocks = (unsigned)((num_locs + 255) / 256);
     normals_backward_u_kernel<<<blocks, 256, 0, st>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    normals_backward_gather_kernel<<<blocks, 256, 0, st>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    return SPSG_OK;
+}
+
+static int normals_views_check(const float *transform, int32_t views_per_chunk) {
+    if (views_per_chunk <= 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "views_per_chunk must be >= 1");
+    if (views_per_chunk > 1 && !transform) return fail(SPSG_ERR_INVALID_ARGUMENT, "per-view normals need a (B*F,4,4) transform");
+    return SPSG_OK;
+}
+
+int spsg_normals_forward_views(const int64_t *locs, int64_t num_locs, const float *vals_sdf, const float *transform,
+                               int32_t views_per_chunk, int32_t *index, int32_t num_chunks, int32_t dimz, int32_t dimy,
+                               int32_t dimx, float *normals, void *stream) {
+    if (int rc = normals_views_check(transform, views_per_chunk)) return rc;
+    if (views_per_chunk == 1)
+        return spsg_normals_forward(locs, num_locs, vals_sdf, transform, index, num_chunks, dimz, dimy, dimx, normals, stream);
+    if (int rc = normals_check(locs, num_locs, vals_sdf, index, num_chunks, dimz, dimy, dimx)) return rc;
+    if ((long long)num_chunks * views_per_chunk >= (1ll << 31)) return fail(SPSG_ERR_INVALID_ARGUMENT, "too many images");
+    if (num_locs > 0 && !normals) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL output pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = spsg_build_index(locs, num_locs, index, num_chunks, dimz, dimy, dimx, stream)) return rc;
+    if (num_locs == 0) return SPSG_OK;
+    NormalsArgs a;
+    memset(&a, 0, sizeof(a));
+    a.locs = (const longlong4 *)locs; a.sdf = vals_sdf; a.transform = transform; a.index = index; a.out = normals;
+    a.n = num_locs; a.dimx = dimx; a.dimy = dimy; a.dimz = dimz;
+    normals_forward_views_kernel<<<(unsigned)((num_locs + 255) / 256), 256, 0, st>>>(a, views_per_chunk);
+    CUDA_TRY(cudaGetLastError());
+    return SPSG_OK;
+}
+
+int spsg_normals_backward_views(const int64_t *locs, int64_t num_locs, const float *vals_sdf, const float *transform,
+                                int32_t views_per_chunk, const int32_t *index, int32_t num_chunks, int32_t dimz,
+                                int32_t dimy, int32_t dimx, const float *grad_normals, float *scratch_u, float *d_sdf,
+                                void *stream) {
+    if (int rc = normals_views_check(transform, views_per_chunk)) return rc;
+    if (views_per_chunk == 1)
+        return spsg_normals_backward(locs, num_locs, vals_sdf, transform, index, num_chunks, dimz, dimy, dimx, grad_normals,
+                                     scratch_u, d_sdf, stream);
+    if (int rc = normals_check(locs, num_locs, vals_sdf, index, num_chunks, dimz, dimy, dimx)) return rc;
+    if ((long long)num_chunks * views_per_chunk >= (1ll << 31)) return fail(SPSG_ERR_INVALID_ARGUMENT, "too many images");
+    if (num_locs == 0) return SPSG_OK;
+    if (!grad_normals || !scratch_u || !d_sdf) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL gradient pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    NormalsArgs a;
+    memset(&a, 0, sizeof(a));
+    a.locs = (const longlong4 *)locs; a.sdf = vals_sdf; a.transform = transform; a.index = index;
+    a.grad_out = grad_normals; a.out = scratch_u; a.d_sdf = d_sdf;
+    a.n = num_locs; a.dimx = dimx; a.dimy = dimy; a.dimz = dimz;
+    const unsigned blocks = (unsigned)((num_locs + 255) / 256);
+    normals_backward_u_views_kernel<<<blocks, 256, 0, st>>>(a, views_per_chunk);
     CUDA_TRY(cudaGetLastError());
     normals_backward_gather_kernel<<<blocks, 256, 0, st>>>(a);
     CUDA_TRY(cudaGetLastError());

@@ -68,24 +68,28 @@ def fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, v
                   clear_grads):
     """``spsg_raycast_forward_loss`` on the buffers of raycaster ``m``: validates every tensor whose pointer crosses the
     C ABI, renders, accumulates the 2D loss terms.  ``targets`` = (target_depth, target_color, weight_color, target_label,
-    class_weight, voxelsize, (w_depth, w_colour, w_semantic)).  Returns (params, targets struct, loss_out[8])."""
+    class_weight, voxelsize, (w_depth, w_colour, w_semantic)).  ``vals_normals`` (N,3) shared or (N,F,3) per view
+    (SPSG_FLAG_VIEW_NORMALS, set in the returned params).  Returns (params, targets struct, loss_out[8])."""
     images = view_matrix.shape[0]
     views = max(1, images // m.batch_size)
     if images != views * m.batch_size or views > m.max_num_frames:
         raise RuntimeError("view_matrix has %d images: expected batch_size (%d) x views <= max_num_frames (%d)"
                            % (images, m.batch_size, m.max_num_frames))
+    per_view = rc.view_normals(vals_normals, views)
     n = rc.check_voxel_inputs(locs, vals_sdf, vals_colors, vals_normals, vals_semantic, view_matrix, intrinsic_params,
-                              images)
+                              images, views if per_view else 1)
     if n * views > m.mapping3dto2d.shape[0]:
         raise RuntimeError("too many voxels for raycast (%d x %d views > %d rows)" % (n, views, m.mapping3dto2d.shape[0]))
-    if clear_grads and (m.d_depth.shape[0] < n or m.d_color.shape[0] < n or m.d_normal.shape[0] < n or
-                        m.d_semantic.shape[0] < n):
+    d_normal = rc.normal_grad_buffer(m, per_view)
+    if clear_grads and (m.d_depth.shape[0] < n or m.d_color.shape[0] < n or
+                        d_normal.shape[0] < n * (views if per_view else 1) or m.d_semantic.shape[0] < n):
         raise RuntimeError("d_* buffers hold fewer than N = %d rows" % n)
     dev = vals_sdf.device
     if m.image_depth.device != dev:
         raise RuntimeError("raycaster buffers live on %s, inputs on %s" % (m.image_depth.device, dev))
     p = N.make_params(m.width, m.height, m.depth_min, m.depth_max, m.thresh_sample_dist, m.ray_increment,
-                      m.dims3d[2], m.dims3d[1], m.dims3d[0], m.batch_size, views, m.mapping3dto2d.shape[1], n, m.flags)
+                      m.dims3d[2], m.dims3d[1], m.dims3d[0], m.batch_size, views, m.mapping3dto2d.shape[1], n,
+                      m.flags | (N.SPSG_FLAG_VIEW_NORMALS if per_view else 0))
     if rc.is_packed_locs(locs):
         p.flags |= N.SPSG_FLAG_PACKED_LOCS
     target_depth, target_color, weight_color, target_label, class_weight, voxelsize, weights = targets
@@ -93,7 +97,7 @@ def fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, v
                          voxelsize, weights)
     # terms, total and normalisers of THIS call (the backward reads the normalisers back)
     loss_out = torch.empty(N.SPSG_LOSS_OUT_FLOATS, device=dev)
-    gb = N.grad_buffers(m.d_color, m.d_depth, m.d_normal, m.d_semantic) if clear_grads else None
+    gb = N.grad_buffers(m.d_color, m.d_depth, d_normal, m.d_semantic) if clear_grads else None
     owner = _module_workspace(m)
     with rc.device_guard(dev):
         nbytes = N.workspace_bytes(p)
@@ -131,8 +135,20 @@ def _upstream_struct(m, p, upstream):
     return N.UpstreamGrads(*ptrs)
 
 
+def _per_view(p):
+    return bool(p.flags & N.SPSG_FLAG_VIEW_NORMALS)
+
+
+def _voxel_grads(m, p, n):
+    """(d_sdf, d_color, d_normal, d_semantic): rows [0, N) of ``m.d_*``; per-view normals as (N,F,3)."""
+    d_normal = rc.normal_grad_buffer(m, _per_view(p))
+    d_normal = d_normal[:n * p.views_per_chunk].view(n, p.views_per_chunk, 3) if _per_view(p) else d_normal[:n]
+    return m.d_depth[:n], m.d_color[:n], d_normal, m.d_semantic[:n]
+
+
 def fused_backward(m, p, tg, loss_out, grad_scale, grads_cleared, upstream=None):
-    """``spsg_raycast_backward_loss``: voxel gradients of ``grad_scale * total`` into rows [0, N) of ``m.d_*``.
+    """``spsg_raycast_backward_loss``: voxel gradients of ``grad_scale * total`` into rows [0, N) of ``m.d_*`` (the
+    per-view normal rows of ``raycast_rgbd_cuda.normal_grad_buffer`` when ``p`` has SPSG_FLAG_VIEW_NORMALS).
     ``upstream`` = (grad_color, grad_depth, grad_normal, grad_semantic) gradient images of the renderings (any of them
     None; contiguous float32): ``spsg_raycast_backward_loss_upstream`` then adds them, unscaled, in the same gather.
     ``grad_scale`` None means 1."""
@@ -144,6 +160,7 @@ def fused_backward(m, p, tg, loss_out, grad_scale, grads_cleared, upstream=None)
         rc._check_input(grad_scale, "grad_scale")
         rc._check_dtype(grad_scale, torch.float32, "grad_scale")
     up = _upstream_struct(m, p, upstream) if upstream is not None else None
+    d_normal = rc.normal_grad_buffer(m, _per_view(p))
     owner = _module_workspace(m)
     with rc.device_guard(dev):
         ws = owner.check(p, N.workspace_bytes(p))  # the work list of the forward that rendered m's images
@@ -151,14 +168,14 @@ def fused_backward(m, p, tg, loss_out, grad_scale, grads_cleared, upstream=None)
             N.check(N.lib.spsg_raycast_backward_loss(
                 ctypes.byref(p), N.ptr(m.image_color), N.ptr(m.image_depth), N.ptr(m.image_semantic),
                 ctypes.byref(tg), N.ptr(loss_out), N.ptr(grad_scale), N.ptr(m.sparse_mapping), N.ptr(m.mapping3dto2d),
-                N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth), N.ptr(m.d_normal), N.ptr(m.d_semantic),
+                N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth), N.ptr(d_normal), N.ptr(m.d_semantic),
                 N.ptr(ws), ws.numel(), rc._stream(dev)))
         else:
             N.check(N.lib.spsg_raycast_backward_loss_upstream(
                 ctypes.byref(p), N.ptr(m.image_color), N.ptr(m.image_depth), N.ptr(m.image_semantic),
                 ctypes.byref(tg), N.ptr(loss_out), N.ptr(grad_scale), ctypes.byref(up), N.ptr(m.sparse_mapping),
                 N.ptr(m.mapping3dto2d), N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth),
-                N.ptr(m.d_normal), N.ptr(m.d_semantic), N.ptr(ws), ws.numel(), rc._stream(dev)))
+                N.ptr(d_normal), N.ptr(m.d_semantic), N.ptr(ws), ws.numel(), rc._stream(dev)))
 
 
 def _targets_off(tg):
@@ -224,7 +241,7 @@ class FusedRaycastLossFunction(Function):
             fused_backward(m, ctx.params, ctx.targets, ctx.loss_out, grad_total.to(torch.float32).contiguous(),
                            ctx.grads_cleared, upstream)
         ctx.grads_cleared = False  # the forward cleared the rows once: a second backward (retain_graph) clears its own
-        grads = (m.d_depth[:n], m.d_color[:n], m.d_normal[:n], m.d_semantic[:n])
+        grads = _voxel_grads(m, ctx.params, n)
         m.workspace.grad_views = grads  # leaves get copies, not the buffers (raycast_rgbd_cuda.ModuleWorkspace)
         return (None, None) + grads + (None,) * 10
 
@@ -236,7 +253,8 @@ def render_loss_and_voxel_grads(raycaster, locs, vals_sdf, vals_colors, vals_nor
     """The fused forward + backward pair without autograd, for callers that own the voxel tensors' gradients themselves
     (and for CUDA-graph capture: nothing but the two native calls is enqueued).  Returns ``(loss_out, (d_sdf, d_color,
     d_normal, d_semantic))``: ``loss_out[0:3]`` = depth / colour / semantic terms, ``loss_out[3]`` = weighted total; the
-    gradients of ``grad_scale * total`` (default 1) are views of rows [0, N) of the raycaster's ``d_*`` buffers."""
+    gradients of ``grad_scale * total`` (default 1) are views of rows [0, N) of the raycaster's ``d_*`` buffers; with
+    per-view normals ``(N,F,3)`` the normal gradient is ``(N,F,3)`` too."""
     c = lambda t: None if t is None else t.contiguous()
     m, n = raycaster, locs.shape[0]
     p, tg, loss_out = fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantics, view_matrix,
@@ -248,7 +266,7 @@ def render_loss_and_voxel_grads(raycaster, locs, vals_sdf, vals_colors, vals_nor
         if grad_scale is None or grad_scale.device != loss_out.device:
             grad_scale = m._unit_scale = torch.ones((), device=loss_out.device)
     fused_backward(m, p, tg, loss_out, grad_scale, n > 0)
-    return loss_out, (m.d_depth[:n], m.d_color[:n], m.d_normal[:n], m.d_semantic[:n])
+    return loss_out, _voxel_grads(m, p, n)
 
 
 def render_with_2d_losses(raycaster, locs, vals_sdf, vals_colors, vals_normals, vals_semantics, view_matrix,

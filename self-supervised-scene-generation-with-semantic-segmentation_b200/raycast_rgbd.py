@@ -9,6 +9,9 @@ Differences, all behind defaulted extras or unobservable through the reference A
   * several views per chunk: pass ``view_matrix`` / ``intrinsic_params`` with ``B*F`` rows (image ``i`` renders
     chunk ``i // F``, the ordering of reference ``style.compute_view_matrix``, style.py:9-16), ``F <= max_num_frames``.
     The voxel gradient is then the sum over views of the per-view means = F reference calls accumulated by autograd.
+  * per-view normals: with ``vals_normals`` of shape ``(N,F,3)``, image ``b*F + f`` renders row ``(v, f)`` -- each view's
+    normals in its own camera frame, as F reference calls with their own ``transform`` give (train.py:542-544).  Its
+    gradient is ``(N,F,3)``, view f's mean in row ``(v, f)``; ``(N,3)`` keeps the shared payload.
   * no host synchronisation: the reference reads ``locs[-1, -1]`` back to the host (raycast_rgbd.py:22,30).
   * the upstream ``RaycastOcc.forward`` NameError (``raycast_color_cuda``, raycast_rgbd.py:103) is fixed.
 """
@@ -16,6 +19,7 @@ import torch
 from torch import nn
 from torch.autograd import Function
 
+from . import _native as N
 from . import raycast_rgbd_cuda
 
 
@@ -58,6 +62,12 @@ class RayCastRGBDFunction(Function):
         return image_color[:images], image_depth[:images], image_normal[:images], image_semantic[:images]
 
     @staticmethod
+    def _normal_grad(ctx, d_normal, n):
+        if ctx.flags & N.SPSG_FLAG_VIEW_NORMALS:
+            return d_normal[:n * ctx.views_per_chunk].view(n, ctx.views_per_chunk, 3)
+        return d_normal[:n]
+
+    @staticmethod
     def backward(ctx, grad_color, grad_depth, grad_normal, grad_semantic):
         sparse_mapping, mapping3dto2d, mapping3dto2d_num, d_color, d_depth, d_normal, d_semantic = ctx.saved_tensors
         n = ctx.dims[4]
@@ -70,7 +80,7 @@ class RayCastRGBDFunction(Function):
             views_per_chunk=ctx.views_per_chunk, grads_cleared=ctx.grads_cleared, workspace_owner=owner,
             flags=ctx.flags)
         ctx.grads_cleared = False  # the forward cleared the rows once: a second backward (retain_graph) clears its own
-        grads = (d_depth[:n], d_color[:n], d_normal[:n], d_semantic[:n])
+        grads = (d_depth[:n], d_color[:n], RayCastRGBDFunction._normal_grad(ctx, d_normal, n), d_semantic[:n])
         if owner is not None:
             owner.grad_views = grads  # leaves get copies, not the buffers (ModuleWorkspace)
         # raycast_rgbd.py:42-43: (locs, vals_sdf, vals_colors, vals_normals, vals_semantic, None...)
@@ -108,6 +118,7 @@ class RaycastRGBD(nn.Module):
         self.d_normal = torch.zeros(batch_size * max_num_locs_per_sample, 3, device=device)
         self.d_depth = torch.zeros(batch_size * max_num_locs_per_sample, 1, device=device)
         self.d_semantic = torch.zeros(batch_size * max_num_locs_per_sample, 14, device=device)
+        self.d_normal_views = None  # (N*F,3) gradient rows of per-view normals (raycast_rgbd_cuda.normal_grad_buffer)
         self.flags = 0  # SPSG_FLAG_* (e.g. _native.SPSG_FLAG_DETERMINISTIC_GRADS for bit-reproducible multi-view gradients)
         # scratch of the native calls (block maps, the backward's work list): owned by the module like the buffers above
         self.workspace = raycast_rgbd_cuda.ModuleWorkspace()
@@ -123,12 +134,15 @@ class RaycastRGBD(nn.Module):
         if images != views * self.batch_size or views > self.max_num_frames:
             raise RuntimeError("view_matrix has %d images: expected batch_size (%d) x views with views <= "
                                "max_num_frames (%d)" % (images, self.batch_size, self.max_num_frames))
+        per_view = raycast_rgbd_cuda.view_normals(vals_normals, views)
+        flags = self.flags | (N.SPSG_FLAG_VIEW_NORMALS if per_view else 0)
         return RayCastRGBDFunction.apply(locs, vals_sdf, vals_colors, vals_normals, vals_semantics, view_matrix,
                                          intrinsic_params, self.dims3d, self.width, self.height, self.depth_min,
                                          self.depth_max, self.thresh_sample_dist, self.ray_increment, self.image_color,
                                          self.image_depth, self.image_normal, self.image_semantic, self.sparse_mapping,
                                          self.mapping3dto2d, self.mapping3dto2d_num, self.d_color, self.d_depth,
-                                         self.d_normal, self.d_semantic, views, self.flags, self.workspace)
+                                         raycast_rgbd_cuda.normal_grad_buffer(self, per_view), self.d_semantic, views,
+                                         flags, self.workspace)
 
 
 class RaycastOcc(nn.Module):

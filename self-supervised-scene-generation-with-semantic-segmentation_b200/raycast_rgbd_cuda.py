@@ -46,9 +46,11 @@ def _check_dtype(t, dtype, name):
         raise RuntimeError("%s must have dtype %s, got %s" % (name, dtype, t.dtype))
 
 
-def check_voxel_inputs(locs, vals_sdf, vals_color, vals_normals, vals_semantic, view_matrix, intrinsic_params, images):
+def check_voxel_inputs(locs, vals_sdf, vals_color, vals_normals, vals_semantic, view_matrix, intrinsic_params, images,
+                       normal_views=1):
     """What every raw-pointer entry point relies on: CUDA + contiguous, int64 `locs` rows of 4, float32 payloads with at
-    least N rows of 1 / 3 / 3 / 14, cameras for every image.  Raises RuntimeError like the reference's AT_ASSERTM."""
+    least N rows of 1 / 3 / 3 / 14 (normals: N * ``normal_views`` rows of 3 with SPSG_FLAG_VIEW_NORMALS), cameras for every
+    image.  Raises RuntimeError like the reference's AT_ASSERTM."""
     for t, name in ((locs, "locs"), (vals_sdf, "vals_sdf"), (vals_color, "vals_color"), (vals_normals, "vals_normals"),
                     (vals_semantic, "vals_semantic"), (view_matrix, "viewMatrixInv"), (intrinsic_params, "intrinsicParams")):
         _check_input(t, name)
@@ -60,7 +62,8 @@ def check_voxel_inputs(locs, vals_sdf, vals_color, vals_normals, vals_semantic, 
     n = locs.shape[0]
     if not is_packed_locs(locs) and locs.numel() != 4 * n:
         raise RuntimeError("locs must be (N, 4) rows of (z, y, x, chunk)")
-    if vals_sdf.numel() < n or vals_color.numel() < 3 * n or vals_normals.numel() < 3 * n or vals_semantic.numel() < 14 * n:
+    if vals_sdf.numel() < n or vals_color.numel() < 3 * n or vals_normals.numel() < 3 * n * normal_views or \
+            vals_semantic.numel() < 14 * n:
         raise RuntimeError("voxel value tensors hold fewer than N = %d rows" % n)
     if view_matrix.numel() < images * 16 or intrinsic_params.numel() < images * 4:
         raise RuntimeError("viewMatrixInv / intrinsicParams hold fewer than %d images" % images)
@@ -95,9 +98,31 @@ def pack_locs_host(locs, num_chunks, dims3d, out=None, threads=0):
     return out
 
 
+def view_normals(vals_normals, views):
+    """Normal payload mode of a render with ``views`` images per chunk: False for the shared ``(N,3)`` payload, True for
+    per-view normals ``(N,views,3)`` (SPSG_FLAG_VIEW_NORMALS; the gradient is ``(N,views,3)`` too)."""
+    if vals_normals.dim() != 3:
+        return False
+    if vals_normals.shape[1] != views or vals_normals.shape[2] != 3:
+        raise RuntimeError("per-view vals_normals must be (N, %d, 3) for %d views per chunk, got %s"
+                           % (views, views, tuple(vals_normals.shape)))
+    return True
+
+
+def normal_grad_buffer(m, per_view):
+    """The ``d_normal`` rows a backward of raycaster ``m`` writes: ``m.d_normal`` (N,3), or with per-view normals a
+    separate buffer of ``m.d_normal.shape[0] * m.max_num_frames`` rows, allocated on first use."""
+    if not per_view:
+        return m.d_normal
+    buf = getattr(m, "d_normal_views", None)
+    if buf is None:
+        buf = m.d_normal_views = torch.zeros(m.d_normal.shape[0] * m.max_num_frames, 3, device=m.d_normal.device)
+    return buf
+
+
 def _stamp(p):
     return (int(p.num_locs), int(p.views_per_chunk), int(p.num_chunks), int(p.width), int(p.height),
-            int(p.max_pixels_per_voxel))
+            int(p.max_pixels_per_voxel), bool(p.flags & N.SPSG_FLAG_VIEW_NORMALS))
 
 
 def workspace(device, nbytes, owner=None, stamp=None, expect=None):
@@ -229,6 +254,7 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
     """Reference signature (``raycast_color_forward``, raycast_rgbd_cuda.cpp:57-91) plus keyword extensions with
     reference-preserving defaults.  ``clear_grads`` = (d_color, d_depth, d_normals, d_semantic) lets the forward's fill
     pass clear the rows the matching ``backward(..., grads_cleared=True)`` will write (needs ``build_index=True``).
+    ``flags`` with SPSG_FLAG_VIEW_NORMALS: ``vals_normals`` (and ``d_normals`` of ``clear_grads``) hold N*F rows.
     ``workspace_owner`` = the calling module's ``ModuleWorkspace`` (else the scratch is looked up by ``sparse_mapping``)."""
     for t, name in ((sparse_mapping, "sparse_mapping"), (imageColor, "imageColor"), (imageDepth, "imageDepth"),
                     (imageNormal, "imageNormal"), (imageSemantic, "imageSemantic"), (mapping3dto2d, "mapping3dto2d"),
@@ -246,7 +272,9 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
             raise RuntimeError("packed locs need build_index=True")
         p.flags |= N.SPSG_FLAG_PACKED_LOCS
     images = p.num_chunks * p.views_per_chunk
-    n = check_voxel_inputs(locs, vals_sdf, vals_color, vals_normals, vals_semantic, viewMatrixInv, intrinsicParams, images)
+    nv = p.views_per_chunk if flags & N.SPSG_FLAG_VIEW_NORMALS else 1
+    n = check_voxel_inputs(locs, vals_sdf, vals_color, vals_normals, vals_semantic, viewMatrixInv, intrinsicParams, images,
+                           nv)
     if mapping3dto2d_num.numel() < p.views_per_chunk * n or mapping3dto2d.shape[0] < p.views_per_chunk * n:
         raise RuntimeError("mapping3dto2d has %d rows, needs views_per_chunk*N = %d" %
                            (mapping3dto2d.shape[0], p.views_per_chunk * n))
@@ -270,7 +298,7 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
         if build_index:
             gb = None
             if clear_grads is not None:
-                for t, rows in zip(clear_grads, (3, 1, 3, 14)):
+                for t, rows in zip(clear_grads, (3, 1, 3 * nv, 14)):
                     _check_input(t, "clear_grads")
                     _check_dtype(t, torch.float32, "clear_grads")
                     if t.numel() < n * rows:
@@ -292,7 +320,8 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
              dims, d_color, d_depth, d_normals, d_semantic, views_per_chunk=1, grads_cleared=False, workspace_owner=None,
              flags=0):
     """Reference signature (``raycast_color_backward``, raycast_rgbd_cuda.cpp:102-140).
-    ``dims`` = int32 CPU tensor (or sequence) [batch, Dx, Dy, Dz, N] (raycast_rgbd.py:30-31)."""
+    ``dims`` = int32 CPU tensor (or sequence) [batch, Dx, Dy, Dz, N] (raycast_rgbd.py:30-31).  ``flags``: the forward's
+    SPSG_FLAG_DETERMINISTIC_GRADS and SPSG_FLAG_VIEW_NORMALS (``d_normals`` then holds N*F rows) are used."""
     for t, name in ((grad_color, "grad_color"), (grad_depth, "grad_depth"), (grad_normal, "grad_normal"),
                     (grad_semantic, "grad_semantic"), (sparse_mapping, "sparse_mapping"),
                     (mapping3dto2d, "mapping3dto2d"), (mapping3dto2d_num, "mapping3dto2d_num"),
@@ -304,13 +333,15 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
         _check_dtype(t, torch.float32, name)
     d = dims.tolist() if isinstance(dims, torch.Tensor) else list(dims)
     n = int(d[4])
-    if d_color.shape[0] < n or d_depth.shape[0] < n or d_normals.shape[0] < n or d_semantic.shape[0] < n:
+    nv = views_per_chunk if flags & N.SPSG_FLAG_VIEW_NORMALS else 1
+    if d_color.shape[0] < n or d_depth.shape[0] < n or d_normals.shape[0] < n * nv or d_semantic.shape[0] < n:
         raise RuntimeError("d_* buffers hold fewer than N = %d rows" % n)
     p = N.make_params(width=grad_color.shape[2], height=grad_color.shape[1], depth_min=0, depth_max=0,
                       thresh_sample_dist=0, ray_increment=0, dimx=int(d[1]), dimy=int(d[2]), dimz=int(d[3]),
                       num_chunks=sparse_mapping.shape[0], views_per_chunk=views_per_chunk,
                       max_pixels_per_voxel=mapping3dto2d.shape[1], num_locs=n,
-                      flags=(N.SPSG_FLAG_GRADS_CLEARED if grads_cleared else 0) | (flags & N.SPSG_FLAG_DETERMINISTIC_GRADS))
+                      flags=(N.SPSG_FLAG_GRADS_CLEARED if grads_cleared else 0) |
+                      (flags & (N.SPSG_FLAG_DETERMINISTIC_GRADS | N.SPSG_FLAG_VIEW_NORMALS)))
     dev = grad_color.device
     px = sparse_mapping.shape[0] * views_per_chunk * p.width * p.height
     if grad_depth.numel() < px or grad_color.numel() < 3 * px or grad_normal.numel() < 3 * px or grad_semantic.numel() < 14 * px:

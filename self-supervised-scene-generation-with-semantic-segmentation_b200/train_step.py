@@ -77,11 +77,21 @@ class ViewGuidedTrainStep:
                                      max_num_locs_per_sample=max_num_locs_per_sample, device=device)
         self.last = {}
 
+    def _normals(self, locs, vals, transform):
+        """train.py:542-544: the voxels' normals in the camera frame of the image that renders them.  With several views
+        per chunk that is one normal per (voxel, view): ``transform`` holds one (4,4) per image, (N,F,3) comes back."""
+        if self.views == 1:
+            return normals.compute_normals_sparse(locs, vals, self.dims3d, transform=transform)
+        return normals.compute_normals_sparse(locs, vals, self.dims3d, transform=transform, views_per_chunk=self.views)
+
     def _target_labels(self, target_for_sdf, target_for_colors, target_for_semantics, view_matrix, intrinsics, transform):
         """train.py:581-622: render the target chunk, its semantics become the per-pixel labels."""
         locs, vals = sparsify.sparsify_predictions(target_for_sdf, self.truncation)
         colors = target_for_colors[locs[:, 3], locs[:, 0], locs[:, 1], locs[:, 2], :].float() / 255.0
-        target_normals = normals.compute_normals_sparse(locs, vals, self.dims3d, transform=transform)
+        if self.views == 1:
+            target_normals = normals.compute_normals_sparse(locs, vals, self.dims3d, transform=transform)
+        else:  # only the labels are read: shared normals in the grid frame
+            target_normals = normals.compute_normals_sparse(locs, vals, self.dims3d, num_chunks=self.batch_size)
         sem = sparsify.gather_dense(locs, target_for_semantics.float())
         onehot = F.one_hot(sem[:, 0].long(), 15)[..., :-1].float().contiguous()
         _, _, _, raycast_semantic = self.raycaster(locs, vals, colors.contiguous(), target_normals, onehot, view_matrix,
@@ -96,7 +106,7 @@ class ViewGuidedTrainStep:
         volume (truncated neighbours count as +-truncation): the two differ at the rim of the input's band."""
         locs, vals, cols = sparsify.sparsify_predictions(inputs[:, :1].contiguous(), self.truncation, None,
                                                          inputs[:, 1:4].contiguous())
-        input_normals = normals.compute_normals_sparse(locs, vals, self.dims3d, transform=transform)
+        input_normals = self._normals(locs, vals, transform)
         raycast_color, _, raycast_normal, _ = self.raycaster(locs, vals, cols, input_normals, None, view_matrix, intrinsics)
         return raycast_color, raycast_normal
 
@@ -141,7 +151,7 @@ class ViewGuidedTrainStep:
         self.last = dict(num_locs=n, loss_occ=loss_occ.detach(), loss_sdf=loss_sdf.detach())
         if 0 < n <= self.raycaster.get_max_num_locs_per_sample() * self.batch_size:          # train.py:524-529
             view_matrix, intrinsics = sample["view_matrix"], sample["images_intrinsic"]
-            transform = torch.inverse(view_matrix)                                             # train.py:544
+            transform = torch.inverse(view_matrix)                    # train.py:544, one per image (I = B * F)
             input2d = None
             if self.render_input:
                 input_color, input_normal = self._render_input(inputs, view_matrix, intrinsics, transform)
@@ -152,7 +162,7 @@ class ViewGuidedTrainStep:
                                                      view_matrix, intrinsics, transform)
             locs, sdf_vals, color_vals, sem_vals = sparsify.sparsify_predictions(
                 output_sdf, T, empty, output_color, output_semantic, raycaster=self.raycaster, counted=counted)
-            output_normals = normals.compute_normals_sparse(locs, sdf_vals, self.dims3d, transform=transform)
+            output_normals = self._normals(locs, sdf_vals, transform)
             color = (color_vals + 1) * 0.5                                                     # train.py:623
             # prediction raycast + depth L1 + colour L1 + 2D semantic CE (train.py:626-643, 744-746), one kernel pair
             total2d, terms, pred = losses.render_with_2d_losses(

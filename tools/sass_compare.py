@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Compare the SASS of two builds of spsg_raycast.cu function by function, instruction offsets and encodings stripped
-(no GPU needed).  The backward gather's template gained a parameter (kUpstream); its old instantiations
-<kFused, kViews> are matched with <kFused, false, kViews>.  The compaction kernels of spsg_sparsify.cu gained the SDF
+(no GPU needed).  The backward gather's template gained parameters (kUpstream, then kViewNormals); its old
+instantiations <kFused, kViews> and <kFused, kUpstream, kViews> are matched with kUpstream / kViewNormals false.  The
+forward kernel's <kLoss, kSmemMaps, kWarps> likewise with <kLoss, kSmemMaps, kWarps, kViewNormals = false>.  The compaction kernels of spsg_sparsify.cu gained the SDF
 element type: the plain sparsify_count_kernel and sparsify_write_kernel<kIndexed> are matched with their <float>
 instantiations.
 
@@ -39,9 +40,12 @@ def functions(cubin):
 
 def key(name):
     name = re.sub(r"_GLOBAL__N__[0-9a-f]+_\d+_\w+?_cu_[0-9a-f]{8}", "", name)  # the anonymous namespace's per-build tag
-    m = re.search(r"backward_gather_kernelI(Lb[01]E)(Lb[01]E)?(Li\dE)E", name)
+    m = re.search(r"backward_gather_kernelI(Lb[01]E)(Lb[01]E)?(Li\dE)(Lb[01]E)?E", name)
     if m:
-        return "backward_gather_kernel" + m.group(1) + (m.group(2) or "Lb0E") + m.group(3)
+        return "backward_gather_kernel" + m.group(1) + (m.group(2) or "Lb0E") + m.group(3) + (m.group(4) or "Lb0E")
+    m = re.search(r"raycast_forward_kernelI(Lb[01]ELb[01]ELi\d+E)(Lb[01]E)?E", name)
+    if m:
+        return "raycast_forward_kernel" + m.group(1) + (m.group(2) or "Lb0E")
     m = re.search(r"sparsify_count_kernel(?:I([a-z])EEv)?", name)
     if m:
         return "sparsify_count_kernel<%s>" % (m.group(1) or "f")
