@@ -126,17 +126,20 @@ __device__ __forceinline__ void median_fill_tile(const float *__restrict__ in, f
 #pragma unroll
         for (int r = 0; r < 4; r++) {
             const int e = lane + 32 * r;  // window element (row i, column j), row-major like the reference
-            int q = -1;
+            int q = 0;
+            bool valid = false;
             if (e < kFillCells) {
                 const int xx = hx + e % kFillDiameter - kFillRadius, yy = y + e / kFillDiameter - kFillRadius;
                 if (xx >= 0 && xx < width && yy >= 0 && yy < height) {
                     const float d = img[yy * width + xx];
-                    if (depth_valid(d)) q = (int)(1000 * d + 0.5f);
+                    valid = depth_valid(d);
+                    if (valid) q = (int)(1000 * d + 0.5f);
                 }
             }
-            // (a valid depth can quantise to a non-positive value only if it is below 0.5 mm or negative; such entries stay
-            // in the ranking, exactly as in the reference's array)
-            alive[r] = q != -1;
+            // (a valid depth can quantise to a non-positive value only if it is below 0.5 mm or negative, -1 included;
+            // such entries stay in the ranking, exactly as in the reference's array: an entry counts by its depth's
+            // validity, not by its value)
+            alive[r] = valid;
             key[r] = (unsigned)q ^ 0x80000000u;
             n += __popc(__ballot_sync(kFull, alive[r]));
         }
