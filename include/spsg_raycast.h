@@ -194,7 +194,10 @@ SPSG_API int spsg_raycast_forward_loss(const spsg_raycast_params *p, int32_t *sp
 
 /* Fused backward of the 2D losses through the raycast: the upstream gradient images are never
  * materialised; each registered pixel's gradient is recomputed from (rendering, target, loss_out).
- * grad_scale: device scalar multiplying everything (d objective / d out[3]); NULL means 1. */
+ * grad_scale: device scalar multiplying everything (d objective / d out[3]); NULL means 1.
+ * The renderings must be those the matching spsg_raycast_forward_loss wrote, unmodified: the forward fills every pixel
+ * registered to a voxel with that voxel's colour and logits, so the backward reads them once per (voxel, view), from one
+ * of its pixels, and reads only the depth and the targets per pixel. */
 SPSG_API int spsg_raycast_backward_loss(const spsg_raycast_params *p, const float *image_color,
                                         const float *image_depth, const float *image_semantic,
                                         const spsg_loss_targets *t, const float *loss_out, const float *grad_scale,
@@ -218,7 +221,7 @@ typedef struct spsg_upstream_grads {   /* d objective / d rendering, same layout
  * Upstream gradients are not multiplied by grad_scale.  Gradients at pixels that hit nothing are ignored, as in
  * spsg_raycast_backward.  Loss targets switched off (NULL target pointers) give exactly spsg_raycast_backward of the
  * upstream images; upstream NULL, or all four planes NULL, gives exactly spsg_raycast_backward_loss.  The renderings must be
- * those of the matching spsg_raycast_forward_loss, unmodified. */
+ * those of the matching spsg_raycast_forward_loss, unmodified (see spsg_raycast_backward_loss). */
 SPSG_API int spsg_raycast_backward_loss_upstream(const spsg_raycast_params *p, const float *image_color,
                                                  const float *image_depth, const float *image_semantic,
                                                  const spsg_loss_targets *t, const float *loss_out,
