@@ -63,6 +63,16 @@ enum {
                                           fill and the index pass (only mapping3dto2d_num is reset)                          */
     SPSG_FLAG_DETERMINISTIC_GRADS = 1u << 4, /* backward, several views per chunk: add a voxel's per-view means in view order
                                                without float atomics (bit-reproducible; the gather takes ~30 % longer) */
+    SPSG_FLAG_DETERMINISTIC = 1u << 10, /* forward and backward: results that depend on nothing but the inputs.  Renderings and
+                                           mapping3dto2d_num are those of the flag off, bit for bit.  Each row r of
+                                           mapping3dto2d holds the min(num[r], P) SMALLEST pixel indices registered to it, in
+                                           ascending order (with num[r] > P a canonical subset: the reference keeps an
+                                           arbitrary P).  The loss block of spsg_raycast_forward_loss is summed in an order
+                                           fixed by pixel position.  The backward gathers the canonical tables; with several
+                                           views the flag implies SPSG_FLAG_DETERMINISTIC_GRADS.  No float atomics.  Pass it
+                                           to the forward and to its backward alike: spsg_workspace_bytes grows by the loss
+                                           partials (8 doubles per 4096 pixels of the batch) and always records the per-pixel
+                                           hits the tables are rebuilt from. */
     SPSG_FLAG_VIEW_NORMALS = 1u << 9    /* forward and backward, several views per chunk: one normal per (voxel, view).
                                            vals_normal is (N,F,3) voxel-major: row (v, f) is voxel v's normal as image
                                            chunk(v)*F + f sees it, and that image's normal rendering reads it (a row of
@@ -164,10 +174,12 @@ SPSG_API int spsg_raycast_forward_indexed(const spsg_raycast_params *p, int32_t 
  *    voxel v of grad_x[pixel].  Rows [0, N) of every d_* are fully written (zeros where nothing hit);
  *    rows >= N are left untouched (the reference zero-fills the whole buffer, Python only ever
  *    returns [:N], raycast_rgbd.py:42).  Per-voxel sums are accumulated in double precision and rounded once.  With one view
- *    per chunk (the reference's case) results are written with plain stores: no float atomics, gradients bit-identical from
- *    run to run.  With several views per chunk the per-view means are added with float atomics (last-bit differences between
- *    runs, like the reference's own atomics) unless SPSG_FLAG_DETERMINISTIC_GRADS is set, which adds them in view order with
- *    plain stores. */
+ *    per chunk (the reference's case) results are written with plain stores, no float atomics.  They are bit-identical from
+ *    run to run only when no row got more than max_pixels_per_voxel pixels: which pixels an overflowing row keeps depends on
+ *    which warp of the forward reached it first.  With several views per chunk the per-view means are added with float
+ *    atomics (last-bit differences between runs, like the reference's own atomics) unless SPSG_FLAG_DETERMINISTIC_GRADS is
+ *    set, which adds them in view order with plain stores.  With SPSG_FLAG_DETERMINISTIC (forward and backward) gradients
+ *    are always bit-identical from run to run. */
 SPSG_API int spsg_raycast_backward(const spsg_raycast_params *p, const float *grad_color, const float *grad_depth,
                                    const float *grad_normal, const float *grad_semantic,
                                    const int32_t *sparse_mapping, const int32_t *mapping3dto2d,
@@ -273,7 +285,15 @@ SPSG_API int spsg_losses2d_forward(const spsg_loss_targets *t, const float *imag
                                    const float *image_semantic, int64_t num_pixels, float *loss_out, void *scratch,
                                    size_t scratch_bytes, void *stream);
 
-/* Gradient images of grad_scale * loss_out[3] w.r.t. the renderings: d_color (P,3), d_depth (P), d_semantic (P,14), any
+/* spsg_losses2d_forward with the sums in an order fixed by pixel position (SPSG_FLAG_DETERMINISTIC): bit-identical
+ *    loss_out from run to run, whatever the device's SM count.  scratch: spsg_losses2d_deterministic_scratch_bytes(num_pixels)
+ *    bytes, 8-byte aligned. */
+SPSG_API size_t spsg_losses2d_deterministic_scratch_bytes(int64_t num_pixels);
+SPSG_API int spsg_losses2d_forward_deterministic(const spsg_loss_targets *t, const float *image_color,
+                                                 const float *image_depth, const float *image_semantic, int64_t num_pixels,
+                                                 float *loss_out, void *scratch, size_t scratch_bytes, void *stream);
+
+/* Gradient images of grad_scale * loss_out[3] w.r.t. the renderings (one thread per pixel, no atomics: deterministic): d_color (P,3), d_depth (P), d_semantic (P,14), any
  *    of them NULL to skip; pixels outside a term's valid set get 0. */
 SPSG_API int spsg_losses2d_backward(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
                                     const float *image_semantic, int64_t num_pixels, const float *loss_out,

@@ -20,6 +20,7 @@ SPSG_FLAG_GLOBAL_MAPS = 1 << 6
 SPSG_FLAG_INDEX_PREBUILT = 1 << 7
 SPSG_FLAG_PACKED_LOCS = 1 << 8
 SPSG_FLAG_VIEW_NORMALS = 1 << 9
+SPSG_FLAG_DETERMINISTIC = 1 << 10
 SPSG_LOSS_OUT_FLOATS = 8
 SPSG_DTYPE_F32 = 0
 SPSG_DTYPE_BF16 = 1
@@ -31,7 +32,8 @@ EXPORTS = (
     "spsg_raycast_forward_indexed", "spsg_raycast_backward", "spsg_raycast_occ", "spsg_raycast_forward_loss",
     "spsg_raycast_backward_loss", "spsg_raycast_backward_loss_upstream", "spsg_timing_enable", "spsg_timing_read",
     "spsg_normals_forward", "spsg_normals_backward", "spsg_normals_forward_views", "spsg_normals_backward_views",
-    "spsg_losses2d_forward", "spsg_losses2d_backward",
+    "spsg_losses2d_forward", "spsg_losses2d_backward", "spsg_losses2d_deterministic_scratch_bytes",
+    "spsg_losses2d_forward_deterministic",
     "spsg_depth_bilateral_filter", "spsg_depth_median_fill", "spsg_depth_to_cameraspace", "spsg_depth_to_normals",
     "spsg_depth_compute_normals",
     "spsg_sparsify_scratch_bytes", "spsg_sparsify_count", "spsg_sparsify_locs", "spsg_sparsify_locs_indexed",
@@ -133,6 +135,10 @@ def _load():
     lib.spsg_normals_backward_views.argtypes = [vp, i64, vp, vp, i32, vp, i32, i32, i32, i32, vp, vp, vp, vp]
     lib.spsg_losses2d_forward.restype = ctypes.c_int
     lib.spsg_losses2d_forward.argtypes = [lt, vp, vp, vp, i64, vp, vp, sz, vp]
+    lib.spsg_losses2d_deterministic_scratch_bytes.restype = sz
+    lib.spsg_losses2d_deterministic_scratch_bytes.argtypes = [i64]
+    lib.spsg_losses2d_forward_deterministic.restype = ctypes.c_int
+    lib.spsg_losses2d_forward_deterministic.argtypes = [lt, vp, vp, vp, i64, vp, vp, sz, vp]
     lib.spsg_losses2d_backward.restype = ctypes.c_int
     lib.spsg_losses2d_backward.argtypes = [lt, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp]
     f32 = ctypes.c_float

@@ -32,6 +32,11 @@ int fail_cuda(cudaError_t e, const char *where) {
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+constexpr int kDetLossPix = 4096;  // pixels per partial of the deterministic loss sums (spsg_deterministic.cuh)
+inline size_t det_loss_partials_bytes(long long num_pixels) {
+    return align_up((size_t)((num_pixels + kDetLossPix - 1) / kDetLossPix) * 8 * sizeof(double), 256);
+}
+
 // Optional per-kernel timing (bench.py's roofline leg): CUDA event pairs recorded on the launch stream around the
 // two dominant kernels.  Off by default; not usable during stream capture.
 struct EventPair { cudaEvent_t a, b; };
@@ -75,6 +80,7 @@ struct Layout {
     size_t loss_off, loss_bytes;    // double[kLossSlots][8] loss accumulators
     size_t list_off, list_bytes;    // int2 (voxel, image) per (voxel, view) pair that received a pixel
     size_t hits_off, hits_bytes;    // optional int32 per-pixel hit voxel
+    size_t det_off, det_bytes;      // SPSG_FLAG_DETERMINISTIC only: double[8] loss partials per kDetLossPix pixels
     size_t total;
 };
 
@@ -120,6 +126,11 @@ Layout make_layout(const spsg_raycast_params *p) {
     L.hits_off = off;
     L.hits_bytes = align_up((size_t)p->num_chunks * F * p->width * p->height * sizeof(int32_t), 256);
     off += L.hits_bytes;
+    L.det_off = off;
+    L.det_bytes = 0;
+    if (p->flags & SPSG_FLAG_DETERMINISTIC)
+        L.det_bytes = det_loss_partials_bytes((long long)p->num_chunks * F * p->width * p->height);
+    off += L.det_bytes;
     L.total = off;
     return L;
 }

@@ -18,8 +18,11 @@
 //   * rendered pixels are staged in shared memory and written with coalesced 128-bit stores;
 //   * the forward appends every (voxel, view) pair that received a pixel to a list, so the backward is one launch:
 //     a per-voxel gather over that list (no float atomics for one view per chunk, no 524288-block
-//     launch, no 164 MB memsets), optionally fused with the 2D losses.
+//     launch, no 164 MB memsets), optionally fused with the 2D losses;
+//   * SPSG_FLAG_DETERMINISTIC adds passes after the forward that make the voxel -> pixel tables and the loss sums
+//     independent of the schedule (spsg_deterministic.cuh).
 #include <cuda_runtime.h>
+#include <limits.h>
 #include <math_constants.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -40,6 +43,7 @@ namespace {
 #include "spsg_forward.cuh"
 #include "spsg_backward.cuh"
 #include "spsg_losses2d.cuh"
+#include "spsg_deterministic.cuh"
 #include "spsg_occ.cuh"
 #include "spsg_normals.cuh"
 
@@ -189,7 +193,9 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
     a.num_chunks = p->num_chunks;
     a.list_count = (int32_t *)(ws + L.head_off);
     a.list = (int2 *)(ws + L.list_off);
-    a.hits = (p->flags & SPSG_FLAG_RECORD_HITS) ? (int32_t *)(ws + L.hits_off) : nullptr;
+    // deterministic mode rebuilds overflowed tables from the per-pixel hits
+    const bool det = (p->flags & SPSG_FLAG_DETERMINISTIC) != 0;
+    a.hits = (p->flags & SPSG_FLAG_RECORD_HITS) || det ? (int32_t *)(ws + L.hits_off) : nullptr;
     a.width = p->width; a.height = p->height;
     a.depth_min = p->depth_min; a.depth_max = p->depth_max; a.thresh = p->thresh_sample_dist; a.inc = p->ray_increment;
     a.dimx = p->dimx; a.dimy = p->dimy; a.dimz = p->dimz;
@@ -256,7 +262,7 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
     do {                                                                                                          \
         if (view_normals) SPSG_LAUNCH_VN(L, M, true); else SPSG_LAUNCH_VN(L, M, false);                           \
     } while (0)
-        if (targets) {
+        if (targets && !det) {  // (deterministic mode sums the losses in a pass of its own, below)
             if (a.maps_in_smem) SPSG_LAUNCH(true, true); else SPSG_LAUNCH(true, false);
         } else {
             if (a.maps_in_smem) SPSG_LAUNCH(false, true); else SPSG_LAUNCH(false, false);
@@ -265,6 +271,34 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
 #undef SPSG_LAUNCH_VN
     }
     CUDA_TRY(cudaGetLastError());
+    if (det) {
+        // canonical tables: listed rows sorted, or reset and rebuilt from the hit records
+        CanonArgs c;
+        c.list_count = a.list_count; c.list = a.list; c.num = mapping3dto2d_num; c.map = mapping3dto2d; c.hits = a.hits;
+        c.max_pixels = p->max_pixels_per_voxel; c.views = p->views_per_chunk; c.num_locs = p->num_locs;
+        c.image_pixels = (unsigned)(p->width * p->height);
+        c.total_pixels = (long long)p->num_chunks * p->views_per_chunk * p->width * p->height;
+        if (p->num_locs > 0) {
+            const long long rows = p->num_locs * p->views_per_chunk;
+            canon_rows_kernel<<<(unsigned)std::min<long long>((rows + kCanonWarps - 1) / kCanonWarps, (long long)sms * 8),
+                                kCanonWarps * 32, 0, st>>>(c);
+            CUDA_TRY(cudaGetLastError());
+            canon_insert_kernel<<<(unsigned)std::min<long long>((c.total_pixels + 255) / 256, (long long)sms * 8), 256, 0, st>>>(c);
+            CUDA_TRY(cudaGetLastError());
+        }
+        if (targets) {
+            // the loss terms of the renderings just written, summed in pixel order
+            Losses2DArgs la;
+            memset(&la, 0, sizeof(la));
+            la.image_color = image_color; la.image_depth = image_depth; la.image_semantic = image_semantic;
+            la.num_pixels = c.total_pixels;
+            la.loss = a.loss;
+            la.loss.done = (int32_t *)(ws + L.head_off) + 32;  // zeroed header, apart from the forward kernel's counters
+            losses2d_det_kernel<<<(unsigned)((c.total_pixels + kDetLossPix - 1) / kDetLossPix), kDetLossThreads, 0, st>>>(
+                la, (double *)(ws + L.det_off));
+            CUDA_TRY(cudaGetLastError());
+        }
+    }
     return SPSG_OK;
 }
 
@@ -320,7 +354,8 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
     const unsigned gather_blocks = (unsigned)std::max<long long>(1, std::min<long long>((max_items + (32 / kGatherGroup) * kGatherWarps - 1) / ((32 / kGatherGroup) * kGatherWarps), (long long)sms * 8));
     const unsigned zero_blocks = (unsigned)std::min<long long>((p->num_locs + 255) / 256, (long long)sms * 4);
     const bool cleared = (p->flags & SPSG_FLAG_GRADS_CLEARED) != 0;  // the forward's fill pass cleared rows [0, N)
-    const bool multi = p->views_per_chunk > 1, exact = (p->flags & SPSG_FLAG_DETERMINISTIC_GRADS) != 0;
+    const bool multi = p->views_per_chunk > 1,
+               exact = (p->flags & (SPSG_FLAG_DETERMINISTIC_GRADS | SPSG_FLAG_DETERMINISTIC)) != 0;
     const bool view_normals = multi && (p->flags & SPSG_FLAG_VIEW_NORMALS);  // d_normal (N,F,3), one row per view
 #define SPSG_GATHER(FUSED, UP, VIEWS, VN, BLOCKS) backward_gather_kernel<FUSED, UP, VIEWS, VN><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a)
 #define SPSG_GATHER_VIEWS(VIEWS, VN, BLOCKS)                                                                      \
@@ -646,6 +681,45 @@ int spsg_losses2d_forward(const spsg_loss_targets *t, const float *image_color, 
     finalize_loss_kernel<<<1, 32, 0, st>>>((const double *)scratch, loss_out, t->weight_depth, t->weight_color_loss,
                                            t->weight_semantic, t->target_depth != nullptr, t->target_color != nullptr,
                                            t->target_label != nullptr);
+    CUDA_TRY(cudaGetLastError());
+    return SPSG_OK;
+}
+
+size_t spsg_losses2d_deterministic_scratch_bytes(int64_t num_pixels) {
+    if (num_pixels < 0) return 0;
+    return (size_t)kLossSlots * 8 * sizeof(double) + 256 + det_loss_partials_bytes(num_pixels);
+}
+
+int spsg_losses2d_forward_deterministic(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                                        const float *image_semantic, int64_t num_pixels, float *loss_out, void *scratch,
+                                        size_t scratch_bytes, void *stream) {
+    if (!t || !loss_out) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL loss targets / loss_out");
+    if (num_pixels < 0 || num_pixels * 14 >= (1ll << 32)) return fail(SPSG_ERR_INVALID_ARGUMENT, "bad pixel count");
+    if ((t->target_depth && !image_depth) || (t->target_color && !image_color) || (t->target_label && !image_semantic))
+        return fail(SPSG_ERR_INVALID_ARGUMENT, "a target is set but its rendering is NULL");
+    if (image_semantic && (reinterpret_cast<uintptr_t>(image_semantic) & 7u)) return fail(SPSG_ERR_INVALID_ARGUMENT, "image_semantic must be 8-byte aligned");
+    if (!scratch || scratch_bytes < spsg_losses2d_deterministic_scratch_bytes(num_pixels) ||
+        (reinterpret_cast<uintptr_t>(scratch) & 7u))
+        return fail(SPSG_ERR_WORKSPACE_TOO_SMALL, "scratch too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    // [slots of the final stage | done counter | per-block partials]
+    const size_t slots = (size_t)kLossSlots * 8 * sizeof(double);
+    CUDA_TRY(cudaMemsetAsync(scratch, 0, slots + 256, st));
+    Losses2DArgs a;
+    memset(&a, 0, sizeof(a));
+    a.image_color = image_color; a.image_depth = image_depth; a.image_semantic = image_semantic;
+    a.loss = make_loss_args(t, (double *)scratch);
+    a.loss.loss_out = loss_out;
+    a.loss.done = (int32_t *)((uint8_t *)scratch + slots);
+    a.num_pixels = num_pixels;
+    if (num_pixels > 0) {
+        losses2d_det_kernel<<<(unsigned)((num_pixels + kDetLossPix - 1) / kDetLossPix), kDetLossThreads, 0, st>>>(
+            a, (double *)((uint8_t *)scratch + slots + 256));
+    } else {
+        finalize_loss_kernel<<<1, 32, 0, st>>>((const double *)scratch, loss_out, t->weight_depth, t->weight_color_loss,
+                                               t->weight_semantic, t->target_depth != nullptr, t->target_color != nullptr,
+                                               t->target_label != nullptr);
+    }
     CUDA_TRY(cudaGetLastError());
     return SPSG_OK;
 }

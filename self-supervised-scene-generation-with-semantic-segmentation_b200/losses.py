@@ -89,7 +89,7 @@ def fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, v
         raise RuntimeError("raycaster buffers live on %s, inputs on %s" % (m.image_depth.device, dev))
     p = N.make_params(m.width, m.height, m.depth_min, m.depth_max, m.thresh_sample_dist, m.ray_increment,
                       m.dims3d[2], m.dims3d[1], m.dims3d[0], m.batch_size, views, m.mapping3dto2d.shape[1], n,
-                      m.flags | (N.SPSG_FLAG_VIEW_NORMALS if per_view else 0))
+                      rc.with_torch_mode(m.flags | (N.SPSG_FLAG_VIEW_NORMALS if per_view else 0)))
     if rc.is_packed_locs(locs):
         p.flags |= N.SPSG_FLAG_PACKED_LOCS
     target_depth, target_color, weight_color, target_label, class_weight, voxelsize, weights = targets
@@ -151,10 +151,14 @@ def fused_backward(m, p, tg, loss_out, grad_scale, grads_cleared, upstream=None)
     per-view normal rows of ``raycast_rgbd_cuda.normal_grad_buffer`` when ``p`` has SPSG_FLAG_VIEW_NORMALS).
     ``upstream`` = (grad_color, grad_depth, grad_normal, grad_semantic) gradient images of the renderings (any of them
     None; contiguous float32): ``spsg_raycast_backward_loss_upstream`` then adds them, unscaled, in the same gather.
-    ``grad_scale`` None means 1."""
-    if grads_cleared:
+    ``grad_scale`` None means 1.  Runs in the deterministic mode of this call (``m.flags`` or torch's switch): the
+    workspace check refuses a forward that ran in the other."""
+    det = rc.with_torch_mode(m.flags) & N.SPSG_FLAG_DETERMINISTIC
+    if grads_cleared or (p.flags & N.SPSG_FLAG_DETERMINISTIC) != det:
         p = type(p).from_buffer_copy(p)  # the caller's params stay as the forward left them
-        p.flags |= N.SPSG_FLAG_GRADS_CLEARED
+        p.flags = (p.flags & ~N.SPSG_FLAG_DETERMINISTIC) | det
+        if grads_cleared:
+            p.flags |= N.SPSG_FLAG_GRADS_CLEARED
     dev = m.image_depth.device
     if grad_scale is not None:
         rc._check_input(grad_scale, "grad_scale")
@@ -329,11 +333,14 @@ class _Losses2D(Function):
         tg = _targets_struct(1, 1, num_pixels, target_depth, target_color, weight_color, target_label, class_weight,
                              voxelsize, weights)
         loss_out = torch.empty(N.SPSG_LOSS_OUT_FLOATS, device=dev)
-        scratch = torch.empty(4096, dtype=torch.uint8, device=dev)
+        # deterministic algorithms: the sums in pixel order (per-block partials in a scratch that grows with the image)
+        det = torch.are_deterministic_algorithms_enabled()
+        forward = N.lib.spsg_losses2d_forward_deterministic if det else N.lib.spsg_losses2d_forward
+        scratch = torch.empty(N.lib.spsg_losses2d_deterministic_scratch_bytes(num_pixels) if det else 4096,
+                              dtype=torch.uint8, device=dev)
         with rc.device_guard(dev):
-            N.check(N.lib.spsg_losses2d_forward(ctypes.byref(tg), N.ptr(image_color), N.ptr(image_depth),
-                                                N.ptr(image_semantic), num_pixels, N.ptr(loss_out), N.ptr(scratch),
-                                                scratch.numel(), rc._stream(dev)))
+            N.check(forward(ctypes.byref(tg), N.ptr(image_color), N.ptr(image_depth), N.ptr(image_semantic), num_pixels,
+                            N.ptr(loss_out), N.ptr(scratch), scratch.numel(), rc._stream(dev)))
         ctx.targets, ctx.num_pixels, ctx.loss_out = tg, num_pixels, loss_out
         ctx.keep = (target_depth, target_color, weight_color, target_label, class_weight)
         ctx.save_for_backward(*[t for t in (image_color, image_depth, image_semantic) if t is not None])

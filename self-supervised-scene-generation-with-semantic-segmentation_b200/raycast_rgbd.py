@@ -14,6 +14,8 @@ Differences, all behind defaulted extras or unobservable through the reference A
     gradient is ``(N,F,3)``, view f's mean in row ``(v, f)``; ``(N,3)`` keeps the shared payload.
   * no host synchronisation: the reference reads ``locs[-1, -1]`` back to the host (raycast_rgbd.py:22,30).
   * the upstream ``RaycastOcc.forward`` NameError (``raycast_color_cuda``, raycast_rgbd.py:103) is fixed.
+  * deterministic mode: under ``torch.use_deterministic_algorithms(True)`` (or with SPSG_FLAG_DETERMINISTIC in ``flags``)
+    the voxel -> pixel tables are canonical and the gradients bit-reproducible; forward and backward must agree on it.
 """
 import torch
 from torch import nn
@@ -119,7 +121,9 @@ class RaycastRGBD(nn.Module):
         self.d_depth = torch.zeros(batch_size * max_num_locs_per_sample, 1, device=device)
         self.d_semantic = torch.zeros(batch_size * max_num_locs_per_sample, 14, device=device)
         self.d_normal_views = None  # (N*F,3) gradient rows of per-view normals (raycast_rgbd_cuda.normal_grad_buffer)
-        self.flags = 0  # SPSG_FLAG_* (e.g. _native.SPSG_FLAG_DETERMINISTIC_GRADS for bit-reproducible multi-view gradients)
+        # SPSG_FLAG_* (e.g. _native.SPSG_FLAG_DETERMINISTIC for bit-reproducible tables, losses and gradients; it is also on
+        # whenever torch.use_deterministic_algorithms(True) is)
+        self.flags = 0
         # scratch of the native calls (block maps, the backward's work list): owned by the module like the buffers above
         self.workspace = raycast_rgbd_cuda.ModuleWorkspace()
 

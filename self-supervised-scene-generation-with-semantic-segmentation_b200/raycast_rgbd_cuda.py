@@ -120,9 +120,17 @@ def normal_grad_buffer(m, per_view):
     return buf
 
 
+def with_torch_mode(flags):
+    """``flags`` plus SPSG_FLAG_DETERMINISTIC while ``torch.use_deterministic_algorithms(True)`` is in effect: every raycast
+    and 2D-loss call then gives results that depend on its inputs alone (canonical voxel -> pixel tables, loss sums in pixel
+    order, no float atomics).  Read at each call, forward and backward alike."""
+    return flags | N.SPSG_FLAG_DETERMINISTIC if torch.are_deterministic_algorithms_enabled() else flags
+
+
 def _stamp(p):
     return (int(p.num_locs), int(p.views_per_chunk), int(p.num_chunks), int(p.width), int(p.height),
-            int(p.max_pixels_per_voxel), bool(p.flags & N.SPSG_FLAG_VIEW_NORMALS))
+            int(p.max_pixels_per_voxel), bool(p.flags & N.SPSG_FLAG_VIEW_NORMALS),
+            "deterministic" if p.flags & N.SPSG_FLAG_DETERMINISTIC else "default")
 
 
 def workspace(device, nbytes, owner=None, stamp=None, expect=None):
@@ -255,7 +263,10 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
     reference-preserving defaults.  ``clear_grads`` = (d_color, d_depth, d_normals, d_semantic) lets the forward's fill
     pass clear the rows the matching ``backward(..., grads_cleared=True)`` will write (needs ``build_index=True``).
     ``flags`` with SPSG_FLAG_VIEW_NORMALS: ``vals_normals`` (and ``d_normals`` of ``clear_grads``) hold N*F rows.
-    ``workspace_owner`` = the calling module's ``ModuleWorkspace`` (else the scratch is looked up by ``sparse_mapping``)."""
+    ``workspace_owner`` = the calling module's ``ModuleWorkspace`` (else the scratch is looked up by ``sparse_mapping``).
+    Deterministic mode (SPSG_FLAG_DETERMINISTIC) is on when ``flags`` has it or torch's deterministic algorithms are enabled;
+    the matching ``backward`` must run in the same mode."""
+    flags = with_torch_mode(flags)
     for t, name in ((sparse_mapping, "sparse_mapping"), (imageColor, "imageColor"), (imageDepth, "imageDepth"),
                     (imageNormal, "imageNormal"), (imageSemantic, "imageSemantic"), (mapping3dto2d, "mapping3dto2d"),
                     (mapping3dto2d_num, "mapping3dto2d_num")):
@@ -321,7 +332,10 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
              flags=0):
     """Reference signature (``raycast_color_backward``, raycast_rgbd_cuda.cpp:102-140).
     ``dims`` = int32 CPU tensor (or sequence) [batch, Dx, Dy, Dz, N] (raycast_rgbd.py:30-31).  ``flags``: the forward's
-    SPSG_FLAG_DETERMINISTIC_GRADS and SPSG_FLAG_VIEW_NORMALS (``d_normals`` then holds N*F rows) are used."""
+    SPSG_FLAG_DETERMINISTIC_GRADS, SPSG_FLAG_VIEW_NORMALS (``d_normals`` then holds N*F rows) and SPSG_FLAG_DETERMINISTIC
+    are used; the last is also on under torch's deterministic algorithms, and a backward in another mode than its forward
+    raises RuntimeError."""
+    flags = with_torch_mode(flags)
     for t, name in ((grad_color, "grad_color"), (grad_depth, "grad_depth"), (grad_normal, "grad_normal"),
                     (grad_semantic, "grad_semantic"), (sparse_mapping, "sparse_mapping"),
                     (mapping3dto2d, "mapping3dto2d"), (mapping3dto2d_num, "mapping3dto2d_num"),
@@ -341,7 +355,7 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
                       num_chunks=sparse_mapping.shape[0], views_per_chunk=views_per_chunk,
                       max_pixels_per_voxel=mapping3dto2d.shape[1], num_locs=n,
                       flags=(N.SPSG_FLAG_GRADS_CLEARED if grads_cleared else 0) |
-                      (flags & (N.SPSG_FLAG_DETERMINISTIC_GRADS | N.SPSG_FLAG_VIEW_NORMALS)))
+                      (flags & (N.SPSG_FLAG_DETERMINISTIC_GRADS | N.SPSG_FLAG_VIEW_NORMALS | N.SPSG_FLAG_DETERMINISTIC)))
     dev = grad_color.device
     px = sparse_mapping.shape[0] * views_per_chunk * p.width * p.height
     if grad_depth.numel() < px or grad_color.numel() < 3 * px or grad_normal.numel() < 3 * px or grad_semantic.numel() < 14 * px:

@@ -123,9 +123,10 @@ def sparse_locs(sdf, truncation, empty=None, raycaster=None, counted=None):
         if raycaster is not None and _feeds(raycaster, sdf, n):
             m = raycaster
             # the workspace of the forward to come, sized for the most views the module renders (the brick sits at its start)
+            # and for the mode that forward will run in (deterministic mode needs more)
             p = N.make_params(m.width, m.height, m.depth_min, m.depth_max, m.thresh_sample_dist, m.ray_increment,
                               m.dims3d[2], m.dims3d[1], m.dims3d[0], m.batch_size, m.max_num_frames,
-                              m.mapping3dto2d.shape[1], n, 0)
+                              m.mapping3dto2d.shape[1], n, rc.with_torch_mode(m.flags) & N.SPSG_FLAG_DETERMINISTIC)
             ws = m.workspace.get(dev, N.workspace_bytes(p))
             indexed = N.lib.spsg_sparsify_locs_indexed_bf16 if bf16 else N.lib.spsg_sparsify_locs_indexed
             N.check(indexed(N.ptr(sdf), N.ptr(empty), B, dz, dy, dx, float(truncation),
