@@ -18,6 +18,7 @@
  *   image_color     f32 (I,H,W,3)   image_depth f32 (I,H,W)   image_normal f32 (I,H,W,3)
  *   image_semantic  f32 (I,H,W,14)                           miss == -inf in every channel
  *   mapping3dto2d   int32 (R,max_pixels_per_voxel)           mapping3dto2d_num int32 (R),  R >= F*N
+ *                   (mapping3dto2d: NULL allowed with SPSG_FLAG_ALL_PIXELS)
  *   d_color (N,3)   d_depth (N,1)   d_normal (N,3)   d_semantic (N,14)
  * with I = num_chunks * views_per_chunk images; image i renders chunk i / views_per_chunk
  * (reference style.py:9-16); views_per_chunk == 1 is exactly the reference.
@@ -73,7 +74,7 @@ enum {
                                            to the forward and to its backward alike: spsg_workspace_bytes grows by the loss
                                            partials (8 doubles per 4096 pixels of the batch) and always records the per-pixel
                                            hits the tables are rebuilt from. */
-    SPSG_FLAG_VIEW_NORMALS = 1u << 9    /* forward and backward, several views per chunk: one normal per (voxel, view).
+    SPSG_FLAG_VIEW_NORMALS = 1u << 9,   /* forward and backward, several views per chunk: one normal per (voxel, view).
                                            vals_normal is (N,F,3) voxel-major: row (v, f) is voxel v's normal as image
                                            chunk(v)*F + f sees it, and that image's normal rendering reads it (a row of
                                            zeros renders -inf, per row).  d_normal is (N,F,3): row (v, f) is the mean of
@@ -81,6 +82,20 @@ enum {
                                            forward's clear_grads->d_normal must hold N*F rows.  Colour, depth and semantic
                                            are unchanged.  With views_per_chunk == 1 the flag changes nothing.  Pass it
                                            to the forward and to its backward alike. */
+    SPSG_FLAG_ALL_PIXELS = 1u << 11     /* forward and backward: the gradient of row (v, f) is the mean over EVERY pixel of view f
+                                           whose hit voxel is v, not over the first max_pixels_per_voxel of them:
+                                               d_x[v] = sum_f (1 / num[f*N + v]) * sum over S(v, f) of grad_x[pixel]
+                                           with num = mapping3dto2d_num = |S(v, f)|.  No table is written or read:
+                                           mapping3dto2d may be NULL on every forward and backward entry point and
+                                           max_pixels_per_voxel is ignored.  Renderings, mapping3dto2d_num and loss_out are
+                                           those of the flag off, bit for bit.  The backward builds one segment of pixel
+                                           indices per (voxel, view) row from the forward's per-pixel hit records, then
+                                           gathers it.  Without SPSG_FLAG_DETERMINISTIC each row is summed in double in any
+                                           order and rounded once; with it every segment is summed in ascending pixel
+                                           order, the views' means are added in view order and no kernel uses float
+                                           atomics.  Composes with VIEW_NORMALS, DETERMINISTIC_GRADS, GRADS_CLEARED,
+                                           PACKED_LOCS, INDEX_PREBUILT and the fused losses.  Pass it to the forward and to
+                                           its backward alike; spsg_workspace_bytes grows as stated there. */
 };
 
 /* Replaces the reference's `opts` CPU tensor [W,H,depth_min,depth_max,thresh,ray_inc,Dx,Dy,Dz]
@@ -140,7 +155,10 @@ SPSG_API void spsg_timing_enable(int on);
 SPSG_API int spsg_timing_read(int which, double *total_ms, int *launches);
 
 /* Scratch shared by forward and backward of one call pair: dense SDF brick (4*B*Dz*Dy*Dx bytes), skip-level map,
- * hit-voxel list, loss accumulators, optional per-pixel hit records.  Must be 256-byte aligned. */
+ * hit-voxel list, loss accumulators, optional per-pixel hit records.  Must be 256-byte aligned.
+ * SPSG_FLAG_ALL_PIXELS adds, with R = F*N rows, X = B*F*W*H pixels and A(b) = b rounded up to a multiple of 256:
+ *     256 + A(4*R) + A(4*X)                        (counters, per-row segment ends, one int32 per rendered pixel)
+ *     + A(4*(floor(X / 65) + 1))                   (with SPSG_FLAG_DETERMINISTIC: the rows longer than 64 pixels) */
 SPSG_API size_t spsg_workspace_bytes(const spsg_raycast_params *p);
 
 /* == raycast_rgbd_cuda.construct_dense_sparse_mapping (raycast_rgbd_cuda.cpp:93-100,

@@ -21,6 +21,7 @@ SPSG_FLAG_INDEX_PREBUILT = 1 << 7
 SPSG_FLAG_PACKED_LOCS = 1 << 8
 SPSG_FLAG_VIEW_NORMALS = 1 << 9
 SPSG_FLAG_DETERMINISTIC = 1 << 10
+SPSG_FLAG_ALL_PIXELS = 1 << 11
 SPSG_LOSS_OUT_FLOATS = 8
 SPSG_DTYPE_F32 = 0
 SPSG_DTYPE_BF16 = 1

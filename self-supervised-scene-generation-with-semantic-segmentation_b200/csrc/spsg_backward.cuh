@@ -27,6 +27,12 @@ struct BackwardArgs {
     const float *up_color, *up_depth, *up_normal, *up_semantic;
 };
 
+// SPSG_FLAG_ALL_PIXELS (the gather's kSegments): row r's pixels are pix[end[r] - num[r], end[r]) (spsg_segments.cuh).  A
+// kernel parameter of its own, after BackwardArgs, so that the struct -- and every kernel that takes it -- keeps its layout.
+struct SegRows {
+    const int32_t *end, *pix;
+};
+
 // Clears the 21 gradient slots of voxels [0, N) (replaces the 4 whole-buffer memsets of kernel.cu:557-560): a warp
 // takes 32 consecutive voxels, so every store instruction writes one contiguous run of the AoS arrays.
 // kSkipHit (one view per chunk): rows of voxels that received pixels are left to the gather, which overwrites them.
@@ -276,11 +282,16 @@ constexpr int kGatherGroup = SPSG_GATHER_GROUP;  // lanes per (voxel, view) item
 // kUpstream (needs kFused): each pixel's row is the recomputed loss gradient plus the caller's upstream gradient images
 // kViewNormals (needs kViews != 0, SPSG_FLAG_VIEW_NORMALS): the normal channels of item (voxel, view) are that view's mean,
 // stored to row (voxel, view) of the (N,F,3) d_normal; the other channels are gathered as without it
-template <bool kFused, bool kUpstream, int kViews, bool kViewNormals>
+// kSegments (SPSG_FLAG_ALL_PIXELS): a row's pixels are its segment of seg_pix, all num[row] of them (no cap), instead of
+// the first min(num, max_pixels) entries of its mapping3dto2d row
+template <bool kFused, bool kUpstream, int kViews, bool kViewNormals, bool kSegments = false>
 #ifndef SPSG_GATHER_MIN_BLOCKS
 #define SPSG_GATHER_MIN_BLOCKS 8  // 32 registers: full occupancy hides the dependent gathers (the fused variants spill 24-92 B and are still faster)
 #endif
-__global__ void __launch_bounds__(kGatherWarps * 32, SPSG_GATHER_MIN_BLOCKS) backward_gather_kernel(const BackwardArgs a) {
+// kSegments: the row's segment start is one more dependent load; at 8 CTAs per SM (32 registers) that variant spills more
+// than the table variant of the same instantiation, at 5 (48 registers) less than it
+__global__ void __launch_bounds__(kGatherWarps * 32, kSegments ? 5 : SPSG_GATHER_MIN_BLOCKS) backward_gather_kernel(const BackwardArgs a,
+                                                                                                    const SegRows seg) {
     static_assert(kFused || !kUpstream, "upstream images are added to the fused variant's recomputed gradients");
     static_assert(kViews != 0 || !kViewNormals, "per-view normal rows need several views per chunk");
     if ((int)blockIdx.x < a.zero_blocks) {
@@ -327,9 +338,11 @@ __global__ void __launch_bounds__(kGatherWarps * 32, SPSG_GATHER_MIN_BLOCKS) bac
             for (int j = 0; j < kSlots; j++) tot[j] = 0.0f;
             for (int view = view0; view < (kViews == 2 ? a.views : view0 + 1); view++) {
                 const size_t row = (size_t)view * a.num_locs + idx;
-                const int32_t *prow = a.mapping3dto2d + row * a.max_pixels;
-                const int cnt = min(max(__ldg(a.mapping3dto2d_num + row), 0), a.max_pixels);  // kernel.cu:392-393
+                const int32_t *prow = kSegments ? seg.pix : a.mapping3dto2d + row * a.max_pixels;
+                const int num = max(__ldg(a.mapping3dto2d_num + row), 0);
+                const int cnt = kSegments ? num : min(num, a.max_pixels);  // kernel.cu:392-393
                 if (cnt == 0) continue;
+                if (kSegments) prow += __ldg(seg.end + row) - cnt;
                 const unsigned pixbase = (unsigned)(image0 + view) * P;  // global pixel index < 2^32 / 14 (check_params)
                 const float inv = __frcp_rn((float)cnt);
                 FusedItem it;

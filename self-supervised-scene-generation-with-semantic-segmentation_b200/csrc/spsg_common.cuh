@@ -33,6 +33,7 @@ int fail_cuda(cudaError_t e, const char *where) {
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 constexpr int kDetLossPix = 4096;  // pixels per partial of the deterministic loss sums (spsg_deterministic.cuh)
+constexpr int kSegWarpSort = 64;   // SPSG_FLAG_ALL_PIXELS + DETERMINISTIC: longest segment one warp sorts (spsg_segments.cuh)
 inline size_t det_loss_partials_bytes(long long num_pixels) {
     return align_up((size_t)((num_pixels + kDetLossPix - 1) / kDetLossPix) * 8 * sizeof(double), 256);
 }
@@ -81,6 +82,11 @@ struct Layout {
     size_t list_off, list_bytes;    // int2 (voxel, image) per (voxel, view) pair that received a pixel
     size_t hits_off, hits_bytes;    // optional int32 per-pixel hit voxel
     size_t det_off, det_bytes;      // SPSG_FLAG_DETERMINISTIC only: double[8] loss partials per kDetLossPix pixels
+    // SPSG_FLAG_ALL_PIXELS only (else 0 bytes): the backward's per-row pixel segments (spsg_segments.cuh)
+    size_t seg_head_off, seg_head_bytes;  // int32 counters: [0] segment allocator, [1] long rows
+    size_t seg_end_off, seg_end_bytes;    // int32 [F*N]: end of row r's segment in the entries
+    size_t seg_pix_off, seg_pix_bytes;    // int32 [B*F*W*H]: in-image pixel indices, one segment per listed row
+    size_t seg_long_off, seg_long_bytes;  // with SPSG_FLAG_DETERMINISTIC: work-list items of rows longer than a warp sorts
     size_t total;
 };
 
@@ -131,6 +137,21 @@ Layout make_layout(const spsg_raycast_params *p) {
     if (p->flags & SPSG_FLAG_DETERMINISTIC)
         L.det_bytes = det_loss_partials_bytes((long long)p->num_chunks * F * p->width * p->height);
     off += L.det_bytes;
+    const bool all = (p->flags & SPSG_FLAG_ALL_PIXELS) != 0;
+    const size_t rows = (size_t)(p->num_locs > 0 ? p->num_locs : 0) * F;
+    const size_t pixels = (size_t)p->num_chunks * F * p->width * p->height;
+    L.seg_head_off = off;
+    L.seg_head_bytes = all ? 256 : 0;
+    off += L.seg_head_bytes;
+    L.seg_end_off = off;
+    L.seg_end_bytes = all ? align_up(rows * sizeof(int32_t), 256) : 0;
+    off += L.seg_end_bytes;
+    L.seg_pix_off = off;
+    L.seg_pix_bytes = all ? align_up(pixels * sizeof(int32_t), 256) : 0;
+    off += L.seg_pix_bytes;
+    L.seg_long_off = off;
+    L.seg_long_bytes = all && (p->flags & SPSG_FLAG_DETERMINISTIC) ? align_up((pixels / (kSegWarpSort + 1) + 1) * sizeof(int32_t), 256) : 0;
+    off += L.seg_long_bytes;
     L.total = off;
     return L;
 }

@@ -20,7 +20,9 @@
 //     a per-voxel gather over that list (no float atomics for one view per chunk, no 524288-block
 //     launch, no 164 MB memsets), optionally fused with the 2D losses;
 //   * SPSG_FLAG_DETERMINISTIC adds passes after the forward that make the voxel -> pixel tables and the loss sums
-//     independent of the schedule (spsg_deterministic.cuh).
+//     independent of the schedule (spsg_deterministic.cuh);
+//   * SPSG_FLAG_ALL_PIXELS drops the fixed voxel -> pixel table: the backward gathers every pixel of a row from segments it
+//     builds out of the forward's per-pixel hit records (spsg_segments.cuh).
 #include <cuda_runtime.h>
 #include <limits.h>
 #include <math_constants.h>
@@ -44,6 +46,7 @@ namespace {
 #include "spsg_backward.cuh"
 #include "spsg_losses2d.cuh"
 #include "spsg_deterministic.cuh"
+#include "spsg_segments.cuh"
 #include "spsg_occ.cuh"
 #include "spsg_normals.cuh"
 
@@ -101,9 +104,10 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
                    int32_t *mapping3dto2d_num, const spsg_loss_targets *targets, float *loss_out,
                    const spsg_grad_buffers *clear_grads, void *workspace, size_t workspace_bytes, cudaStream_t st) {
     if (int rc = check_params(p)) return rc;
-    if (p->max_pixels_per_voxel <= 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "max_pixels_per_voxel must be positive");
+    const bool all = (p->flags & SPSG_FLAG_ALL_PIXELS) != 0;  // no table: the backward builds segments from the hits
+    if (!all && p->max_pixels_per_voxel <= 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "max_pixels_per_voxel must be positive");
     if (!sparse_mapping || !view_matrix || !intrinsics || !image_color || !image_depth || !image_normal ||
-        !image_semantic || !mapping3dto2d || !mapping3dto2d_num)
+        !image_semantic || (!all && !mapping3dto2d) || !mapping3dto2d_num)
         return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL tensor pointer");
     if (p->num_locs > 0 && (!locs || !vals_sdf || !vals_color || !vals_normal || !vals_semantic))
         return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL voxel tensor pointer");
@@ -187,7 +191,7 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
     a.view_matrix = view_matrix; a.intrinsics = intrinsics;
     a.image_color = image_color; a.image_depth = image_depth; a.image_normal = image_normal;
     a.image_semantic = image_semantic;
-    a.mapping3dto2d = mapping3dto2d; a.mapping3dto2d_num = mapping3dto2d_num;
+    a.mapping3dto2d = all ? nullptr : mapping3dto2d; a.mapping3dto2d_num = mapping3dto2d_num;
     a.dense = dense; a.vbits = vbits; a.bmap = bmap; a.vpc = L.vpc; a.bpc = L.bpc; a.wpr = L.wpr;
     a.tile_counter = (int32_t *)(ws + L.tiles_off);
     a.num_chunks = p->num_chunks;
@@ -195,7 +199,7 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
     a.list = (int2 *)(ws + L.list_off);
     // deterministic mode rebuilds overflowed tables from the per-pixel hits
     const bool det = (p->flags & SPSG_FLAG_DETERMINISTIC) != 0;
-    a.hits = (p->flags & SPSG_FLAG_RECORD_HITS) || det ? (int32_t *)(ws + L.hits_off) : nullptr;
+    a.hits = (p->flags & SPSG_FLAG_RECORD_HITS) || det || all ? (int32_t *)(ws + L.hits_off) : nullptr;
     a.width = p->width; a.height = p->height;
     a.depth_min = p->depth_min; a.depth_max = p->depth_max; a.thresh = p->thresh_sample_dist; a.inc = p->ray_increment;
     a.dimx = p->dimx; a.dimy = p->dimy; a.dimz = p->dimz;
@@ -204,7 +208,7 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
         a.vx = maps ? p->dimx - 1 : 0; a.vy = maps ? p->dimy - 1 : 0; a.vz = maps ? p->dimz - 1 : 0;
     }
     a.nbx = L.nbx; a.nby = L.nby; a.nbz = L.nbz;
-    a.views = p->views_per_chunk; a.max_pixels = p->max_pixels_per_voxel;
+    a.views = p->views_per_chunk; a.max_pixels = all ? 0 : p->max_pixels_per_voxel;  // 0: the kernel writes no table entry
     a.num_locs = p->num_locs;
     a.flags = p->flags;
     a.vec_ok = (p->width % 4 == 0) && aligned16(image_color) && aligned16(image_depth) && aligned16(image_normal) &&
@@ -278,7 +282,7 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
         c.max_pixels = p->max_pixels_per_voxel; c.views = p->views_per_chunk; c.num_locs = p->num_locs;
         c.image_pixels = (unsigned)(p->width * p->height);
         c.total_pixels = (long long)p->num_chunks * p->views_per_chunk * p->width * p->height;
-        if (p->num_locs > 0) {
+        if (p->num_locs > 0 && !all) {
             const long long rows = p->num_locs * p->views_per_chunk;
             canon_rows_kernel<<<(unsigned)std::min<long long>((rows + kCanonWarps - 1) / kCanonWarps, (long long)sms * 8),
                                 kCanonWarps * 32, 0, st>>>(c);
@@ -309,8 +313,9 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
                     float *d_normal, float *d_semantic, void *workspace, size_t workspace_bytes, cudaStream_t st,
                     const spsg_upstream_grads *upstream = nullptr) {
     if (int rc = check_params(p)) return rc;
+    const bool all = (p->flags & SPSG_FLAG_ALL_PIXELS) != 0;  // rows gathered from segments built here, not from a table
     if (!g_or_img_color || !g_or_img_depth || !g_or_img_semantic || (!fused && !grad_normal) || !sparse_mapping ||
-        !mapping3dto2d || !mapping3dto2d_num)
+        (!all && !mapping3dto2d) || !mapping3dto2d_num)
         return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL tensor pointer");
     if (fused && (!targets || !loss_out)) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL loss targets");
     // upstream images (fused only): any plane may be NULL; none at all is exactly the fused backward without them
@@ -318,7 +323,7 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
                     (upstream->grad_color || upstream->grad_depth || upstream->grad_normal || upstream->grad_semantic);
     if (up && (reinterpret_cast<uintptr_t>(upstream->grad_semantic) & 7u))
         return fail(SPSG_ERR_INVALID_ARGUMENT, "upstream grad_semantic must be 8-byte aligned");
-    if (p->max_pixels_per_voxel <= 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "max_pixels_per_voxel must be positive");
+    if (!all && p->max_pixels_per_voxel <= 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "max_pixels_per_voxel must be positive");
     if (p->num_locs == 0) return SPSG_OK;
     if (!d_color || !d_depth || !d_normal || !d_semantic) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL gradient pointer");
     if (reinterpret_cast<uintptr_t>(d_semantic) & 7u) return fail(SPSG_ERR_INVALID_ARGUMENT, "d_semantic must be 8-byte aligned");
@@ -357,7 +362,39 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
     const bool multi = p->views_per_chunk > 1,
                exact = (p->flags & (SPSG_FLAG_DETERMINISTIC_GRADS | SPSG_FLAG_DETERMINISTIC)) != 0;
     const bool view_normals = multi && (p->flags & SPSG_FLAG_VIEW_NORMALS);  // d_normal (N,F,3), one row per view
-#define SPSG_GATHER(FUSED, UP, VIEWS, VN, BLOCKS) backward_gather_kernel<FUSED, UP, VIEWS, VN><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a)
+    SegRows seg = {nullptr, nullptr};
+    if (all) {
+        // this call's segments, rebuilt from the forward's work list and hit records (a second backward rebuilds them
+        // alike); the sort passes only with SPSG_FLAG_DETERMINISTIC
+        const bool sorted = (p->flags & SPSG_FLAG_DETERMINISTIC) != 0;
+        SegArgs sa;
+        sa.list_count = a.list_count; sa.list = a.list; sa.num = mapping3dto2d_num;
+        sa.hits = (const int32_t *)(ws + L.hits_off);
+        sa.seg_end = (int32_t *)(ws + L.seg_end_off); sa.seg_pix = (int32_t *)(ws + L.seg_pix_off);
+        sa.counters = (int32_t *)(ws + L.seg_head_off);
+        sa.long_items = sorted ? (int32_t *)(ws + L.seg_long_off) : nullptr;
+        sa.views = p->views_per_chunk; sa.num_locs = p->num_locs;
+        sa.image_pixels = (unsigned)(p->width * p->height);
+        sa.total_pixels = (long long)p->num_chunks * p->views_per_chunk * p->width * p->height;
+        const long long rows = p->num_locs * p->views_per_chunk;
+        CUDA_TRY(cudaMemsetAsync(sa.counters, 0, L.seg_head_bytes, st));
+        seg_alloc_kernel<<<(unsigned)std::min<long long>((rows + 255) / 256, (long long)sms * 8), 256, 0, st>>>(sa);
+        CUDA_TRY(cudaGetLastError());
+        seg_scatter_kernel<<<(unsigned)std::min<long long>((sa.total_pixels + 255) / 256, (long long)sms * 8), 256, 0, st>>>(sa);
+        CUDA_TRY(cudaGetLastError());
+        if (sorted) {
+            seg_sort_warp_kernel<<<(unsigned)std::min<long long>((rows + 7) / 8, (long long)sms * 8), 256, 0, st>>>(sa);
+            CUDA_TRY(cudaGetLastError());
+            seg_sort_long_kernel<<<(unsigned)sms * 2, kSegThreads, 0, st>>>(sa);
+            CUDA_TRY(cudaGetLastError());
+        }
+        seg.end = sa.seg_end; seg.pix = sa.seg_pix;
+    }
+#define SPSG_GATHER(FUSED, UP, VIEWS, VN, BLOCKS)                                                                     \
+    do {                                                                                                              \
+        if (all) backward_gather_kernel<FUSED, UP, VIEWS, VN, true><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a, seg);  \
+        else backward_gather_kernel<FUSED, UP, VIEWS, VN><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a, seg);            \
+    } while (0)
 #define SPSG_GATHER_VIEWS(VIEWS, VN, BLOCKS)                                                                      \
     do {                                                                                                          \
         if (up) SPSG_GATHER(true, true, VIEWS, VN, BLOCKS);                                                       \

@@ -78,8 +78,10 @@ def fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, v
     per_view = rc.view_normals(vals_normals, views)
     n = rc.check_voxel_inputs(locs, vals_sdf, vals_colors, vals_normals, vals_semantic, view_matrix, intrinsic_params,
                               images, views if per_view else 1)
-    if n * views > m.mapping3dto2d.shape[0]:
-        raise RuntimeError("too many voxels for raycast (%d x %d views > %d rows)" % (n, views, m.mapping3dto2d.shape[0]))
+    flags = rc.with_torch_mode(m.flags | (N.SPSG_FLAG_VIEW_NORMALS if per_view else 0))
+    rows, max_pixels = rc.table_shape(m.mapping3dto2d, m.mapping3dto2d_num, flags)
+    if n * views > rows:
+        raise RuntimeError("too many voxels for raycast (%d x %d views > %d rows)" % (n, views, rows))
     d_normal = rc.normal_grad_buffer(m, per_view)
     if clear_grads and (m.d_depth.shape[0] < n or m.d_color.shape[0] < n or
                         d_normal.shape[0] < n * (views if per_view else 1) or m.d_semantic.shape[0] < n):
@@ -88,8 +90,7 @@ def fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, v
     if m.image_depth.device != dev:
         raise RuntimeError("raycaster buffers live on %s, inputs on %s" % (m.image_depth.device, dev))
     p = N.make_params(m.width, m.height, m.depth_min, m.depth_max, m.thresh_sample_dist, m.ray_increment,
-                      m.dims3d[2], m.dims3d[1], m.dims3d[0], m.batch_size, views, m.mapping3dto2d.shape[1], n,
-                      rc.with_torch_mode(m.flags | (N.SPSG_FLAG_VIEW_NORMALS if per_view else 0)))
+                      m.dims3d[2], m.dims3d[1], m.dims3d[0], m.batch_size, views, max_pixels, n, flags)
     if rc.is_packed_locs(locs):
         p.flags |= N.SPSG_FLAG_PACKED_LOCS
     target_depth, target_color, weight_color, target_label, class_weight, voxelsize, weights = targets
@@ -108,7 +109,7 @@ def fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, v
             ctypes.byref(p), N.ptr(m.sparse_mapping), N.ptr(locs), N.ptr(vals_sdf), N.ptr(vals_colors),
             N.ptr(vals_normals), N.ptr(vals_semantic), N.ptr(view_matrix), N.ptr(intrinsic_params),
             N.ptr(m.image_color), N.ptr(m.image_depth), N.ptr(m.image_normal), N.ptr(m.image_semantic),
-            N.ptr(m.mapping3dto2d), N.ptr(m.mapping3dto2d_num), ctypes.byref(tg), N.ptr(loss_out),
+            rc.table_ptr(m.mapping3dto2d, p.flags), N.ptr(m.mapping3dto2d_num), ctypes.byref(tg), N.ptr(loss_out),
             ctypes.byref(gb) if gb is not None else None, N.ptr(ws), ws.numel(), rc._stream(dev)))
         owner.filled(p)
         if prebuilt:
@@ -151,12 +152,13 @@ def fused_backward(m, p, tg, loss_out, grad_scale, grads_cleared, upstream=None)
     per-view normal rows of ``raycast_rgbd_cuda.normal_grad_buffer`` when ``p`` has SPSG_FLAG_VIEW_NORMALS).
     ``upstream`` = (grad_color, grad_depth, grad_normal, grad_semantic) gradient images of the renderings (any of them
     None; contiguous float32): ``spsg_raycast_backward_loss_upstream`` then adds them, unscaled, in the same gather.
-    ``grad_scale`` None means 1.  Runs in the deterministic mode of this call (``m.flags`` or torch's switch): the
-    workspace check refuses a forward that ran in the other."""
-    det = rc.with_torch_mode(m.flags) & N.SPSG_FLAG_DETERMINISTIC
-    if grads_cleared or (p.flags & N.SPSG_FLAG_DETERMINISTIC) != det:
+    ``grad_scale`` None means 1.  Runs in the deterministic mode of this call (``m.flags`` or torch's switch) and the
+    all-pixels mode of ``m.flags``: the workspace check refuses a forward that ran in another."""
+    modes = N.SPSG_FLAG_DETERMINISTIC | N.SPSG_FLAG_ALL_PIXELS
+    mode = rc.with_torch_mode(m.flags) & modes
+    if grads_cleared or (p.flags & modes) != mode:
         p = type(p).from_buffer_copy(p)  # the caller's params stay as the forward left them
-        p.flags = (p.flags & ~N.SPSG_FLAG_DETERMINISTIC) | det
+        p.flags = (p.flags & ~modes) | mode
         if grads_cleared:
             p.flags |= N.SPSG_FLAG_GRADS_CLEARED
     dev = m.image_depth.device
@@ -171,14 +173,14 @@ def fused_backward(m, p, tg, loss_out, grad_scale, grads_cleared, upstream=None)
         if up is None:
             N.check(N.lib.spsg_raycast_backward_loss(
                 ctypes.byref(p), N.ptr(m.image_color), N.ptr(m.image_depth), N.ptr(m.image_semantic),
-                ctypes.byref(tg), N.ptr(loss_out), N.ptr(grad_scale), N.ptr(m.sparse_mapping), N.ptr(m.mapping3dto2d),
-                N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth), N.ptr(d_normal), N.ptr(m.d_semantic),
+                ctypes.byref(tg), N.ptr(loss_out), N.ptr(grad_scale), N.ptr(m.sparse_mapping),
+                rc.table_ptr(m.mapping3dto2d, p.flags), N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth), N.ptr(d_normal), N.ptr(m.d_semantic),
                 N.ptr(ws), ws.numel(), rc._stream(dev)))
         else:
             N.check(N.lib.spsg_raycast_backward_loss_upstream(
                 ctypes.byref(p), N.ptr(m.image_color), N.ptr(m.image_depth), N.ptr(m.image_semantic),
                 ctypes.byref(tg), N.ptr(loss_out), N.ptr(grad_scale), ctypes.byref(up), N.ptr(m.sparse_mapping),
-                N.ptr(m.mapping3dto2d), N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth),
+                rc.table_ptr(m.mapping3dto2d, p.flags), N.ptr(m.mapping3dto2d_num), N.ptr(m.d_color), N.ptr(m.d_depth),
                 N.ptr(d_normal), N.ptr(m.d_semantic), N.ptr(ws), ws.numel(), rc._stream(dev)))
 
 

@@ -16,6 +16,8 @@ Differences, all behind defaulted extras or unobservable through the reference A
   * the upstream ``RaycastOcc.forward`` NameError (``raycast_color_cuda``, raycast_rgbd.py:103) is fixed.
   * deterministic mode: under ``torch.use_deterministic_algorithms(True)`` (or with SPSG_FLAG_DETERMINISTIC in ``flags``)
     the voxel -> pixel tables are canonical and the gradients bit-reproducible; forward and backward must agree on it.
+  * ``max_pixels_per_voxel=None``: the gradient of a (voxel, view) is the mean over every pixel it received, not over the
+    first ``max_pixels_per_voxel`` (SPSG_FLAG_ALL_PIXELS in ``flags``); no ``mapping3dto2d`` table is allocated.
 """
 import torch
 from torch import nn
@@ -31,9 +33,11 @@ class RayCastRGBDFunction(Function):
                 dims3d, width, height, depth_min, depth_max, thresh_sample_dist, ray_increment, image_color,
                 image_depth, image_normal, image_semantic, sparse_mapping, mapping3dto2d, mapping3dto2d_num, d_color,
                 d_depth, d_normal, d_semantic, views_per_chunk=1, flags=0, workspace_owner=None):
-        if locs.shape[0] * views_per_chunk > mapping3dto2d.shape[0]:  # raycast_rgbd.py:16-21
-            print('ERROR: locs size %s vs mapping3dto2d size %s' % (str(locs.shape), str(mapping3dto2d.shape)))
-            keep = mapping3dto2d.shape[0] // views_per_chunk
+        rows = raycast_rgbd_cuda.table_shape(mapping3dto2d, mapping3dto2d_num, flags)[0]
+        if locs.shape[0] * views_per_chunk > rows:  # raycast_rgbd.py:16-21
+            print('ERROR: locs size %s vs mapping3dto2d size %s' % (str(locs.shape), str(mapping3dto2d_num.shape if
+                  raycast_rgbd_cuda.all_pixels(flags) else mapping3dto2d.shape)))
+            keep = rows // views_per_chunk
             locs = locs[:keep]
             vals_sdf = vals_sdf[:keep]
             vals_colors = vals_colors[:keep]
@@ -113,7 +117,9 @@ class RaycastRGBD(nn.Module):
         self.image_normal = torch.zeros(images, height, width, 3, device=device)
         self.image_color = torch.zeros(images, height, width, 3, device=device)
         self.image_semantic = torch.zeros(images, height, width, 14, device=device)
-        self.mapping3dto2d = torch.zeros(rows, max_pixels_per_voxel, dtype=torch.int, device=device)
+        # max_pixels_per_voxel=None: every pixel of a (voxel, view) enters its gradient (SPSG_FLAG_ALL_PIXELS), no table
+        self.mapping3dto2d = torch.zeros(rows, max_pixels_per_voxel, dtype=torch.int, device=device) \
+            if max_pixels_per_voxel is not None else torch.empty(0, dtype=torch.int, device=device)
         self.mapping3dto2d_num = torch.zeros(rows, dtype=torch.int, device=device)
         self.sparse_mapping = torch.zeros(batch_size, dims3d[0], dims3d[1], dims3d[2], dtype=torch.int, device=device)
         self.d_color = torch.zeros(batch_size * max_num_locs_per_sample, 3, device=device)
@@ -122,8 +128,9 @@ class RaycastRGBD(nn.Module):
         self.d_semantic = torch.zeros(batch_size * max_num_locs_per_sample, 14, device=device)
         self.d_normal_views = None  # (N*F,3) gradient rows of per-view normals (raycast_rgbd_cuda.normal_grad_buffer)
         # SPSG_FLAG_* (e.g. _native.SPSG_FLAG_DETERMINISTIC for bit-reproducible tables, losses and gradients; it is also on
-        # whenever torch.use_deterministic_algorithms(True) is)
-        self.flags = 0
+        # whenever torch.use_deterministic_algorithms(True) is).  SPSG_FLAG_ALL_PIXELS marks the module without a table:
+        # keep it when adding flags (``m.flags |= ...``)
+        self.flags = N.SPSG_FLAG_ALL_PIXELS if max_pixels_per_voxel is None else 0
         # scratch of the native calls (block maps, the backward's work list): owned by the module like the buffers above
         self.workspace = raycast_rgbd_cuda.ModuleWorkspace()
 

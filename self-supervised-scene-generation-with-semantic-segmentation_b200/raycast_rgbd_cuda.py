@@ -127,10 +127,33 @@ def with_torch_mode(flags):
     return flags | N.SPSG_FLAG_DETERMINISTIC if torch.are_deterministic_algorithms_enabled() else flags
 
 
+def all_pixels(flags):
+    """SPSG_FLAG_ALL_PIXELS: the gradient of a (voxel, view) row is the mean over every pixel registered to it, and no
+    ``mapping3dto2d`` table is used (``RaycastRGBD(..., max_pixels_per_voxel=None)``)."""
+    return bool(flags & N.SPSG_FLAG_ALL_PIXELS)
+
+
+def table_shape(mapping3dto2d, mapping3dto2d_num, flags):
+    """(rows, max_pixels_per_voxel) of a raycaster's registration buffers: the table's, or in the all-pixels mode the
+    counters' rows and 0 (the table may then be None or empty)."""
+    if all_pixels(flags):
+        return mapping3dto2d_num.shape[0], 0
+    if mapping3dto2d is None or mapping3dto2d.dim() != 2:
+        raise RuntimeError("mapping3dto2d must be a (rows, max_pixels_per_voxel) table (only SPSG_FLAG_ALL_PIXELS, i.e. "
+                           "RaycastRGBD(..., max_pixels_per_voxel=None), runs without one)")
+    return mapping3dto2d.shape[0], mapping3dto2d.shape[1]
+
+
+def table_ptr(mapping3dto2d, flags):
+    """Device pointer of the table, NULL in the all-pixels mode."""
+    return None if all_pixels(flags) else N.ptr(mapping3dto2d)
+
+
 def _stamp(p):
     return (int(p.num_locs), int(p.views_per_chunk), int(p.num_chunks), int(p.width), int(p.height),
             int(p.max_pixels_per_voxel), bool(p.flags & N.SPSG_FLAG_VIEW_NORMALS),
-            "deterministic" if p.flags & N.SPSG_FLAG_DETERMINISTIC else "default")
+            "deterministic" if p.flags & N.SPSG_FLAG_DETERMINISTIC else "default",
+            "all pixels" if p.flags & N.SPSG_FLAG_ALL_PIXELS else "table")
 
 
 def workspace(device, nbytes, owner=None, stamp=None, expect=None):
@@ -248,12 +271,12 @@ def construct_dense_sparse_mapping(locs, sparse_mapping):
                                        _stream(sparse_mapping.device)))
 
 
-def _forward_params(sparse_mapping, locs, mapping3dto2d, opts, views_per_chunk=1, flags=0):
+def _forward_params(sparse_mapping, locs, max_pixels, opts, views_per_chunk=1, flags=0):
     o = opts.tolist() if isinstance(opts, torch.Tensor) else list(opts)
     return N.make_params(width=_opt_int(o[0]), height=_opt_int(o[1]), depth_min=o[2], depth_max=o[3],
                          thresh_sample_dist=o[4], ray_increment=o[5], dimx=_opt_int(o[6]), dimy=_opt_int(o[7]),
                          dimz=_opt_int(o[8]), num_chunks=sparse_mapping.shape[0], views_per_chunk=views_per_chunk,
-                         max_pixels_per_voxel=mapping3dto2d.shape[1], num_locs=locs.shape[0], flags=flags)
+                         max_pixels_per_voxel=max_pixels, num_locs=locs.shape[0], flags=flags)
 
 
 def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_semantic, viewMatrixInv, imageColor,
@@ -265,19 +288,23 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
     ``flags`` with SPSG_FLAG_VIEW_NORMALS: ``vals_normals`` (and ``d_normals`` of ``clear_grads``) hold N*F rows.
     ``workspace_owner`` = the calling module's ``ModuleWorkspace`` (else the scratch is looked up by ``sparse_mapping``).
     Deterministic mode (SPSG_FLAG_DETERMINISTIC) is on when ``flags`` has it or torch's deterministic algorithms are enabled;
-    the matching ``backward`` must run in the same mode."""
+    the matching ``backward`` must run in the same mode.  With SPSG_FLAG_ALL_PIXELS in ``flags`` no table is written:
+    ``mapping3dto2d`` may be None or empty, and the backward (same flag) averages every pixel of a row."""
     flags = with_torch_mode(flags)
+    table = () if all_pixels(flags) else ((mapping3dto2d, "mapping3dto2d"),)
     for t, name in ((sparse_mapping, "sparse_mapping"), (imageColor, "imageColor"), (imageDepth, "imageDepth"),
-                    (imageNormal, "imageNormal"), (imageSemantic, "imageSemantic"), (mapping3dto2d, "mapping3dto2d"),
-                    (mapping3dto2d_num, "mapping3dto2d_num")):
+                    (imageNormal, "imageNormal"), (imageSemantic, "imageSemantic")) + table + \
+            ((mapping3dto2d_num, "mapping3dto2d_num"),):
         _check_input(t, name)
     _check_dtype(sparse_mapping, torch.int32, "sparse_mapping")
-    _check_dtype(mapping3dto2d, torch.int32, "mapping3dto2d")
+    if table:
+        _check_dtype(mapping3dto2d, torch.int32, "mapping3dto2d")
     _check_dtype(mapping3dto2d_num, torch.int32, "mapping3dto2d_num")
     for t, name in ((imageColor, "imageColor"), (imageDepth, "imageDepth"), (imageNormal, "imageNormal"),
                     (imageSemantic, "imageSemantic")):
         _check_dtype(t, torch.float32, name)
-    p = _forward_params(sparse_mapping, locs, mapping3dto2d, opts, views_per_chunk, flags)
+    rows, max_pixels = table_shape(mapping3dto2d, mapping3dto2d_num, flags)
+    p = _forward_params(sparse_mapping, locs, max_pixels, opts, views_per_chunk, flags)
     if is_packed_locs(locs):
         if not build_index:
             raise RuntimeError("packed locs need build_index=True")
@@ -286,9 +313,8 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
     nv = p.views_per_chunk if flags & N.SPSG_FLAG_VIEW_NORMALS else 1
     n = check_voxel_inputs(locs, vals_sdf, vals_color, vals_normals, vals_semantic, viewMatrixInv, intrinsicParams, images,
                            nv)
-    if mapping3dto2d_num.numel() < p.views_per_chunk * n or mapping3dto2d.shape[0] < p.views_per_chunk * n:
-        raise RuntimeError("mapping3dto2d has %d rows, needs views_per_chunk*N = %d" %
-                           (mapping3dto2d.shape[0], p.views_per_chunk * n))
+    if mapping3dto2d_num.numel() < p.views_per_chunk * n or rows < p.views_per_chunk * n:
+        raise RuntimeError("mapping3dto2d has %d rows, needs views_per_chunk*N = %d" % (rows, p.views_per_chunk * n))
     px = images * p.width * p.height
     if imageDepth.numel() < px or imageColor.numel() < 3 * px or imageNormal.numel() < 3 * px or \
             imageSemantic.numel() < 14 * px:
@@ -305,7 +331,7 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
         args = (ctypes.byref(p), N.ptr(sparse_mapping), N.ptr(locs), N.ptr(vals_sdf), N.ptr(vals_color),
                 N.ptr(vals_normals), N.ptr(vals_semantic), N.ptr(viewMatrixInv), N.ptr(intrinsicParams),
                 N.ptr(imageColor), N.ptr(imageDepth), N.ptr(imageNormal), N.ptr(imageSemantic),
-                N.ptr(mapping3dto2d), N.ptr(mapping3dto2d_num))
+                table_ptr(mapping3dto2d, flags), N.ptr(mapping3dto2d_num))
         if build_index:
             gb = None
             if clear_grads is not None:
@@ -334,12 +360,13 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
     ``dims`` = int32 CPU tensor (or sequence) [batch, Dx, Dy, Dz, N] (raycast_rgbd.py:30-31).  ``flags``: the forward's
     SPSG_FLAG_DETERMINISTIC_GRADS, SPSG_FLAG_VIEW_NORMALS (``d_normals`` then holds N*F rows) and SPSG_FLAG_DETERMINISTIC
     are used; the last is also on under torch's deterministic algorithms, and a backward in another mode than its forward
-    raises RuntimeError."""
+    raises RuntimeError.  SPSG_FLAG_ALL_PIXELS (as in the forward): ``mapping3dto2d`` may be None or empty."""
     flags = with_torch_mode(flags)
+    table = () if all_pixels(flags) else ((mapping3dto2d, "mapping3dto2d"),)
     for t, name in ((grad_color, "grad_color"), (grad_depth, "grad_depth"), (grad_normal, "grad_normal"),
-                    (grad_semantic, "grad_semantic"), (sparse_mapping, "sparse_mapping"),
-                    (mapping3dto2d, "mapping3dto2d"), (mapping3dto2d_num, "mapping3dto2d_num"),
-                    (d_color, "d_color"), (d_depth, "d_depth"), (d_normals, "d_normals"), (d_semantic, "d_semantic")):
+                    (grad_semantic, "grad_semantic"), (sparse_mapping, "sparse_mapping")) + table + \
+            ((mapping3dto2d_num, "mapping3dto2d_num"), (d_color, "d_color"), (d_depth, "d_depth"),
+             (d_normals, "d_normals"), (d_semantic, "d_semantic")):
         _check_input(t, name)
     for t, name in ((grad_color, "grad_color"), (grad_depth, "grad_depth"), (grad_normal, "grad_normal"),
                     (grad_semantic, "grad_semantic"), (d_color, "d_color"), (d_depth, "d_depth"), (d_normals, "d_normals"),
@@ -353,9 +380,11 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
     p = N.make_params(width=grad_color.shape[2], height=grad_color.shape[1], depth_min=0, depth_max=0,
                       thresh_sample_dist=0, ray_increment=0, dimx=int(d[1]), dimy=int(d[2]), dimz=int(d[3]),
                       num_chunks=sparse_mapping.shape[0], views_per_chunk=views_per_chunk,
-                      max_pixels_per_voxel=mapping3dto2d.shape[1], num_locs=n,
+                      max_pixels_per_voxel=0 if all_pixels(flags) or mapping3dto2d.dim() != 2 else mapping3dto2d.shape[1],
+                      num_locs=n,
                       flags=(N.SPSG_FLAG_GRADS_CLEARED if grads_cleared else 0) |
-                      (flags & (N.SPSG_FLAG_DETERMINISTIC_GRADS | N.SPSG_FLAG_VIEW_NORMALS | N.SPSG_FLAG_DETERMINISTIC)))
+                      (flags & (N.SPSG_FLAG_DETERMINISTIC_GRADS | N.SPSG_FLAG_VIEW_NORMALS | N.SPSG_FLAG_DETERMINISTIC |
+                                N.SPSG_FLAG_ALL_PIXELS)))
     dev = grad_color.device
     px = sparse_mapping.shape[0] * views_per_chunk * p.width * p.height
     if grad_depth.numel() < px or grad_color.numel() < 3 * px or grad_normal.numel() < 3 * px or grad_semantic.numel() < 14 * px:
@@ -366,7 +395,7 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
         ws = workspace_owner.check(p, nbytes) if workspace_owner is not None else \
             workspace(dev, nbytes, sparse_mapping, expect=_stamp(p))
         N.check(N.lib.spsg_raycast_backward(ctypes.byref(p), N.ptr(grad_color), N.ptr(grad_depth), N.ptr(grad_normal),
-                                            N.ptr(grad_semantic), N.ptr(sparse_mapping), N.ptr(mapping3dto2d),
+                                            N.ptr(grad_semantic), N.ptr(sparse_mapping), table_ptr(mapping3dto2d, flags),
                                             N.ptr(mapping3dto2d_num), N.ptr(d_color), N.ptr(d_depth),
                                             N.ptr(d_normals), N.ptr(d_semantic), N.ptr(ws), ws.numel(), _stream(dev)))
 

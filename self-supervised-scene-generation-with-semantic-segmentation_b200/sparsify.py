@@ -124,9 +124,10 @@ def sparse_locs(sdf, truncation, empty=None, raycaster=None, counted=None):
             m = raycaster
             # the workspace of the forward to come, sized for the most views the module renders (the brick sits at its start)
             # and for the mode that forward will run in (deterministic mode needs more)
+            flags = rc.with_torch_mode(m.flags) & (N.SPSG_FLAG_DETERMINISTIC | N.SPSG_FLAG_ALL_PIXELS)
             p = N.make_params(m.width, m.height, m.depth_min, m.depth_max, m.thresh_sample_dist, m.ray_increment,
                               m.dims3d[2], m.dims3d[1], m.dims3d[0], m.batch_size, m.max_num_frames,
-                              m.mapping3dto2d.shape[1], n, rc.with_torch_mode(m.flags) & N.SPSG_FLAG_DETERMINISTIC)
+                              rc.table_shape(m.mapping3dto2d, m.mapping3dto2d_num, flags)[1], n, flags)
             ws = m.workspace.get(dev, N.workspace_bytes(p))
             indexed = N.lib.spsg_sparsify_locs_indexed_bf16 if bf16 else N.lib.spsg_sparsify_locs_indexed
             N.check(indexed(N.ptr(sdf), N.ptr(empty), B, dz, dy, dx, float(truncation),
@@ -144,7 +145,7 @@ def _feeds(m, sdf, n):
     ws = getattr(m, "workspace", None)
     return (ws is not None and n > 0 and tuple(sdf.shape) == (m.batch_size,) + tuple(m.dims3d) and
             m.sparse_mapping.device == sdf.device and tuple(m.sparse_mapping.shape) == tuple(sdf.shape) and
-            n * m.max_num_frames <= m.mapping3dto2d.shape[0])
+            n * m.max_num_frames <= rc.table_shape(m.mapping3dto2d, m.mapping3dto2d_num, m.flags)[0])
 
 
 def _payload_array(dense, sparse):

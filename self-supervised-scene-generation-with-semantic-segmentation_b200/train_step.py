@@ -51,13 +51,17 @@ class ViewGuidedTrainStep:
                 The bfloat16 heads (NDHWC with ``prepare_generator``) go to the producer glue as they are; from the voxel
                 payloads on (normals, the three raycasts, the 2D losses, ``image_loss``) everything stays float32.  No
                 gradient scaler: bfloat16 has float32's exponent range.  False: the float32 step.
+    max_pixels_per_voxel  the raycaster's voxel -> pixel table width (64, the reference's): a (voxel, view)'s gradient is
+                the mean over the first that many of its pixels.  None: over all of them, without the table
+                (``RaycastRGBD(..., max_pixels_per_voxel=None)``; at B = 8, F = 1 and the default row bound that drops a
+                1.31 GB allocation).
     """
 
     def __init__(self, model, loss_util, batch_size, dims3d, width, height, class_weight, voxelsize=0.02, truncation=3.0,
                  weight_occ_loss=1.0, weight_sdf_loss=0.1, weight_depth_loss=1.0, weight_color_loss=1.0,
                  weight_semantic_loss=0.1, weight_surf_geo=1.0, weight_missing_geo=5.0, logweight_sdf=True,
                  max_num_locs_per_sample=640000, views_per_chunk=1, render_input=True, device=None, image_loss=None,
-                 autocast_bf16=False):
+                 autocast_bf16=False, max_pixels_per_voxel=64):
         self.model, self.loss_util = model, loss_util
         self.image_loss = image_loss
         self.autocast_bf16 = autocast_bf16
@@ -74,7 +78,8 @@ class ViewGuidedTrainStep:
         self.raycaster = RaycastRGBD(batch_size, self.dims3d, width, height, depth_min=0.1 / voxelsize,
                                      depth_max=6.0 / voxelsize, thresh_sample_dist=thresh_sample_dist,
                                      ray_increment=ray_increment, max_num_frames=views_per_chunk,
-                                     max_num_locs_per_sample=max_num_locs_per_sample, device=device)
+                                     max_num_locs_per_sample=max_num_locs_per_sample,
+                                     max_pixels_per_voxel=max_pixels_per_voxel, device=device)
         self.last = {}
 
     def _normals(self, locs, vals, transform):
