@@ -22,6 +22,18 @@
  *   d_color (N,3)   d_depth (N,1)   d_normal (N,3)   d_semantic (N,14)
  * with I = num_chunks * views_per_chunk images; image i renders chunk i / views_per_chunk
  * (reference style.py:9-16); views_per_chunk == 1 is exactly the reference.
+ *
+ * Semantic class count C (spsg_raycast_params.semantic_channels; 0 means 14, the reference's float14): every "14" of the
+ * layouts above and of the loss structs below is C -- vals_semantic (N,C), image_semantic (I,H,W,C), d_semantic (N,C),
+ * grad_semantic / upstream grad_semantic (I,H,W,C), class_weight (C), and target_label == C means ignore.  A miss is -inf in
+ * all C channels.  C = 1..64; anything else is SPSG_ERR_INVALID_ARGUMENT.  Nothing but the semantic channels depends on C:
+ * the colour, depth and normal renderings, mapping3dto2d(_num), the backward's work list and the SPSG_FLAG_DETERMINISTIC
+ * tables are bit-identical to those of the C = 14 call on the same voxels, and each semantic pixel is a copy of its hit
+ * voxel's row.  The cross-entropy (fused and stand-alone) is valid where label < C and logit 0 != -inf and equals
+ * sum w[y] * nll / sum w[y] over C logits, with the 14-channel path's arithmetic in the same order.  C != 14 runs
+ * C-generic kernels (SPSG_FLAG_GENERIC_SEMANTIC forces them at C = 14); C = 14 without that flag runs exactly the
+ * 14-channel kernels.  spsg_workspace_bytes does not depend on C.  C composes with every flag.  A backward must be called
+ * with the C of its forward (the library cannot tell: the workspace does not record it).
  */
 #ifndef SPSG_RAYCAST_H_
 #define SPSG_RAYCAST_H_
@@ -41,6 +53,7 @@ extern "C" {
 
 #define SPSG_SEMANTIC_CHANNELS 14 /* float14, raycast_rgbd_cuda_kernel.cu:18-21 */
 #define SPSG_GRAD_CHANNELS 21     /* colour 3 + depth 1 + normal 3 + semantic 14 */
+#define SPSG_MAX_SEMANTIC_CHANNELS 64 /* largest spsg_raycast_params.semantic_channels */
 
 enum {
     SPSG_OK = 0,
@@ -82,7 +95,7 @@ enum {
                                            forward's clear_grads->d_normal must hold N*F rows.  Colour, depth and semantic
                                            are unchanged.  With views_per_chunk == 1 the flag changes nothing.  Pass it
                                            to the forward and to its backward alike. */
-    SPSG_FLAG_ALL_PIXELS = 1u << 11     /* forward and backward: the gradient of row (v, f) is the mean over EVERY pixel of view f
+    SPSG_FLAG_ALL_PIXELS = 1u << 11,    /* forward and backward: the gradient of row (v, f) is the mean over EVERY pixel of view f
                                            whose hit voxel is v, not over the first max_pixels_per_voxel of them:
                                                d_x[v] = sum_f (1 / num[f*N + v]) * sum over S(v, f) of grad_x[pixel]
                                            with num = mapping3dto2d_num = |S(v, f)|.  No table is written or read:
@@ -96,6 +109,10 @@ enum {
                                            atomics.  Composes with VIEW_NORMALS, DETERMINISTIC_GRADS, GRADS_CLEARED,
                                            PACKED_LOCS, INDEX_PREBUILT and the fused losses.  Pass it to the forward and to
                                            its backward alike; spsg_workspace_bytes grows as stated there. */
+    SPSG_FLAG_GENERIC_SEMANTIC = 1u << 12 /* debug: run the C-generic semantic kernels (forward epilogue, gather, loss sums)
+                                           even at C = 14, where the 14-channel kernels run otherwise.  Results are those of
+                                           the 14-channel kernels; under SPSG_FLAG_DETERMINISTIC bit for bit (renderings,
+                                           tables, loss_out, gradients).  For tests and timing of the two paths. */
 };
 
 /* Replaces the reference's `opts` CPU tensor [W,H,depth_min,depth_max,thresh,ray_inc,Dx,Dy,Dz]
@@ -110,7 +127,7 @@ typedef struct spsg_raycast_params {
     int32_t max_pixels_per_voxel; /* mapping3dto2d.size(1)                             */
     int64_t num_locs;             /* N = locs.size(0)                                  */
     uint32_t flags;               /* SPSG_FLAG_*                                       */
-    uint32_t reserved;
+    uint32_t semantic_channels;   /* C, semantic classes per voxel / pixel: 1..64, 0 = 14 (see the top of this file) */
 } spsg_raycast_params;
 
 /* Fused 2D losses (reference: depth L1 train.py:635-638, colour L1 loss.py:246-257,
@@ -120,8 +137,8 @@ typedef struct spsg_loss_targets {
     const float *target_depth;    /* (I,H,W) metres; 0 = hole (ignored)                               */
     const float *target_color;    /* (I,H,W,3) already permuted to channels-last                      */
     const float *weight_color;    /* (I,H,W) optional per-pixel colour weight or NULL (loss.py:250-253) */
-    const uint8_t *target_label;  /* (I,H,W) class id, 14 = ignore (train.py:614-616)                 */
-    const float *class_weight;    /* (14) cross-entropy class weights (train.py:118-119) or NULL = 1  */
+    const uint8_t *target_label;  /* (I,H,W) class id, 14 (C) = ignore (train.py:614-616)             */
+    const float *class_weight;    /* (14) / (C) cross-entropy class weights (train.py:118-119) or NULL = 1 */
     float voxelsize;              /* depth scale applied to the rendering (train.py:635)              */
     float weight_depth, weight_color_loss, weight_semantic; /* loss = sum_k weight_k * loss_k         */
 } spsg_loss_targets;
@@ -318,6 +335,21 @@ SPSG_API int spsg_losses2d_backward(const spsg_loss_targets *t, const float *ima
                                     const float *grad_scale, float *d_color, float *d_depth, float *d_semantic,
                                     void *stream);
 
+/* The three stand-alone 2D-loss calls above with C = num_classes logits per pixel (1..64): image_semantic and d_semantic
+ *    (P,C), class_weight (C), target_label C = ignore; no alignment beyond 4 bytes.  These always run the C-generic kernels,
+ *    also at C = 14, where they give the results of the 14-channel calls (the deterministic forward bit for bit). */
+SPSG_API int spsg_losses2d_forward_classes(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                                           const float *image_semantic, int32_t num_classes, int64_t num_pixels,
+                                           float *loss_out, void *scratch, size_t scratch_bytes, void *stream);
+SPSG_API int spsg_losses2d_forward_deterministic_classes(const spsg_loss_targets *t, const float *image_color,
+                                                         const float *image_depth, const float *image_semantic,
+                                                         int32_t num_classes, int64_t num_pixels, float *loss_out,
+                                                         void *scratch, size_t scratch_bytes, void *stream);
+SPSG_API int spsg_losses2d_backward_classes(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                                            const float *image_semantic, int32_t num_classes, int64_t num_pixels,
+                                            const float *loss_out, const float *grad_scale, float *d_color,
+                                            float *d_depth, float *d_semantic, void *stream);
+
 /* ---- host side of a host-fed call.  The reference hands its voxel rows to the GPU as int64 (z,y,x,b) -- 32 bytes per voxel, 28
  *      of them zero -- (raycast_rgbd.py:22-28; data_util.py builds them from the chunk file's uint32 triples).  This packs them,
  *      on the host, into what the index pass derives from them anyway: one uint32 linear cell index ((b*Dz+z)*Dy+y)*Dx+x per
@@ -453,6 +485,11 @@ SPSG_API int spsg_dense_scatter_strided(const spsg_dense_head *heads, int32_t co
  *    hist: 15 device int64 (cleared, then the number of pixels per label) or NULL. */
 SPSG_API int spsg_labels_from_render(const float *semantic, int64_t num_pixels, uint8_t *labels, int64_t *hist,
                                      void *stream);
+
+/* spsg_labels_from_render over C = num_classes (1..64) channels: semantic (P,C), 4-byte aligned; label C = miss or
+ *    unlabeled; hist: C + 1 device int64 or NULL. */
+SPSG_API int spsg_labels_from_render_classes(const float *semantic, int32_t num_classes, int64_t num_pixels,
+                                             uint8_t *labels, int64_t *hist, void *stream);
 
 #ifdef __cplusplus
 }

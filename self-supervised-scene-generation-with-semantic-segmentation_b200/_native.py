@@ -22,6 +22,8 @@ SPSG_FLAG_PACKED_LOCS = 1 << 8
 SPSG_FLAG_VIEW_NORMALS = 1 << 9
 SPSG_FLAG_DETERMINISTIC = 1 << 10
 SPSG_FLAG_ALL_PIXELS = 1 << 11
+SPSG_FLAG_GENERIC_SEMANTIC = 1 << 12
+SPSG_MAX_SEMANTIC_CHANNELS = 64
 SPSG_LOSS_OUT_FLOATS = 8
 SPSG_DTYPE_F32 = 0
 SPSG_DTYPE_BF16 = 1
@@ -42,6 +44,8 @@ EXPORTS = (
     "spsg_sparsify_count_bf16", "spsg_sparsify_locs_bf16", "spsg_sparsify_locs_indexed_bf16",
     "spsg_dense_gather_strided", "spsg_dense_scatter_strided",
     "spsg_labels_from_render", "spsg_pack_locs_host",
+    "spsg_losses2d_forward_classes", "spsg_losses2d_forward_deterministic_classes", "spsg_losses2d_backward_classes",
+    "spsg_labels_from_render_classes",
 )
 
 
@@ -55,7 +59,7 @@ class Params(ctypes.Structure):
         ("num_chunks", ctypes.c_int32), ("views_per_chunk", ctypes.c_int32),
         ("max_pixels_per_voxel", ctypes.c_int32),
         ("num_locs", ctypes.c_int64),
-        ("flags", ctypes.c_uint32), ("reserved", ctypes.c_uint32),
+        ("flags", ctypes.c_uint32), ("semantic_channels", ctypes.c_uint32),
     ]
 
 
@@ -142,6 +146,12 @@ def _load():
     lib.spsg_losses2d_forward_deterministic.argtypes = [lt, vp, vp, vp, i64, vp, vp, sz, vp]
     lib.spsg_losses2d_backward.restype = ctypes.c_int
     lib.spsg_losses2d_backward.argtypes = [lt, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp]
+    lib.spsg_losses2d_forward_classes.restype = ctypes.c_int
+    lib.spsg_losses2d_forward_classes.argtypes = [lt, vp, vp, vp, i32, i64, vp, vp, sz, vp]
+    lib.spsg_losses2d_forward_deterministic_classes.restype = ctypes.c_int
+    lib.spsg_losses2d_forward_deterministic_classes.argtypes = [lt, vp, vp, vp, i32, i64, vp, vp, sz, vp]
+    lib.spsg_losses2d_backward_classes.restype = ctypes.c_int
+    lib.spsg_losses2d_backward_classes.argtypes = [lt, vp, vp, vp, i32, i64, vp, vp, vp, vp, vp, vp]
     f32 = ctypes.c_float
     lib.spsg_depth_bilateral_filter.restype = ctypes.c_int
     lib.spsg_depth_bilateral_filter.argtypes = [vp, vp, i32, i32, i32, f32, f32, vp]
@@ -181,6 +191,8 @@ def _load():
     lib.spsg_dense_scatter_strided.argtypes = [dh, i32, vp, i64, i32, i32, i32, i32, vp]
     lib.spsg_labels_from_render.restype = ctypes.c_int
     lib.spsg_labels_from_render.argtypes = [vp, i64, vp, vp, vp]
+    lib.spsg_labels_from_render_classes.restype = ctypes.c_int
+    lib.spsg_labels_from_render_classes.argtypes = [vp, i32, i64, vp, vp, vp]
     lib.spsg_timing_enable.restype = None
     lib.spsg_timing_enable.argtypes = [ctypes.c_int]
     lib.spsg_timing_read.restype = ctypes.c_int
@@ -205,10 +217,11 @@ def version():
 
 
 def make_params(width, height, depth_min, depth_max, thresh_sample_dist, ray_increment, dimx, dimy, dimz, num_chunks,
-                views_per_chunk=1, max_pixels_per_voxel=64, num_locs=0, flags=0):
+                views_per_chunk=1, max_pixels_per_voxel=64, num_locs=0, flags=0, semantic_channels=0):
+    """``semantic_channels``: C, the semantic classes per voxel / pixel (0 = 14)."""
     return Params(int(width), int(height), float(depth_min), float(depth_max), float(thresh_sample_dist),
                   float(ray_increment), int(dimx), int(dimy), int(dimz), int(num_chunks), int(views_per_chunk),
-                  int(max_pixels_per_voxel), int(num_locs), int(flags), 0)
+                  int(max_pixels_per_voxel), int(num_locs), int(flags), int(semantic_channels))
 
 
 def workspace_bytes(params):

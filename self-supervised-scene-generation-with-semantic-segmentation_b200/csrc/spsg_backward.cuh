@@ -70,6 +70,38 @@ __global__ void __launch_bounds__(256) backward_zero_view_normals_kernel(const B
     zero_rows<false, true>(a, ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5, ((long long)gridDim.x * blockDim.x) >> 5);
 }
 
+// zero_rows with C = a.loss.sem_channels semantic slots per voxel (kGenericSem launches)
+template <bool kSkipHit, bool kViewNormals = false>
+__device__ __forceinline__ void zero_rows_sem(const BackwardArgs &a, long long first_warp, long long num_warps) {
+    const int lane = threadIdx.x & 31, C = a.loss.sem_channels;
+    for (long long base = first_warp * 32; base < a.num_locs; base += num_warps * 32) {
+        const long long i = base + lane;
+        const bool keep = kSkipHit && i < a.num_locs && __ldg(a.mapping3dto2d_num + i) > 0;
+        const unsigned kept = __ballot_sync(0xffffffffu, keep);
+        const int n = (int)min((long long)32, a.num_locs - base);
+        float *s = a.d_semantic + (size_t)base * C;
+        for (int e = lane; e < n * C; e += 32)
+            if (!((kept >> (e / C)) & 1u)) s[e] = 0.0f;
+        float *c = a.d_color + (size_t)base * 3, *nm = a.d_normal + (size_t)base * 3;
+        for (int e = lane; e < n * 3; e += 32)
+            if (!((kept >> (e / 3)) & 1u)) {
+                c[e] = 0.0f;
+                if (!kViewNormals) nm[e] = 0.0f;
+            }
+        if (kViewNormals) {
+            float *nv = a.d_normal + (size_t)base * 3 * a.views;
+            for (int e = lane; e < n * 3 * a.views; e += 32) nv[e] = 0.0f;
+        }
+        if (lane < n && !keep) a.d_depth[i] = 0.0f;
+    }
+}
+
+template <bool kViewNormals>
+__global__ void __launch_bounds__(256) backward_zero_sem_kernel(const BackwardArgs a) {
+    zero_rows_sem<false, kViewNormals>(a, ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5,
+                                       ((long long)gridDim.x * blockDim.x) >> 5);
+}
+
 // Upstream gradient of one pixel, all 21 channels (g[0..13] semantic, [14..16] colour, [17] depth->sdf, [18..20] normal).
 // Plain variant: read from the four gradient images.  Fused variant (pixel_grads_fused): recomputed from the rendering and
 // the targets of the 2D losses.
@@ -264,6 +296,154 @@ __device__ __forceinline__ void add_upstream_grads(const BackwardArgs &a, unsign
     }
 }
 
+// ---- C-generic twins of the four per-pixel helpers above (kGenericSem).  A pixel's row has R = C + 7 channels: [0, C)
+// semantic, [C, C+3) colour, C+3 depth->sdf, [C+4, C+7) normal -- at C = 14 exactly the 21-channel layout.  Every term is
+// rounded as its 14-channel counterpart rounds it.
+__device__ __forceinline__ void pixel_grads_sem(const BackwardArgs &a, int C, unsigned gpix, float *__restrict__ t) {
+    const float *s = a.grad_semantic + (size_t)gpix * C;
+#pragma unroll 1
+    for (int k = 0; k < C; k++) t[k] = __ldg(s + k);
+    const float *c = a.grad_color + (size_t)gpix * 3, *n = a.grad_normal + (size_t)gpix * 3;
+    t[C] = __ldg(c); t[C + 1] = __ldg(c + 1); t[C + 2] = __ldg(c + 2);
+    t[C + 3] = __ldg(a.grad_depth + gpix);
+    t[C + 4] = __ldg(n); t[C + 5] = __ldg(n + 1); t[C + 6] = __ldg(n + 2);
+}
+
+// pixel_grads_fused over C logits (the stand-alone backward's gradient images)
+__device__ __forceinline__ void pixel_grads_fused_sem(const BackwardArgs &a, const FusedCoef &fc, int C, unsigned gpix,
+                                                      float *__restrict__ t) {
+    const LossArgs &L = a.loss;
+    const int y = L.target_label ? (int)L.target_label[gpix] : C;
+    const float *l = a.image_semantic + (size_t)gpix * C;
+    if (y < C && __ldg(l) != -CUDART_INF_F) {  // valid = (label < C) & (logit0 != -inf)
+        float m = __ldg(l);
+#pragma unroll 1
+        for (int k = 1; k < C; k++) m = fmaxf(m, __ldg(l + k));
+        float sum = 0.0f;
+#pragma unroll 1
+        for (int k = 0; k < C; k++) {
+            const float e = __expf(__ldg(l + k) - m);
+            t[k] = e;
+            sum += e;
+        }
+        const float w = L.class_weight ? __ldg(L.class_weight + y) : 1.0f;
+        const float f = fc.sem * w, fs = f * __frcp_rn(sum);
+#pragma unroll 1
+        for (int k = 0; k < C; k++) t[k] = t[k] * fs - (k == y ? f : 0.0f);
+    } else {
+#pragma unroll 1
+        for (int k = 0; k < C; k++) t[k] = 0.0f;
+    }
+    float g0 = 0.0f, g1 = 0.0f, g2 = 0.0f;
+    if (L.target_color) {
+        const float w = L.weight_color ? __ldg(L.weight_color + gpix) : 1.0f;
+        const float *c = a.image_color + (size_t)gpix * 3, *tc = L.target_color + (size_t)gpix * 3;
+        const float c0 = __ldg(c), c1 = __ldg(c + 1), c2 = __ldg(c + 2);
+        const float d0 = __fadd_rn(__fmul_rn(c0, w), -__fmul_rn(__ldg(tc), w));
+        const float d1 = __fadd_rn(__fmul_rn(c1, w), -__fmul_rn(__ldg(tc + 1), w));
+        const float d2 = __fadd_rn(__fmul_rn(c2, w), -__fmul_rn(__ldg(tc + 2), w));
+        const float f = fc.col * w;
+        if (c0 != -CUDART_INF_F) g0 = f * (float)((d0 > 0.0f) - (d0 < 0.0f));
+        if (c1 != -CUDART_INF_F) g1 = f * (float)((d1 > 0.0f) - (d1 < 0.0f));
+        if (c2 != -CUDART_INF_F) g2 = f * (float)((d2 > 0.0f) - (d2 < 0.0f));
+    }
+    t[C] = g0; t[C + 1] = g1; t[C + 2] = g2;
+    float gd = 0.0f;
+    if (L.target_depth) {
+        const float td = __ldg(L.target_depth + gpix);
+        const float r = __ldg(a.image_depth + gpix);
+        if (td != 0.0f && r != -CUDART_INF_F) {
+            const float d = __fmul_rn(r, L.voxelsize) - td;
+            gd = fc.dep * (float)((d > 0.0f) - (d < 0.0f));
+        }
+    }
+    t[C + 3] = gd; t[C + 4] = 0.0f; t[C + 5] = 0.0f; t[C + 6] = 0.0f;
+}
+
+// fused_item over C logits: lane c of the group loads logits c, c + G, ...; e_k goes to e[k], the sum is taken in k order
+// from there (what the 14-channel shuffles add, in the same order)
+template <int G>
+__device__ __forceinline__ FusedItem fused_item_sem(const BackwardArgs &a, int C, unsigned gpix0, int hl, unsigned hmask,
+                                                    float *__restrict__ e) {
+    FusedItem it = {0.0f, false, 0.0f, 0.0f, 0.0f};
+    if (a.loss.target_label) {
+        const float *l = a.image_semantic + (size_t)gpix0 * C;
+        float m = CUDART_NAN_F;  // fmaxf drops it: lanes without a channel do not take part
+        for (int k = hl; k < C; k += G) m = fmaxf(m, __ldg(l + k));
+        it.sem = __ldg(l) != -CUDART_INF_F;
+        if (it.sem) {
+#pragma unroll
+            for (int o = G / 2; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(hmask, m, o, G));
+            for (int k = hl; k < C; k += G) e[k] = __expf(__ldg(l + k) - m);
+            __syncwarp(hmask);
+            float sum = 0.0f;
+            for (int k = 0; k < C; k++) sum += e[k];
+            it.rs = __frcp_rn(sum);
+        }
+    }
+    if (a.loss.target_color) {
+        const float *c = a.image_color + (size_t)gpix0 * 3;
+        it.c0 = __ldg(c); it.c1 = __ldg(c + 1); it.c2 = __ldg(c + 2);
+    }
+    __syncwarp(hmask);
+    return it;
+}
+
+// fused_pixel_grads over C logits
+__device__ __forceinline__ void fused_pixel_grads_sem(const BackwardArgs &a, const FusedCoef &fc, const FusedItem &it, int C,
+                                                      const float *__restrict__ e, unsigned gpix, float *__restrict__ t) {
+    const LossArgs &L = a.loss;
+    const int y = it.sem ? (int)L.target_label[gpix] : C;
+    if (y < C) {
+        const float f = __fmul_rn(fc.sem, L.class_weight ? __ldg(L.class_weight + y) : 1.0f), fs = __fmul_rn(f, it.rs);
+#pragma unroll 1
+        for (int k = 0; k < C; k++) t[k] = __fmaf_rn(e[k], fs, -(k == y ? f : 0.0f));
+    } else {
+#pragma unroll 1
+        for (int k = 0; k < C; k++) t[k] = 0.0f;
+    }
+    float g0 = 0.0f, g1 = 0.0f, g2 = 0.0f;
+    if (L.target_color) {
+        const float w = L.weight_color ? __ldg(L.weight_color + gpix) : 1.0f;
+        const float *tc = L.target_color + (size_t)gpix * 3;
+        const float d0 = __fadd_rn(__fmul_rn(it.c0, w), -__fmul_rn(__ldg(tc), w));
+        const float d1 = __fadd_rn(__fmul_rn(it.c1, w), -__fmul_rn(__ldg(tc + 1), w));
+        const float d2 = __fadd_rn(__fmul_rn(it.c2, w), -__fmul_rn(__ldg(tc + 2), w));
+        const float fw = fc.col * w;
+        if (it.c0 != -CUDART_INF_F) g0 = fw * (float)((d0 > 0.0f) - (d0 < 0.0f));
+        if (it.c1 != -CUDART_INF_F) g1 = fw * (float)((d1 > 0.0f) - (d1 < 0.0f));
+        if (it.c2 != -CUDART_INF_F) g2 = fw * (float)((d2 > 0.0f) - (d2 < 0.0f));
+    }
+    t[C] = g0; t[C + 1] = g1; t[C + 2] = g2;
+    float gd = 0.0f;
+    if (L.target_depth) {
+        const float td = __ldg(L.target_depth + gpix);
+        const float r = __ldg(a.image_depth + gpix);
+        if (td != 0.0f && r != -CUDART_INF_F) {
+            const float d = __fmul_rn(r, L.voxelsize) - td;
+            gd = fc.dep * (float)((d > 0.0f) - (d < 0.0f));
+        }
+    }
+    t[C + 3] = gd; t[C + 4] = 0.0f; t[C + 5] = 0.0f; t[C + 6] = 0.0f;
+}
+
+__device__ __forceinline__ void add_upstream_grads_sem(const BackwardArgs &a, int C, unsigned gpix, float *__restrict__ t) {
+    if (a.up_semantic) {
+        const float *s = a.up_semantic + (size_t)gpix * C;
+#pragma unroll 1
+        for (int k = 0; k < C; k++) t[k] += __ldg(s + k);
+    }
+    if (a.up_color) {
+        const float *c = a.up_color + (size_t)gpix * 3;
+        t[C] += __ldg(c); t[C + 1] += __ldg(c + 1); t[C + 2] += __ldg(c + 2);
+    }
+    if (a.up_depth) t[C + 3] += __ldg(a.up_depth + gpix);
+    if (a.up_normal) {
+        const float *n = a.up_normal + (size_t)gpix * 3;
+        t[C + 4] += __ldg(n); t[C + 5] += __ldg(n + 1); t[C + 6] += __ldg(n + 2);
+    }
+}
+
 // The gather (kernel.cu:391-419 turned inside out).  Work items are the (voxel, view) pairs the forward listed; one
 // warp per item.  Lane k fetches the k-th registered pixel id (one coalesced load) and that pixel's 21 upstream
 // gradients (independent 8- and 4-byte loads; the fused variant reads only its targets and depth, see FusedItem), parks
@@ -284,7 +464,10 @@ constexpr int kGatherGroup = SPSG_GATHER_GROUP;  // lanes per (voxel, view) item
 // stored to row (voxel, view) of the (N,F,3) d_normal; the other channels are gathered as without it
 // kSegments (SPSG_FLAG_ALL_PIXELS): a row's pixels are its segment of seg_pix, all num[row] of them (no cap), instead of
 // the first min(num, max_pixels) entries of its mapping3dto2d row
-template <bool kFused, bool kUpstream, int kViews, bool kViewNormals, bool kSegments = false>
+// kGenericSem (C = a.loss.sem_channels != 14, or SPSG_FLAG_GENERIC_SEMANTIC): rows of R = C + 7 channels, staged in dynamic
+// shared memory (kGatherWarps * 32 / G * G * R floats: 21.5 KB at C = 14, 72.7 KB at C = 64), the per-pixel helpers'
+// *_sem twins; lane c of a group sums channels c, c + G, ... as without it
+template <bool kFused, bool kUpstream, int kViews, bool kViewNormals, bool kSegments = false, bool kGenericSem = false>
 #ifndef SPSG_GATHER_MIN_BLOCKS
 #define SPSG_GATHER_MIN_BLOCKS 8  // 32 registers: full occupancy hides the dependent gathers (the fused variants spill 24-92 B and are still faster)
 #endif
@@ -295,18 +478,26 @@ __global__ void __launch_bounds__(kGatherWarps * 32, kSegments ? 5 : SPSG_GATHER
     static_assert(kFused || !kUpstream, "upstream images are added to the fused variant's recomputed gradients");
     static_assert(kViews != 0 || !kViewNormals, "per-view normal rows need several views per chunk");
     if ((int)blockIdx.x < a.zero_blocks) {
+        if (kGenericSem) {
+            zero_rows_sem<true>(a, ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5, ((long long)a.zero_blocks * blockDim.x) >> 5);
+            return;
+        }
         zero_rows<true>(a, ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5, ((long long)a.zero_blocks * blockDim.x) >> 5);
         return;
     }
     // kGatherGroup lanes per item, 32 / kGatherGroup items in flight per warp: the groups work on different items
-    constexpr int G = kGatherGroup, kPerWarp = 32 / G, kSlots = (21 + G - 1) / G;
+    constexpr int G = kGatherGroup, kPerWarp = 32 / G;
+    constexpr int kSlots = ((kGenericSem ? kMaxSemanticChannels + 7 : 21) + G - 1) / G;
     static_assert(!kFused || G >= 14, "the fused variant's softmax takes one lane per semantic channel");
-    __shared__ float s_g[kGatherWarps * kPerWarp][G * 21];
-    __shared__ __align__(16) float s_e[kFused ? kGatherWarps * kPerWarp : 1][16];  // fused: the item's e_k (FusedItem)
+    __shared__ float s_g[kGenericSem ? 1 : kGatherWarps * kPerWarp][kGenericSem ? 1 : G * 21];
+    extern __shared__ float s_dyn[];  // kGenericSem: the groups' rows of R floats
+    constexpr int kE = kGenericSem ? kMaxSemanticChannels : 16;
+    __shared__ __align__(16) float s_e[kFused ? kGatherWarps * kPerWarp : 1][kE];  // fused: the item's e_k (FusedItem)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int hl = lane & (G - 1), half = lane / G;
     const unsigned hmask = (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << (G * half);
-    float *tile = s_g[warp * kPerWarp + half];
+    const int C = kGenericSem ? a.loss.sem_channels : 14, R = kGenericSem ? C + 7 : 21;
+    float *tile = kGenericSem ? s_dyn + (size_t)(warp * kPerWarp + half) * G * R : s_g[warp * kPerWarp + half];
     const int groups_total = (int)(gridDim.x - a.zero_blocks) * kGatherWarps * kPerWarp;
     const int count = *a.list_count;
     const unsigned P = (unsigned)(a.width * a.height);
@@ -346,7 +537,10 @@ __global__ void __launch_bounds__(kGatherWarps * 32, kSegments ? 5 : SPSG_GATHER
                 const unsigned pixbase = (unsigned)(image0 + view) * P;  // global pixel index < 2^32 / 14 (check_params)
                 const float inv = __frcp_rn((float)cnt);
                 FusedItem it;
-                if (kFused) it = fused_item<G>(a, pixbase + (unsigned)__ldg(prow), hl, hmask, s_e[warp * kPerWarp + half]);
+                if (kFused && kGenericSem)
+                    it = fused_item_sem<G>(a, C, pixbase + (unsigned)__ldg(prow), hl, hmask, s_e[warp * kPerWarp + half]);
+                else if (kFused)
+                    it = fused_item<G>(a, pixbase + (unsigned)__ldg(prow), hl, hmask, s_e[warp * kPerWarp + half]);
                 double acc[kSlots];  // channels hl + G j; double: the sum does not depend on the pixel order to fp32 precision
 #pragma unroll
                 for (int j = 0; j < kSlots; j++) acc[j] = 0.0;
@@ -354,7 +548,14 @@ __global__ void __launch_bounds__(kGatherWarps * 32, kSegments ? 5 : SPSG_GATHER
                     const int m = min(G, cnt - k0);
                     if (hl < m) {
                         const unsigned gpix = pixbase + (unsigned)__ldg(prow + k0 + hl);
-                        if (kFused) {
+                        if (kGenericSem) {
+                            if (kFused) {
+                                fused_pixel_grads_sem(a, fc, it, C, s_e[warp * kPerWarp + half], gpix, tile + hl * R);
+                                if (kUpstream) add_upstream_grads_sem(a, C, gpix, tile + hl * R);
+                            } else {
+                                pixel_grads_sem(a, C, gpix, tile + hl * R);
+                            }
+                        } else if (kFused) {
                             fused_pixel_grads(a, fc, it, s_e[warp * kPerWarp + half], gpix, tile + hl * 21);
                             if (kUpstream) add_upstream_grads(a, gpix, tile + hl * 21);
                         } else {
@@ -368,7 +569,7 @@ __global__ void __launch_bounds__(kGatherWarps * 32, kSegments ? 5 : SPSG_GATHER
                     for (int r = 0; r < m; r++) {
 #pragma unroll
                         for (int j = 0; j < kSlots; j++)
-                            if (hl + G * j < 21) acc[j] += (double)tile[r * 21 + hl + G * j];
+                            if (hl + G * j < R) acc[j] += (double)tile[r * R + hl + G * j];
                     }
                     __syncwarp(hmask);
                 }
@@ -376,18 +577,18 @@ __global__ void __launch_bounds__(kGatherWarps * 32, kSegments ? 5 : SPSG_GATHER
                 for (int j = 0; j < kSlots; j++) {
                     const float mean = (float)(acc[j] * (double)inv);  // mean = sum / count (kernel.cu:398-418)
                     const int c = hl + G * j;
-                    if (kViewNormals && c >= 18 && c < 21) a.d_normal[((size_t)idx * a.views + view) * 3 + (c - 18)] = mean;
+                    if (kViewNormals && c >= R - 3 && c < R) a.d_normal[((size_t)idx * a.views + view) * 3 + (c - (R - 3))] = mean;
                     else tot[j] += mean;
                 }
             }
-            // channel c -> destination: 0-13 semantic, 14-16 colour, 17 depth->sdf, 18-20 normal
+            // channel c -> destination: 0-13 semantic, 14-16 colour, 17 depth->sdf, 18-20 normal (generic: C, C+3, C+4)
 #pragma unroll
             for (int j = 0; j < kSlots; j++) {
                 const int c = hl + G * j;
-                if (c < (kViewNormals ? 18 : 21)) {
-                    float *d = c < 14 ? a.d_semantic + (size_t)idx * 14 + c
-                             : c < 17 ? a.d_color + (size_t)idx * 3 + (c - 14)
-                             : c == 17 ? a.d_depth + idx : a.d_normal + (size_t)idx * 3 + (c - 18);
+                if (c < (kViewNormals ? R - 3 : R)) {
+                    float *d = c < C ? a.d_semantic + (size_t)idx * C + c
+                             : c < C + 3 ? a.d_color + (size_t)idx * 3 + (c - C)
+                             : c == C + 3 ? a.d_depth + idx : a.d_normal + (size_t)idx * 3 + (c - (C + 4));
                     if (kViews == 1) atomicAdd(d, tot[j]);
                     else *d = tot[j];
                 }

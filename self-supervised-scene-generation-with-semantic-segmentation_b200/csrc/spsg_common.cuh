@@ -10,6 +10,7 @@ constexpr float kBoxEps = 1.0f / 64.0f;  // shrink of skip regions; >> every fp3
 constexpr float kFracGuard = 1.0f / 256.0f;  // fast corner path needs frac(p) in [guard, 1-guard]
 constexpr int kMaxFastDim = 8192;        // fast corner path proven for coordinates < 2^13
 constexpr int kLossSlots = 64;           // copies of the loss accumulators (spreads atomic contention)
+constexpr int kMaxSemanticChannels = 64; // largest C of spsg_raycast_params.semantic_channels
 
 // block map byte = kind << 3 | level; level k >= 1: the aligned region of edge 2^(k+1) voxels around the block
 enum { kKindSurface = 0, kKindEmpty = 1, kKindPos = 2, kKindNeg = 3 };

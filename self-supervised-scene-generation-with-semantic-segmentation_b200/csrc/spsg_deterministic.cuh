@@ -85,7 +85,8 @@ constexpr int kDetLossThreads = 256;
 static_assert(kDetLossPix % kDetLossThreads == 0, "whole pixel rounds per block");
 
 // a.loss.accum: kLossSlots * 8 doubles of scratch for the final stage; a.loss.done: a zeroed int32; partials: 8 doubles
-// per block
+// per block.  kGenericSem: C = a.loss.sem_channels logits per pixel.
+template <bool kGenericSem = false>
 __global__ void __launch_bounds__(kDetLossThreads) losses2d_det_kernel(const Losses2DArgs a, double *__restrict__ partials) {
     __shared__ float s_warp[kDetLossThreads / 32][6];
     __shared__ int s_last;
@@ -94,7 +95,7 @@ __global__ void __launch_bounds__(kDetLossThreads) losses2d_det_kernel(const Los
 #pragma unroll 1
     for (int k = 0; k < kDetLossPix / kDetLossThreads; k++) {
         const long long p = p0 + k * kDetLossThreads + threadIdx.x;
-        if (p < a.num_pixels) loss_terms_pixel(a, p, acc);
+        if (p < a.num_pixels) loss_terms_pixel<kGenericSem>(a, p, acc);
     }
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll

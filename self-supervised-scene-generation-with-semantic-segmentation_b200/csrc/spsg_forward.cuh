@@ -34,6 +34,7 @@ struct LossArgs {
     float *loss_out;
     int32_t *done;  // CTAs finished (zeroed per call)
     float w_depth, w_color, w_sem;
+    int sem_channels;  // C of the kGenericSem kernels (in the struct's tail padding: no kernel parameter offset moves)
 };
 
 __device__ __forceinline__ void finalize_loss_warp(const double *acc, float *__restrict__ out, float w_depth, float w_color,
@@ -145,6 +146,42 @@ __device__ __forceinline__ void store_warp_tile(const float *__restrict__ s, flo
     }
 }
 
+// Write-out of the C-channel semantic rows of a warp's 8x4 pixel tile (kGenericSem).  Each tile row is 8*C contiguous
+// floats of the image; lane l writes floats l, l + 32, ... of it, taking the pixel's hit voxel from its lane by shuffle and
+// the value from that voxel's payload row.  Every store instruction covers 128 contiguous bytes, so unlike the 14-channel
+// path no staging is needed, and no payload is held in registers.  Loop bounds are uniform over the warp (the shuffles).
+__device__ __forceinline__ void store_semantic_rows(const float *__restrict__ vals, int C, int hit, float *__restrict__ g,
+                                                    size_t pix0, int x0, int y0, int width, int height, int lane) {
+    const int rows = min(kWarpH, height - y0), cols = min(kWarpW, width - x0);
+    if (rows <= 0 || cols <= 0) return;
+    const int n = cols * C;
+    float *__restrict__ base = g + pix0 * C;
+    const size_t stride = (size_t)width * C;
+#pragma unroll 1
+    for (int r = 0; r < rows; r++) {
+#pragma unroll 1
+        for (int k0 = 0; k0 < n; k0 += 32) {
+            const int k = k0 + lane, px = min(k / C, kWarpW - 1);
+            const int h = __shfl_sync(0xffffffffu, hit, r * kWarpW + px);
+            if (k < n) __stcs(base + r * stride + k, h >= 0 ? __ldg(vals + (size_t)h * C + (k - px * C)) : -CUDART_INF_F);
+        }
+    }
+}
+
+// Cross-entropy of one pixel over the C logits of row l (kGenericSem): max, sum of exp(l_k - max) in k order, log, in the
+// order of the 14-channel code it stands beside (kFast: __expf / __logf as the fused forward, else expf / logf as the
+// stand-alone losses).
+template <bool kFast>
+__device__ __forceinline__ float ce_nll(const float *__restrict__ l, int C, int y) {
+    float m = __ldg(l);
+#pragma unroll 1
+    for (int k = 1; k < C; k++) m = fmaxf(m, __ldg(l + k));
+    float s = 0.0f;
+#pragma unroll 1
+    for (int k = 0; k < C; k++) s += kFast ? __expf(__ldg(l + k) - m) : expf(__ldg(l + k) - m);
+    return (kFast ? __logf(s) : logf(s)) + m - __ldg(l + y);
+}
+
 // words [0, n) of p := 0, this warp's share of a launch-wide sweep: 16-byte stores where p is aligned
 __device__ __forceinline__ void clear_span(float *__restrict__ p, size_t n, size_t warp_id, size_t num_warps, int lane) {
     if ((reinterpret_cast<uintptr_t>(p) & 15u) == 0) {
@@ -165,7 +202,10 @@ __device__ __forceinline__ void clear_span(float *__restrict__ p, size_t n, size
 // the SM; tiles of the chunk's images are dealt to warps first statically, then from a global counter.
 // kViewNormals (SPSG_FLAG_VIEW_NORMALS, several views): vals_normal is (N,F,3) and image chunk*F + f reads row (hit, f); the
 // backward's normal rows to clear are N*F.
-template <bool kLoss, bool kSmemMaps, int kWarps, bool kViewNormals>
+// kGenericSem (C != 14, or SPSG_FLAG_GENERIC_SEMANTIC): vals_semantic / image_semantic hold a.loss.sem_channels channels; the
+// semantic rows are written by store_semantic_rows and the fused cross-entropy reads the hit voxel's payload row.  The
+// march, the registration and every other rendering are the same code.
+template <bool kLoss, bool kSmemMaps, int kWarps, bool kViewNormals, bool kGenericSem = false>
 __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const ForwardArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ float4 s_steps[kStepEntries];
@@ -181,7 +221,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
         // The backward's output rows are zeroed here (the reference memsets its whole d_* buffers, kernel.cu:557-560): a few
         // fire-and-forget stores per warp that overlap the march, instead of a longer fill pass in front of the index build.
         const size_t wid = (size_t)blockIdx.x * kWarps + warp, nw = (size_t)gridDim.x * kWarps, n = (size_t)a.clear_rows;
-        clear_span(a.clear.d_semantic, n * 14, wid, nw, lane);
+        clear_span(a.clear.d_semantic, n * (kGenericSem ? (size_t)a.loss.sem_channels : 14), wid, nw, lane);
         clear_span(a.clear.d_color, n * 3, wid, nw, lane);
         clear_span(a.clear.d_normal, n * 3 * (kViewNormals ? (size_t)a.views : 1), wid, nw, lane);
         clear_span(a.clear.d_depth, n, wid, nw, lane);
@@ -616,11 +656,13 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
                     const float m0 = __ldg(n + 0), m1 = __ldg(n + 1), m2 = __ldg(n + 2);
                     if (!(m0 == 0.0f && m1 == 0.0f && m2 == 0.0f)) { n0 = m0; n1 = m1; n2 = m2; }  // :220
                     dep = depth;
+                    if (!kGenericSem) {
                     const float2 *s2 = reinterpret_cast<const float2 *>(a.vals_semantic + (size_t)hit * 14);
 #pragma unroll
                     for (int k = 0; k < 7; k++) {
                         const float2 t2 = __ldg(s2 + k);
                         sem[2 * k] = t2.x; sem[2 * k + 1] = t2.y;
+                    }
                     }
                 }
                 {
@@ -658,10 +700,15 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
                 // the staging buffer is reused: semantic first, then colour + normal + depth
                 const bool vec = a.vec_ok != 0;
                 const size_t tile_pix0 = ((size_t)img * a.height + wy0) * a.width + wx0;
+                if (kGenericSem) {
+                    store_semantic_rows(a.vals_semantic, a.loss.sem_channels, hit, a.image_semantic, tile_pix0, wx0, wy0, a.width,
+                                        a.height, lane);
+                } else {
 #pragma unroll
                 for (int k = 0; k < 7; k++) reinterpret_cast<float2 *>(stage + lane * 14)[k] = make_float2(sem[2 * k], sem[2 * k + 1]);
                 __syncwarp();
                 store_warp_tile<14>(stage, a.image_semantic, tile_pix0, wx0, wy0, a.width, a.height, vec, lane);
+                }
                 if (kLoss) {
                     // The three 2D loss terms of this pixel.  The logits are read back from the staging row (still intact: the
                     // stores above only read it), one at a time, so the 14 payload registers are dead by now and the fused
@@ -681,7 +728,16 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
                                      fabsf(__fadd_rn(__fmul_rn(col2, w), -__fmul_rn(__ldg(t + 2), w)));
                             acc[3] = 3.0f;
                         }
-                        if (L.target_label) {  // train.py:744-746
+                        if (kGenericSem && L.target_label) {  // the same over the hit voxel's C logits
+                            const int y = L.target_label[gpix];
+                            const int C = a.loss.sem_channels;
+                            const float *lg = a.vals_semantic + (size_t)hit * C;
+                            if (y < C && __ldg(lg) != ninf) {
+                                const float w = L.class_weight ? __ldg(L.class_weight + y) : 1.0f;
+                                acc[4] = w * ce_nll<true>(lg, C, y);
+                                acc[5] = w;
+                            }
+                        } else if (L.target_label) {  // train.py:744-746
                             const int y = L.target_label[gpix];
                             const float *lg = stage + lane * 14;
                             if (y < 14 && lg[0] != ninf) {  // valid = (label < 14) & (logit0 != -inf), train.py:744

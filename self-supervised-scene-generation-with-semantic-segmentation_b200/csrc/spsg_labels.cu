@@ -19,6 +19,7 @@
 namespace {
 
 constexpr int kClasses = 14;
+constexpr int kMaxClasses = 64;  // spsg_labels_from_render_classes
 
 __global__ void __launch_bounds__(256) labels_kernel(const float *__restrict__ semantic, long long num_pixels,
                                                      uint8_t *__restrict__ labels, unsigned long long *__restrict__ hist) {
@@ -49,7 +50,51 @@ __global__ void __launch_bounds__(256) labels_kernel(const float *__restrict__ s
     }
 }
 
+// labels_kernel over C channels per pixel (label C = miss or unlabeled, hist of C + 1 bins): the same first-maximum scan,
+// the values read one at a time
+__global__ void __launch_bounds__(256) labels_classes_kernel(const float *__restrict__ semantic, int C, long long num_pixels,
+                                                             uint8_t *__restrict__ labels, unsigned long long *__restrict__ hist) {
+    __shared__ unsigned s_hist[kMaxClasses + 1];
+    if (hist && threadIdx.x <= C) s_hist[threadIdx.x] = 0u;
+    if (hist) __syncthreads();
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < num_pixels; i += stride) {
+        const float *p = semantic + i * C;
+        float best = __ldg(p);
+        int arg = 0;
+#pragma unroll 1
+        for (int k = 1; k < C; k++) {
+            const float v = __ldg(p + k);
+            if (best == best && (v > best || v != v)) { best = v; arg = k; }  // first maximum; NaN wins
+        }
+        const int label = (best != best || best >= 1.0f) ? arg : C;
+        labels[i] = (uint8_t)label;
+        if (hist) atomicAdd(&s_hist[label], 1u);
+    }
+    if (hist) {
+        __syncthreads();
+        if (threadIdx.x <= C && s_hist[threadIdx.x]) atomicAdd(hist + threadIdx.x, (unsigned long long)s_hist[threadIdx.x]);
+    }
+}
+
 }  // namespace
+
+extern "C" SPSG_API int spsg_labels_from_render_classes(const float *semantic, int32_t num_classes, int64_t num_pixels,
+                                                        uint8_t *labels, int64_t *hist, void *stream) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (num_classes < 1 || num_classes > kMaxClasses)
+        return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "num_classes must be in 1..64");
+    if (num_pixels < 0 || (num_pixels > 0 && (!semantic || !labels)))
+        return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "bad semantic / labels / num_pixels");
+    if (reinterpret_cast<uintptr_t>(semantic) & 3u) return spsg_internal_fail(SPSG_ERR_INVALID_ARGUMENT, "semantic must be 4-byte aligned");
+    if (hist) SPSG_CUDA_TRY(cudaMemsetAsync(hist, 0, (num_classes + 1) * sizeof(int64_t), st));
+    if (num_pixels == 0) return SPSG_OK;
+    const unsigned grid = (unsigned)std::min<long long>((num_pixels + 255) / 256, (long long)spsg_internal_sm_count() * 8);
+    labels_classes_kernel<<<grid, 256, 0, st>>>(semantic, num_classes, num_pixels, labels,
+                                                 reinterpret_cast<unsigned long long *>(hist));
+    SPSG_CUDA_TRY(cudaGetLastError());
+    return SPSG_OK;
+}
 
 extern "C" SPSG_API int spsg_labels_from_render(const float *semantic, int64_t num_pixels, uint8_t *labels,
                                                 int64_t *hist, void *stream) {

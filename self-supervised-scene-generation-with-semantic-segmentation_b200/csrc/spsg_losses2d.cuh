@@ -15,6 +15,8 @@ struct Losses2DArgs {
 };
 
 // one thread per pixel: the same six sums the fused forward accumulates in its epilogue
+// kGenericSem: C = a.loss.sem_channels logits per pixel (spsg_losses2d_forward_classes), label C = ignore
+template <bool kGenericSem = false>
 __global__ void __launch_bounds__(256) losses2d_forward_kernel(const Losses2DArgs a) {
     const float ninf = -CUDART_INF_F;
     float acc[6] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
@@ -35,7 +37,15 @@ __global__ void __launch_bounds__(256) losses2d_forward_kernel(const Losses2DArg
                 }
             }
         }
-        if (L.target_label) {  // train.py:744-746
+        if (kGenericSem && L.target_label) {  // the same over C logits
+            const int y = L.target_label[p], C = a.loss.sem_channels;
+            const float *l = a.image_semantic + p * C;
+            if (y < C && __ldg(l) != ninf) {
+                const float w = L.class_weight ? __ldg(L.class_weight + y) : 1.0f;
+                acc[4] += w * ce_nll<false>(l, C, y);
+                acc[5] += w;
+            }
+        } else if (L.target_label) {  // train.py:744-746
             const int y = L.target_label[p];
             if (y < 14) {
                 float l[14];
@@ -75,6 +85,7 @@ __global__ void __launch_bounds__(256) losses2d_forward_kernel(const Losses2DArg
 
 // pixel p's share of the six sums, added onto acc: the body of losses2d_forward_kernel's loop, for the deterministic
 // variant (spsg_deterministic.cuh).  (Kept apart so that losses2d_forward_kernel compiles exactly as before.)
+template <bool kGenericSem>
 __device__ __forceinline__ void loss_terms_pixel(const Losses2DArgs &a, long long p, float (&acc)[6]) {
     const float ninf = -CUDART_INF_F;
     const LossArgs &L = a.loss;
@@ -93,7 +104,15 @@ __device__ __forceinline__ void loss_terms_pixel(const Losses2DArgs &a, long lon
             }
         }
     }
-    if (L.target_label) {  // train.py:744-746
+    if (kGenericSem && L.target_label) {  // the same over C logits
+        const int y = L.target_label[p], C = a.loss.sem_channels;
+        const float *l = a.image_semantic + p * C;
+        if (y < C && __ldg(l) != ninf) {
+            const float w = L.class_weight ? __ldg(L.class_weight + y) : 1.0f;
+            acc[4] += w * ce_nll<false>(l, C, y);
+            acc[5] += w;
+        }
+    } else if (L.target_label) {  // train.py:744-746
         const int y = L.target_label[p];
         if (y < 14) {
             float l[14];
@@ -122,9 +141,23 @@ __device__ __forceinline__ void loss_terms_pixel(const Losses2DArgs &a, long lon
 }
 
 // gradient images of the weighted total w.r.t. the renderings (zero where a pixel is not part of a term)
+// kGenericSem: C = a.loss.sem_channels; each thread's row of C + 7 gradients is built in dynamic shared memory
+template <bool kGenericSem = false>
 __global__ void __launch_bounds__(256) losses2d_backward_kernel(const BackwardArgs a, long long num_pixels, float *d_color,
                                                                float *d_depth, float *d_semantic) {
     const FusedCoef fc = fused_coef(a);
+    if constexpr (kGenericSem) {
+        extern __shared__ float s_rows[];
+        const int C = a.loss.sem_channels;
+        float *g = s_rows + (size_t)threadIdx.x * (C + 7);
+        for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < num_pixels; p += (long long)gridDim.x * blockDim.x) {
+            pixel_grads_fused_sem(a, fc, C, (unsigned)p, g);
+            if (d_semantic)
+                for (int k = 0; k < C; k++) d_semantic[p * C + k] = g[k];
+            if (d_color) { d_color[p * 3] = g[C]; d_color[p * 3 + 1] = g[C + 1]; d_color[p * 3 + 2] = g[C + 2]; }
+            if (d_depth) d_depth[p] = g[C + 3];
+        }
+    } else {
     for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < num_pixels; p += (long long)gridDim.x * blockDim.x) {
         float g[21];
         pixel_grads_fused(a, fc, (unsigned)p, g);
@@ -134,5 +167,6 @@ __global__ void __launch_bounds__(256) losses2d_backward_kernel(const BackwardAr
         }
         if (d_color) { d_color[p * 3] = g[14]; d_color[p * 3 + 1] = g[15]; d_color[p * 3 + 2] = g[16]; }
         if (d_depth) d_depth[p] = g[17];
+    }
     }
 }

@@ -54,6 +54,14 @@ namespace {
 // host side
 // ---------------------------------------------------------------------------------------------
 
+// C of a call: 0 stands for the reference's 14
+int semantic_channels(const spsg_raycast_params *p) { return p->semantic_channels ? (int)p->semantic_channels : 14; }
+
+// the C-generic kernels run for C != 14, and at C = 14 when the debug flag asks for them
+bool generic_semantic(const spsg_raycast_params *p) {
+    return semantic_channels(p) != 14 || (p->flags & SPSG_FLAG_GENERIC_SEMANTIC) != 0;
+}
+
 int check_params(const spsg_raycast_params *p) {
     if (!p) return fail(SPSG_ERR_INVALID_ARGUMENT, "params is NULL");
     if (p->width <= 0 || p->height <= 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "width/height must be positive");
@@ -63,7 +71,9 @@ int check_params(const spsg_raycast_params *p) {
     if (p->num_locs < 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "num_locs must be >= 0");
     if ((long long)p->num_chunks * p->dimx * p->dimy * p->dimz >= (1ll << 31))
         return fail(SPSG_ERR_INVALID_ARGUMENT, "dense grid exceeds 32-bit indexing (reference limit, SURVEY 3.5)");
-    if ((long long)p->num_chunks * p->views_per_chunk * p->width * p->height * 14 >= (1ll << 32))
+    if (p->semantic_channels > (uint32_t)kMaxSemanticChannels)
+        return fail(SPSG_ERR_INVALID_ARGUMENT, "semantic_channels must be 0 (= 14) or 1..64");
+    if ((long long)p->num_chunks * p->views_per_chunk * p->width * p->height * std::max(14, semantic_channels(p)) >= (1ll << 32))
         return fail(SPSG_ERR_INVALID_ARGUMENT, "image batch exceeds 32-bit indexing (reference limit, SURVEY 3.5)");
     if ((long long)p->num_locs * p->views_per_chunk >= (1ll << 31))
         return fail(SPSG_ERR_INVALID_ARGUMENT, "num_locs * views_per_chunk exceeds 32-bit indexing");
@@ -221,6 +231,8 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
     a.loss = make_loss_args(targets, accum);
     a.loss.loss_out = loss_out;
     a.loss.done = (int32_t *)(ws + L.head_off) + 16;  // in the per-call zeroed header, next to the list counter
+    const bool gsem = generic_semantic(p);
+    a.loss.sem_channels = semantic_channels(p);
     if (clear_grads && p->num_locs > 0) {  // rows [0, N) of the backward's outputs (kernel.cu:557-560), cleared by the forward's warps
         a.clear = *clear_grads;
         a.clear_rows = p->num_locs;
@@ -242,7 +254,9 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
         CUDA_TRY(cudaGetDevice(&dev));
         std::lock_guard<std::mutex> lk(mu);
         if (dev < 0 || dev >= 64 || !configured[dev]) {
-#define SPSG_SET_SMEM(L, M, W, VN) CUDA_TRY(cudaFuncSetAttribute(raycast_forward_kernel<L, M, W, VN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmemMax))
+#define SPSG_SET_SMEM(L, M, W, VN) \
+    CUDA_TRY(cudaFuncSetAttribute(raycast_forward_kernel<L, M, W, VN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmemMax)); \
+    CUDA_TRY(cudaFuncSetAttribute(raycast_forward_kernel<L, M, W, VN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmemMax))
 #define SPSG_SET_SMEM_ALL(VN)                                                                                   \
     SPSG_SET_SMEM(true, true, kFwdWarps, VN); SPSG_SET_SMEM(false, true, kFwdWarps, VN);                         \
     SPSG_SET_SMEM(true, false, kFwdWarps, VN); SPSG_SET_SMEM(false, false, kFwdWarps, VN);                       \
@@ -259,7 +273,9 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
         ScopedKernelTimer timer(0, st);
 #define SPSG_LAUNCH_VN(L, M, VN)                                                                                  \
     do {                                                                                                          \
-        if (large) raycast_forward_kernel<L, M, kFwdWarpsLarge, VN><<<grid, kFwdWarpsLarge * 32, dyn, st>>>(a);  \
+        if (gsem && large) raycast_forward_kernel<L, M, kFwdWarpsLarge, VN, true><<<grid, kFwdWarpsLarge * 32, dyn, st>>>(a); \
+        else if (gsem) raycast_forward_kernel<L, M, kFwdWarps, VN, true><<<grid, kFwdWarps * 32, dyn, st>>>(a);  \
+        else if (large) raycast_forward_kernel<L, M, kFwdWarpsLarge, VN><<<grid, kFwdWarpsLarge * 32, dyn, st>>>(a); \
         else raycast_forward_kernel<L, M, kFwdWarps, VN><<<grid, kFwdWarps * 32, dyn, st>>>(a);                  \
     } while (0)
 #define SPSG_LAUNCH(L, M)                                                                                         \
@@ -298,8 +314,9 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
             la.num_pixels = c.total_pixels;
             la.loss = a.loss;
             la.loss.done = (int32_t *)(ws + L.head_off) + 32;  // zeroed header, apart from the forward kernel's counters
-            losses2d_det_kernel<<<(unsigned)((c.total_pixels + kDetLossPix - 1) / kDetLossPix), kDetLossThreads, 0, st>>>(
-                la, (double *)(ws + L.det_off));
+            const unsigned blocks = (unsigned)((c.total_pixels + kDetLossPix - 1) / kDetLossPix);
+            if (gsem) losses2d_det_kernel<true><<<blocks, kDetLossThreads, 0, st>>>(la, (double *)(ws + L.det_off));
+            else losses2d_det_kernel<<<blocks, kDetLossThreads, 0, st>>>(la, (double *)(ws + L.det_off));
             CUDA_TRY(cudaGetLastError());
         }
     }
@@ -353,6 +370,34 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
     a.width = p->width; a.height = p->height;
     a.views = p->views_per_chunk; a.max_pixels = p->max_pixels_per_voxel;
     a.num_locs = p->num_locs;
+    const bool gsem = generic_semantic(p);
+    a.loss.sem_channels = semantic_channels(p);
+    // kGenericSem: the gather's rows of C + 7 floats in dynamic shared memory (above 48 KB from C = 41 on)
+    const size_t gather_dyn = gsem ? (size_t)kGatherWarps * 32 * (a.loss.sem_channels + 7) * sizeof(float) : 0;
+    if (gsem) {
+        // the opt-in limit of every generic gather, once per device and for the largest C: the attribute is process-wide,
+        // so a per-call value could be lowered by another thread between its set and this launch
+        static std::mutex mu;
+        static bool configured[64] = {false};
+        int dev = 0;
+        CUDA_TRY(cudaGetDevice(&dev));
+        std::lock_guard<std::mutex> lk(mu);
+        if (dev < 0 || dev >= 64 || !configured[dev]) {
+            constexpr int kMaxDyn = kGatherWarps * 32 * (kMaxSemanticChannels + 7) * (int)sizeof(float);
+#define SPSG_SET_GATHER(FUSED, UP, VIEWS, VN)                                                                            \
+    CUDA_TRY(cudaFuncSetAttribute(backward_gather_kernel<FUSED, UP, VIEWS, VN, false, true>,                              \
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxDyn));                                 \
+    CUDA_TRY(cudaFuncSetAttribute(backward_gather_kernel<FUSED, UP, VIEWS, VN, true, true>,                               \
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxDyn))
+#define SPSG_SET_GATHER_ROUTES(VIEWS, VN)                                                                               \
+    SPSG_SET_GATHER(false, false, VIEWS, VN); SPSG_SET_GATHER(true, false, VIEWS, VN); SPSG_SET_GATHER(true, true, VIEWS, VN)
+            SPSG_SET_GATHER_ROUTES(0, false); SPSG_SET_GATHER_ROUTES(1, false); SPSG_SET_GATHER_ROUTES(1, true);
+            SPSG_SET_GATHER_ROUTES(2, false); SPSG_SET_GATHER_ROUTES(2, true);
+#undef SPSG_SET_GATHER_ROUTES
+#undef SPSG_SET_GATHER
+            if (dev >= 0 && dev < 64) configured[dev] = true;
+        }
+    }
     const int sms = sm_count();
     // half a warp per listed (voxel, view) pair; the list length is only known on the device: size for its bound N * F
     const long long max_items = p->num_locs * p->views_per_chunk;
@@ -390,9 +435,15 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
         }
         seg.end = sa.seg_end; seg.pix = sa.seg_pix;
     }
+#define SPSG_GATHER_SEM(FUSED, UP, VIEWS, VN, SEG, BLOCKS)                                                            \
+    do {                                                                                                              \
+        backward_gather_kernel<FUSED, UP, VIEWS, VN, SEG, true><<<(BLOCKS), kGatherWarps * 32, gather_dyn, st>>>(a, seg); \
+    } while (0)
 #define SPSG_GATHER(FUSED, UP, VIEWS, VN, BLOCKS)                                                                     \
     do {                                                                                                              \
-        if (all) backward_gather_kernel<FUSED, UP, VIEWS, VN, true><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a, seg);  \
+        if (gsem && all) SPSG_GATHER_SEM(FUSED, UP, VIEWS, VN, true, BLOCKS);                                          \
+        else if (gsem) SPSG_GATHER_SEM(FUSED, UP, VIEWS, VN, false, BLOCKS);                                           \
+        else if (all) backward_gather_kernel<FUSED, UP, VIEWS, VN, true><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a, seg); \
         else backward_gather_kernel<FUSED, UP, VIEWS, VN><<<(BLOCKS), kGatherWarps * 32, 0, st>>>(a, seg);            \
     } while (0)
 #define SPSG_GATHER_VIEWS(VIEWS, VN, BLOCKS)                                                                      \
@@ -420,7 +471,9 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
         SPSG_GATHER_ANY(zero_blocks + gather_blocks);
     } else {
         a.zero_blocks = 0;
-        if (view_normals) backward_zero_view_normals_kernel<<<zero_blocks, 256, 0, st>>>(a);
+        if (gsem && view_normals) backward_zero_sem_kernel<true><<<zero_blocks, 256, 0, st>>>(a);
+        else if (gsem) backward_zero_sem_kernel<false><<<zero_blocks, 256, 0, st>>>(a);
+        else if (view_normals) backward_zero_view_normals_kernel<<<zero_blocks, 256, 0, st>>>(a);
         else backward_zero_kernel<<<zero_blocks, 256, 0, st>>>(a);
         CUDA_TRY(cudaGetLastError());
         ScopedKernelTimer timer(1, st);
@@ -429,6 +482,7 @@ int launch_backward(const spsg_raycast_params *p, bool fused, const float *g_or_
 #undef SPSG_GATHER_ANY
 #undef SPSG_GATHER_VIEWS
 #undef SPSG_GATHER
+#undef SPSG_GATHER_SEM
     CUDA_TRY(cudaGetLastError());
     return SPSG_OK;
 }
@@ -693,26 +747,39 @@ int spsg_normals_backward_views(const int64_t *locs, int64_t num_locs, const flo
     return SPSG_OK;
 }
 
-int spsg_losses2d_forward(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
-                          const float *image_semantic, int64_t num_pixels, float *loss_out, void *scratch,
-                          size_t scratch_bytes, void *stream) {
-    if (!t || !loss_out) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL loss targets / loss_out");
-    if (num_pixels < 0 || num_pixels * 14 >= (1ll << 32)) return fail(SPSG_ERR_INVALID_ARGUMENT, "bad pixel count");
+}  // extern "C"
+
+// The stand-alone 2D losses, with C logits per pixel: C = 14 and !generic are the 14-channel kernels of the original entry
+// points, anything else their kGenericSem twins.
+static int losses2d_check(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                          const float *image_semantic, int C, int64_t num_pixels, bool generic) {
+    if (C < 1 || C > kMaxSemanticChannels) return fail(SPSG_ERR_INVALID_ARGUMENT, "num_classes must be in 1..64");
+    if (num_pixels < 0 || num_pixels * std::max(14, C) >= (1ll << 32)) return fail(SPSG_ERR_INVALID_ARGUMENT, "bad pixel count");
     if ((t->target_depth && !image_depth) || (t->target_color && !image_color) || (t->target_label && !image_semantic))
         return fail(SPSG_ERR_INVALID_ARGUMENT, "a target is set but its rendering is NULL");
-    if (image_semantic && (reinterpret_cast<uintptr_t>(image_semantic) & 7u)) return fail(SPSG_ERR_INVALID_ARGUMENT, "image_semantic must be 8-byte aligned");
+    if (!generic && image_semantic && (reinterpret_cast<uintptr_t>(image_semantic) & 7u))
+        return fail(SPSG_ERR_INVALID_ARGUMENT, "image_semantic must be 8-byte aligned");
+    return SPSG_OK;
+}
+
+static int losses2d_forward_impl(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                                 const float *image_semantic, int C, bool generic, int64_t num_pixels, float *loss_out,
+                                 void *scratch, size_t scratch_bytes, cudaStream_t st) {
+    if (!t || !loss_out) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL loss targets / loss_out");
+    if (int rc = losses2d_check(t, image_color, image_depth, image_semantic, C, num_pixels, generic)) return rc;
     const size_t need = (size_t)kLossSlots * 8 * sizeof(double);
     if (!scratch || scratch_bytes < need || (reinterpret_cast<uintptr_t>(scratch) & 7u)) return fail(SPSG_ERR_WORKSPACE_TOO_SMALL, "scratch too small");
-    cudaStream_t st = (cudaStream_t)stream;
     CUDA_TRY(cudaMemsetAsync(scratch, 0, need, st));
     Losses2DArgs a;
     memset(&a, 0, sizeof(a));
     a.image_color = image_color; a.image_depth = image_depth; a.image_semantic = image_semantic;
     a.loss = make_loss_args(t, (double *)scratch);
     a.num_pixels = num_pixels;
+    a.loss.sem_channels = C;
     if (num_pixels > 0) {
         const unsigned blocks = (unsigned)std::min<long long>((num_pixels + 255) / 256, (long long)sm_count() * 8);
-        losses2d_forward_kernel<<<blocks, 256, 0, st>>>(a);
+        if (generic) losses2d_forward_kernel<true><<<blocks, 256, 0, st>>>(a);
+        else losses2d_forward_kernel<<<blocks, 256, 0, st>>>(a);
         CUDA_TRY(cudaGetLastError());
     }
     finalize_loss_kernel<<<1, 32, 0, st>>>((const double *)scratch, loss_out, t->weight_depth, t->weight_color_loss,
@@ -722,23 +789,14 @@ int spsg_losses2d_forward(const spsg_loss_targets *t, const float *image_color, 
     return SPSG_OK;
 }
 
-size_t spsg_losses2d_deterministic_scratch_bytes(int64_t num_pixels) {
-    if (num_pixels < 0) return 0;
-    return (size_t)kLossSlots * 8 * sizeof(double) + 256 + det_loss_partials_bytes(num_pixels);
-}
-
-int spsg_losses2d_forward_deterministic(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
-                                        const float *image_semantic, int64_t num_pixels, float *loss_out, void *scratch,
-                                        size_t scratch_bytes, void *stream) {
+static int losses2d_forward_det_impl(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                                     const float *image_semantic, int C, bool generic, int64_t num_pixels, float *loss_out,
+                                     void *scratch, size_t scratch_bytes, cudaStream_t st) {
     if (!t || !loss_out) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL loss targets / loss_out");
-    if (num_pixels < 0 || num_pixels * 14 >= (1ll << 32)) return fail(SPSG_ERR_INVALID_ARGUMENT, "bad pixel count");
-    if ((t->target_depth && !image_depth) || (t->target_color && !image_color) || (t->target_label && !image_semantic))
-        return fail(SPSG_ERR_INVALID_ARGUMENT, "a target is set but its rendering is NULL");
-    if (image_semantic && (reinterpret_cast<uintptr_t>(image_semantic) & 7u)) return fail(SPSG_ERR_INVALID_ARGUMENT, "image_semantic must be 8-byte aligned");
+    if (int rc = losses2d_check(t, image_color, image_depth, image_semantic, C, num_pixels, generic)) return rc;
     if (!scratch || scratch_bytes < spsg_losses2d_deterministic_scratch_bytes(num_pixels) ||
         (reinterpret_cast<uintptr_t>(scratch) & 7u))
         return fail(SPSG_ERR_WORKSPACE_TOO_SMALL, "scratch too small");
-    cudaStream_t st = (cudaStream_t)stream;
     // [slots of the final stage | done counter | per-block partials]
     const size_t slots = (size_t)kLossSlots * 8 * sizeof(double);
     CUDA_TRY(cudaMemsetAsync(scratch, 0, slots + 256, st));
@@ -749,9 +807,12 @@ int spsg_losses2d_forward_deterministic(const spsg_loss_targets *t, const float 
     a.loss.loss_out = loss_out;
     a.loss.done = (int32_t *)((uint8_t *)scratch + slots);
     a.num_pixels = num_pixels;
+    a.loss.sem_channels = C;
     if (num_pixels > 0) {
-        losses2d_det_kernel<<<(unsigned)((num_pixels + kDetLossPix - 1) / kDetLossPix), kDetLossThreads, 0, st>>>(
-            a, (double *)((uint8_t *)scratch + slots + 256));
+        const unsigned blocks = (unsigned)((num_pixels + kDetLossPix - 1) / kDetLossPix);
+        double *partials = (double *)((uint8_t *)scratch + slots + 256);
+        if (generic) losses2d_det_kernel<true><<<blocks, kDetLossThreads, 0, st>>>(a, partials);
+        else losses2d_det_kernel<<<blocks, kDetLossThreads, 0, st>>>(a, partials);
     } else {
         finalize_loss_kernel<<<1, 32, 0, st>>>((const double *)scratch, loss_out, t->weight_depth, t->weight_color_loss,
                                                t->weight_semantic, t->target_depth != nullptr, t->target_color != nullptr,
@@ -761,14 +822,12 @@ int spsg_losses2d_forward_deterministic(const spsg_loss_targets *t, const float 
     return SPSG_OK;
 }
 
-int spsg_losses2d_backward(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
-                           const float *image_semantic, int64_t num_pixels, const float *loss_out,
-                           const float *grad_scale, float *d_color, float *d_depth, float *d_semantic, void *stream) {
+static int losses2d_backward_impl(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                                  const float *image_semantic, int C, bool generic, int64_t num_pixels, const float *loss_out,
+                                  const float *grad_scale, float *d_color, float *d_depth, float *d_semantic, cudaStream_t st) {
     if (!t || !loss_out) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL loss targets / loss_out");
-    if (num_pixels < 0 || num_pixels * 14 >= (1ll << 32)) return fail(SPSG_ERR_INVALID_ARGUMENT, "bad pixel count");
-    if ((t->target_depth && !image_depth) || (t->target_color && !image_color) || (t->target_label && !image_semantic))
-        return fail(SPSG_ERR_INVALID_ARGUMENT, "a target is set but its rendering is NULL");
-    if (d_semantic && (reinterpret_cast<uintptr_t>(d_semantic) & 7u)) return fail(SPSG_ERR_INVALID_ARGUMENT, "d_semantic must be 8-byte aligned");
+    if (int rc = losses2d_check(t, image_color, image_depth, image_semantic, C, num_pixels, generic)) return rc;
+    if (!generic && d_semantic && (reinterpret_cast<uintptr_t>(d_semantic) & 7u)) return fail(SPSG_ERR_INVALID_ARGUMENT, "d_semantic must be 8-byte aligned");
     if (num_pixels == 0) return SPSG_OK;
     BackwardArgs a;
     memset(&a, 0, sizeof(a));
@@ -777,10 +836,68 @@ int spsg_losses2d_backward(const spsg_loss_targets *t, const float *image_color,
     a.loss_out = loss_out;
     a.w_depth = t->weight_depth; a.w_color = t->weight_color_loss; a.w_sem = t->weight_semantic;
     a.grad_scale = grad_scale;
-    const unsigned blocks = (unsigned)std::min<long long>((num_pixels + 255) / 256, (long long)sm_count() * 8);
-    losses2d_backward_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(a, num_pixels, d_color, d_depth, d_semantic);
+    a.loss.sem_channels = C;
+    if (generic) {
+        // 128 threads: each thread's row of C + 7 gradients in shared memory stays under 48 KB up to C = 64
+        const unsigned blocks = (unsigned)std::min<long long>((num_pixels + 127) / 128, (long long)sm_count() * 16);
+        losses2d_backward_kernel<true><<<blocks, 128, 128 * (C + 7) * sizeof(float), st>>>(a, num_pixels, d_color, d_depth, d_semantic);
+    } else {
+        const unsigned blocks = (unsigned)std::min<long long>((num_pixels + 255) / 256, (long long)sm_count() * 8);
+        losses2d_backward_kernel<<<blocks, 256, 0, st>>>(a, num_pixels, d_color, d_depth, d_semantic);
+    }
     CUDA_TRY(cudaGetLastError());
     return SPSG_OK;
+}
+
+extern "C" {
+
+int spsg_losses2d_forward(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                          const float *image_semantic, int64_t num_pixels, float *loss_out, void *scratch,
+                          size_t scratch_bytes, void *stream) {
+    return losses2d_forward_impl(t, image_color, image_depth, image_semantic, 14, false, num_pixels, loss_out, scratch,
+                                 scratch_bytes, (cudaStream_t)stream);
+}
+
+int spsg_losses2d_forward_classes(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                                  const float *image_semantic, int32_t num_classes, int64_t num_pixels, float *loss_out,
+                                  void *scratch, size_t scratch_bytes, void *stream) {
+    return losses2d_forward_impl(t, image_color, image_depth, image_semantic, num_classes, true, num_pixels, loss_out,
+                                 scratch, scratch_bytes, (cudaStream_t)stream);
+}
+
+size_t spsg_losses2d_deterministic_scratch_bytes(int64_t num_pixels) {
+    if (num_pixels < 0) return 0;
+    return (size_t)kLossSlots * 8 * sizeof(double) + 256 + det_loss_partials_bytes(num_pixels);
+}
+
+int spsg_losses2d_forward_deterministic(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                                        const float *image_semantic, int64_t num_pixels, float *loss_out, void *scratch,
+                                        size_t scratch_bytes, void *stream) {
+    return losses2d_forward_det_impl(t, image_color, image_depth, image_semantic, 14, false, num_pixels, loss_out, scratch,
+                                     scratch_bytes, (cudaStream_t)stream);
+}
+
+int spsg_losses2d_forward_deterministic_classes(const spsg_loss_targets *t, const float *image_color,
+                                                const float *image_depth, const float *image_semantic, int32_t num_classes,
+                                                int64_t num_pixels, float *loss_out, void *scratch, size_t scratch_bytes,
+                                                void *stream) {
+    return losses2d_forward_det_impl(t, image_color, image_depth, image_semantic, num_classes, true, num_pixels, loss_out,
+                                     scratch, scratch_bytes, (cudaStream_t)stream);
+}
+
+int spsg_losses2d_backward(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                           const float *image_semantic, int64_t num_pixels, const float *loss_out,
+                           const float *grad_scale, float *d_color, float *d_depth, float *d_semantic, void *stream) {
+    return losses2d_backward_impl(t, image_color, image_depth, image_semantic, 14, false, num_pixels, loss_out, grad_scale,
+                                  d_color, d_depth, d_semantic, (cudaStream_t)stream);
+}
+
+int spsg_losses2d_backward_classes(const spsg_loss_targets *t, const float *image_color, const float *image_depth,
+                                   const float *image_semantic, int32_t num_classes, int64_t num_pixels,
+                                   const float *loss_out, const float *grad_scale, float *d_color, float *d_depth,
+                                   float *d_semantic, void *stream) {
+    return losses2d_backward_impl(t, image_color, image_depth, image_semantic, num_classes, true, num_pixels, loss_out,
+                                  grad_scale, d_color, d_depth, d_semantic, (cudaStream_t)stream);
 }
 
 }  // extern "C"

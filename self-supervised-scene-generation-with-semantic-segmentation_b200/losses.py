@@ -7,6 +7,9 @@ kernel, accumulates the reference's three 2D loss terms
     colour L1     mean |colour * w - target * w|            over hit pixels x 3 channels      loss.py:246-257
     semantic CE   sum w[y] * nll / sum w[y]                 over (hit & label < 14)           train.py:744-746
 
+With C semantic classes (``RaycastRGBD(..., num_classes=C)``, or C-channel renderings for the stand-alone ops) every 14
+is C: C logits, label C = ignore, ``class_weight`` of length C.  C is taken from the tensors.
+
 Its backward never materialises the loss terms' gradient images: every registered pixel's gradient is recomputed from
 (rendering, target, normalisers) inside the per-voxel gather, which can also add the caller's own gradient images of the
 renderings (``differentiable_images=True``).  No CPU path.
@@ -22,25 +25,31 @@ from . import raycast_rgbd_cuda as rc
 
 def labels_from_render(raycast_semantic, histogram=False):
     """target2d_label of train.py:614-616 / pred2d_label of :749-752: ``argmax(cat(render, ones), -1)`` as uint8
-    (14 = miss or unlabeled), shape ``raycast_semantic.shape[:-1]``, in one pass over the rendering.  With
-    ``histogram=True`` also returns the number of pixels per label (15 int64, on the device) from the same pass."""
+    (C = miss or unlabeled, C = ``raycast_semantic.shape[-1]``, 14 in the reference), shape ``raycast_semantic.shape[:-1]``,
+    in one pass over the rendering.  With ``histogram=True`` also returns the number of pixels per label (C + 1 int64, on
+    the device) from the same pass."""
     sem = raycast_semantic.detach()
     rc._check_input(sem, "raycast_semantic")
     rc._check_dtype(sem, torch.float32, "raycast_semantic")
-    if sem.shape[-1] != 14:
-        raise RuntimeError("raycast_semantic must have 14 channels")
-    if sem.data_ptr() % 8:
+    c = int(sem.shape[-1])
+    if not 1 <= c <= N.SPSG_MAX_SEMANTIC_CHANNELS:
+        raise RuntimeError("raycast_semantic must have 1..%d channels, got %d" % (N.SPSG_MAX_SEMANTIC_CHANNELS, c))
+    if c == 14 and sem.data_ptr() % 8:
         sem = sem.clone()
     labels = torch.empty(sem.shape[:-1], dtype=torch.uint8, device=sem.device)
-    hist = torch.empty(15, dtype=torch.int64, device=sem.device) if histogram else None
+    hist = torch.empty(c + 1, dtype=torch.int64, device=sem.device) if histogram else None
     with rc.device_guard(sem.device):
-        N.check(N.lib.spsg_labels_from_render(N.ptr(sem), labels.numel(), N.ptr(labels), N.ptr(hist),
-                                              rc._stream(sem.device)))
+        if c == 14:
+            N.check(N.lib.spsg_labels_from_render(N.ptr(sem), labels.numel(), N.ptr(labels), N.ptr(hist),
+                                                  rc._stream(sem.device)))
+        else:
+            N.check(N.lib.spsg_labels_from_render_classes(N.ptr(sem), c, labels.numel(), N.ptr(labels), N.ptr(hist),
+                                                          rc._stream(sem.device)))
     return (labels, hist) if histogram else labels
 
 
 def _targets_struct(images, h, w, target_depth, target_color, weight_color, target_label, class_weight, voxelsize,
-                    weights):
+                    weights, classes=14):
     def chk(t, numel, dtype, name):
         if t is None:
             return None
@@ -52,7 +61,7 @@ def _targets_struct(images, h, w, target_depth, target_color, weight_color, targ
                       N.ptr(chk(target_color, 3 * px, torch.float32, "target_color")),
                       N.ptr(chk(weight_color, px, torch.float32, "weight_color")),
                       N.ptr(chk(target_label, px, torch.uint8, "target_label")),
-                      N.ptr(chk(class_weight, 14, torch.float32, "class_weight")),
+                      N.ptr(chk(class_weight, classes, torch.float32, "class_weight")),
                       float(voxelsize), float(weights[0]), float(weights[1]), float(weights[2]))
     return t
 
@@ -76,26 +85,30 @@ def fused_forward(m, locs, vals_sdf, vals_colors, vals_normals, vals_semantic, v
         raise RuntimeError("view_matrix has %d images: expected batch_size (%d) x views <= max_num_frames (%d)"
                            % (images, m.batch_size, m.max_num_frames))
     per_view = rc.view_normals(vals_normals, views)
+    c = rc.semantic_channels(m.image_semantic)
+    if c != 14 and (vals_semantic.dim() != 2 or vals_semantic.shape[1] != c):
+        raise RuntimeError("vals_semantics must be (N, %d), got %s" % (c, tuple(vals_semantic.shape)))
     n = rc.check_voxel_inputs(locs, vals_sdf, vals_colors, vals_normals, vals_semantic, view_matrix, intrinsic_params,
-                              images, views if per_view else 1)
+                              images, views if per_view else 1, c)
     flags = rc.with_torch_mode(m.flags | (N.SPSG_FLAG_VIEW_NORMALS if per_view else 0))
     rows, max_pixels = rc.table_shape(m.mapping3dto2d, m.mapping3dto2d_num, flags)
     if n * views > rows:
         raise RuntimeError("too many voxels for raycast (%d x %d views > %d rows)" % (n, views, rows))
     d_normal = rc.normal_grad_buffer(m, per_view)
     if clear_grads and (m.d_depth.shape[0] < n or m.d_color.shape[0] < n or
-                        d_normal.shape[0] < n * (views if per_view else 1) or m.d_semantic.shape[0] < n):
+                        d_normal.shape[0] < n * (views if per_view else 1) or m.d_semantic.shape[0] < n or
+                        m.d_semantic.numel() < c * n):
         raise RuntimeError("d_* buffers hold fewer than N = %d rows" % n)
     dev = vals_sdf.device
     if m.image_depth.device != dev:
         raise RuntimeError("raycaster buffers live on %s, inputs on %s" % (m.image_depth.device, dev))
     p = N.make_params(m.width, m.height, m.depth_min, m.depth_max, m.thresh_sample_dist, m.ray_increment,
-                      m.dims3d[2], m.dims3d[1], m.dims3d[0], m.batch_size, views, max_pixels, n, flags)
+                      m.dims3d[2], m.dims3d[1], m.dims3d[0], m.batch_size, views, max_pixels, n, flags, c)
     if rc.is_packed_locs(locs):
         p.flags |= N.SPSG_FLAG_PACKED_LOCS
     target_depth, target_color, weight_color, target_label, class_weight, voxelsize, weights = targets
     tg = _targets_struct(images, m.height, m.width, target_depth, target_color, weight_color, target_label, class_weight,
-                         voxelsize, weights)
+                         voxelsize, weights, c)
     # terms, total and normalisers of THIS call (the backward reads the normalisers back)
     loss_out = torch.empty(N.SPSG_LOSS_OUT_FLOATS, device=dev)
     gb = N.grad_buffers(m.d_color, m.d_depth, d_normal, m.d_semantic) if clear_grads else None
@@ -125,7 +138,8 @@ def _upstream_struct(m, p, upstream):
     images = p.num_chunks * p.views_per_chunk
     px = images * p.height * p.width
     ptrs = []
-    for g, ch, name in zip(upstream, (3, 1, 3, 14), ("grad_color", "grad_depth", "grad_normal", "grad_semantic")):
+    for g, ch, name in zip(upstream, (3, 1, 3, p.semantic_channels or 14),
+                           ("grad_color", "grad_depth", "grad_normal", "grad_semantic")):
         if g is not None:
             rc._check_input(g, name)
             rc._check_dtype(g, torch.float32, name)
@@ -286,7 +300,8 @@ def render_with_2d_losses(raycaster, locs, vals_sdf, vals_colors, vals_normals, 
     images_depth     (I,H,W) or (I,1,H,W) metres, 0 = hole;  None switches the depth term off
     images_color     (I,H,W,3) channels-last (the reference passes images_color.permute(0,2,3,1)); None = off
     weight_color     (I,H,W) or (I,1,H,W) per-pixel colour weight or None
-    target2d_label   (I,H,W) or (I,H,W,1) uint8, 14 = ignore; None switches the semantic term off
+    target2d_label   (I,H,W) or (I,H,W,1) uint8, 14 (C) = ignore; None switches the semantic term off
+    weight_semantic_class  (C) class weights or None; C = the raycaster's ``num_classes``
     Returns (total, terms[3] = (depth, colour, semantic), (color, depth, normal, semantic) renderings).
     ``total = weight_depth_loss*depth + weight_color_loss*colour + weight_semantic_loss*semantic``; ``terms`` are
     reported values, like the ``.item()`` logging in train.py.  Gradients flow from ``total`` and, with
@@ -298,7 +313,7 @@ def render_with_2d_losses(raycaster, locs, vals_sdf, vals_colors, vals_normals, 
     ``differentiable_images=True`` they are saved for the backward, and modifying one in place before ``backward()``
     raises autograd's version-counter error."""
     if vals_semantics is None:
-        vals_semantics = torch.zeros(vals_sdf.shape[0], 14, device=vals_sdf.device)
+        vals_semantics = torch.zeros(vals_sdf.shape[0], raycaster.image_semantic.shape[-1], device=vals_sdf.device)
     out = FusedRaycastLossFunction.apply(
         raycaster, locs, vals_sdf, vals_colors, vals_normals, vals_semantics, view_matrix, intrinsic_params,
         None if images_depth is None else images_depth.contiguous(),
@@ -322,9 +337,10 @@ class _Losses2D(Function):
                 class_weight, voxelsize, weights):
         some = next(t for t in (image_color, image_depth, image_semantic) if t is not None)
         dev = some.device
+        classes = 14 if image_semantic is None else rc.semantic_channels(image_semantic)
         px = {"c": None if image_color is None else image_color.numel() // 3,
               "d": None if image_depth is None else image_depth.numel(),
-              "s": None if image_semantic is None else image_semantic.numel() // 14}
+              "s": None if image_semantic is None else image_semantic.numel() // classes}
         num_pixels = next(v for v in px.values() if v is not None)
         if any(v is not None and v != num_pixels for v in px.values()):
             raise RuntimeError("renderings disagree on the number of pixels")
@@ -333,17 +349,23 @@ class _Losses2D(Function):
                 rc._check_input(t, name)
                 rc._check_dtype(t, torch.float32, name)
         tg = _targets_struct(1, 1, num_pixels, target_depth, target_color, weight_color, target_label, class_weight,
-                             voxelsize, weights)
+                             voxelsize, weights, classes)
         loss_out = torch.empty(N.SPSG_LOSS_OUT_FLOATS, device=dev)
         # deterministic algorithms: the sums in pixel order (per-block partials in a scratch that grows with the image)
         det = torch.are_deterministic_algorithms_enabled()
-        forward = N.lib.spsg_losses2d_forward_deterministic if det else N.lib.spsg_losses2d_forward
         scratch = torch.empty(N.lib.spsg_losses2d_deterministic_scratch_bytes(num_pixels) if det else 4096,
                               dtype=torch.uint8, device=dev)
+        imgs = (N.ptr(image_color), N.ptr(image_depth), N.ptr(image_semantic))
         with rc.device_guard(dev):
-            N.check(forward(ctypes.byref(tg), N.ptr(image_color), N.ptr(image_depth), N.ptr(image_semantic), num_pixels,
-                            N.ptr(loss_out), N.ptr(scratch), scratch.numel(), rc._stream(dev)))
-        ctx.targets, ctx.num_pixels, ctx.loss_out = tg, num_pixels, loss_out
+            if classes == 14:
+                forward = N.lib.spsg_losses2d_forward_deterministic if det else N.lib.spsg_losses2d_forward
+                N.check(forward(ctypes.byref(tg), *imgs, num_pixels, N.ptr(loss_out), N.ptr(scratch), scratch.numel(),
+                                rc._stream(dev)))
+            else:
+                forward = N.lib.spsg_losses2d_forward_deterministic_classes if det else N.lib.spsg_losses2d_forward_classes
+                N.check(forward(ctypes.byref(tg), *imgs, classes, num_pixels, N.ptr(loss_out), N.ptr(scratch),
+                                scratch.numel(), rc._stream(dev)))
+        ctx.targets, ctx.num_pixels, ctx.loss_out, ctx.classes = tg, num_pixels, loss_out, classes
         ctx.keep = (target_depth, target_color, weight_color, target_label, class_weight)
         ctx.save_for_backward(*[t for t in (image_color, image_depth, image_semantic) if t is not None])
         ctx.present = tuple(t is not None for t in (image_color, image_depth, image_semantic))
@@ -359,10 +381,14 @@ class _Losses2D(Function):
         need = ctx.needs_input_grad[:3]
         grads = [torch.empty_like(t) if (t is not None and n) else None for t, n in zip(imgs, need)]
         scale = grad_total.to(torch.float32).contiguous()
+        ptrs = (N.ptr(imgs[0]), N.ptr(imgs[1]), N.ptr(imgs[2]))
+        outs = (N.ptr(ctx.loss_out), N.ptr(scale), N.ptr(grads[0]), N.ptr(grads[1]), N.ptr(grads[2]), rc._stream(dev))
         with rc.device_guard(dev):
-            N.check(N.lib.spsg_losses2d_backward(ctypes.byref(ctx.targets), N.ptr(imgs[0]), N.ptr(imgs[1]), N.ptr(imgs[2]),
-                                                 ctx.num_pixels, N.ptr(ctx.loss_out), N.ptr(scale), N.ptr(grads[0]),
-                                                 N.ptr(grads[1]), N.ptr(grads[2]), rc._stream(dev)))
+            if ctx.classes == 14:
+                N.check(N.lib.spsg_losses2d_backward(ctypes.byref(ctx.targets), *ptrs, ctx.num_pixels, *outs))
+            else:
+                N.check(N.lib.spsg_losses2d_backward_classes(ctypes.byref(ctx.targets), *ptrs, ctx.classes, ctx.num_pixels,
+                                                             *outs))
         return (grads[0], grads[1], grads[2]) + (None,) * 7
 
 
@@ -390,6 +416,6 @@ def color_l1_loss(raycast_color, target_color, weight_color=None):
 
 
 def semantic_2d_ce_loss(raycast_semantic, target2d_label, weight_semantic_class=None):
-    """train.py:744-746: class-weighted cross-entropy over (label < 14 & rendered)."""
+    """train.py:744-746: class-weighted cross-entropy over (label < C & rendered), C = ``raycast_semantic.shape[-1]``."""
     return losses_2d(raycast_semantic=raycast_semantic, target2d_label=target2d_label,
                      weight_semantic_class=weight_semantic_class)[0]

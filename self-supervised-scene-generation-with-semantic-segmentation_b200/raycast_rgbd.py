@@ -18,6 +18,8 @@ Differences, all behind defaulted extras or unobservable through the reference A
     the voxel -> pixel tables are canonical and the gradients bit-reproducible; forward and backward must agree on it.
   * ``max_pixels_per_voxel=None``: the gradient of a (voxel, view) is the mean over every pixel it received, not over the
     first ``max_pixels_per_voxel`` (SPSG_FLAG_ALL_PIXELS in ``flags``); no ``mapping3dto2d`` table is allocated.
+  * ``num_classes=C``: semantic payloads, renderings and gradients of C channels instead of the reference's 14 (1..64;
+    e.g. 20 for ScanNet, 41 for NYU40 / mpcat40).  Geometry does not depend on C.
 """
 import torch
 from torch import nn
@@ -95,7 +97,7 @@ class RayCastRGBDFunction(Function):
 
 class RaycastRGBD(nn.Module):
     def __init__(self, batch_size, dims3d, width, height, depth_min, depth_max, thresh_sample_dist, ray_increment,
-                 max_num_frames=1, max_num_locs_per_sample=200000, max_pixels_per_voxel=64, device=None):
+                 max_num_frames=1, max_num_locs_per_sample=200000, max_pixels_per_voxel=64, device=None, num_classes=14):
         super(RaycastRGBD, self).__init__()
         if not torch.cuda.is_available():
             raise RuntimeError("RaycastRGBD needs a CUDA device: this implementation has no CPU path")
@@ -110,13 +112,16 @@ class RaycastRGBD(nn.Module):
         self.thresh_sample_dist = thresh_sample_dist
         self.ray_increment = ray_increment
         self.max_num_locs_per_sample = max_num_locs_per_sample
+        if not 1 <= num_classes <= N.SPSG_MAX_SEMANTIC_CHANNELS:
+            raise RuntimeError("num_classes must be in 1..%d, got %d" % (N.SPSG_MAX_SEMANTIC_CHANNELS, num_classes))
+        self.num_classes = num_classes
         images = batch_size * max_num_frames
         rows = batch_size * max_num_frames * max_num_locs_per_sample
         # same buffers, shapes and dtypes as raycast_rgbd.py:59-72, allocated directly on the device
         self.image_depth = torch.zeros(images, height, width, device=device)
         self.image_normal = torch.zeros(images, height, width, 3, device=device)
         self.image_color = torch.zeros(images, height, width, 3, device=device)
-        self.image_semantic = torch.zeros(images, height, width, 14, device=device)
+        self.image_semantic = torch.zeros(images, height, width, num_classes, device=device)
         # max_pixels_per_voxel=None: every pixel of a (voxel, view) enters its gradient (SPSG_FLAG_ALL_PIXELS), no table
         self.mapping3dto2d = torch.zeros(rows, max_pixels_per_voxel, dtype=torch.int, device=device) \
             if max_pixels_per_voxel is not None else torch.empty(0, dtype=torch.int, device=device)
@@ -125,7 +130,7 @@ class RaycastRGBD(nn.Module):
         self.d_color = torch.zeros(batch_size * max_num_locs_per_sample, 3, device=device)
         self.d_normal = torch.zeros(batch_size * max_num_locs_per_sample, 3, device=device)
         self.d_depth = torch.zeros(batch_size * max_num_locs_per_sample, 1, device=device)
-        self.d_semantic = torch.zeros(batch_size * max_num_locs_per_sample, 14, device=device)
+        self.d_semantic = torch.zeros(batch_size * max_num_locs_per_sample, num_classes, device=device)
         self.d_normal_views = None  # (N*F,3) gradient rows of per-view normals (raycast_rgbd_cuda.normal_grad_buffer)
         # SPSG_FLAG_* (e.g. _native.SPSG_FLAG_DETERMINISTIC for bit-reproducible tables, losses and gradients; it is also on
         # whenever torch.use_deterministic_algorithms(True) is).  SPSG_FLAG_ALL_PIXELS marks the module without a table:
@@ -139,7 +144,10 @@ class RaycastRGBD(nn.Module):
 
     def forward(self, locs, vals_sdf, vals_colors, vals_normals, vals_semantics, view_matrix, intrinsic_params):
         if vals_semantics is None:
-            vals_semantics = torch.zeros(vals_sdf.shape[0], 14, device=vals_sdf.device)  # unlabeled class
+            vals_semantics = torch.zeros(vals_sdf.shape[0], self.num_classes, device=vals_sdf.device)  # unlabeled class
+        elif self.num_classes != 14 and (vals_semantics.dim() != 2 or vals_semantics.shape[1] != self.num_classes):
+            # (at 14 the reference's behaviour stays: any payload with at least 14 * N values is read as (N,14))
+            raise RuntimeError("vals_semantics must be (N, %d), got %s" % (self.num_classes, tuple(vals_semantics.shape)))
         images = view_matrix.shape[0]
         views = max(1, images // self.batch_size)
         if images != views * self.batch_size or views > self.max_num_frames:

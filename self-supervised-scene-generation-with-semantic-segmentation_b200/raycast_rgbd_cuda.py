@@ -47,10 +47,10 @@ def _check_dtype(t, dtype, name):
 
 
 def check_voxel_inputs(locs, vals_sdf, vals_color, vals_normals, vals_semantic, view_matrix, intrinsic_params, images,
-                       normal_views=1):
+                       normal_views=1, semantic_channels=14):
     """What every raw-pointer entry point relies on: CUDA + contiguous, int64 `locs` rows of 4, float32 payloads with at
-    least N rows of 1 / 3 / 3 / 14 (normals: N * ``normal_views`` rows of 3 with SPSG_FLAG_VIEW_NORMALS), cameras for every
-    image.  Raises RuntimeError like the reference's AT_ASSERTM."""
+    least N rows of 1 / 3 / 3 / C (normals: N * ``normal_views`` rows of 3 with SPSG_FLAG_VIEW_NORMALS; C =
+    ``semantic_channels``), cameras for every image.  Raises RuntimeError like the reference's AT_ASSERTM."""
     for t, name in ((locs, "locs"), (vals_sdf, "vals_sdf"), (vals_color, "vals_color"), (vals_normals, "vals_normals"),
                     (vals_semantic, "vals_semantic"), (view_matrix, "viewMatrixInv"), (intrinsic_params, "intrinsicParams")):
         _check_input(t, name)
@@ -63,7 +63,7 @@ def check_voxel_inputs(locs, vals_sdf, vals_color, vals_normals, vals_semantic, 
     if not is_packed_locs(locs) and locs.numel() != 4 * n:
         raise RuntimeError("locs must be (N, 4) rows of (z, y, x, chunk)")
     if vals_sdf.numel() < n or vals_color.numel() < 3 * n or vals_normals.numel() < 3 * n * normal_views or \
-            vals_semantic.numel() < 14 * n:
+            vals_semantic.numel() < semantic_channels * n:
         raise RuntimeError("voxel value tensors hold fewer than N = %d rows" % n)
     if view_matrix.numel() < images * 16 or intrinsic_params.numel() < images * 4:
         raise RuntimeError("viewMatrixInv / intrinsicParams hold fewer than %d images" % images)
@@ -149,9 +149,18 @@ def table_ptr(mapping3dto2d, flags):
     return None if all_pixels(flags) else N.ptr(mapping3dto2d)
 
 
+def semantic_channels(t):
+    """C of a call, from the last dimension of its semantic image (or gradient image): the reference's buffers are
+    (I,H,W,14).  1..64, else RuntimeError."""
+    c = int(t.shape[-1]) if t.dim() >= 2 else 14
+    if not 1 <= c <= N.SPSG_MAX_SEMANTIC_CHANNELS:
+        raise RuntimeError("semantic images must have 1..%d channels, got %d" % (N.SPSG_MAX_SEMANTIC_CHANNELS, c))
+    return c
+
+
 def _stamp(p):
     return (int(p.num_locs), int(p.views_per_chunk), int(p.num_chunks), int(p.width), int(p.height),
-            int(p.max_pixels_per_voxel), bool(p.flags & N.SPSG_FLAG_VIEW_NORMALS),
+            int(p.max_pixels_per_voxel), "%d classes" % (p.semantic_channels or 14), bool(p.flags & N.SPSG_FLAG_VIEW_NORMALS),
             "deterministic" if p.flags & N.SPSG_FLAG_DETERMINISTIC else "default",
             "all pixels" if p.flags & N.SPSG_FLAG_ALL_PIXELS else "table")
 
@@ -271,12 +280,13 @@ def construct_dense_sparse_mapping(locs, sparse_mapping):
                                        _stream(sparse_mapping.device)))
 
 
-def _forward_params(sparse_mapping, locs, max_pixels, opts, views_per_chunk=1, flags=0):
+def _forward_params(sparse_mapping, locs, max_pixels, opts, views_per_chunk=1, flags=0, semantic_channels=14):
     o = opts.tolist() if isinstance(opts, torch.Tensor) else list(opts)
     return N.make_params(width=_opt_int(o[0]), height=_opt_int(o[1]), depth_min=o[2], depth_max=o[3],
                          thresh_sample_dist=o[4], ray_increment=o[5], dimx=_opt_int(o[6]), dimy=_opt_int(o[7]),
                          dimz=_opt_int(o[8]), num_chunks=sparse_mapping.shape[0], views_per_chunk=views_per_chunk,
-                         max_pixels_per_voxel=max_pixels, num_locs=locs.shape[0], flags=flags)
+                         max_pixels_per_voxel=max_pixels, num_locs=locs.shape[0], flags=flags,
+                         semantic_channels=semantic_channels)
 
 
 def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_semantic, viewMatrixInv, imageColor,
@@ -289,7 +299,8 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
     ``workspace_owner`` = the calling module's ``ModuleWorkspace`` (else the scratch is looked up by ``sparse_mapping``).
     Deterministic mode (SPSG_FLAG_DETERMINISTIC) is on when ``flags`` has it or torch's deterministic algorithms are enabled;
     the matching ``backward`` must run in the same mode.  With SPSG_FLAG_ALL_PIXELS in ``flags`` no table is written:
-    ``mapping3dto2d`` may be None or empty, and the backward (same flag) averages every pixel of a row."""
+    ``mapping3dto2d`` may be None or empty, and the backward (same flag) averages every pixel of a row.  The semantic class
+    count C is ``imageSemantic.shape[-1]`` (14 for the reference's buffers): ``vals_semantic`` is then read as (N,C)."""
     flags = with_torch_mode(flags)
     table = () if all_pixels(flags) else ((mapping3dto2d, "mapping3dto2d"),)
     for t, name in ((sparse_mapping, "sparse_mapping"), (imageColor, "imageColor"), (imageDepth, "imageDepth"),
@@ -304,7 +315,8 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
                     (imageSemantic, "imageSemantic")):
         _check_dtype(t, torch.float32, name)
     rows, max_pixels = table_shape(mapping3dto2d, mapping3dto2d_num, flags)
-    p = _forward_params(sparse_mapping, locs, max_pixels, opts, views_per_chunk, flags)
+    c = semantic_channels(imageSemantic)
+    p = _forward_params(sparse_mapping, locs, max_pixels, opts, views_per_chunk, flags, c)
     if is_packed_locs(locs):
         if not build_index:
             raise RuntimeError("packed locs need build_index=True")
@@ -312,12 +324,12 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
     images = p.num_chunks * p.views_per_chunk
     nv = p.views_per_chunk if flags & N.SPSG_FLAG_VIEW_NORMALS else 1
     n = check_voxel_inputs(locs, vals_sdf, vals_color, vals_normals, vals_semantic, viewMatrixInv, intrinsicParams, images,
-                           nv)
+                           nv, c)
     if mapping3dto2d_num.numel() < p.views_per_chunk * n or rows < p.views_per_chunk * n:
         raise RuntimeError("mapping3dto2d has %d rows, needs views_per_chunk*N = %d" % (rows, p.views_per_chunk * n))
     px = images * p.width * p.height
     if imageDepth.numel() < px or imageColor.numel() < 3 * px or imageNormal.numel() < 3 * px or \
-            imageSemantic.numel() < 14 * px:
+            imageSemantic.numel() < c * px:
         raise RuntimeError("image buffers are smaller than %d x %d x %d" % (images, p.height, p.width))
     dev = vals_sdf.device
     with device_guard(dev):
@@ -335,7 +347,7 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
         if build_index:
             gb = None
             if clear_grads is not None:
-                for t, rows in zip(clear_grads, (3, 1, 3 * nv, 14)):
+                for t, rows in zip(clear_grads, (3, 1, 3 * nv, c)):
                     _check_input(t, "clear_grads")
                     _check_dtype(t, torch.float32, "clear_grads")
                     if t.numel() < n * rows:
@@ -360,7 +372,8 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
     ``dims`` = int32 CPU tensor (or sequence) [batch, Dx, Dy, Dz, N] (raycast_rgbd.py:30-31).  ``flags``: the forward's
     SPSG_FLAG_DETERMINISTIC_GRADS, SPSG_FLAG_VIEW_NORMALS (``d_normals`` then holds N*F rows) and SPSG_FLAG_DETERMINISTIC
     are used; the last is also on under torch's deterministic algorithms, and a backward in another mode than its forward
-    raises RuntimeError.  SPSG_FLAG_ALL_PIXELS (as in the forward): ``mapping3dto2d`` may be None or empty."""
+    raises RuntimeError.  SPSG_FLAG_ALL_PIXELS (as in the forward): ``mapping3dto2d`` may be None or empty.  C =
+    ``grad_semantic.shape[-1]`` must be the forward's (else RuntimeError); ``d_semantic`` holds N rows of C."""
     flags = with_torch_mode(flags)
     table = () if all_pixels(flags) else ((mapping3dto2d, "mapping3dto2d"),)
     for t, name in ((grad_color, "grad_color"), (grad_depth, "grad_depth"), (grad_normal, "grad_normal"),
@@ -375,7 +388,9 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
     d = dims.tolist() if isinstance(dims, torch.Tensor) else list(dims)
     n = int(d[4])
     nv = views_per_chunk if flags & N.SPSG_FLAG_VIEW_NORMALS else 1
-    if d_color.shape[0] < n or d_depth.shape[0] < n or d_normals.shape[0] < n * nv or d_semantic.shape[0] < n:
+    c = semantic_channels(grad_semantic)
+    if d_color.shape[0] < n or d_depth.shape[0] < n or d_normals.shape[0] < n * nv or d_semantic.shape[0] < n or \
+            d_semantic.numel() < c * n:
         raise RuntimeError("d_* buffers hold fewer than N = %d rows" % n)
     p = N.make_params(width=grad_color.shape[2], height=grad_color.shape[1], depth_min=0, depth_max=0,
                       thresh_sample_dist=0, ray_increment=0, dimx=int(d[1]), dimy=int(d[2]), dimz=int(d[3]),
@@ -384,10 +399,10 @@ def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping,
                       num_locs=n,
                       flags=(N.SPSG_FLAG_GRADS_CLEARED if grads_cleared else 0) |
                       (flags & (N.SPSG_FLAG_DETERMINISTIC_GRADS | N.SPSG_FLAG_VIEW_NORMALS | N.SPSG_FLAG_DETERMINISTIC |
-                                N.SPSG_FLAG_ALL_PIXELS)))
+                                N.SPSG_FLAG_ALL_PIXELS | N.SPSG_FLAG_GENERIC_SEMANTIC)), semantic_channels=c)
     dev = grad_color.device
     px = sparse_mapping.shape[0] * views_per_chunk * p.width * p.height
-    if grad_depth.numel() < px or grad_color.numel() < 3 * px or grad_normal.numel() < 3 * px or grad_semantic.numel() < 14 * px:
+    if grad_depth.numel() < px or grad_color.numel() < 3 * px or grad_normal.numel() < 3 * px or grad_semantic.numel() < c * px:
         raise RuntimeError("gradient images are smaller than %d x %d x %d" % (px // (p.width * p.height), p.height, p.width))
     with device_guard(dev):
         nbytes = N.workspace_bytes(p)

@@ -55,13 +55,16 @@ class ViewGuidedTrainStep:
                 the mean over the first that many of its pixels.  None: over all of them, without the table
                 (``RaycastRGBD(..., max_pixels_per_voxel=None)``; at B = 8, F = 1 and the default row bound that drops a
                 1.31 GB allocation).
+    num_classes the semantic label set's size C (14, the reference's; e.g. 20 for ScanNet, 41 for NYU40): the generator's
+                semantic head has C channels, ``sample["semantics"]`` holds labels 0..C (C = unlabeled) and ``class_weight``
+                C weights.  The raycaster, the target one-hot and the 2D labels are C wide.
     """
 
     def __init__(self, model, loss_util, batch_size, dims3d, width, height, class_weight, voxelsize=0.02, truncation=3.0,
                  weight_occ_loss=1.0, weight_sdf_loss=0.1, weight_depth_loss=1.0, weight_color_loss=1.0,
                  weight_semantic_loss=0.1, weight_surf_geo=1.0, weight_missing_geo=5.0, logweight_sdf=True,
                  max_num_locs_per_sample=640000, views_per_chunk=1, render_input=True, device=None, image_loss=None,
-                 autocast_bf16=False, max_pixels_per_voxel=64):
+                 autocast_bf16=False, max_pixels_per_voxel=64, num_classes=14):
         self.model, self.loss_util = model, loss_util
         self.image_loss = image_loss
         self.autocast_bf16 = autocast_bf16
@@ -72,6 +75,7 @@ class ViewGuidedTrainStep:
         self.weight_surf_geo, self.weight_missing_geo, self.logweight_sdf = weight_surf_geo, weight_missing_geo, logweight_sdf
         self.class_weight = class_weight
         self.views = views_per_chunk
+        self.num_classes = num_classes
         self.render_input = render_input
         ray_increment = 0.3 * truncation            # train.py:134
         thresh_sample_dist = 50.5 * ray_increment   # train.py:135
@@ -79,7 +83,7 @@ class ViewGuidedTrainStep:
                                      depth_max=6.0 / voxelsize, thresh_sample_dist=thresh_sample_dist,
                                      ray_increment=ray_increment, max_num_frames=views_per_chunk,
                                      max_num_locs_per_sample=max_num_locs_per_sample,
-                                     max_pixels_per_voxel=max_pixels_per_voxel, device=device)
+                                     max_pixels_per_voxel=max_pixels_per_voxel, device=device, num_classes=num_classes)
         self.last = {}
 
     def _normals(self, locs, vals, transform):
@@ -98,10 +102,10 @@ class ViewGuidedTrainStep:
         else:  # only the labels are read: shared normals in the grid frame
             target_normals = normals.compute_normals_sparse(locs, vals, self.dims3d, num_chunks=self.batch_size)
         sem = sparsify.gather_dense(locs, target_for_semantics.float())
-        onehot = F.one_hot(sem[:, 0].long(), 15)[..., :-1].float().contiguous()
+        onehot = F.one_hot(sem[:, 0].long(), self.num_classes + 1)[..., :-1].float().contiguous()
         _, _, _, raycast_semantic = self.raycaster(locs, vals, colors.contiguous(), target_normals, onehot, view_matrix,
                                                    intrinsics)
-        return losses.labels_from_render(raycast_semantic)  # (I,H,W) uint8, 14 = miss / unlabeled
+        return losses.labels_from_render(raycast_semantic)  # (I,H,W) uint8, C = miss / unlabeled
 
     def _render_input(self, inputs, view_matrix, intrinsics, transform):
         """train.py:556-578: the input scan's colour / normal rendering (the discriminator's conditioning; with no
