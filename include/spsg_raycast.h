@@ -204,6 +204,22 @@ SPSG_API int spsg_raycast_forward_indexed(const spsg_raycast_params *p, int32_t 
                                           int32_t *mapping3dto2d_num, const spsg_grad_buffers *clear_grads,
                                           void *workspace, size_t workspace_bytes, void *stream);
 
+/* Label render: the march of spsg_raycast_forward_indexed (same hit voxel per pixel, bit for bit), with one uint8 label per
+ *    voxel as its only payload and one uint8 label per pixel as its only output -- what label maps of a one-hot render
+ *    (argmax of cat(render, ones), train.py:590-616) give, without the C-wide semantic image:
+ *        image_label[pixel] = hit voxel v ? min(voxel_labels[v], C) : C          C = p->semantic_channels (0 = 14)
+ *    voxel_labels: (N) uint8; a label above C renders as C.  image_label: (I,H,W) uint8.  hist: C + 1 device int64, cleared
+ *    and then the number of pixels per label (integer atomics: deterministic), or NULL.  Index routes as in
+ *    spsg_raycast_forward_indexed (int64 rows, SPSG_FLAG_PACKED_LOCS, SPSG_FLAG_INDEX_PREBUILT); SPSG_FLAG_NO_CLIP,
+ *    NO_BRICK_SKIP, SMEM_MAPS and GLOBAL_MAPS act as in the forward; every other flag is ignored.  Nothing else is
+ *    written: no float image, no mapping3dto2d(_num), no work list, no hit records, no gradient rows -- so no backward may
+ *    follow it on this workspace.  Needs no more workspace than spsg_workspace_bytes(p); 256-byte aligned. */
+SPSG_API int spsg_raycast_labels(const spsg_raycast_params *p, int32_t *sparse_mapping, const int64_t *locs,
+                                 const float *vals_sdf, const uint8_t *voxel_labels,
+                                 const float *view_matrix, const float *intrinsics,
+                                 uint8_t *image_label, int64_t *hist,
+                                 void *workspace, size_t workspace_bytes, void *stream);
+
 /* == raycast_rgbd_cuda.backward (raycast_rgbd_cuda.cpp:102-140, raycast_rgbd_cuda_kernel.cu:365-423,
  *    535-586): d_x[v] = sum over views of mean over the first min(num, max_pixels) pixels registered to
  *    voxel v of grad_x[pixel].  Rows [0, N) of every d_* are fully written (zeros where nothing hit);

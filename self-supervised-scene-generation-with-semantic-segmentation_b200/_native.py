@@ -45,7 +45,7 @@ EXPORTS = (
     "spsg_dense_gather_strided", "spsg_dense_scatter_strided",
     "spsg_labels_from_render", "spsg_pack_locs_host",
     "spsg_losses2d_forward_classes", "spsg_losses2d_forward_deterministic_classes", "spsg_losses2d_backward_classes",
-    "spsg_labels_from_render_classes",
+    "spsg_labels_from_render_classes", "spsg_raycast_labels",
 )
 
 
@@ -119,6 +119,8 @@ def _load():
     lib.spsg_raycast_forward.argtypes = [pp] + [vp] * 14 + [vp, sz, vp]
     lib.spsg_raycast_forward_indexed.restype = ctypes.c_int
     lib.spsg_raycast_forward_indexed.argtypes = [pp] + [vp] * 14 + [gb, vp, sz, vp]
+    lib.spsg_raycast_labels.restype = ctypes.c_int
+    lib.spsg_raycast_labels.argtypes = [pp] + [vp] * 8 + [vp, sz, vp]
     lib.spsg_raycast_backward.restype = ctypes.c_int
     lib.spsg_raycast_backward.argtypes = [pp] + [vp] * 11 + [vp, sz, vp]
     lib.spsg_raycast_occ.restype = ctypes.c_int

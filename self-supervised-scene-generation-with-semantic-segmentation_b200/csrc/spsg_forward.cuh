@@ -69,6 +69,11 @@ struct ForwardArgs {
     LossArgs loss;
     spsg_grad_buffers clear;  // gradient rows [0, clear_rows) to zero for the backward that follows (or clear_rows = 0)
     long long clear_rows;
+    // kLabels (spsg_raycast_labels), after every other field so that no kernel parameter offset moves: uint8 label per
+    // voxel in, uint8 label per pixel out, optional C + 1 counters (C = loss.sem_channels)
+    const uint8_t *voxel_labels;
+    uint8_t *image_label;
+    unsigned long long *hist;
 };
 
 constexpr int kTileW = 16, kTileH = 8;  // pixels per CTA of the occupancy kernel: 4 warps of 8x4 pixels
@@ -205,7 +210,11 @@ __device__ __forceinline__ void clear_span(float *__restrict__ p, size_t n, size
 // kGenericSem (C != 14, or SPSG_FLAG_GENERIC_SEMANTIC): vals_semantic / image_semantic hold a.loss.sem_channels channels; the
 // semantic rows are written by store_semantic_rows and the fused cross-entropy reads the hit voxel's payload row.  The
 // march, the registration and every other rendering are the same code.
-template <bool kLoss, bool kSmemMaps, int kWarps, bool kViewNormals, bool kGenericSem = false>
+// kLabels (spsg_raycast_labels): the same march, then an epilogue that writes one byte per pixel -- the hit voxel's
+// label, min(voxel_labels[hit], C), or C on a miss -- and, with a.hist, counts pixels per label in a shared-memory
+// histogram (the staging area, which this epilogue does not use) flushed once per CTA with integer atomics.  No payload
+// loads, no float image, no registration, no work list, no hit records, no gradient rows.
+template <bool kLoss, bool kSmemMaps, int kWarps, bool kViewNormals, bool kGenericSem = false, bool kLabels = false>
 __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const ForwardArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ float4 s_steps[kStepEntries];
@@ -217,7 +226,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
     const unsigned kFull = 0xffffffffu;
     const float kInf = CUDART_INF_F;
 
-    if (a.clear_rows > 0) {
+    if (!kLabels && a.clear_rows > 0) {
         // The backward's output rows are zeroed here (the reference memsets its whole d_* buffers, kernel.cu:557-560): a few
         // fire-and-forget stores per warp that overlap the march, instead of a longer fill pass in front of the index build.
         const size_t wid = (size_t)blockIdx.x * kWarps + warp, nw = (size_t)gridDim.x * kWarps, n = (size_t)a.clear_rows;
@@ -228,6 +237,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
     }
     if (threadIdx.x < kStepEntries) step_table_fill(s_steps, threadIdx.x, a.inc);
     if (kSmemMaps && threadIdx.x == 0) mbar_init(mbar, 1);
+    if (kLabels && a.hist && threadIdx.x <= a.loss.sem_channels) reinterpret_cast<unsigned *>(smem + 128)[threadIdx.x] = 0u;
     __syncthreads();
     unsigned phase = 0;
     const float inv_inc = rcp_approx(a.inc);
@@ -641,6 +651,18 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
                 const long long clk2 = clock64();
 #endif
 
+                if (kLabels) {
+                    // ---- label epilogue: one byte per pixel (a tile row is 8 contiguous bytes), one shared atomic per
+                    // distinct label of the warp
+                    const int C = a.loss.sem_channels;
+                    const int label = hit >= 0 ? min((int)__ldg(a.voxel_labels + hit), C) : C;
+                    if (active) a.image_label[gpix] = (uint8_t)label;
+                    if (a.hist) {
+                        const unsigned peers = __match_any_sync(kFull, active ? label : -1);
+                        if (active && lane == __ffs(peers) - 1)
+                            atomicAdd(reinterpret_cast<unsigned *>(smem + 128) + label, (unsigned)__popc(peers));
+                    }
+                } else {
                 // ---- write-out (kernel.cu:276-285 init, :217-239 hit) through shared memory
                 const float ninf = __int_as_float(0xff800000);
                 float col0 = ninf, col1 = ninf, col2 = ninf, dep = ninf;
@@ -811,11 +833,18 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
                     STAT_ADD(32 + min(bucket, 9), 1);
                 }
 #endif
+                }  // !kLabels
             }
             tile = __shfl_sync(kFull, next, 0);
             if (tile < tile_limit) prepare(bind_chunk(tile), q);
         }
         if (kSmemMaps) phase ^= 1u;
+    }
+    if (kLabels && a.hist) {
+        __syncthreads();
+        const unsigned *s_hist = reinterpret_cast<const unsigned *>(smem + 128);
+        if (threadIdx.x <= a.loss.sem_channels && s_hist[threadIdx.x])
+            atomicAdd(a.hist + threadIdx.x, (unsigned long long)s_hist[threadIdx.x]);
     }
     if (kLoss) {
         // Every loss atomic of this CTA is ordered before its arrival; the CTA that arrives last sees them all in L2 and

@@ -107,25 +107,48 @@ LossArgs make_loss_args(const spsg_loss_targets *t, double *accum) {
     return L;
 }
 
+// Outputs of the label render (spsg_raycast_labels), which runs launch_forward with the kLabels kernels
+struct LabelOut {
+    const uint8_t *voxel_labels;
+    uint8_t *image_label;
+    int64_t *hist;
+};
+
+// the flags a label render acts on: the march's debug switches and the index routes (everything else concerns tables,
+// gradients, normals or the semantic payload kernels)
+constexpr uint32_t kLabelFlags = SPSG_FLAG_NO_CLIP | SPSG_FLAG_NO_BRICK_SKIP | SPSG_FLAG_SMEM_MAPS | SPSG_FLAG_GLOBAL_MAPS |
+                                 SPSG_FLAG_PACKED_LOCS | SPSG_FLAG_INDEX_PREBUILT;
+
 int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *sparse_mapping, const int64_t *locs,
                    const float *vals_sdf, const float *vals_color, const float *vals_normal,
                    const float *vals_semantic, const float *view_matrix, const float *intrinsics, float *image_color,
                    float *image_depth, float *image_normal, float *image_semantic, int32_t *mapping3dto2d,
                    int32_t *mapping3dto2d_num, const spsg_loss_targets *targets, float *loss_out,
-                   const spsg_grad_buffers *clear_grads, void *workspace, size_t workspace_bytes, cudaStream_t st) {
+                   const spsg_grad_buffers *clear_grads, void *workspace, size_t workspace_bytes, cudaStream_t st,
+                   const LabelOut *lab = nullptr) {
     if (int rc = check_params(p)) return rc;
     const bool all = (p->flags & SPSG_FLAG_ALL_PIXELS) != 0;  // no table: the backward builds segments from the hits
-    if (!all && p->max_pixels_per_voxel <= 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "max_pixels_per_voxel must be positive");
-    if (!sparse_mapping || !view_matrix || !intrinsics || !image_color || !image_depth || !image_normal ||
-        !image_semantic || (!all && !mapping3dto2d) || !mapping3dto2d_num)
-        return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL tensor pointer");
-    if (p->num_locs > 0 && (!locs || !vals_sdf || !vals_color || !vals_normal || !vals_semantic))
-        return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL voxel tensor pointer");
+    const bool packed = (p->flags & SPSG_FLAG_PACKED_LOCS) != 0;
+    if (lab) {
+        // label render: no payload, image, table or gradient pointers (the caller passes p with kLabelFlags only)
+        if (!sparse_mapping || !view_matrix || !intrinsics || !lab->image_label) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL tensor pointer");
+        if (p->num_locs > 0 && (!locs || !vals_sdf || !lab->voxel_labels))
+            return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL voxel tensor pointer");
+        if (reinterpret_cast<uintptr_t>(lab->hist) & 7u) return fail(SPSG_ERR_INVALID_ARGUMENT, "hist must be 8-byte aligned");
+        if (p->num_locs > 0 && (reinterpret_cast<uintptr_t>(locs) & (packed ? 3u : 15u)))
+            return fail(SPSG_ERR_INVALID_ARGUMENT, "locs must be 16-byte (packed: 4-byte) aligned");
+    } else {
+        if (!all && p->max_pixels_per_voxel <= 0) return fail(SPSG_ERR_INVALID_ARGUMENT, "max_pixels_per_voxel must be positive");
+        if (!sparse_mapping || !view_matrix || !intrinsics || !image_color || !image_depth || !image_normal ||
+            !image_semantic || (!all && !mapping3dto2d) || !mapping3dto2d_num)
+            return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL tensor pointer");
+        if (p->num_locs > 0 && (!locs || !vals_sdf || !vals_color || !vals_normal || !vals_semantic))
+            return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL voxel tensor pointer");
+        if (p->num_locs > 0 && ((reinterpret_cast<uintptr_t>(vals_semantic) & 7u) || (reinterpret_cast<uintptr_t>(locs) & (packed ? 3u : 15u))))
+            return fail(SPSG_ERR_INVALID_ARGUMENT, "vals_semantic must be 8-byte and locs 16-byte (packed: 4-byte) aligned");
+    }
     if (!aligned16(view_matrix) || !aligned16(intrinsics))
         return fail(SPSG_ERR_INVALID_ARGUMENT, "view_matrix / intrinsics must be 16-byte aligned");
-    const bool packed = (p->flags & SPSG_FLAG_PACKED_LOCS) != 0;
-    if (p->num_locs > 0 && ((reinterpret_cast<uintptr_t>(vals_semantic) & 7u) || (reinterpret_cast<uintptr_t>(locs) & (packed ? 3u : 15u))))
-        return fail(SPSG_ERR_INVALID_ARGUMENT, "vals_semantic must be 8-byte and locs 16-byte (packed: 4-byte) aligned");
     if (packed && !build_index) return fail(SPSG_ERR_INVALID_ARGUMENT, "packed locs need an entry point that builds the index");
     if (packed && (unsigned long long)p->num_chunks * p->dimz * p->dimy * p->dimx >= 0xffffffffull)
         return fail(SPSG_ERR_INVALID_ARGUMENT, "packed locs need fewer than 2^32 - 1 cells");
@@ -237,6 +260,11 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
         a.clear = *clear_grads;
         a.clear_rows = p->num_locs;
     }
+    if (lab) {
+        a.voxel_labels = lab->voxel_labels; a.image_label = lab->image_label;
+        a.hist = reinterpret_cast<unsigned long long *>(lab->hist);
+        if (lab->hist) CUDA_TRY(cudaMemsetAsync(lab->hist, 0, (size_t)(a.loss.sem_channels + 1) * sizeof(int64_t), st));
+    }
     // persistent: one CTA per SM (fewer when there is less than one tile per warp)
     const long long tiles_x = (p->width + kWarpW - 1) / kWarpW, tiles_y = (p->height + kWarpH - 1) / kWarpH;
     const long long all_tiles = ((tiles_x + 1) / 2) * ((tiles_y + 1) / 2) * 4 * p->views_per_chunk * p->num_chunks;
@@ -266,6 +294,11 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
             SPSG_SET_SMEM_ALL(true);
 #undef SPSG_SET_SMEM_ALL
 #undef SPSG_SET_SMEM
+#define SPSG_SET_SMEM_LABELS(M, W) \
+    CUDA_TRY(cudaFuncSetAttribute(raycast_forward_kernel<false, M, W, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmemMax))
+            SPSG_SET_SMEM_LABELS(true, kFwdWarps); SPSG_SET_SMEM_LABELS(false, kFwdWarps);
+            SPSG_SET_SMEM_LABELS(true, kFwdWarpsLarge); SPSG_SET_SMEM_LABELS(false, kFwdWarpsLarge);
+#undef SPSG_SET_SMEM_LABELS
             if (dev >= 0 && dev < 64) configured[dev] = true;
         }
     }
@@ -282,11 +315,19 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
     do {                                                                                                          \
         if (view_normals) SPSG_LAUNCH_VN(L, M, true); else SPSG_LAUNCH_VN(L, M, false);                           \
     } while (0)
-        if (targets && !det) {  // (deterministic mode sums the losses in a pass of its own, below)
+#define SPSG_LAUNCH_LABELS(M)                                                                                     \
+    do {                                                                                                          \
+        if (large) raycast_forward_kernel<false, M, kFwdWarpsLarge, false, false, true><<<grid, kFwdWarpsLarge * 32, dyn, st>>>(a); \
+        else raycast_forward_kernel<false, M, kFwdWarps, false, false, true><<<grid, kFwdWarps * 32, dyn, st>>>(a); \
+    } while (0)
+        if (lab) {
+            if (a.maps_in_smem) SPSG_LAUNCH_LABELS(true); else SPSG_LAUNCH_LABELS(false);
+        } else if (targets && !det) {  // (deterministic mode sums the losses in a pass of its own, below)
             if (a.maps_in_smem) SPSG_LAUNCH(true, true); else SPSG_LAUNCH(true, false);
         } else {
             if (a.maps_in_smem) SPSG_LAUNCH(false, true); else SPSG_LAUNCH(false, false);
         }
+#undef SPSG_LAUNCH_LABELS
 #undef SPSG_LAUNCH
 #undef SPSG_LAUNCH_VN
     }
@@ -584,6 +625,18 @@ int spsg_raycast_forward_indexed(const spsg_raycast_params *p, int32_t *sparse_m
                           intrinsics, image_color, image_depth, image_normal, image_semantic, mapping3dto2d,
                           mapping3dto2d_num, nullptr, nullptr, clear_grads, workspace, workspace_bytes,
                           (cudaStream_t)stream);
+}
+
+int spsg_raycast_labels(const spsg_raycast_params *p, int32_t *sparse_mapping, const int64_t *locs, const float *vals_sdf,
+                        const uint8_t *voxel_labels, const float *view_matrix, const float *intrinsics,
+                        uint8_t *image_label, int64_t *hist, void *workspace, size_t workspace_bytes, void *stream) {
+    if (!p) return fail(SPSG_ERR_INVALID_ARGUMENT, "params is NULL");
+    spsg_raycast_params q = *p;
+    q.flags &= kLabelFlags;
+    const LabelOut lab = {voxel_labels, image_label, hist};
+    return launch_forward(&q, true, sparse_mapping, locs, vals_sdf, nullptr, nullptr, nullptr, view_matrix, intrinsics,
+                          nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, workspace,
+                          workspace_bytes, (cudaStream_t)stream, &lab);
 }
 
 int spsg_raycast_backward(const spsg_raycast_params *p, const float *grad_color, const float *grad_depth,

@@ -20,6 +20,7 @@ Differences, all behind defaulted extras or unobservable through the reference A
     first ``max_pixels_per_voxel`` (SPSG_FLAG_ALL_PIXELS in ``flags``); no ``mapping3dto2d`` table is allocated.
   * ``num_classes=C``: semantic payloads, renderings and gradients of C channels instead of the reference's 14 (1..64;
     e.g. 20 for ScanNet, 41 for NYU40 / mpcat40).  Geometry does not depend on C.
+  * ``RaycastRGBD.render_labels``: the label map of a render from one uint8 label per voxel, without the C-wide image.
 """
 import torch
 from torch import nn
@@ -162,6 +163,25 @@ class RaycastRGBD(nn.Module):
                                          self.mapping3dto2d, self.mapping3dto2d_num, self.d_color, self.d_depth,
                                          raycast_rgbd_cuda.normal_grad_buffer(self, per_view), self.d_semantic, views,
                                          flags, self.workspace)
+
+    def render_labels(self, locs, vals_sdf, voxel_labels, view_matrix, intrinsic_params, histogram=False):
+        """The label map of a render, without rendering the semantic image: a new (I,H,W) uint8 tensor holding the hit
+        voxel's label (``voxel_labels``, (N,) uint8; a label above ``num_classes`` counts as ``num_classes``), or
+        ``num_classes`` where the ray hits nothing.  Same march and hit voxels as ``forward``, so it equals
+        ``losses.labels_from_render`` of a forward with the one-hot of ``voxel_labels`` as semantic payload.  With
+        ``histogram=True`` also returns the (num_classes + 1,) int64 pixel count per label.  The module's images, tables
+        and gradient buffers are not touched; it counts as a forward on the module's workspace, so a backward of an earlier
+        forward raises afterwards.  No autograd."""
+        images = view_matrix.shape[0]
+        views = max(1, images // self.batch_size)
+        if images != views * self.batch_size or views > self.max_num_frames:
+            raise RuntimeError("view_matrix has %d images: expected batch_size (%d) x views with views <= "
+                               "max_num_frames (%d)" % (images, self.batch_size, self.max_num_frames))
+        opts = [self.width, self.height, self.depth_min, self.depth_max, self.thresh_sample_dist, self.ray_increment,
+                self.dims3d[2], self.dims3d[1], self.dims3d[0]]
+        return raycast_rgbd_cuda.render_labels(self.sparse_mapping, locs, vals_sdf, voxel_labels, view_matrix,
+                                               intrinsic_params, opts, self.num_classes, views, self.flags, histogram,
+                                               self.workspace)
 
 
 class RaycastOcc(nn.Module):

@@ -158,6 +158,9 @@ def semantic_channels(t):
     return c
 
 
+_LABEL_STAMP = "label render (no tables)"
+
+
 def _stamp(p):
     return (int(p.num_locs), int(p.views_per_chunk), int(p.num_chunks), int(p.width), int(p.height),
             int(p.max_pixels_per_voxel), "%d classes" % (p.semantic_channels or 14), bool(p.flags & N.SPSG_FLAG_VIEW_NORMALS),
@@ -225,6 +228,12 @@ class ModuleWorkspace:
 
     def filled(self, p):
         self.stamp = _stamp(p)
+        self.forwards += 1
+
+    def labels_rendered(self):
+        """A label render ran on this workspace: it counts as a forward, and its stamp matches no backward's (it leaves no
+        tables or work list), so a backward after it raises instead of gathering what an earlier forward left."""
+        self.stamp = _LABEL_STAMP
         self.forwards += 1
 
     def check_latest(self, forward):
@@ -363,6 +372,61 @@ def forward(sparse_mapping, locs, vals_sdf, vals_color, vals_normals, vals_seman
             if p.flags & N.SPSG_FLAG_INDEX_PREBUILT:
                 workspace_owner.mark_prebuilt(locs)  # index and brick are untouched: still valid for these rows
     return ws
+
+
+def render_labels(sparse_mapping, locs, vals_sdf, voxel_labels, viewMatrixInv, intrinsicParams, opts, num_classes,
+                  views_per_chunk=1, flags=0, histogram=False, workspace_owner=None):
+    """Label render (``spsg_raycast_labels``): the forward's march with a uint8 label per voxel as the only payload.
+    Returns a new ``(I, H, W)`` uint8 tensor, ``min(voxel_labels[hit voxel], C)`` or C on a miss (C = ``num_classes``), and
+    with ``histogram=True`` also its ``(C + 1,)`` int64 pixel count per label.  ``voxel_labels``: (N,) uint8.  ``flags``: the
+    march's debug flags act, the rest is ignored.  ``sparse_mapping`` is rebuilt; nothing else of the caller's is written.
+    The workspace (``workspace_owner``'s, else the one cached for ``sparse_mapping``) is stamped so that no backward runs
+    on it afterwards."""
+    for t, name in ((sparse_mapping, "sparse_mapping"), (locs, "locs"), (vals_sdf, "vals_sdf"), (voxel_labels, "voxel_labels"),
+                    (viewMatrixInv, "viewMatrixInv"), (intrinsicParams, "intrinsicParams")):
+        _check_input(t, name)
+    _check_dtype(sparse_mapping, torch.int32, "sparse_mapping")
+    if not is_packed_locs(locs):
+        _check_dtype(locs, torch.int64, "locs")
+    _check_dtype(vals_sdf, torch.float32, "vals_sdf")
+    _check_dtype(voxel_labels, torch.uint8, "voxel_labels")
+    _check_dtype(viewMatrixInv, torch.float32, "viewMatrixInv")
+    _check_dtype(intrinsicParams, torch.float32, "intrinsicParams")
+    if not 1 <= num_classes <= N.SPSG_MAX_SEMANTIC_CHANNELS:
+        raise RuntimeError("num_classes must be in 1..%d, got %d" % (N.SPSG_MAX_SEMANTIC_CHANNELS, num_classes))
+    p = _forward_params(sparse_mapping, locs, 0, opts, views_per_chunk, flags, num_classes)
+    if is_packed_locs(locs):
+        p.flags |= N.SPSG_FLAG_PACKED_LOCS
+    n = locs.shape[0]
+    if not is_packed_locs(locs) and locs.numel() != 4 * n:
+        raise RuntimeError("locs must be (N, 4) rows of (z, y, x, chunk)")
+    if vals_sdf.numel() < n or voxel_labels.numel() < n:
+        raise RuntimeError("vals_sdf / voxel_labels hold fewer than N = %d rows" % n)
+    images = p.num_chunks * p.views_per_chunk
+    if viewMatrixInv.numel() < images * 16 or intrinsicParams.numel() < images * 4:
+        raise RuntimeError("viewMatrixInv / intrinsicParams hold fewer than %d images" % images)
+    dev = vals_sdf.device
+    devs = {t.device for t in (sparse_mapping, locs, vals_sdf, voxel_labels, viewMatrixInv, intrinsicParams)}
+    if len(devs) != 1:
+        raise RuntimeError("raycast inputs live on different devices: %s" % sorted(str(d) for d in devs))
+    image_label = torch.empty(images, p.height, p.width, dtype=torch.uint8, device=dev)
+    hist = torch.empty(num_classes + 1, dtype=torch.int64, device=dev) if histogram else None
+    with device_guard(dev):
+        nbytes = N.workspace_bytes(p)
+        if workspace_owner is not None:
+            prebuilt = workspace_owner.take_prebuilt(locs, nbytes)
+            ws = workspace_owner.get(dev, nbytes)
+            p.flags |= prebuilt
+        else:
+            ws = workspace(dev, nbytes, sparse_mapping, stamp=_LABEL_STAMP)
+        N.check(N.lib.spsg_raycast_labels(ctypes.byref(p), N.ptr(sparse_mapping), N.ptr(locs), N.ptr(vals_sdf),
+                                          N.ptr(voxel_labels), N.ptr(viewMatrixInv), N.ptr(intrinsicParams),
+                                          N.ptr(image_label), N.ptr(hist), N.ptr(ws), ws.numel(), _stream(dev)))
+        if workspace_owner is not None:
+            workspace_owner.labels_rendered()
+            if p.flags & N.SPSG_FLAG_INDEX_PREBUILT:
+                workspace_owner.mark_prebuilt(locs)  # index and brick are untouched: still valid for these rows
+    return (image_label, hist) if histogram else image_label
 
 
 def backward(grad_color, grad_depth, grad_normal, grad_semantic, sparse_mapping, mapping3dto2d, mapping3dto2d_num,

@@ -20,7 +20,6 @@ import torch
 from . import parallel as P
 from . import synthetic as S
 from .losses import labels_from_render
-from .normals import compute_normals_sparse
 from .raycast_rgbd import RaycastRGBD
 
 
@@ -128,7 +127,6 @@ def render_room(predict, room_dims_zyx, device, views_per_chunk=5, chunks_per_la
     view_np, intr_np = window_views(F, chunk_dims)
     view = torch.from_numpy(np.tile(view_np, (B, 1, 1))).to(device)
     intr = torch.from_numpy(np.tile(intr_np, (B, 1))).to(device)
-    grid2cam = torch.inverse(view[::F]).contiguous()          # one rotation per chunk for the normals (train.py:544)
     hist = torch.zeros(S.NUM_CLASSES + 1, dtype=torch.int64, device=device)
     images, rendered, rays = [], 0, 0
     predict_group = getattr(predict, "predict_group", None)
@@ -154,13 +152,15 @@ def render_room(predict, room_dims_zyx, device, views_per_chunk=5, chunks_per_la
         if not present:  # the reference skips empty windows (test_scene_as_chunks.py:160-161)
             continue
         with torch.no_grad():
-            normals = compute_normals_sparse(locs, sdf, chunk_dims, grid2cam, num_chunks=B)
-            _, depth, _, sem_img = rc(locs, sdf, color, normals, sem, view, intr)
-            # pred2d_label of train.py:749-752 and its per-class pixel counts in one pass over the rendering
-            labels, h = labels_from_render(sem_img[:slots * F], histogram=True)
-            labels = labels.view(slots, F, height, width)
-            if len(present) < slots:  # idle slots rendered nothing: all their pixels are label 14
-                h[S.NUM_CLASSES] -= (slots - len(present)) * F * width * height
+            # pred2d_label of train.py:749-752 and its per-class pixel counts.  A pixel's rendered logits are its hit
+            # voxel's row, so its label is the label of that row: one byte per voxel, then the label render (which writes
+            # no float image and needs no normals or colours)
+            voxel_labels = labels_from_render(sem)
+            labels, h = rc.render_labels(locs, sdf, voxel_labels, view, intr, histogram=True)
+            labels = labels[:slots * F].view(slots, F, height, width)
+            # idle slots, and the slots past this group's windows, rendered nothing: all their pixels are label 14
+            h[S.NUM_CLASSES] -= (B - len(present)) * F * width * height
+            if len(present) < slots:
                 labels = labels[torch.tensor(present, device=device)]
             hist += h
         rendered += len(present)

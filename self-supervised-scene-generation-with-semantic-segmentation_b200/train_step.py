@@ -8,7 +8,7 @@ and the prediction (``:626-632``) -- -> depth L1 / colour L1 / 2D semantic cross
 
 ``ViewGuidedTrainStep`` runs exactly that data flow with every op between the generator's dense heads and the scalar loss
 replaced by this package's CUDA ops: ordered stream compaction + fused gathers (``sparsify``), the sparse normals kernel
-(``normals``), the persistent raycast kernel, the fused label map (``losses.labels_from_render``) and the raycast with the
+(``normals``), the persistent raycast kernel, its label render (``RaycastRGBD.render_labels``) and the raycast with the
 three 2D losses fused into its epilogue (``losses.render_with_2d_losses``).  The generator and the dense 3D losses are the
 caller's (the reference's own ``model.Generator`` / ``loss`` module in bench.py and the tests): they are stock PyTorch and
 outside the hot path (SURVEY.md section 8).  Data parallelism is ``torch.nn.parallel.DistributedDataParallel`` around the
@@ -17,7 +17,6 @@ generator: its gradient all-reduce is the step's only collective (SURVEY.md sect
 import contextlib
 
 import torch
-import torch.nn.functional as F
 
 from . import losses, normals, sparsify
 from .raycast_rgbd import RaycastRGBD
@@ -57,7 +56,7 @@ class ViewGuidedTrainStep:
                 1.31 GB allocation).
     num_classes the semantic label set's size C (14, the reference's; e.g. 20 for ScanNet, 41 for NYU40): the generator's
                 semantic head has C channels, ``sample["semantics"]`` holds labels 0..C (C = unlabeled) and ``class_weight``
-                C weights.  The raycaster, the target one-hot and the 2D labels are C wide.
+                C weights.  The raycaster and the 2D labels are C wide.
     """
 
     def __init__(self, model, loss_util, batch_size, dims3d, width, height, class_weight, voxelsize=0.02, truncation=3.0,
@@ -94,18 +93,14 @@ class ViewGuidedTrainStep:
         return normals.compute_normals_sparse(locs, vals, self.dims3d, transform=transform, views_per_chunk=self.views)
 
     def _target_labels(self, target_for_sdf, target_for_colors, target_for_semantics, view_matrix, intrinsics, transform):
-        """train.py:581-622: render the target chunk, its semantics become the per-pixel labels."""
+        """train.py:581-622: render the target chunk, its semantics become the per-pixel labels.  The reference renders
+        colours, normals and a one-hot semantic image and takes its argmax (train.py:590-616); each pixel's label is that
+        of its hit voxel (C where the ray misses, or the voxel is unlabeled), which the label render writes directly.  The
+        target colours and the cameras' ``transform`` are not needed for that."""
         locs, vals = sparsify.sparsify_predictions(target_for_sdf, self.truncation)
-        colors = target_for_colors[locs[:, 3], locs[:, 0], locs[:, 1], locs[:, 2], :].float() / 255.0
-        if self.views == 1:
-            target_normals = normals.compute_normals_sparse(locs, vals, self.dims3d, transform=transform)
-        else:  # only the labels are read: shared normals in the grid frame
-            target_normals = normals.compute_normals_sparse(locs, vals, self.dims3d, num_chunks=self.batch_size)
         sem = sparsify.gather_dense(locs, target_for_semantics.float())
-        onehot = F.one_hot(sem[:, 0].long(), self.num_classes + 1)[..., :-1].float().contiguous()
-        _, _, _, raycast_semantic = self.raycaster(locs, vals, colors.contiguous(), target_normals, onehot, view_matrix,
-                                                   intrinsics)
-        return losses.labels_from_render(raycast_semantic)  # (I,H,W) uint8, C = miss / unlabeled
+        voxel_labels = sem[:, 0].to(torch.uint8).contiguous()
+        return self.raycaster.render_labels(locs, vals, voxel_labels, view_matrix, intrinsics)  # (I,H,W) uint8
 
     def _render_input(self, inputs, view_matrix, intrinsics, transform):
         """train.py:556-578: the input scan's colour / normal rendering (the discriminator's conditioning; with no
