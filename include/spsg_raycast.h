@@ -220,6 +220,31 @@ SPSG_API int spsg_raycast_labels(const spsg_raycast_params *p, int32_t *sparse_m
                                  uint8_t *image_label, int64_t *hist,
                                  void *workspace, size_t workspace_bytes, void *stream);
 
+/* Eval render: the march of spsg_raycast_labels (same hit voxel per pixel) with an epilogue for evaluation without a
+ *    backward.  One call gives, for the prediction (vals_color (N,3), vals_semantic (N,C) logits, pred_labels (N) uint8 --
+ *    the voxels' predicted labels, e.g. spsg_labels_from_render_classes of the logits; a label above C counts as C):
+ *      loss_out     SPSG_LOSS_OUT_FLOATS floats, the loss block of spsg_raycast_forward_loss for the same inputs and targets
+ *                   (same per-pixel arithmetic and per-warp partials as its C-generic epilogue; the partials are added in
+ *                   double in an order fixed by tile position, so the result is bit-reproducible in every mode, and the
+ *                   normalisers out[4..6] equal the fused forward's).  t: as there; any target may be NULL.
+ *      image_label  (I,H,W) uint8: hit voxel v ? min(pred_labels[v], C) : C, or NULL.
+ *      confusion    (C+1)^2 device uint64, cleared and then confusion[min(target_label, C) * (C + 1) + label] = number of
+ *                   pixels (integer atomics: deterministic), or NULL.  Needs t->target_label.
+ *    vals_color may be NULL without t->target_color, vals_semantic without t->target_label.  No normals are read; nothing else
+ *    is written: no float image, no mapping3dto2d(_num), no work list, no hit records, no gradient rows -- so no backward
+ *    may follow it on this workspace.  Index routes and flags as in spsg_raycast_labels (every flag but the march's debug
+ *    switches and the index routes is ignored, SPSG_FLAG_DETERMINISTIC included: the result does not depend on it).  Needs
+ *    no more workspace than spsg_workspace_bytes(p), and scratch_bytes >= spsg_raycast_eval_scratch_bytes(p); both
+ *    256-byte aligned.  Every argument is checked before anything is enqueued. */
+SPSG_API int spsg_raycast_eval(const spsg_raycast_params *p, int32_t *sparse_mapping, const int64_t *locs,
+                               const float *vals_sdf, const float *vals_color, const float *vals_semantic,
+                               const uint8_t *pred_labels, const float *view_matrix, const float *intrinsics,
+                               const spsg_loss_targets *t, float *loss_out, uint8_t *image_label, uint64_t *confusion,
+                               void *scratch, size_t scratch_bytes, void *workspace, size_t workspace_bytes, void *stream);
+
+/* Scratch of spsg_raycast_eval (8 floats per 8x4-pixel warp tile of the batch, plus a few KB); 0 for invalid params. */
+SPSG_API size_t spsg_raycast_eval_scratch_bytes(const spsg_raycast_params *p);
+
 /* == raycast_rgbd_cuda.backward (raycast_rgbd_cuda.cpp:102-140, raycast_rgbd_cuda_kernel.cu:365-423,
  *    535-586): d_x[v] = sum over views of mean over the first min(num, max_pixels) pixels registered to
  *    voxel v of grad_x[pixel].  Rows [0, N) of every d_* are fully written (zeros where nothing hit);

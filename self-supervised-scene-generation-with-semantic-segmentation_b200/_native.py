@@ -45,7 +45,7 @@ EXPORTS = (
     "spsg_dense_gather_strided", "spsg_dense_scatter_strided",
     "spsg_labels_from_render", "spsg_pack_locs_host",
     "spsg_losses2d_forward_classes", "spsg_losses2d_forward_deterministic_classes", "spsg_losses2d_backward_classes",
-    "spsg_labels_from_render_classes", "spsg_raycast_labels",
+    "spsg_labels_from_render_classes", "spsg_raycast_labels", "spsg_raycast_eval", "spsg_raycast_eval_scratch_bytes",
 )
 
 
@@ -121,6 +121,10 @@ def _load():
     lib.spsg_raycast_forward_indexed.argtypes = [pp] + [vp] * 14 + [gb, vp, sz, vp]
     lib.spsg_raycast_labels.restype = ctypes.c_int
     lib.spsg_raycast_labels.argtypes = [pp] + [vp] * 8 + [vp, sz, vp]
+    lib.spsg_raycast_eval.restype = ctypes.c_int
+    lib.spsg_raycast_eval.argtypes = [pp] + [vp] * 8 + [lt, vp, vp, vp, vp, sz, vp, sz, vp]
+    lib.spsg_raycast_eval_scratch_bytes.restype = sz
+    lib.spsg_raycast_eval_scratch_bytes.argtypes = [pp]
     lib.spsg_raycast_backward.restype = ctypes.c_int
     lib.spsg_raycast_backward.argtypes = [pp] + [vp] * 11 + [vp, sz, vp]
     lib.spsg_raycast_occ.restype = ctypes.c_int

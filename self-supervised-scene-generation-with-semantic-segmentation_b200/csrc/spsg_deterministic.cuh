@@ -131,3 +131,64 @@ __global__ void __launch_bounds__(kDetLossThreads) losses2d_det_kernel(const Los
                            a.loss.target_depth != nullptr, a.loss.target_color != nullptr, a.loss.target_label != nullptr,
                            lane);
 }
+
+// ---------------------------------------------------------------------------------------------
+// loss sums of the eval render (spsg_raycast_eval): the forward's kEval epilogue leaves each (image, tile)'s six per-warp
+// partials in its own slot of 8 floats; block b adds tiles [b * kEvalSumTiles, (b + 1) * kEvalSumTiles) in double in a fixed
+// order, and the block that finishes last adds the blocks' partials and finalises as losses2d_det_kernel does.
+// Bit-reproducible whatever the forward's schedule.
+// ---------------------------------------------------------------------------------------------
+
+constexpr int kEvalSumTiles = 2048;
+static_assert(kEvalSumTiles % kDetLossThreads == 0, "whole tile rounds per block");
+
+// loss.accum: kLossSlots * 8 doubles of scratch for the final stage; loss.done: a zeroed int32; partials: 8 doubles per block
+__global__ void __launch_bounds__(kDetLossThreads) eval_loss_sum_kernel(const float *__restrict__ tiles, long long num_tiles,
+                                                                        const LossArgs loss, double *__restrict__ partials) {
+    __shared__ double s_warp[kDetLossThreads / 32][6];
+    __shared__ int s_last;
+    double acc[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    const long long t0 = (long long)blockIdx.x * kEvalSumTiles;
+#pragma unroll 1
+    for (int k = 0; k < kEvalSumTiles / kDetLossThreads; k++) {
+        const long long t = t0 + k * kDetLossThreads + threadIdx.x;
+        if (t < num_tiles) {
+            const float4 lo = __ldg(reinterpret_cast<const float4 *>(tiles + t * 8));
+            const float2 hi = __ldg(reinterpret_cast<const float2 *>(tiles + t * 8 + 4));
+            acc[0] += lo.x; acc[1] += lo.y; acc[2] += lo.z; acc[3] += lo.w; acc[4] += hi.x; acc[5] += hi.y;
+        }
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < 6; k++) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], o);
+        if (lane == 0) s_warp[warp][k] = acc[k];
+    }
+    __syncthreads();
+    if (threadIdx.x < 6) {
+        double s = 0.0;
+        for (int w = 0; w < kDetLossThreads / 32; w++) s += s_warp[w][threadIdx.x];
+        partials[(size_t)blockIdx.x * 8 + threadIdx.x] = s;
+        __threadfence();
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) s_last = atomicAdd(loss.done, 1) == (int)gridDim.x - 1;
+    __syncthreads();
+    if (!s_last) return;
+    __threadfence();
+    if (threadIdx.x < kLossSlots) {
+        // slot t = blocks t, t + kLossSlots, ... in block order; finalize_loss_warp then adds the slots in a fixed tree
+        double t[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+        for (unsigned b = threadIdx.x; b < gridDim.x; b += kLossSlots)
+#pragma unroll
+            for (int k = 0; k < 6; k++) t[k] += __ldcg(partials + (size_t)b * 8 + k);
+#pragma unroll
+        for (int k = 0; k < 6; k++) loss.accum[threadIdx.x * 8 + k] = t[k];
+        __threadfence();
+    }
+    __syncthreads();
+    if (warp == 0)
+        finalize_loss_warp(loss.accum, loss.loss_out, loss.w_depth, loss.w_color, loss.w_sem, loss.target_depth != nullptr,
+                           loss.target_color != nullptr, loss.target_label != nullptr, lane);
+}

@@ -74,6 +74,10 @@ struct ForwardArgs {
     const uint8_t *voxel_labels;
     uint8_t *image_label;
     unsigned long long *hist;
+    // kEval (spsg_raycast_eval), after the kLabels fields (voxel_labels = predicted label per voxel, image_label = optional
+    // per-pixel output): optional (C + 1)^2 confusion counters, and 8 floats per (image, tile) for the six loss partials
+    unsigned long long *confusion;
+    float *eval_tiles;
 };
 
 constexpr int kTileW = 16, kTileH = 8;  // pixels per CTA of the occupancy kernel: 4 warps of 8x4 pixels
@@ -214,7 +218,14 @@ __device__ __forceinline__ void clear_span(float *__restrict__ p, size_t n, size
 // label, min(voxel_labels[hit], C), or C on a miss -- and, with a.hist, counts pixels per label in a shared-memory
 // histogram (the staging area, which this epilogue does not use) flushed once per CTA with integer atomics.  No payload
 // loads, no float image, no registration, no work list, no hit records, no gradient rows.
-template <bool kLoss, bool kSmemMaps, int kWarps, bool kViewNormals, bool kGenericSem = false, bool kLabels = false>
+// kEval (spsg_raycast_eval): the same march, then an epilogue for evaluation without a backward: the predicted label of
+// the pixel (as kLabels, from voxel_labels), optionally stored; the (C + 1)^2 confusion of min(target label, C) against it,
+// counted in shared memory (the staging area) and flushed once per CTA with integer atomics; and the three 2D loss terms
+// with kLoss's per-pixel arithmetic (the C-generic cross-entropy at every C), whose six per-warp partials go to the tile's
+// own slot of a.eval_tiles for eval_loss_sum_kernel to add in a fixed order.  Reads the hit voxel's colour and logits, no
+// normals; no float atomics, no image, registration, work list or hit records.
+template <bool kLoss, bool kSmemMaps, int kWarps, bool kViewNormals, bool kGenericSem = false, bool kLabels = false,
+          bool kEval = false>
 __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const ForwardArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ float4 s_steps[kStepEntries];
@@ -226,7 +237,7 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
     const unsigned kFull = 0xffffffffu;
     const float kInf = CUDART_INF_F;
 
-    if (!kLabels && a.clear_rows > 0) {
+    if (!kLabels && !kEval && a.clear_rows > 0) {
         // The backward's output rows are zeroed here (the reference memsets its whole d_* buffers, kernel.cu:557-560): a few
         // fire-and-forget stores per warp that overlap the march, instead of a longer fill pass in front of the index build.
         const size_t wid = (size_t)blockIdx.x * kWarps + warp, nw = (size_t)gridDim.x * kWarps, n = (size_t)a.clear_rows;
@@ -238,6 +249,9 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
     if (threadIdx.x < kStepEntries) step_table_fill(s_steps, threadIdx.x, a.inc);
     if (kSmemMaps && threadIdx.x == 0) mbar_init(mbar, 1);
     if (kLabels && a.hist && threadIdx.x <= a.loss.sem_channels) reinterpret_cast<unsigned *>(smem + 128)[threadIdx.x] = 0u;
+    const int conf_cells = (a.loss.sem_channels + 1) * (a.loss.sem_channels + 1);  // (kEval)
+    if (kEval && a.confusion)
+        for (int i = threadIdx.x; i < conf_cells; i += kWarps * 32) reinterpret_cast<unsigned *>(smem + 128)[i] = 0u;
     __syncthreads();
     unsigned phase = 0;
     const float inv_inc = rcp_approx(a.inc);
@@ -662,6 +676,56 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
                         if (active && lane == __ffs(peers) - 1)
                             atomicAdd(reinterpret_cast<unsigned *>(smem + 128) + label, (unsigned)__popc(peers));
                     }
+                } else if (kEval) {
+                    // ---- eval epilogue: predicted label, confusion count (one shared atomic per distinct cell of the
+                    // warp), the loss terms of kLoss from the hit voxel's payload rows
+                    const LossArgs &L = a.loss;
+                    const int C = L.sem_channels;
+                    const int label = hit >= 0 ? min((int)__ldg(a.voxel_labels + hit), C) : C;
+                    if (a.image_label && active) a.image_label[gpix] = (uint8_t)label;
+                    if (a.confusion) {
+                        const int cell = active ? min((int)L.target_label[gpix], C) * (C + 1) + label : -1;
+                        const unsigned peers = __match_any_sync(kFull, cell);
+                        if (active && lane == __ffs(peers) - 1)
+                            atomicAdd(reinterpret_cast<unsigned *>(smem + 128) + cell, (unsigned)__popc(peers));
+                    }
+                    float acc[6] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
+                    if (hit >= 0) {
+                        if (L.target_depth) {  // train.py:635-638
+                            const float t = __ldg(L.target_depth + gpix);
+                            if (t != 0.0f) { acc[0] = fabsf(__fmul_rn(depth, L.voxelsize) - t); acc[1] = 1.0f; }
+                        }
+                        if (L.target_color) {  // loss.py:246-257
+                            const float *c = a.vals_color + (size_t)hit * 3;
+                            const float w = L.weight_color ? __ldg(L.weight_color + gpix) : 1.0f;
+                            const float *t = L.target_color + gpix * 3;
+                            acc[2] = fabsf(__fadd_rn(__fmul_rn(__ldg(c + 0), w), -__fmul_rn(__ldg(t + 0), w))) +
+                                     fabsf(__fadd_rn(__fmul_rn(__ldg(c + 1), w), -__fmul_rn(__ldg(t + 1), w))) +
+                                     fabsf(__fadd_rn(__fmul_rn(__ldg(c + 2), w), -__fmul_rn(__ldg(t + 2), w)));
+                            acc[3] = 3.0f;
+                        }
+                        if (L.target_label) {  // train.py:744-746, over the hit voxel's C logits
+                            const int y = L.target_label[gpix];
+                            const float *lg = a.vals_semantic + (size_t)hit * C;
+                            if (y < C && __ldg(lg) != -kInf) {
+                                const float w = L.class_weight ? __ldg(L.class_weight + y) : 1.0f;
+                                acc[4] = w * ce_nll<true>(lg, C, y);
+                                acc[5] = w;
+                            }
+                        }
+                    }
+                    // the partials exactly as kLoss forms them, stored instead of added
+                    float mine = 0.0f;
+                    const int n_depth = __popc(__ballot_sync(kFull, acc[1] != 0.0f)), n_color = __popc(__ballot_sync(kFull, acc[3] != 0.0f));
+                    if (lane == 1) mine = (float)n_depth;
+                    if (lane == 3) mine = 3.0f * (float)n_color;
+#pragma unroll
+                    for (int k = 0; k < 6; k++) {
+                        if (k == 1 || k == 3) continue;
+                        const float t = warp_sum(acc[k]);
+                        if (lane == k) mine = t;
+                    }
+                    if (lane < 6) a.eval_tiles[((size_t)img * tiles_per_image + tile % tiles_per_image) * 8 + lane] = mine;
                 } else {
                 // ---- write-out (kernel.cu:276-285 init, :217-239 hit) through shared memory
                 const float ninf = __int_as_float(0xff800000);
@@ -833,7 +897,9 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
                     STAT_ADD(32 + min(bucket, 9), 1);
                 }
 #endif
-                }  // !kLabels
+                }  // !kLabels && !kEval
+            } else if (kEval && lane < 6) {
+                a.eval_tiles[((size_t)q.img * tiles_per_image + tile % tiles_per_image) * 8 + lane] = 0.0f;  // no pixel
             }
             tile = __shfl_sync(kFull, next, 0);
             if (tile < tile_limit) prepare(bind_chunk(tile), q);
@@ -845,6 +911,12 @@ __global__ void __launch_bounds__(kWarps * 32, 1) raycast_forward_kernel(const F
         const unsigned *s_hist = reinterpret_cast<const unsigned *>(smem + 128);
         if (threadIdx.x <= a.loss.sem_channels && s_hist[threadIdx.x])
             atomicAdd(a.hist + threadIdx.x, (unsigned long long)s_hist[threadIdx.x]);
+    }
+    if (kEval && a.confusion) {
+        __syncthreads();
+        const unsigned *s_conf = reinterpret_cast<const unsigned *>(smem + 128);
+        for (int i = threadIdx.x; i < conf_cells; i += kWarps * 32)
+            if (s_conf[i]) atomicAdd(a.confusion + i, (unsigned long long)s_conf[i]);
     }
     if (kLoss) {
         // Every loss atomic of this CTA is ordered before its arrival; the CTA that arrives last sees them all in L2 and

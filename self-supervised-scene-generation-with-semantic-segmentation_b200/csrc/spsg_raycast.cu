@@ -107,12 +107,41 @@ LossArgs make_loss_args(const spsg_loss_targets *t, double *accum) {
     return L;
 }
 
-// Outputs of the label render (spsg_raycast_labels), which runs launch_forward with the kLabels kernels
+// Outputs of the label render (spsg_raycast_labels), which runs launch_forward with the kLabels kernels, and of the eval
+// render (spsg_raycast_eval: eval set), which runs it with the kEval kernels and then eval_loss_sum_kernel
 struct LabelOut {
     const uint8_t *voxel_labels;
     uint8_t *image_label;
     int64_t *hist;
+    bool eval;
+    uint64_t *confusion;
+    void *scratch;  // EvalScratch layout, checked by the caller
 };
+
+// warp tiles of a forward launch: 16x8-pixel blocks of four 8x4 tiles, per image
+long long forward_tiles(const spsg_raycast_params *p) {
+    const long long tiles_x = (p->width + kWarpW - 1) / kWarpW, tiles_y = (p->height + kWarpH - 1) / kWarpH;
+    return ((tiles_x + 1) / 2) * ((tiles_y + 1) / 2) * 4 * p->views_per_chunk * p->num_chunks;
+}
+
+// Scratch of spsg_raycast_eval: [kLossSlots * 8 doubles for the final stage | done counter (256 B) | 8 doubles per block of
+// eval_loss_sum_kernel | 8 floats per warp tile of the forward]
+struct EvalScratch {
+    long long tiles;
+    unsigned blocks;
+    size_t done_off, partials_off, tiles_off, total;
+};
+
+EvalScratch eval_scratch_layout(const spsg_raycast_params *p) {
+    EvalScratch s;
+    s.tiles = forward_tiles(p);
+    s.blocks = (unsigned)((s.tiles + kEvalSumTiles - 1) / kEvalSumTiles);
+    s.done_off = (size_t)kLossSlots * 8 * sizeof(double);
+    s.partials_off = s.done_off + 256;
+    s.tiles_off = s.partials_off + align_up((size_t)s.blocks * 8 * sizeof(double), 256);
+    s.total = s.tiles_off + align_up((size_t)s.tiles * 8 * sizeof(float), 256);
+    return s;
+}
 
 // the flags a label render acts on: the march's debug switches and the index routes (everything else concerns tables,
 // gradients, normals or the semantic payload kernels)
@@ -130,9 +159,12 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
     const bool all = (p->flags & SPSG_FLAG_ALL_PIXELS) != 0;  // no table: the backward builds segments from the hits
     const bool packed = (p->flags & SPSG_FLAG_PACKED_LOCS) != 0;
     if (lab) {
-        // label render: no payload, image, table or gradient pointers (the caller passes p with kLabelFlags only)
-        if (!sparse_mapping || !view_matrix || !intrinsics || !lab->image_label) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL tensor pointer");
-        if (p->num_locs > 0 && (!locs || !vals_sdf || !lab->voxel_labels))
+        // label / eval render: no normals, image, table or gradient pointers (the caller passes p with kLabelFlags only);
+        // the eval render's label image is optional, and it reads colour / logits for the colour / semantic terms
+        if (!sparse_mapping || !view_matrix || !intrinsics || (!lab->eval && !lab->image_label))
+            return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL tensor pointer");
+        if (p->num_locs > 0 && (!locs || !vals_sdf || !lab->voxel_labels ||
+                                (lab->eval && ((targets->target_color && !vals_color) || (targets->target_label && !vals_semantic)))))
             return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL voxel tensor pointer");
         if (reinterpret_cast<uintptr_t>(lab->hist) & 7u) return fail(SPSG_ERR_INVALID_ARGUMENT, "hist must be 8-byte aligned");
         if (p->num_locs > 0 && (reinterpret_cast<uintptr_t>(locs) & (packed ? 3u : 15u)))
@@ -264,10 +296,19 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
         a.voxel_labels = lab->voxel_labels; a.image_label = lab->image_label;
         a.hist = reinterpret_cast<unsigned long long *>(lab->hist);
         if (lab->hist) CUDA_TRY(cudaMemsetAsync(lab->hist, 0, (size_t)(a.loss.sem_channels + 1) * sizeof(int64_t), st));
+        if (lab->eval) {
+            const EvalScratch es = eval_scratch_layout(p);
+            a.confusion = reinterpret_cast<unsigned long long *>(lab->confusion);
+            a.eval_tiles = (float *)((uint8_t *)lab->scratch + es.tiles_off);
+            a.loss.accum = (double *)lab->scratch;
+            a.loss.done = (int32_t *)((uint8_t *)lab->scratch + es.done_off);
+            CUDA_TRY(cudaMemsetAsync(a.loss.done, 0, 256, st));
+            const size_t cells = (size_t)(a.loss.sem_channels + 1) * (a.loss.sem_channels + 1);
+            if (lab->confusion) CUDA_TRY(cudaMemsetAsync(lab->confusion, 0, cells * sizeof(uint64_t), st));
+        }
     }
     // persistent: one CTA per SM (fewer when there is less than one tile per warp)
-    const long long tiles_x = (p->width + kWarpW - 1) / kWarpW, tiles_y = (p->height + kWarpH - 1) / kWarpH;
-    const long long all_tiles = ((tiles_x + 1) / 2) * ((tiles_y + 1) / 2) * 4 * p->views_per_chunk * p->num_chunks;
+    const long long all_tiles = forward_tiles(p);
     const unsigned grid = (unsigned)std::max<long long>(1, std::min<long long>(sms, all_tiles));
     // CTA size: 24 warps when every warp gets about one tile (latency-bound), 28 when there are many tiles per SM
     const bool large = all_tiles >= (long long)sms * 4 * kFwdWarpsLarge;
@@ -299,6 +340,11 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
             SPSG_SET_SMEM_LABELS(true, kFwdWarps); SPSG_SET_SMEM_LABELS(false, kFwdWarps);
             SPSG_SET_SMEM_LABELS(true, kFwdWarpsLarge); SPSG_SET_SMEM_LABELS(false, kFwdWarpsLarge);
 #undef SPSG_SET_SMEM_LABELS
+#define SPSG_SET_SMEM_EVAL(M, W) \
+    CUDA_TRY(cudaFuncSetAttribute(raycast_forward_kernel<false, M, W, false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmemMax))
+            SPSG_SET_SMEM_EVAL(true, kFwdWarps); SPSG_SET_SMEM_EVAL(false, kFwdWarps);
+            SPSG_SET_SMEM_EVAL(true, kFwdWarpsLarge); SPSG_SET_SMEM_EVAL(false, kFwdWarpsLarge);
+#undef SPSG_SET_SMEM_EVAL
             if (dev >= 0 && dev < 64) configured[dev] = true;
         }
     }
@@ -320,18 +366,33 @@ int launch_forward(const spsg_raycast_params *p, bool build_index, int32_t *spar
         if (large) raycast_forward_kernel<false, M, kFwdWarpsLarge, false, false, true><<<grid, kFwdWarpsLarge * 32, dyn, st>>>(a); \
         else raycast_forward_kernel<false, M, kFwdWarps, false, false, true><<<grid, kFwdWarps * 32, dyn, st>>>(a); \
     } while (0)
-        if (lab) {
+#define SPSG_LAUNCH_EVAL(M)                                                                                       \
+    do {                                                                                                          \
+        if (large) raycast_forward_kernel<false, M, kFwdWarpsLarge, false, false, false, true><<<grid, kFwdWarpsLarge * 32, dyn, st>>>(a); \
+        else raycast_forward_kernel<false, M, kFwdWarps, false, false, false, true><<<grid, kFwdWarps * 32, dyn, st>>>(a); \
+    } while (0)
+        if (lab && lab->eval) {
+            if (a.maps_in_smem) SPSG_LAUNCH_EVAL(true); else SPSG_LAUNCH_EVAL(false);
+        } else if (lab) {
             if (a.maps_in_smem) SPSG_LAUNCH_LABELS(true); else SPSG_LAUNCH_LABELS(false);
         } else if (targets && !det) {  // (deterministic mode sums the losses in a pass of its own, below)
             if (a.maps_in_smem) SPSG_LAUNCH(true, true); else SPSG_LAUNCH(true, false);
         } else {
             if (a.maps_in_smem) SPSG_LAUNCH(false, true); else SPSG_LAUNCH(false, false);
         }
+#undef SPSG_LAUNCH_EVAL
 #undef SPSG_LAUNCH_LABELS
 #undef SPSG_LAUNCH
 #undef SPSG_LAUNCH_VN
     }
     CUDA_TRY(cudaGetLastError());
+    if (lab && lab->eval) {
+        // the tiles' loss partials, added in a fixed order
+        const EvalScratch es = eval_scratch_layout(p);
+        eval_loss_sum_kernel<<<es.blocks, kDetLossThreads, 0, st>>>(a.eval_tiles, es.tiles, a.loss,
+                                                                    (double *)((uint8_t *)lab->scratch + es.partials_off));
+        CUDA_TRY(cudaGetLastError());
+    }
     if (det) {
         // canonical tables: listed rows sorted, or reset and rebuilt from the hit records
         CanonArgs c;
@@ -633,9 +694,33 @@ int spsg_raycast_labels(const spsg_raycast_params *p, int32_t *sparse_mapping, c
     if (!p) return fail(SPSG_ERR_INVALID_ARGUMENT, "params is NULL");
     spsg_raycast_params q = *p;
     q.flags &= kLabelFlags;
-    const LabelOut lab = {voxel_labels, image_label, hist};
+    const LabelOut lab = {voxel_labels, image_label, hist, false, nullptr, nullptr};
     return launch_forward(&q, true, sparse_mapping, locs, vals_sdf, nullptr, nullptr, nullptr, view_matrix, intrinsics,
                           nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, workspace,
+                          workspace_bytes, (cudaStream_t)stream, &lab);
+}
+
+size_t spsg_raycast_eval_scratch_bytes(const spsg_raycast_params *p) {
+    if (check_params(p)) return 0;
+    return eval_scratch_layout(p).total;
+}
+
+int spsg_raycast_eval(const spsg_raycast_params *p, int32_t *sparse_mapping, const int64_t *locs, const float *vals_sdf,
+                      const float *vals_color, const float *vals_semantic, const uint8_t *pred_labels,
+                      const float *view_matrix, const float *intrinsics, const spsg_loss_targets *t, float *loss_out,
+                      uint8_t *image_label, uint64_t *confusion, void *scratch, size_t scratch_bytes, void *workspace,
+                      size_t workspace_bytes, void *stream) {
+    if (int rc = check_params(p)) return rc;
+    if (!t || !loss_out) return fail(SPSG_ERR_INVALID_ARGUMENT, "NULL loss targets / loss_out");
+    if (confusion && !t->target_label) return fail(SPSG_ERR_INVALID_ARGUMENT, "the confusion matrix needs target labels");
+    if (reinterpret_cast<uintptr_t>(confusion) & 7u) return fail(SPSG_ERR_INVALID_ARGUMENT, "confusion must be 8-byte aligned");
+    spsg_raycast_params q = *p;
+    q.flags &= kLabelFlags;
+    if (!scratch || scratch_bytes < eval_scratch_layout(&q).total) return fail(SPSG_ERR_WORKSPACE_TOO_SMALL, "scratch too small");
+    if (reinterpret_cast<uintptr_t>(scratch) & 255u) return fail(SPSG_ERR_INVALID_ARGUMENT, "scratch must be 256-byte aligned");
+    const LabelOut lab = {pred_labels, image_label, nullptr, true, confusion, scratch};
+    return launch_forward(&q, true, sparse_mapping, locs, vals_sdf, vals_color, nullptr, vals_semantic, view_matrix,
+                          intrinsics, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, t, loss_out, nullptr, workspace,
                           workspace_bytes, (cudaStream_t)stream, &lab);
 }
 

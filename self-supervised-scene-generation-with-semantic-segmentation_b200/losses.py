@@ -325,6 +325,97 @@ def render_with_2d_losses(raycaster, locs, vals_sdf, vals_colors, vals_normals, 
     return out[0], out[1], out[2:]
 
 
+def evaluate_2d(raycaster, locs, vals_sdf, vals_colors, vals_semantics, view_matrix, intrinsic_params, images_depth=None,
+                images_color=None, weight_color=None, target2d_label=None, weight_semantic_class=None, voxelsize=0.02,
+                weight_depth_loss=1.0, weight_color_loss=1.0, weight_semantic_loss=1.0, labels=False):
+    """Evaluation of a prediction without training (train.py ``test()``, :1088-1090 and :1193-1196): the three 2D loss
+    terms of ``render_with_2d_losses``, the predicted label map and the semantic confusion matrix, from one ray march
+    (``spsg_raycast_eval``) with no rendered image, no registration tables and no backward.
+
+    Arguments as ``render_with_2d_losses`` without ``vals_normals``; ``vals_semantics`` (N, C) logits, C = the raycaster's
+    ``num_classes``.  Returns ``(total, terms, confusion, pred_labels)``:
+      total, terms  the weighted total and (depth, colour, semantic), the values ``render_with_2d_losses`` reports for the
+                    same inputs (same per-pixel arithmetic and per-warp partials; bit-reproducible sums in any mode)
+      confusion     (C+1, C+1) int64, [min(target label, C), predicted label] pixel counts, or None without target labels
+      pred_labels   (I, H, W) uint8 with ``labels=True``: ``labels_from_render`` of the prediction's semantic rendering
+                    (the hit voxel's argmax of ``cat(logits, ones)``, C on a miss), else None
+    Plain tensors, no autograd.  Rebuilds only the raycaster's ``sparse_mapping`` and workspace (it takes the index
+    prebuilt by ``sparsify.sparsify_predictions(..., raycaster=raycaster)``); its images, tables and gradient buffers are
+    untouched, and a backward of an earlier forward on it raises afterwards."""
+    m = raycaster
+    images = view_matrix.shape[0]
+    views = max(1, images // m.batch_size)
+    if images != views * m.batch_size or views > m.max_num_frames:
+        raise RuntimeError("view_matrix has %d images: expected batch_size (%d) x views with views <= max_num_frames (%d)"
+                           % (images, m.batch_size, m.max_num_frames))
+    c = m.num_classes
+    n = locs.shape[0]
+    if vals_semantics is None:
+        vals_semantics = torch.zeros(n, c, device=vals_sdf.device)
+    if vals_semantics.dim() != 2 or vals_semantics.shape[1] != c:
+        raise RuntimeError("vals_semantics must be (N, %d), got %s" % (c, tuple(vals_semantics.shape)))
+    for t, name in ((m.sparse_mapping, "sparse_mapping"), (locs, "locs"), (vals_sdf, "vals_sdf"), (vals_colors, "vals_colors"),
+                    (vals_semantics, "vals_semantics"), (view_matrix, "view_matrix"), (intrinsic_params, "intrinsic_params")):
+        rc._check_input(t, name)
+    if not rc.is_packed_locs(locs):
+        rc._check_dtype(locs, torch.int64, "locs")
+        if locs.numel() != 4 * n:
+            raise RuntimeError("locs must be (N, 4) rows of (z, y, x, chunk)")
+    for t, name in ((vals_sdf, "vals_sdf"), (vals_colors, "vals_colors"), (vals_semantics, "vals_semantics"),
+                    (view_matrix, "view_matrix"), (intrinsic_params, "intrinsic_params")):
+        rc._check_dtype(t, torch.float32, name)
+    if vals_sdf.numel() < n or vals_colors.numel() < 3 * n:
+        raise RuntimeError("vals_sdf / vals_colors hold fewer than N = %d rows" % n)
+    if view_matrix.numel() < images * 16 or intrinsic_params.numel() < images * 4:
+        raise RuntimeError("view_matrix / intrinsic_params hold fewer than %d images" % images)
+    dev = vals_sdf.device
+    devs = {t.device for t in (m.sparse_mapping, locs, vals_sdf, vals_colors, vals_semantics, view_matrix, intrinsic_params)}
+    if len(devs) != 1:
+        raise RuntimeError("evaluate_2d inputs live on different devices: %s" % sorted(str(d) for d in devs))
+    cont = lambda t: None if t is None else t.contiguous()  # noqa: E731
+    target2d_label = cont(target2d_label)
+    keep = (cont(images_depth), cont(images_color), cont(weight_color), target2d_label, weight_semantic_class)
+    tg = _targets_struct(images, m.height, m.width, *keep, voxelsize,
+                         (weight_depth_loss, weight_color_loss, weight_semantic_loss), c)
+    pred_voxel = labels_from_render(vals_semantics)  # the existing argmax rules (NaN, +-inf, ties, max < 1 -> C)
+    loss_out = torch.empty(N.SPSG_LOSS_OUT_FLOATS, device=dev)
+    confusion = torch.empty(c + 1, c + 1, dtype=torch.int64, device=dev) if target2d_label is not None else None
+    pred_labels = torch.empty(images, m.height, m.width, dtype=torch.uint8, device=dev) if labels else None
+    p = N.make_params(m.width, m.height, m.depth_min, m.depth_max, m.thresh_sample_dist, m.ray_increment, m.dims3d[2],
+                      m.dims3d[1], m.dims3d[0], m.batch_size, views, 0, n, m.flags, c)
+    if rc.is_packed_locs(locs):
+        p.flags |= N.SPSG_FLAG_PACKED_LOCS
+    owner = _module_workspace(m)
+    with rc.device_guard(dev):
+        nbytes = N.workspace_bytes(p)
+        prebuilt = owner.take_prebuilt(locs, nbytes)  # index + brick written with locs by sparsify_predictions(raycaster=m)
+        ws = owner.get(dev, nbytes)
+        p.flags |= prebuilt
+        scratch = owner.get_eval_scratch(dev, N.lib.spsg_raycast_eval_scratch_bytes(ctypes.byref(p)))
+        N.check(N.lib.spsg_raycast_eval(
+            ctypes.byref(p), N.ptr(m.sparse_mapping), N.ptr(locs), N.ptr(vals_sdf), N.ptr(vals_colors),
+            N.ptr(vals_semantics), N.ptr(pred_voxel), N.ptr(view_matrix), N.ptr(intrinsic_params), ctypes.byref(tg),
+            N.ptr(loss_out), N.ptr(pred_labels), N.ptr(confusion), N.ptr(scratch), scratch.numel(), N.ptr(ws), ws.numel(),
+            rc._stream(dev)))
+        owner.labels_rendered(rc._EVAL_STAMP)
+        if prebuilt:
+            owner.mark_prebuilt(locs)  # index and brick are untouched: still valid for these rows
+    return loss_out[3], loss_out[:3], confusion, pred_labels
+
+
+def semantic_metrics(confusion):
+    """Pixel accuracy, per-class IoU and mean IoU of a ``(C+1, C+1)`` confusion matrix of ``evaluate_2d`` (rows: target
+    label, the last one unlabelled; columns: predicted label, the last one a miss).  Only rows < C (labelled pixels) count;
+    a labelled pixel predicted C is wrong.  Returns ``(accuracy, iou, mean_iou)`` as float64 device tensors: ``iou`` (C,),
+    NaN for a class with an empty union, ``mean_iou`` over the classes with a non-empty union (NaN if none)."""
+    c = confusion.shape[0] - 1
+    m = confusion[:c].to(torch.float64)
+    tp = torch.diagonal(m[:, :c])
+    union = m.sum(1) + m[:, :c].sum(0) - tp
+    iou = tp / union
+    return tp.sum() / m.sum(), iou, iou[union > 0].mean()
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # The same three terms as stand-alone ops on rendered images: the boundary at which the reference applies them
 # (loss.compute_2dcolor_loss, loss.py:246-257; the inline expressions of train.py:635-638 and :744-746).  One pass over

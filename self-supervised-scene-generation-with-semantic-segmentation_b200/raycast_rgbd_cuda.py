@@ -159,6 +159,7 @@ def semantic_channels(t):
 
 
 _LABEL_STAMP = "label render (no tables)"
+_EVAL_STAMP = "eval render (no tables)"
 
 
 def _stamp(p):
@@ -204,6 +205,7 @@ class ModuleWorkspace:
         self.ws, self.stamp, self._prebuilt = None, None, None
         self.forwards = 0
         self.grad_views = None
+        self.eval_scratch = None  # spsg_raycast_eval's scratch (losses.evaluate_2d)
 
     def get(self, device, nbytes):
         if self.ws is None or self.ws.numel() < nbytes or self.ws.device != device:
@@ -230,11 +232,17 @@ class ModuleWorkspace:
         self.stamp = _stamp(p)
         self.forwards += 1
 
-    def labels_rendered(self):
-        """A label render ran on this workspace: it counts as a forward, and its stamp matches no backward's (it leaves no
-        tables or work list), so a backward after it raises instead of gathering what an earlier forward left."""
-        self.stamp = _LABEL_STAMP
+    def labels_rendered(self, stamp=_LABEL_STAMP):
+        """A label (or eval, ``stamp=_EVAL_STAMP``) render ran on this workspace: it counts as a forward, and its stamp
+        matches no backward's (it leaves no tables or work list), so a backward after it raises instead of gathering what an
+        earlier forward left."""
+        self.stamp = stamp
         self.forwards += 1
+
+    def get_eval_scratch(self, device, nbytes):
+        if self.eval_scratch is None or self.eval_scratch.numel() < nbytes or self.eval_scratch.device != device:
+            self.eval_scratch = torch.empty(max(int(nbytes), 1 << 16), dtype=torch.uint8, device=device)
+        return self.eval_scratch
 
     def check_latest(self, forward):
         """``forward`` = ``self.forwards`` right after the forward whose backward is about to run."""

@@ -185,3 +185,46 @@ class ViewGuidedTrainStep:
             loss.backward()                                                                    # train.py:756
             optimizer.step()                                                                   # train.py:757
         return loss.detach()
+
+    def validate(self, sample):
+        """The 2D branch of train.py ``test()`` (:870-1275; the losses of :1088-1090, :1193-1196): the step's forward and
+        losses without training.  Under ``torch.no_grad()``: the generator forward and dense 3D losses as in ``__call__``,
+        the target labels, then the prediction's depth / colour / semantic terms and its confusion matrix against the target
+        labels from one ``losses.evaluate_2d`` call -- no input render, normals, ``image_loss`` or backward.  Returns the
+        weighted total; ``self.last`` holds ``num_locs``, ``loss_occ``, ``loss_sdf`` and, when the prediction is rendered,
+        ``terms2d`` and ``confusion`` ((C+1, C+1) int64, see ``losses.semantic_metrics``).  No parameter's ``.grad`` is
+        touched; the generator's train / eval mode is the caller's."""
+        lu, T = self.loss_util, self.truncation
+        with torch.no_grad():
+            inputs, mask, known = sample["input"], sample["mask"], sample.get("known")
+            target_for_sdf, target_for_colors = lu.compute_targets(sample["sdf"], T, True, known, sample["colors"])
+            dense_region = (torch.autocast("cuda", dtype=torch.bfloat16) if self.autocast_bf16 else contextlib.nullcontext())
+            with dense_region:
+                output_occ, output_sdf, output_color, output_semantic = self.model(
+                    inputs, mask, pred_sdf=[True, True], pred_color=True, pred_semantic=True)
+                input_occ = torch.abs(inputs[:, :1]) < (T - 0.01)
+                weight = lu.compute_dense_geo_weights(target_for_sdf, input_occ, T, self.weight_surf_geo,
+                                                      self.weight_missing_geo)
+                empty = torch.sigmoid(output_occ) < 0.5
+                weight[empty] = 0
+                loss_occ = lu.compute_geo_occ_loss(target_for_sdf, output_occ, known, weight, T)
+                loss_sdf = lu.compute_geo_loss(target_for_sdf, None, output_sdf, known, weight, self.logweight_sdf)
+                loss = self.w["occ"] * loss_occ + self.w["sdf"] * loss_sdf
+            counted = sparsify.count_locs(output_sdf, T, empty)
+            n = counted.n
+            self.last = dict(num_locs=n, loss_occ=loss_occ, loss_sdf=loss_sdf)
+            if 0 < n <= self.raycaster.get_max_num_locs_per_sample() * self.batch_size:
+                view_matrix, intrinsics = sample["view_matrix"], sample["images_intrinsic"]
+                target2d_label = self._target_labels(target_for_sdf, target_for_colors, sample["semantics"], view_matrix,
+                                                     intrinsics, None)
+                locs, sdf_vals, color_vals, sem_vals = sparsify.sparsify_predictions(
+                    output_sdf, T, empty, output_color, output_semantic, raycaster=self.raycaster, counted=counted)
+                total2d, terms, confusion, _ = losses.evaluate_2d(
+                    self.raycaster, locs, sdf_vals, (color_vals + 1) * 0.5, sem_vals, view_matrix, intrinsics,
+                    images_depth=sample["images_depth"], images_color=sample["images_color"].permute(0, 2, 3, 1),
+                    target2d_label=target2d_label, weight_semantic_class=self.class_weight, voxelsize=self.voxelsize,
+                    weight_depth_loss=self.w["depth"], weight_color_loss=self.w["color"],
+                    weight_semantic_loss=self.w["semantic"])
+                loss = loss + total2d
+                self.last.update(terms2d=terms, confusion=confusion)
+        return loss

@@ -3,7 +3,7 @@
 (no GPU needed).  The backward gather's template gained parameters (kUpstream, then kViewNormals, then kSegments); its old
 instantiations <kFused, kViews> and <kFused, kUpstream, kViews> are matched with kUpstream / kViewNormals / kSegments /
 kGenericSem false.  The forward kernel's <kLoss, kSmemMaps, kWarps> likewise with <kLoss, kSmemMaps, kWarps, kViewNormals =
-false, kGenericSem = false, kLabels = false>, and the stand-alone loss kernels (losses2d_forward/backward/det_kernel) with their
+false, kGenericSem = false, kLabels = false, kEval = false>, and the stand-alone loss kernels (losses2d_forward/backward/det_kernel) with their
 <kGenericSem = false> instantiations.  The compaction kernels of spsg_sparsify.cu gained the SDF
 element type: the plain sparsify_count_kernel and sparsify_write_kernel<kIndexed> are matched with their <float>
 instantiations.
@@ -46,10 +46,10 @@ def key(name):
     if m:
         return "backward_gather_kernel" + m.group(1) + (m.group(2) or "Lb0E") + m.group(3) + (m.group(4) or "Lb0E") + \
             (m.group(5) or "Lb0E") + (m.group(6) or "Lb0E")
-    m = re.search(r"raycast_forward_kernelI(Lb[01]ELb[01]ELi\d+E)(Lb[01]E)?(Lb[01]E)?(Lb[01]E)?E", name)
+    m = re.search(r"raycast_forward_kernelI(Lb[01]ELb[01]ELi\d+E)(Lb[01]E)?(Lb[01]E)?(Lb[01]E)?(Lb[01]E)?E", name)
     if m:
         return "raycast_forward_kernel" + m.group(1) + (m.group(2) or "Lb0E") + (m.group(3) or "Lb0E") + \
-            (m.group(4) or "Lb0E")
+            (m.group(4) or "Lb0E") + (m.group(5) or "Lb0E")
     m = re.search(r"(losses2d_(?:forward|backward|det)_kernel)(?:ILb([01])EE)?", name)
     if m:
         return "%s<%s>" % (m.group(1), m.group(2) or "0")
